@@ -1,13 +1,14 @@
 #!/usr/bin/env python
 """bench.py -- Arnoldi steps/s on BASELINE.json's config C2 (5-point Poisson 4096^2, fp64, kdim=128).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 One bench "step" = one pass of the hot path over one start vector = one full kstart=1..kend=128
 Arnoldi factorisation (128 Arnoldi steps: matvec + CGS2 + Hessenberg update each).  `value` is
 Arnoldi steps per second = 128*K / time, the strong-scaling metric BASELINE.json names (global
-n = 16.8M rows sharded by grid rows over the N ranks).
+n = 16.8M rows sharded by grid rows over the N ranks).  The start vector is seeded, so two builds run with the same
+arguments and --dump-outputs can be compared output for output.
 
 Prints ONE JSON line on rank 0 (see DESIGN.md "Measurement" for every key).
 """
@@ -32,6 +33,17 @@ if os.environ.get("NCCL_DEBUG", "VERSION").upper() == "VERSION":
 METRIC = "arnoldi_steps_per_s"
 UNIT = "steps/s"
 POISSON5 = (4.0, -1.0, -1.0, -1.0, -1.0)
+# --dump-outputs keeps the whole H and a fixed row sample of the basis (17 GB at full size): at most 16384 rows, fewer when
+# kdim is so large that H and the sample would exceed DUMP_BYTES (default size: 16384 x 129 fp64 = 17 MB)
+DUMP_ROWS = 16384
+DUMP_BYTES = 64 << 20
+DUMP_SEED = 2024
+
+
+def dump_rows(n: int, kdim: int) -> np.ndarray:
+    """The sorted global rows of the basis that --dump-outputs keeps, drawn from a fixed seed."""
+    budget = (DUMP_BYTES - (kdim + 1) * kdim * 8) // ((kdim + 1) * 8)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=min(n, DUMP_ROWS, budget), replace=False))
 
 
 def parse():
@@ -50,7 +62,18 @@ def parse():
     ap.add_argument("--no-p2p", action="store_true", help="use ncclAllReduce instead of the in-kernel NVLink allreduce (A/B)")
     ap.add_argument("--opt", action="append", default=[], metavar="NAME=0|1",
                     help="lkb_set_option A/B switches: fused, fin (fused final pass), fused_halo, p2p, graphs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR: H.npy (the Hessenberg matrix) and X_sample.npy "
+                         f"(all columns of the Krylov basis at up to {DUMP_ROWS} fixed, seeded, sorted global rows), float64, "
+                         f"{DUMP_BYTES >> 20} MB at most")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm times sampled steps, not whole factorisations)")
+    if args.dump_outputs and (args.kdim + 1) ** 2 * 8 > DUMP_BYTES:
+        ap.error(f"--dump-outputs: H and one row of the basis exceed {DUMP_BYTES >> 20} MB at this --kdim")
+    return args
 
 
 def alg_bytes_step(j: int, n: int, s: int = 8) -> int:
@@ -209,6 +232,28 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------
+def basis_sample(X, rows: np.ndarray, row0: int, world: int):
+    """All columns of the (row-sharded) basis X at the given ascending global rows, gathered on rank 0 (None on the other
+    ranks).  The rows are picked on the device, so only the sample crosses to the host."""
+    import torch
+    import torch.distributed as dist
+
+    class _Column:                                   # a device column of X as a torch tensor, without a copy
+        def __init__(self, v):
+            self.__cuda_array_interface__ = {"shape": (v.n,), "typestr": "<f8", "data": (v.ptr, False), "version": 2}
+
+    X.ctx.sync()
+    mine = rows[(rows >= row0) & (rows < row0 + X.n)] - row0
+    idx = torch.as_tensor(mine, device=torch.cuda.current_device())
+    part = torch.stack([torch.as_tensor(_Column(X.col(j)), device=idx.device)[idx] for j in range(X.ncols)], dim=1)
+    part = part.cpu().numpy()
+    if world == 1:
+        return part
+    parts = [None] * world if dist.get_rank() == 0 else None
+    dist.gather_object(part, parts, dst=0)       # rank r holds the r-th slab of grid rows: rank order is row order
+    return np.concatenate(parts) if parts else None
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -284,6 +329,13 @@ def run_ours(args):
     launches = ctx.kernel_launches - l0
     clocks = sampler.stop() if rank == 0 else None
     value = args.steps * kdim / (ms_total * 1e-3)
+    # ---- the outputs of the last timed step, taken before anything below runs the factorisation again ----------
+    if args.dump_outputs:
+        outputs = {"H": H.copy(), "X_sample": basis_sample(X, dump_rows(n, kdim), row0, world)}
+        if rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
 
     # ---- parity record (outside the timed region): H and Ritz values of THIS run, at THIS number of ranks, against the
     # committed oracle Hessenberg matrix of the same workload (tests/golden/c2_full_H.npz, all 128 steps on the CPU) ----

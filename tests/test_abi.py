@@ -7,6 +7,8 @@ import re
 
 import pytest
 
+from oracle import ref_exec
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -421,7 +423,7 @@ def test_fortran_shim_identifiers_are_declared():
     assert [p[1] for p in bad] == ["lkb_vec_zer0"]
 
 
-REFERENCE = "/root/reference/src"
+REFERENCE = os.path.join(ref_exec.REF, "src")      # the LightKrylov checkout the interpreter tests use ($LK_REFERENCE)
 _REF_ROUTINES = {          # try-function -> (reference file, reference routine)
     "arnoldi": ("Krylov/BaseKrylov.fypp", "arnoldi"), "lanczos": ("Krylov/BaseKrylov.fypp", "lanczos_tridiagonalization"),
     "bidiagonalization": ("Krylov/BaseKrylov.fypp", "lanczos_bidiagonalization"), "qr": ("Krylov/BaseKrylov.fypp", "qr_no_pivoting"),
