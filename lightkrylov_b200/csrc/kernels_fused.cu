@@ -358,7 +358,7 @@ static bool axpy_dot_t(cudaStream_t s, const void* V, int64_t ld, int j, const v
     if (nb > ntiles) nb = ntiles;
     if (nb > RT_MAXROWS) nb = RT_MAXROWS;
     launch_ex(k_axpy_dot<K>, (unsigned)nb, FZ_THREADS, sh, s, pdl_take(4), tmap, j, tp, nst, elt_per_pack, (const W*)c1, (E*)w, n, (W*)partial, (W*)out, counter, flags, p2p ? *p2p : P2P(),
-              sweep_dir() | (((size_t)n * sizeof(E) <= w_keep_bytes()) ? 2 : 0));
+              sweep_dir() | (((size_t)n * sizeof(E) <= W_KEEP_BYTES) ? 2 : 0));
     return true;
 }
 

@@ -8,7 +8,6 @@
 // registers; X is streamed once per group of PB outputs with 128-bit loads, Z is broadcast from
 // shared memory.  PB = 16 (real) / 8 (complex) keeps the fp64 FMA rate needed at full HBM speed below the
 // B200 fp64 pipe, so this stays HBM-bound without tensor cores (a DMMA variant is a later row).
-#include <stdlib.h>
 #include "lkb_kernels.h"
 
 namespace lkb {
@@ -180,8 +179,7 @@ k_basis_gemm_dmma(const double* __restrict__ X, int64_t ldx, int k, const double
 }
 
 static bool gemm_dmma(cudaStream_t s, const void* X, int64_t ldx, int k, const void* Z, int ldz, int p, void* Y, int64_t ldy, int64_t n) {
-    static const int variant = getenv("LKB_GEMM_VARIANT") ? atoi(getenv("LKB_GEMM_VARIANT")) : 1;      // 0 = FMA kernel (A/B)
-    if (variant == 0 || k < 1 || p < 1 || n < 1) return false;
+    if (k < 1 || p < 1 || n < 1) return false;
     if (((uintptr_t)X & 15) || (ldx % 2)) return false;                 // 16-byte cp.async
     const int kpad = (k + GM_KS - 1) / GM_KS * GM_KS;
     const size_t sh = ((size_t)kpad * GM_ZS + (size_t)GM_STAGES * GM_KS * GM_XS) * sizeof(double);

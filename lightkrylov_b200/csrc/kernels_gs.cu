@@ -749,7 +749,7 @@ static void multidot_t(cudaStream_t s, const void* V, int64_t ld, int j, const v
     static const SmemAttrOnce attr((const void*)k_multidot<K>, 160 * 1024);
     attr.ensure();
     launch_ex(k_multidot<K>, (unsigned)nb, MD_THREADS, sh, s, pdl_take(2), (const E*)V, ld, j, (const E*)w, n, (W*)partial, (W*)out, counter, flags, pp,
-              sweep_dir() | (((size_t)n * sizeof(E) <= w_keep_bytes()) ? 2 : 0));
+              sweep_dir() | (((size_t)n * sizeof(E) <= W_KEEP_BYTES) ? 2 : 0));
 }
 void launch_multidot(int kind, cudaStream_t s, const void* V, int64_t ld, int j, const void* w, int64_t n,
                      void* partial, void* out, unsigned* counter, const int* flags, int sms, const P2P* p2p) {
@@ -806,7 +806,7 @@ static void multiaxpy_fin_t(cudaStream_t s, const void* V, int64_t ld, int j, co
     fp.kstep = kstep; fp.mode = mode;
     launch_ex(k_multiaxpy_fin<K>, (unsigned)nb, 256, sh, s, pdl_take(8), (const E*)V, ld, j, (const W*)c2, (E*)w, n, (double*)partial,
               (W*)nrm2_out, counter, fp, p2p ? *p2p : P2P(), hp ? *hp : HaloP2P(),
-              sweep_dir() | (((size_t)n * sizeof(E) <= w_keep_bytes()) ? 2 : 0));
+              sweep_dir() | (((size_t)n * sizeof(E) <= W_KEEP_BYTES) ? 2 : 0));
 }
 void launch_multiaxpy_fin(int kind, cudaStream_t s, const void* V, int64_t ld, int j, const void* c1, const void* c2, void* w,
                           int64_t n, void* partial, void* nrm2_out, unsigned* counter, void* hcol, double tol, double atol,

@@ -4,7 +4,6 @@
 // intent(out)).  Stencil index convention: p = i + nx*(j + ny*k); coef = (center,-x,+x,-y,+y,-z,+z),
 // homogeneous Dirichlet outside the global grid.  The slowest axis (y in 2-D, z in 3-D) is the
 // row-sharded one: the neighbouring slab's boundary row / plane arrives in halo_lo / halo_hi.
-#include <stdlib.h>
 #include <algorithm>
 #include "lkb_kernels.h"
 #include "lkb_p2p.cuh"
@@ -52,24 +51,15 @@ template <typename E, int PW> struct PackOps {
 };
 
 
-// Block decode shared by the two stencil kernels.  1-D grid, column block fastest (consecutive CTAs stream
-// consecutive segments of the same grid rows); the row groups are rotated by one so that the two groups that
-// read the inter-GPU halos (first / last row group in 2-D, first / last plane in 3-D) are scheduled LAST: the
-// slab interior is computed while the neighbours' halo rows are still in flight (SURVEY 8e: "overlapped with the
-// interior update").  halo_wait: the halo-reading CTAs wait until the neighbours published the epoch the local
-// counter says (k_halo_push has already waited, so this is one load; after a push fused into k_multiaxpy_fin /
-// k_scale_dev nobody has waited yet and this is where the exchange is synchronised).
-struct StBlock { int64_t cb, rb, k; };
-template <int DIM>
-LKB_DI StBlock st_decode(int64_t ncb, int64_t nyb, int64_t nz) {
-    StBlock b;
-    const int64_t bid = blockIdx.x;
-    b.cb = bid % ncb;
-    const int64_t rg = bid / ncb;
-    if (DIM == 2) { b.k = 0; b.rb = (rg + 1) % nyb; }
-    else { b.rb = rg % nyb; b.k = (rg / nyb + 1) % nz; }
-    return b;
-}
+// Both stencil kernels take one CTA per (column block, row block[, plane]) of a 1-D grid, column block fastest
+// (consecutive CTAs stream consecutive segments of the same grid rows).  The row blocks (2-D) / planes (3-D) are rotated
+// by one so that the CTAs that read the inter-GPU halos (first / last row block in 2-D, first / last plane in 3-D) are
+// scheduled LAST: the slab interior is computed while the neighbours' halo rows are still in flight (SURVEY 8e:
+// "overlapped with the interior update").  halo_wait: the halo-reading CTAs wait until the neighbours published the
+// epoch the local counter says (k_halo_push has already waited, so this is one load; after a push fused into
+// k_multiaxpy_fin / k_scale_dev nobody has waited yet and this is where the exchange is synchronised).
+// Both kernels take the same argument list; in 2-D, nz is 1 and the z coefficients are unused.
+enum { ST_RY = 8 };           // grid rows per CTA
 LKB_DI void halo_wait(const unsigned* halo_epoch, const unsigned* flag_lo, const unsigned* flag_hi, bool need_lo, bool need_hi) {
     if (!halo_epoch || !(need_lo || need_hi)) return;      // uniform over the CTA
     if (threadIdx.x == 0) {
@@ -81,14 +71,21 @@ LKB_DI void halo_wait(const unsigned* halo_epoch, const unsigned* flag_lo, const
     __syncthreads();
 }
 
-// One CTA = 256 threads side by side along x (256*PW points of one grid row), marching RY rows in y
-// (2.5-D blocking): the south / centre / north packs of a column live in registers, so every x
-// element is loaded from HBM once per CTA (+2 halo rows per RY rows, served by L2 because the
-// neighbouring CTA streams them at the same time).  The x-halo (west / east neighbour of a pack)
-// comes from L1 (the neighbouring thread loaded that line) or, with SHFL, through warp shuffles.
-// UN > 1 prefetches UN north rows up front.  Inter-GPU halos arrive in halo_lo / halo_hi (slab
-// edges, filled by ncclSend/Recv).  HBM traffic ~ (2 + 2/RY) * n * s.
-template <int K, int PW, int DIM, int RY, int UN, bool SHFL>
+// ------------------------------------------------------------------------------------------
+// 3-D 7-point stencil: register y-march (2.5-D blocking).  One CTA = blockDim.x threads side by side along x
+// (blockDim.x * PW points of one grid row of plane k), marching ST_RY rows in y: the south / centre / north packs of a
+// column live in registers, so every x element of the plane is loaded from HBM once per CTA (+2 halo rows per ST_RY
+// rows, served by L2 because the neighbouring CTA streams them at the same time).  The x-halo (west / east neighbour of
+// a pack) comes from L1 (the neighbouring thread loaded that line), the z-neighbours from L2 (the CTAs of planes k-1 /
+// k+1 stream them) or, at the slab edges, from the inter-GPU halo planes halo_lo / halo_hi.
+// HBM traffic ~ (2 + 2/ST_RY) * n * s.
+// Why this kernel (B200, fp64, 384^3, profiles/stencil_ab.py -> profiles/r02_stencil_ab.txt): 5.15 TB/s, against
+// 2.9-3.7 TB/s for the 2-D kernel's shared-memory staging extended by the planes k-1 / k+1 (3 * ST_RY + 2 staged rows
+// per CTA cut the occupancy) and 3.95 TB/s for a z-march with the planes in registers (y-neighbours re-read through L1;
+// a deeper plane prefetch thrashed L1).  A z-march with the plane staged in shared memory (two block barriers per
+// plane, round 1) reached 2.8 TB/s.
+// ------------------------------------------------------------------------------------------
+template <int K, int PW>
 __global__ void __launch_bounds__(256)
 k_stencil(const typename Tr<K>::E* __restrict__ x, typename Tr<K>::E* __restrict__ y,
           int64_t nx, int64_t ny, int64_t nz, Coef7<typename Tr<K>::E> cf,
@@ -110,53 +107,31 @@ k_stencil(const typename Tr<K>::E* __restrict__ x, typename Tr<K>::E* __restrict
     }
     using P = typename PO::P;
     const int64_t npk_row = nx / PW;
-    const int64_t nyb = (ny + RY - 1) / RY;
-    const StBlock sb = st_decode<DIM>(ncb, nyb, nz);
-    const int64_t ip = sb.cb * blockDim.x + threadIdx.x;
-    const bool active = ip < npk_row;                 // inactive lanes still take part in the shuffles
+    const int64_t nyb = (ny + ST_RY - 1) / ST_RY;
+    const int64_t bid = blockIdx.x;
+    const int64_t cb = bid % ncb, rg = bid / ncb;
+    const int64_t rb = rg % nyb, k = (rg / nyb + 1) % nz;
+    const int64_t ip = cb * blockDim.x + threadIdx.x;
+    const bool active = ip < npk_row;                 // idle lanes march the row's last pack and store nothing
     const int64_t i0 = (active ? ip : npk_row - 1) * PW;
-    const int64_t k = sb.k;
-    const int64_t j0 = sb.rb * RY;
-    const int64_t j1 = min(ny, j0 + RY);
-    halo_wait(halo_epoch, flag_lo, flag_hi, halo_lo && (DIM == 2 ? j0 == 0 : k == 0),
-              halo_hi && (DIM == 2 ? j1 >= ny : k == nz - 1));
+    const int64_t j0 = rb * ST_RY;
+    const int64_t j1 = min(ny, j0 + ST_RY);
+    halo_wait(halo_epoch, flag_lo, flag_hi, halo_lo && k == 0, halo_hi && k == nz - 1);
     const int64_t plane = nx * ny;
     const E* xk = x + k * plane;
-    const int lane = threadIdx.x & 31;
 
     auto getrow = [&](int64_t j) -> P {
-        if (DIM == 2) {
-            if (j < 0) return halo_lo ? PO::ld_cg(halo_lo + i0) : PO::zero();
-            if (j >= ny) return halo_hi ? PO::ld_cg(halo_hi + i0) : PO::zero();
-        } else {
-            if (j < 0 || j >= ny) return PO::zero();
-        }
+        if (j < 0 || j >= ny) return PO::zero();
         return PO::ld(xk + j * nx + i0);
     };
-    auto shfl_e = [&](E v, int src) -> E {
-        if constexpr (sizeof(E) == 4) return __shfl_sync(0xffffffffu, v, src);
-        else if constexpr (sizeof(E) == 8 && !Tr<K>::cplx) return __shfl_sync(0xffffffffu, v, src);
-        else if constexpr (sizeof(E) == 8) { E r; r.x = __shfl_sync(0xffffffffu, v.x, src); r.y = __shfl_sync(0xffffffffu, v.y, src); return r; }
-        else { E r; r.x = __shfl_sync(0xffffffffu, v.x, src); r.y = __shfl_sync(0xffffffffu, v.y, src); return r; }
-    };
-    auto do_row = [&](int64_t j, const P& south, const P& center, const P& north) {
+    P south = getrow(j0 - 1), center = getrow(j0);
+    for (int64_t j = j0; j < j1; ++j) {
+        const P north = getrow(j + 1);
         const int64_t p = j * nx + i0;
-        // x-halo through warp shuffles; edge lanes of the warp (and of the row) load / zero-fill
-        E west, east;
-        if (SHFL) {
-            west = shfl_e(center.v[PW - 1], (lane + 31) & 31);
-            east = shfl_e(center.v[0], (lane + 1) & 31);
-            if (lane == 0) west = i0 > 0 ? __ldg(xk + p - 1) : zero_v(E());
-            if (lane == 31 || ip + 1 >= npk_row) east = (i0 + PW < nx) ? __ldg(xk + p + PW) : zero_v(E());
-        } else {
-            west = i0 > 0 ? __ldg(xk + p - 1) : zero_v(E());
-            east = (i0 + PW < nx) ? __ldg(xk + p + PW) : zero_v(E());
-        }
-        P down, up;
-        if (DIM == 3) {
-            down = (k > 0) ? PO::ld(xk + p - plane) : (halo_lo ? PO::ld_cg(halo_lo + p) : PO::zero());
-            up = (k < nz - 1) ? PO::ld(xk + p + plane) : (halo_hi ? PO::ld_cg(halo_hi + p) : PO::zero());
-        }
+        const E west = i0 > 0 ? __ldg(xk + p - 1) : zero_v(E());
+        const E east = (i0 + PW < nx) ? __ldg(xk + p + PW) : zero_v(E());
+        const P down = (k > 0) ? PO::ld(xk + p - plane) : (halo_lo ? PO::ld_cg(halo_lo + p) : PO::zero());
+        const P up = (k < nz - 1) ? PO::ld(xk + p + plane) : (halo_hi ? PO::ld_cg(halo_hi + p) : PO::zero());
         P out;
 #pragma unroll
         for (int e = 0; e < PW; ++e) {
@@ -165,40 +140,24 @@ k_stencil(const typename Tr<K>::E* __restrict__ x, typename Tr<K>::E* __restrict
             fmacc(s, (e < PW - 1 ? center.v[e < PW - 1 ? e + 1 : 0] : east), cf.c[2]);
             fmacc(s, south.v[e], cf.c[3]);
             fmacc(s, north.v[e], cf.c[4]);
-            if (DIM == 3) { fmacc(s, down.v[e], cf.c[5]); fmacc(s, up.v[e], cf.c[6]); }
+            fmacc(s, down.v[e], cf.c[5]);
+            fmacc(s, up.v[e], cf.c[6]);
             out.v[e] = s;
         }
         if (active) PO::st_w(y + k * plane + p, out, keep, pol);
-    };
-
-    P south = getrow(j0 - 1), center = getrow(j0);
-    int64_t j = j0;
-    for (; j + UN <= j1; j += UN) {
-        P nb[UN];
-#pragma unroll
-        for (int u = 0; u < UN; ++u) nb[u] = getrow(j + 1 + u);
-#pragma unroll
-        for (int u = 0; u < UN; ++u) {
-            do_row(j + u, south, center, nb[u]);
-            south = center; center = nb[u];
-        }
-    }
-    for (; j < j1; ++j) {
-        const P north = getrow(j + 1);
-        do_row(j, south, center, north);
         south = center; center = north;
     }
 }
 
 // ------------------------------------------------------------------------------------------
-// Shared-memory halo-staged stencil (default).  One CTA = ST_TX packs in x by RY rows in y.  The CTA
-// first issues ALL its loads -- the (RY+2) x ST_TX tile of plane k including the y-halo rows (from
-// the neighbouring rows, from the inter-GPU halo buffers at slab edges, or zero at the Dirichlet
-// boundary) and, in 3-D, the RY x ST_TX centre rows of planes k-1 / k+1 -- as 16-byte cp.async
-// copies straight into shared memory (RY+2 .. 3RY+2 requests in flight per thread, no register
-// staging), waits once, and then computes the RY output rows from shared memory: north / south /
-// west / east neighbours are shared-memory reads, only the west/east scalar of the tile's edge
-// columns comes from global memory.  Every x element is fetched from L2/HBM once per CTA.
+// 2-D 5-point stencil: shared-memory halo staging.  One CTA = ST_TX packs in x by ST_RY rows in y.  The CTA first
+// issues ALL its loads -- the (ST_RY+2) x ST_TX tile including the y-halo rows (from the neighbouring rows, from the
+// inter-GPU halo buffers at slab edges, or zero at the Dirichlet boundary) -- as cp.async copies straight into shared
+// memory (ST_RY+2 requests in flight per thread, no register staging), waits once, and then computes the ST_RY output
+// rows from shared memory: north / south / west / east neighbours are shared-memory reads, only the west/east scalar
+// of the tile's edge columns comes from global memory.  Every x element is fetched from L2/HBM once per CTA.
+// Why this kernel (B200, fp64, 4096^2, profiles/stencil_ab.py -> profiles/r02_stencil_ab.txt): 5.85 TB/s, against
+// 4.85 TB/s for a register y-march like the 3-D kernel's and 5.81 TB/s for the same staging with 4 rows per CTA.
 // ------------------------------------------------------------------------------------------
 enum { ST_TX = 128 };
 
@@ -210,7 +169,7 @@ template <int BYTES> LKB_DI void cp_async(void* smem_dst, const void* gsrc) {
 }
 LKB_DI void cp_async_wait_all() { asm volatile("cp.async.commit_group;\n\tcp.async.wait_group 0;" ::: "memory"); }
 
-template <int K, int PW, int DIM, int RY>
+template <int K, int PW>
 __global__ void __launch_bounds__(ST_TX)
 k_stencil_smem(const typename Tr<K>::E* __restrict__ x, typename Tr<K>::E* __restrict__ y,
                int64_t nx, int64_t ny, int64_t nz, Coef7<typename Tr<K>::E> cf,
@@ -232,22 +191,17 @@ k_stencil_smem(const typename Tr<K>::E* __restrict__ x, typename Tr<K>::E* __res
         if (halo_hi) halo_hi += off;
     }
     extern __shared__ __align__(16) unsigned char st_smem[];
-    P* tile = reinterpret_cast<P*>(st_smem);                       // [(RY+2)][ST_TX]
-    P* dn = tile + (RY + 2) * ST_TX;                               // [RY][ST_TX]  (3-D only)
-    P* up = dn + RY * ST_TX;                                       // [RY][ST_TX]
+    P* tile = reinterpret_cast<P*>(st_smem);                       // [(ST_RY+2)][ST_TX]
     const int tx = threadIdx.x;
     const int64_t npk_row = nx / PW;
-    const int64_t nyb = (ny + RY - 1) / RY;
-    const StBlock sb = st_decode<DIM>(ncb, nyb, nz);
-    const int64_t ip = sb.cb * ST_TX + tx;
+    const int64_t nyb = (ny + ST_RY - 1) / ST_RY;
+    const int64_t bid = blockIdx.x;
+    const int64_t cb = bid % ncb, rb = (bid / ncb + 1) % nyb;
+    const int64_t ip = cb * ST_TX + tx;
     const bool active = ip < npk_row;
     const int64_t i0 = ip * PW;
-    const int64_t k = sb.k;
-    const int64_t j0 = sb.rb * RY;
-    const int64_t plane = nx * ny;
-    halo_wait(halo_epoch, flag_lo, flag_hi, halo_lo && (DIM == 2 ? j0 == 0 : k == 0),
-              halo_hi && (DIM == 2 ? j0 + RY >= ny : k == nz - 1));
-    const E* xk = x + k * plane;
+    const int64_t j0 = rb * ST_RY;
+    halo_wait(halo_epoch, flag_lo, flag_hi, halo_lo && j0 == 0, halo_hi && j0 + ST_RY >= ny);
     P zero;
 #pragma unroll
     for (int e = 0; e < PW; ++e) zero.v[e] = zero_v(E());
@@ -255,44 +209,31 @@ k_stencil_smem(const typename Tr<K>::E* __restrict__ x, typename Tr<K>::E* __res
     if (active) {
         // ---- issue every load of the tile ----
 #pragma unroll
-        for (int r = 0; r < RY + 2; ++r) {
+        for (int r = 0; r < ST_RY + 2; ++r) {
             const int64_t j = j0 - 1 + r;
             const E* src = nullptr;
-            if (j >= 0 && j < ny) src = xk + j * nx + i0;
-            else if (DIM == 2 && j < 0 && halo_lo) src = halo_lo + i0;
-            else if (DIM == 2 && j >= ny && j == ny && halo_hi) src = halo_hi + i0;
+            if (j >= 0 && j < ny) src = x + j * nx + i0;
+            else if (j < 0 && halo_lo) src = halo_lo + i0;
+            else if (j == ny && halo_hi) src = halo_hi + i0;
             if (src && j <= ny) cp_async<PB>(&tile[r * ST_TX + tx], src);
             else tile[r * ST_TX + tx] = zero;
-        }
-        if (DIM == 3) {
-#pragma unroll
-            for (int r = 0; r < RY; ++r) {
-                const int64_t j = j0 + r;
-                if (j < ny) {
-                    const int64_t p = j * nx + i0;
-                    const E* sd = (k > 0) ? xk + p - plane : (halo_lo ? halo_lo + p : nullptr);
-                    const E* su = (k < nz - 1) ? xk + p + plane : (halo_hi ? halo_hi + p : nullptr);
-                    if (sd) cp_async<PB>(&dn[r * ST_TX + tx], sd); else dn[r * ST_TX + tx] = zero;
-                    if (su) cp_async<PB>(&up[r * ST_TX + tx], su); else up[r * ST_TX + tx] = zero;
-                }
-            }
         }
     }
     cp_async_wait_all();
     __syncthreads();
     if (!active) return;
-    // ---- compute RY rows out of shared memory ----
+    // ---- compute ST_RY rows out of shared memory ----
 #pragma unroll
-    for (int r = 0; r < RY; ++r) {
+    for (int r = 0; r < ST_RY; ++r) {
         const int64_t j = j0 + r;
         if (j >= ny) break;
         const int64_t p = j * nx + i0;
         const P center = tile[(r + 1) * ST_TX + tx], south = tile[r * ST_TX + tx], north = tile[(r + 2) * ST_TX + tx];
         E west, east;
         if (tx > 0) west = tile[(r + 1) * ST_TX + tx - 1].v[PW - 1];
-        else west = i0 > 0 ? __ldg(xk + p - 1) : zero_v(E());
+        else west = i0 > 0 ? __ldg(x + p - 1) : zero_v(E());
         if (tx < ST_TX - 1 && ip + 1 < npk_row) east = tile[(r + 1) * ST_TX + tx + 1].v[0];
-        else east = (i0 + PW < nx) ? __ldg(xk + p + PW) : zero_v(E());
+        else east = (i0 + PW < nx) ? __ldg(x + p + PW) : zero_v(E());
         P out;
 #pragma unroll
         for (int e = 0; e < PW; ++e) {
@@ -301,89 +242,9 @@ k_stencil_smem(const typename Tr<K>::E* __restrict__ x, typename Tr<K>::E* __res
             fmacc(sacc, (e < PW - 1 ? center.v[e < PW - 1 ? e + 1 : 0] : east), cf.c[2]);
             fmacc(sacc, south.v[e], cf.c[3]);
             fmacc(sacc, north.v[e], cf.c[4]);
-            if (DIM == 3) {
-                fmacc(sacc, dn[r * ST_TX + tx].v[e], cf.c[5]);
-                fmacc(sacc, up[r * ST_TX + tx].v[e], cf.c[6]);
-            }
             out.v[e] = sacc;
         }
-        PackOps<E, PW>::st_w(y + k * plane + p, out, keep, pol);
-    }
-}
-
-
-// ------------------------------------------------------------------------------------------
-// 3-D z-march (round 2; "3.5-D blocking").  One CTA = ZT_TX packs in x by ZT_TY rows in y, marching LZ planes in z
-// with the below / centre / above packs of its column in REGISTERS and the next plane prefetched one iteration
-// ahead.  The y-neighbours (rows j-1 / j+1 of the centre plane) are re-read through L1: the neighbouring threads
-// of the same CTA loaded exactly those lines one iteration earlier as their "above" pack.  Per point and plane the
-// kernel issues ONE load that can miss L1 -- against three in the y-marching kernel, whose z-neighbours belong to
-// other CTAs and are always served by L2 (ncu, 384^3 fp64: DRAM traffic already equal to the algorithmic 2 n s, but
-// 3.4 n s of L2->L1 traffic and 4.6 TB/s).  No shared memory, no block barrier (the shared-memory z-march of round 1
-// paid two barriers per plane: 2.8 TB/s).  Inter-GPU halo planes (k = -1, k = nz) come from halo_lo / halo_hi.
-// ------------------------------------------------------------------------------------------
-enum { ZT_TX = 32, ZT_TY = 8 };
-
-template <int K, int PW, int LZ>
-__global__ void __launch_bounds__(ZT_TX * ZT_TY)
-k_stencil3d_zmarch(const typename Tr<K>::E* __restrict__ x, typename Tr<K>::E* __restrict__ y,
-                   int64_t nx, int64_t ny, int64_t nz, Coef7<typename Tr<K>::E> cf,
-                   const typename Tr<K>::E* __restrict__ halo_lo, const typename Tr<K>::E* __restrict__ halo_hi,
-                   const unsigned* __restrict__ halo_epoch, int64_t halo_parity_stride, const unsigned* __restrict__ flag_lo,
-                   const unsigned* __restrict__ flag_hi, int64_t ncbx, int64_t ncby, const int* __restrict__ flags)
-{
-    using E = typename Tr<K>::E;
-    using PO = PackOps<E, PW>;
-    using P = typename PO::P;
-    pdl_wait();
-    pdl_trigger();
-    if (flags && flags[F_STOP]) return;
-    if (halo_epoch) {
-        const int64_t off = (int64_t)(*halo_epoch & 1u) * halo_parity_stride;
-        if (halo_lo) halo_lo += off;
-        if (halo_hi) halo_hi += off;
-    }
-    const int64_t nzc = (nz + LZ - 1) / LZ;
-    const int64_t bid = blockIdx.x;
-    const int64_t cbx = bid % ncbx, cby = (bid / ncbx) % ncby;
-    const int64_t zc = ((bid / (ncbx * ncby)) + 1) % nzc;            // the chunks touching the inter-GPU halos run last
-    const int64_t k0 = zc * LZ, k1 = min(nz, k0 + LZ);
-    halo_wait(halo_epoch, flag_lo, flag_hi, halo_lo && k0 == 0, halo_hi && k1 == nz);
-    const int tx = threadIdx.x % ZT_TX, ty = threadIdx.x / ZT_TX;
-    const int64_t npk_row = nx / PW;
-    const int64_t ip = cbx * ZT_TX + tx;
-    const int64_t j = cby * ZT_TY + ty;
-    if (ip >= npk_row || j >= ny) return;
-    const int64_t i0 = ip * PW;
-    const int64_t plane = nx * ny;
-    const int64_t q = j * nx + i0;                                   // offset inside a plane
-    auto load_plane = [&](int64_t k) -> P {
-        if (k < 0) return halo_lo ? PO::ld_cg(halo_lo + q) : PO::zero();
-        if (k >= nz) return halo_hi ? PO::ld_cg(halo_hi + q) : PO::zero();
-        return PO::ld(x + k * plane + q);
-    };
-    P down = load_plane(k0 - 1), center = load_plane(k0), up = load_plane(k0 + 1);
-    for (int64_t k = k0; k < k1; ++k) {
-        const P nxt = (k + 2 <= k1) ? load_plane(k + 2) : PO::zero();          // prefetch: used two iterations later as `up`
-        const E* xc = x + k * plane + q;
-        const P north = (j + 1 < ny) ? PO::ld(xc + nx) : PO::zero();
-        const P south = (j > 0) ? PO::ld(xc - nx) : PO::zero();
-        const E west = i0 > 0 ? __ldg(xc - 1) : zero_v(E());
-        const E east = (i0 + PW < nx) ? __ldg(xc + PW) : zero_v(E());
-        P out;
-#pragma unroll
-        for (int e = 0; e < PW; ++e) {
-            E s = mul_v(cf.c[0], center.v[e]);
-            fmacc(s, (e > 0 ? center.v[e > 0 ? e - 1 : 0] : west), cf.c[1]);
-            fmacc(s, (e < PW - 1 ? center.v[e < PW - 1 ? e + 1 : 0] : east), cf.c[2]);
-            fmacc(s, south.v[e], cf.c[3]);
-            fmacc(s, north.v[e], cf.c[4]);
-            fmacc(s, down.v[e], cf.c[5]);
-            fmacc(s, up.v[e], cf.c[6]);
-            out.v[e] = s;
-        }
-        PO::st(y + k * plane + q, out);
-        down = center; center = up; up = nxt;
+        PackOps<E, PW>::st_w(y + p, out, keep, pol);
     }
 }
 
@@ -400,52 +261,24 @@ static void stencil_launch(cudaStream_t s, const StencilArgs& a, const void* x, 
     }
     for (int q = 0; q < 7; ++q) from_scalar(c[q], cf.c[q]);
     const int64_t npk_row = a.nx / PW;
-    const int keep_w = ((size_t)a.nx * (size_t)a.ny * (size_t)(DIM == 3 ? a.nz : 1) * sizeof(E) <= w_keep_bytes()) ? 1 : 0;
-    // Measured on B200 (profiles/stencil_ab.py, fp64): 2-D 4096^2 -- shared-memory kernel RY=8 5.64 TB/s vs
-    // register march 5.24 TB/s; 3-D 384^3 -- shared-memory kernel 2.1-3.0 TB/s (3RY+2 staged rows per CTA cut
-    // the occupancy) vs register march 4.62 TB/s; a z-march with the plane staged in shared memory (two block
-    // barriers per plane) reached only 2.8 TB/s and was dropped; a register z-march (variant 4, k_stencil3d_zmarch) 3.95 TB/s.
-    // Default: shared-memory staging in 2-D, register y-march in 3-D.
-    // 3-D: the z-march (variant 4) measured 3.95 TB/s against 4.32 TB/s for the y-march at 384^3 in three separate runs
-    // (gpurun_out/r02_stencil_ab*.txt) -- the y-march stays the default
-    static const int env_variant = getenv("LKB_STENCIL_VARIANT") ? atoi(getenv("LKB_STENCIL_VARIANT")) : -1;
-    const int variant = env_variant >= 0 ? env_variant : (a.variant >= 0 ? a.variant : (DIM == 2 ? 1 : 0));
-    if constexpr (DIM == 3) {
-        if (variant == 4) {      // z-march with register planes (A/B only)
-            constexpr int LZ = 32;
-            const int64_t ncbx = (npk_row + ZT_TX - 1) / ZT_TX, ncby = (a.ny + ZT_TY - 1) / ZT_TY, nzc = (a.nz + LZ - 1) / LZ;
-            const unsigned grid = (unsigned)(ncbx * ncby * nzc);
-            launch_ex(k_stencil3d_zmarch<K, PW, LZ>, grid, ZT_TX * ZT_TY, 0, s, pdl_take(1), (const E*)x, (E*)y, a.nx, a.ny, a.nz, cf,
-                (const E*)a.halo_lo, (const E*)a.halo_hi, a.halo_epoch, a.halo_parity_stride, a.flag_lo, a.flag_hi, ncbx, ncby, flags);
-            return;
-        }
+    const int64_t nyb = (a.ny + ST_RY - 1) / ST_RY;
+    const int keep_w = ((size_t)a.nx * (size_t)a.ny * (size_t)a.nz * sizeof(E) <= W_KEEP_BYTES) ? 1 : 0;
+    auto launch = [&](auto kern, int64_t ncb, unsigned block, size_t smem) {
+        const unsigned grid = (unsigned)(nyb * a.nz * ncb);
+        launch_ex(kern, grid, block, smem, s, pdl_take(1), (const E*)x, (E*)y, a.nx, a.ny, a.nz, cf,
+                  (const E*)a.halo_lo, (const E*)a.halo_hi, a.halo_epoch, a.halo_parity_stride, a.flag_lo, a.flag_hi, ncb, flags, keep_w);
+    };
+    if constexpr (DIM == 2) {
+        static const SmemAttrOnce once((const void*)k_stencil_smem<K, PW>, 96 * 1024);
+        once.ensure();
+        launch(k_stencil_smem<K, PW>, (npk_row + ST_TX - 1) / ST_TX, ST_TX, (size_t)(ST_RY + 2) * ST_TX * sizeof(Pack<E, PW>));
+    } else {
+        // CTA width: the narrowest multiple of 32 threads that covers a grid row with the same number of CTAs as 256-wide
+        // ones would (384^3: 192 packs per row -> 192 threads, no idle lanes; a 256-wide CTA left 25 % of its threads idle:
+        // 4.28 TB/s at 384^3 against 5.17 TB/s at 512^3)
+        const int64_t ncb = (npk_row + 255) / 256;
+        launch(k_stencil<K, PW>, ncb, (unsigned)std::min<int64_t>(256, ((npk_row + ncb - 1) / ncb + 31) / 32 * 32), 0);
     }
-    if (variant >= 1 && variant <= 3) {
-        // shared-memory halo-staged kernel
-#define LKB_STS(RY_) { const int64_t nyb_ = (a.ny + RY_ - 1) / RY_; \
-            const int64_t ncb_ = (npk_row + ST_TX - 1) / ST_TX; \
-            const unsigned grid_ = (unsigned)(nyb_ * (DIM == 3 ? a.nz : 1) * ncb_); \
-            const size_t sh_ = (size_t)((RY_ + 2) + (DIM == 3 ? 2 * RY_ : 0)) * ST_TX * sizeof(Pack<E, PW>); \
-            static const SmemAttrOnce once_((const void*)k_stencil_smem<K, PW, DIM, RY_>, 96 * 1024); once_.ensure(); \
-            launch_ex(k_stencil_smem<K, PW, DIM, RY_>, grid_, ST_TX, sh_, s, pdl_take(1), (const E*)x, (E*)y, a.nx, a.ny, a.nz, cf, \
-                (const E*)a.halo_lo, (const E*)a.halo_hi, a.halo_epoch, a.halo_parity_stride, a.flag_lo, a.flag_hi, ncb_, flags, keep_w); }
-        if (variant == 3) LKB_STS(4) else LKB_STS(8)
-#undef LKB_STS
-        return;
-    }
-    // variant 0: register-marching kernel.  RY = 8 rows per CTA, no unrolling, L1-served x-halo
-    // (profiles/stencil_ab.py, B200: 5.2 TB/s 2-D 4096^2 / 4.6 TB/s 3-D 384^3; longer marches or 4x-unrolled
-    // prefetch were slower, warp-shuffle x-halo made no difference).
-    constexpr int RY = 8;
-    const int64_t nyb = (a.ny + RY - 1) / RY;
-    // CTA width: the narrowest multiple of 32 threads that covers a grid row with the same number of CTAs as 256-wide
-    // ones would (384^3: 192 packs per row -> 192 threads, no idle lanes; a 256-wide CTA left 25 % of its threads idle:
-    // 4.28 TB/s at 384^3 against 5.17 TB/s at 512^3)
-    const int64_t ncb = (npk_row + 255) / 256;
-    const unsigned bs = (unsigned)std::min<int64_t>(256, ((npk_row + ncb - 1) / ncb + 31) / 32 * 32);
-    const unsigned grid = (unsigned)(nyb * (DIM == 3 ? a.nz : 1) * ncb);
-    launch_ex(k_stencil<K, PW, DIM, RY, 1, false>, grid, bs, 0, s, pdl_take(1), (const E*)x, (E*)y, a.nx, a.ny, a.nz, cf,
-              (const E*)a.halo_lo, (const E*)a.halo_hi, a.halo_epoch, a.halo_parity_stride, a.flag_lo, a.flag_hi, ncb, flags, keep_w);
 }
 
 template <int K>
@@ -588,10 +421,17 @@ void launch_csr(int kind, cudaStream_t s, int64_t m, const int64_t* rowptr, cons
 // ------------------------------------------------------------------------------------------
 // L2-blocked CSR SpMV (layout: lkb_csr.cu).  One launch per column block; thread-per-row (a row has ~nnz/nb entries
 // in a block: 1-3 for C5), consecutive threads read consecutive table entries and nearly consecutive values.
-// The x gathers of a block all fall into one L2-resident slice; they carry an L2 evict_last policy while the
-// streamed operands (table, col, val, y) are marked evict_first so that they do not push the slice out.
-LKB_DI uint64_t l2_policy_evict_last() { uint64_t p; asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p)); return p; }
-LKB_DI uint64_t l2_policy_evict_first() { uint64_t p; asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p)); return p; }
+// The x gathers of a block all fall into one L2-resident slice and carry an L2 evict_last policy; the streamed
+// operands (table, col, val) carry evict_normal.
+// Why this kernel (B200, full-size C5 matrix, 48 MB slices, matvec ms per sweep, profiles/spmv_ab.py): 16.4 ms
+// (profiles/r02_spmv_ab3_persistL2.jsonl), bandwidth-bound on its actual traffic (ncu: DRAM 6.9 GB per block at
+// 5.3 TB/s, of which ~3 GB are x-gather sectors that missed L2; profiles/r02_ncu_summary.md).  Measured slower:
+//   the same kernel with evict_first streams                              17.2 ms  (profiles/r02_spmv_ab2.jsonl)
+//   CSR-stream: coalesced col / val runs per CTA, products staged in      19.5 ms  (profiles/r02_spmv_ab2.jsonl)
+//     shared memory; latency-bound at 64 registers, 4 CTAs / SM
+//   warp-pipelined CSR-stream (cp.async-staged col / val, no barrier)     20.7 ms  (profiles/r02_spmv_ab4_warp_pipelined.jsonl)
+// All stream forms land at 19-21 ms whatever hides the col / val latency: the L2 gather rate (~100 G sectors/s), not the
+// streams, is what they wait for.  A persisting-L2 set-aside (64 / 79 MB) changed none of them by more than 2 %.
 LKB_DI uint64_t l2_policy_evict_normal() { uint64_t p; asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(p)); return p; }
 template <typename T> LKB_DI T ld_hint(const T* p, uint64_t pol);
 template <> LKB_DI float ld_hint<float>(const float* p, uint64_t pol) {
@@ -611,11 +451,11 @@ template <int K>
 __global__ void __launch_bounds__(256)
 k_csr_blocked(int64_t rows, const uint32_t* __restrict__ tab, const int32_t* __restrict__ col,
               const typename Tr<K>::E* __restrict__ val, const typename Tr<K>::E* __restrict__ x,
-              typename Tr<K>::E* __restrict__ y, bool conj_vals, bool first, const int* __restrict__ flags, bool stream_first)
+              typename Tr<K>::E* __restrict__ y, bool conj_vals, bool first, const int* __restrict__ flags)
 {
     using E = typename Tr<K>::E;
     if (flags && flags[F_STOP]) return;
-    const uint64_t keep = l2_policy_evict_last(), stream = stream_first ? l2_policy_evict_first() : l2_policy_evict_normal();
+    const uint64_t keep = pol_evict_last(), stream = l2_policy_evict_normal();
     for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < rows; r += (int64_t)gridDim.x * blockDim.x) {
         const uint32_t q0 = ld_hint<uint32_t>(tab + r, stream), q1 = ld_hint<uint32_t>(tab + r + 1, stream);
         if (q0 == q1 && !first) continue;                       // nothing in this block for row r
@@ -628,127 +468,17 @@ k_csr_blocked(int64_t rows, const uint32_t* __restrict__ tab, const int32_t* __r
         y[r] = acc;
     }
 }
-// "CSR-stream" variant (default): a CTA owns CS_ROWS consecutive rows of the block, whose entries are ONE contiguous
-// run [tab[r0], tab[r0 + CS_ROWS]) of the blocked arrays.  Phase 1: all threads stride over that run -- perfectly
-// coalesced col / val streams, CS_U independent gathers of x in flight per thread -- and park the products in shared
-// memory; phase 2: every thread sums the products of its rows in position order (the same fixed order as the
-// thread-per-row kernel) and updates y.  The thread-per-row kernel chains tab -> col -> x -> fma with 2-3 entries per
-// row and ran latency-bound (~3.3 TB/s of DRAM traffic on C5); here the three dependent loads of a chain are issued
-// for CS_U entries at a time.  Streamed operands: L1::no_allocate + L2 evict_first; x gathers: L2 evict_last.
-enum { CS_ROWS = 512, CS_CH = 2048 };
-template <typename T> LKB_DI T ld_stream(const T* p, uint64_t pol);
-template <> LKB_DI float ld_stream<float>(const float* p, uint64_t pol) {
-    float v; asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.f32 %0, [%1], %2;" : "=f"(v) : "l"(p), "l"(pol)); return v; }
-template <> LKB_DI double ld_stream<double>(const double* p, uint64_t pol) {
-    double v; asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.f64 %0, [%1], %2;" : "=d"(v) : "l"(p), "l"(pol)); return v; }
-template <> LKB_DI float2 ld_stream<float2>(const float2* p, uint64_t pol) {
-    float2 v; asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v2.f32 {%0, %1}, [%2], %3;" : "=f"(v.x), "=f"(v.y) : "l"(p), "l"(pol)); return v; }
-template <> LKB_DI double2 ld_stream<double2>(const double2* p, uint64_t pol) {
-    double2 v; asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v2.f64 {%0, %1}, [%2], %3;" : "=d"(v.x), "=d"(v.y) : "l"(p), "l"(pol)); return v; }
-template <> LKB_DI int32_t ld_stream<int32_t>(const int32_t* p, uint64_t pol) {
-    int32_t v; asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.s32 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol)); return v; }
-template <> LKB_DI uint32_t ld_stream<uint32_t>(const uint32_t* p, uint64_t pol) {
-    uint32_t v; asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.u32 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol)); return v; }
-
-template <int K, int CS_U, int MINB>
-__global__ void __launch_bounds__(256, MINB)
-k_csr_blocked_stream(int64_t rows, const uint32_t* __restrict__ tab, const int32_t* __restrict__ col,
-                     const typename Tr<K>::E* __restrict__ val, const typename Tr<K>::E* __restrict__ x,
-                     typename Tr<K>::E* __restrict__ y, bool conj_vals, bool first, const int* __restrict__ flags)
-{
-    using E = typename Tr<K>::E;
-    constexpr int RPT = CS_ROWS / 256;                      // rows per thread
-    if (flags && flags[F_STOP]) return;
-    extern __shared__ __align__(16) unsigned char cs_smem[];
-    E* prod = reinterpret_cast<E*>(cs_smem);                // [CS_CH]
-    const uint64_t keep = l2_policy_evict_last(), stream = l2_policy_evict_first();
-    const int tid = threadIdx.x;
-    for (int64_t r0 = (int64_t)blockIdx.x * CS_ROWS; r0 < rows; r0 += (int64_t)gridDim.x * CS_ROWS) {
-        const int64_t rend = min(rows, r0 + CS_ROWS);
-        uint32_t qa[RPT], qb[RPT];
-        E acc[RPT];
-#pragma unroll
-        for (int i = 0; i < RPT; ++i) {
-            const int64_t r = r0 + tid + 256 * i;
-            qa[i] = qb[i] = 0u; acc[i] = zero_v(E());
-            if (r < rend) {
-                qa[i] = ld_stream<uint32_t>(tab + r, stream); qb[i] = ld_stream<uint32_t>(tab + r + 1, stream);
-                if (!first && qa[i] != qb[i]) acc[i] = y[r];
-            }
-        }
-        const uint32_t qs = ld_stream<uint32_t>(tab + r0, stream), qe = ld_stream<uint32_t>(tab + rend, stream);
-        for (uint32_t c0 = qs; c0 < qe; c0 += CS_CH) {
-            const uint32_t c1 = min(c0 + (uint32_t)CS_CH, qe);
-            // ---- phase 1: products of the run [c0, c1) into shared memory ----
-            for (uint32_t e0 = c0 + tid; e0 < c1; e0 += 256 * CS_U) {
-                int32_t cj[CS_U]; E a[CS_U], xv[CS_U];
-#pragma unroll
-                for (int u = 0; u < CS_U; ++u) { const uint32_t e = e0 + 256 * u; if (e < c1) cj[u] = ld_stream<int32_t>(col + e, stream); }
-#pragma unroll
-                for (int u = 0; u < CS_U; ++u) { const uint32_t e = e0 + 256 * u; if (e < c1) a[u] = ld_stream<E>(val + e, stream); }
-#pragma unroll
-                for (int u = 0; u < CS_U; ++u) { const uint32_t e = e0 + 256 * u; if (e < c1) xv[u] = ld_hint<E>(x + cj[u], keep); }
-#pragma unroll
-                for (int u = 0; u < CS_U; ++u) {
-                    const uint32_t e = e0 + 256 * u;
-                    if (e < c1) prod[e - c0] = mul_v(conj_vals ? conj_v(a[u]) : a[u], xv[u]);
-                }
-            }
-            __syncthreads();
-            // ---- phase 2: row sums in position order ----
-#pragma unroll
-            for (int i = 0; i < RPT; ++i) {
-                const uint32_t lo = max(qa[i], c0), hi = min(qb[i], c1);
-                for (uint32_t q = lo; q < hi; ++q) acc[i] = add_v(acc[i], prod[q - c0]);
-            }
-            __syncthreads();
-        }
-#pragma unroll
-        for (int i = 0; i < RPT; ++i) {
-            const int64_t r = r0 + tid + 256 * i;
-            if (r < rend && (first || qa[i] != qb[i])) y[r] = acc[i];
-        }
-    }
-}
 void launch_csr_blocked(int kind, cudaStream_t s, const CsrBlocked& b, const void* x, void* y, bool conj_vals, const int* flags, int sms) {
-    // Variants measured on the full-size C5 matrix (B200, profiles/spmv_ab.py, gpurun_out/r02_spmv_ab*.jsonl; ncu in
-    // profiles/r02_ncu_summary.md), matvec ms per sweep at 48 MB slices:
-    //   0  thread-per-row, streams evict_first    17.2   DRAM 6.9 GB / block at 5.3 TB/s: bandwidth-bound on ACTUAL traffic,
-    //                                                    of which ~3 GB are x-gather sectors that missed L2
-    //   2  thread-per-row, streams evict_normal   16.4   (default)
-    //   1  CSR-stream                             19.5   DRAM 4.9 GB / block (x misses 0.9 GB) but latency-bound at 64 regs,
-    //                                                    4 CTAs / SM; forcing 5-6 CTAs / SM spills and doubles the time
-    //   3  warp-pipelined CSR-stream (cp.async-staged col / val per warp, no block barrier; removed again)   20.7
-    // All stream forms land at 19-21 ms whatever hides the col / val latency: the L2 gather rate (~100 G sectors/s), not the
-    // streams, is what they wait for.  A persisting-L2 set-aside (64 / 79 MB) changed none of them by more than 2 %.
-    static const int env_variant = getenv("LKB_CSR_BLOCKED_VARIANT") ? atoi(getenv("LKB_CSR_BLOCKED_VARIANT")) : -1;
-    const int variant = env_variant >= 0 ? env_variant : b.variant;
-    if (variant == 1) {
-        int64_t nbs = (b.rows + CS_ROWS - 1) / CS_ROWS;
-        if (nbs < 1) nbs = 1;
-        if (nbs > (int64_t)sms * 6) nbs = (int64_t)sms * 6;
-        const size_t sh = (size_t)CS_CH * kind_size(kind);
-        for (int blk = 0; blk < b.nb; ++blk) {
-            const uint32_t* tab = b.tab + (size_t)blk * (b.rows + 1);
-#define LKB_CSS(K_, E_, U_, M_) k_csr_blocked_stream<K_, U_, M_><<<(int)nbs, 256, sh, s>>>(b.rows, tab, b.col, (const E_*)b.val, (const E_*)x, (E_*)y, conj_vals, blk == 0, flags)
-#define LKB_CSS_K(U_, M_) switch (kind) { case KS: LKB_CSS(KS, float, U_, M_); break; case KD: LKB_CSS(KD, double, U_, M_); break; \
-                                          case KC: LKB_CSS(KC, float2, U_, M_); break; default: LKB_CSS(KZ, double2, U_, M_); break; }
-            LKB_CSS_K(4, 4)      // 4 gathers in flight per thread, 4 CTAs / SM (64 registers); 2 x 6 and 3 x 5 spill and run 2x slower
-#undef LKB_CSS_K
-#undef LKB_CSS
-        }
-        return;
-    }
     int64_t nb = (b.rows + 255) / 256;
     if (nb < 1) nb = 1;
     if (nb > (int64_t)sms * 16) nb = (int64_t)sms * 16;
     for (int blk = 0; blk < b.nb; ++blk) {
         const uint32_t* tab = b.tab + (size_t)blk * (b.rows + 1);
         switch (kind) {
-            case KS: k_csr_blocked<KS><<<(int)nb, 256, 0, s>>>(b.rows, tab, b.col, (const float*)b.val, (const float*)x, (float*)y, conj_vals, blk == 0, flags, variant == 0); break;
-            case KD: k_csr_blocked<KD><<<(int)nb, 256, 0, s>>>(b.rows, tab, b.col, (const double*)b.val, (const double*)x, (double*)y, conj_vals, blk == 0, flags, variant == 0); break;
-            case KC: k_csr_blocked<KC><<<(int)nb, 256, 0, s>>>(b.rows, tab, b.col, (const float2*)b.val, (const float2*)x, (float2*)y, conj_vals, blk == 0, flags, variant == 0); break;
-            default: k_csr_blocked<KZ><<<(int)nb, 256, 0, s>>>(b.rows, tab, b.col, (const double2*)b.val, (const double2*)x, (double2*)y, conj_vals, blk == 0, flags, variant == 0); break;
+            case KS: k_csr_blocked<KS><<<(int)nb, 256, 0, s>>>(b.rows, tab, b.col, (const float*)b.val, (const float*)x, (float*)y, conj_vals, blk == 0, flags); break;
+            case KD: k_csr_blocked<KD><<<(int)nb, 256, 0, s>>>(b.rows, tab, b.col, (const double*)b.val, (const double*)x, (double*)y, conj_vals, blk == 0, flags); break;
+            case KC: k_csr_blocked<KC><<<(int)nb, 256, 0, s>>>(b.rows, tab, b.col, (const float2*)b.val, (const float2*)x, (float2*)y, conj_vals, blk == 0, flags); break;
+            default: k_csr_blocked<KZ><<<(int)nb, 256, 0, s>>>(b.rows, tab, b.col, (const double2*)b.val, (const double2*)x, (double2*)y, conj_vals, blk == 0, flags); break;
         }
     }
 }

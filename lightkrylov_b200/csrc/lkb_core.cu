@@ -130,13 +130,6 @@ int allreduce_w(lkb_ctx_s* c, void* buf, size_t ndoubles) {
 }
 int& pdl_state() { static thread_local int s = 0; return s; }
 int& sweep_dir() { static thread_local int d = 0; return d; }
-size_t w_keep_bytes() { static const size_t b = (size_t)(getenv("LKB_W_KEEP_MB") ? atoi(getenv("LKB_W_KEEP_MB")) : 48) << 20; return b; }
-// Which kernel classes are launched programmatically (bits: 1 matvec, 2 multi-dot, 4 fused axpy+dot, 8 multi-axpy, 16 scale).
-// Default 4: only the TMA kernel.  Measured on B200 (profiles/r02_pdl2.sh .. r02_pdl4.sh): a programmatically launched
-// kernel inherits the predecessor's L1 / shared-memory carve-out, which costs the LDG-based multi-dot / multi-axpy
-// kernels up to 11 % (4096 x 512: all classes 1729 steps/s, none 1870, fused only 1876); the TMA kernel is carve-out
-// neutral and gains from filling its ring during the multi-dot's tail (reduction tree + NVLink allreduce).
-int pdl_mask() { static const int m = getenv("LKB_PDL_MASK") ? atoi(getenv("LKB_PDL_MASK")) : 4; return m; }
 // Stream-ordered allocation of vectors / bases / solver work space from the device's default memory pool with an
 // unlimited release threshold: freed blocks stay cached in the pool, so the GB-sized work bases that gmres / cg /
 // eigs allocate per call (`allocate(V(kdim+1), source=b)` in the reference) cost a pool lookup instead of a
@@ -338,11 +331,8 @@ int lkb_set_option(lkb_ctx_t c, const char* name, int value) {
     else if (!strcmp(name, "fin")) c->fin = value != 0;
     else if (!strcmp(name, "pdl")) c->pdl = value != 0;
     else if (!strcmp(name, "serpentine")) c->serpentine = value != 0;
-    else if (!strcmp(name, "write_intermediate")) c->write_intermediate = value != 0;
     else if (!strcmp(name, "csr_slice_kb")) c->csr_slice_kb = value;            // 0 disables the L2 blocking
     else if (!strcmp(name, "csr_block_min_kb")) c->csr_block_min_kb = value;
-    else if (!strcmp(name, "csr_blocked_variant")) c->csr_variant = value;
-    else if (!strcmp(name, "stencil_variant")) c->stencil_variant = value;
     else if (!strcmp(name, "fused_halo")) c->fused_halo = value != 0;
     else if (!strcmp(name, "p2p")) c->p2p_active = (value != 0) && c->p2p.world > 1;
     else { set_error("unknown option %s", name); return LKB_ERR_ARG; }
@@ -845,7 +835,6 @@ int op_apply_enqueue(lkb_op_s* A, const void* x, void* y, bool trans, const int*
             LKB_NCCL(api->GroupEnd());
             pdl_rearm();
         }
-        A->st.variant = c->stencil_variant;
         launch_stencil(A->kind, c->stream, A->st, x, y, trans, flags, c->sms);
     } else if (A->type == 3 && A->dist) {
         const int dt = (A->kind == KS || A->kind == KC) ? 7 : 8;            // ncclFloat32 / ncclFloat64

@@ -288,7 +288,6 @@ int csr_block_device(lkb_ctx_s* c, int kind, int64_t rows, int64_t ncols, int64_
     cudaFree(*rowptr); cudaFree(*col); cudaFree(*val);
     *rowptr = nullptr; *col = nullptr; *val = nullptr;
     blk->nb = nb; blk->cw = cw; blk->rows = rows; blk->nnz = nnz; blk->tab = tab; blk->col = bcol; blk->val = bval;
-    blk->variant = c->csr_variant;
     return 0;
 }
 

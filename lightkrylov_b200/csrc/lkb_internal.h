@@ -57,8 +57,6 @@ struct lkb_ctx_s {
     bool fin = true;            // final CGS2 pass fused with normalisation + column update (k_multiaxpy_fin)
     bool serpentine = true;     // consecutive Gram-Schmidt kernels of a step sweep the rows in opposite directions (lkb_kernels.h)
     bool pdl = true;            // programmatic dependent launch of the step-loop kernels (lkb_kernels.h: PdlScope)
-    int stencil_variant = -1;   // option "stencil_variant": A/B of the stencil kernels (-1 = the measured default per dimension)
-    int csr_variant = 2;        // SpMV kernel of L2-blocked operators created from now on (option "csr_blocked_variant")
     int csr_slice_kb = 48 * 1024, csr_block_min_kb = 96 * 1024;   // L2 blocking of CSR operators (lkb_csr.cu)
     bool write_intermediate = false;   // eigs / eighs / svds rewrite <solver>_output.txt every step (rank 0)
     bool fused_halo = true;     // P2P halo push fused into the kernel that finishes the next matvec input

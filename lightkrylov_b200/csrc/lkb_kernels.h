@@ -55,9 +55,14 @@ struct SmemAttrOnce {
 // aware launch is a normal one (its predecessor in the stream is not one of our kernels: memset, NCCL, user
 // callback), afterwards the chain is on.  pdl_rearm() after anything that is not a kernel of this library.
 int& pdl_state();
-// cls: kernel class bit for the LKB_PDL_MASK experiment switch (1 matvec, 2 multi-dot, 4 fused, 8 multi-axpy, 16 scale)
-int pdl_mask();
-inline bool pdl_take(int cls = 0xff) { int& s = pdl_state(); if (s == 2) return (pdl_mask() & cls) != 0; if (s == 1) s = 2; return false; }
+// Kernel classes launched programmatically (bits: 1 matvec, 2 multi-dot, 4 fused axpy+dot, 8 multi-axpy, 16 scale): only
+// the TMA kernel.  Measured on B200 (profiles/r02_pdl2.sh .. r02_pdl4.sh): a programmatically launched kernel inherits the
+// predecessor's L1 / shared-memory carve-out, which costs the LDG-based multi-dot / multi-axpy kernels up to 11 %
+// (4096 x 512: all classes 1729 steps/s, none 1870, fused only 1876); the TMA kernel is carve-out neutral and gains from
+// filling its ring during the multi-dot's tail (reduction tree + NVLink allreduce).
+constexpr int PDL_CLASSES = 4;
+// cls: the class bit of the launching kernel
+inline bool pdl_take(int cls = 0xff) { int& s = pdl_state(); if (s == 2) return (PDL_CLASSES & cls) != 0; if (s == 1) s = 2; return false; }
 inline void pdl_rearm() { int& s = pdl_state(); if (s == 2) s = 1; }
 struct PdlScope {
     int prev;
@@ -70,8 +75,7 @@ struct PdlScope {
 // directions: a kernel starts on the rows its predecessor read last, which are still L2-resident (126 MB L2: ~10 % of
 // a kernel's bytes at the per-GPU share of N = 8, ~1 % at N = 1).  The direction is a pure function of the step index
 // (dgs_enqueue), so results stay bitwise reproducible (graphs on / off, one-shot vs step-by-step, any launch timing).
-size_t w_keep_bytes(); // slices of w up to this size are kept L2-resident (evict_last), LKB_W_KEEP_MB, default 48; lkb_types.cuh
-int& sweep_dir();      // 0 ascending, 1 descending: read by launch_multidot / launch_axpy_dot / launch_multiaxpy_fin
+int& sweep_dir();     // 0 ascending, 1 descending: read by launch_multidot / launch_axpy_dot / launch_multiaxpy_fin
 struct SweepDir {
     int prev;
     explicit SweepDir(int d) : prev(sweep_dir()) { sweep_dir() = d; }
@@ -94,7 +98,6 @@ struct StencilArgs {
     const void* halo_lo;       // previous slab's last row/plane (nullptr = Dirichlet boundary)
     const void* halo_hi;       // next slab's first row/plane
     int dim;                   // 2 or 3
-    int variant = -1;          // kernel variant (kernels_ops.cu: 0 register y-march, 1-3 shared-memory staging, 4 register z-march); -1 = default
     // p2p halo exchange: halo_lo / halo_hi point at parity 0 of double-buffered regions; the kernel adds
     // (epoch & 1) * halo_parity_stride elements, epoch being the device counter of the push kernel
     const unsigned* halo_epoch = nullptr;
@@ -179,7 +182,6 @@ void launch_narrow(int kind, cudaStream_t s, const void* src, void* dst, int n, 
 // L2-blocked CSR (lkb_csr.cu): non-zeros sorted by column block; tab[b * (rows + 1) + r] = first entry of (block b, row r)
 struct CsrBlocked {
     int nb = 0; int64_t cw = 0, rows = 0, nnz = 0;
-    int variant = 2;           // kernel: 2 thread-per-row (default), 0 same with evict_first streams, 1 CSR-stream (kernels_ops.cu)
     uint32_t* tab = nullptr; int32_t* col = nullptr; void* val = nullptr;
 };
 // y = A x over the blocked layout: one sweep per column block, y accumulated across the blocks

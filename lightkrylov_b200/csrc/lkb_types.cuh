@@ -152,11 +152,13 @@ template <typename P> LKB_DI P ld_pack(const void* p) {      // coherent streami
 #endif
     return *reinterpret_cast<P*>(&r);
 }
-// Accesses of the WORK VECTOR w of a Krylov step.  When a GPU's slice of w is small (<= w_keep_bytes(), default 48 MB: the
+// Accesses of the WORK VECTOR w of a Krylov step.  When a GPU's slice of w is small (<= W_KEEP_BYTES = 48 MB: the
 // 1/4 and 1/8 shares of C2) every access of w carries an L2 evict_last policy, so w survives the j columns of V that
 // stream through L2 between its uses (matvec writes it, the multi-dot, the fused kernel and the final axpy read it):
 // 4096 x 512 1917 -> 1943 steps/s (+1.4 %, the fused kernel +5 %).  At full size (134 MB per vector > L2) the hint costs
-// 0.9 %, hence the size switch (profiles/r02_l2hint.sh with the -DLKB_W_EVICT_LAST experiment build, round 2).
+// 0.9 %, hence the size switch (profiles/r02_l2hint.sh with the -DLKB_W_EVICT_LAST experiment build, round 2; A/B of the
+// threshold in profiles/r02_wkeep_result.txt).
+constexpr size_t W_KEEP_BYTES = (size_t)48 << 20;
 LKB_DI uint64_t pol_evict_last() { uint64_t p; asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p)); return p; }
 template <typename P> LKB_DI P ld_pack_w(const void* p, bool keep, uint64_t pol) {          // coherent (w is rewritten by the kernel)
     if (!keep) return ld_pack<P>(p);

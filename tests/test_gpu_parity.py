@@ -149,10 +149,11 @@ def test_qr_breakdown_refill(lk, ctx):
 # ---------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("kind", ["d", "z", "s"])
 @pytest.mark.parametrize("dims", [(512, 40), (260, 33), (96, 24, 40), (33, 17), (30, 9, 35)])
-def test_stencil_kernel_variants_agree(lk, ctx, oracle, kind, dims):
-    """Every stencil kernel kept for A/B (option "stencil_variant": 0 register y-march, 1 / 3 shared-memory staging with 8 / 4
-    rows, 4 register z-march in 3-D) computes the same matvec / rmatvec as the oracle -- incl. rows that are not a multiple
-    of the pack width (partial packs) and row lengths that leave lanes of a CTA idle."""
+def test_stencil_ragged_shapes_vs_oracle(lk, ctx, oracle, kind, dims):
+    """The 2-D (shared-memory staging) and 3-D (register y-march) stencil kernels compute the same matvec / rmatvec as the
+    oracle on awkward shapes: rows that are not a multiple of the pack width (partial packs), row lengths that leave lanes
+    of a CTA idle, and row counts that are not a multiple of the rows per CTA.  There is one kernel per dimension and no
+    option to select another."""
     dt = lk.DTYPES[kind]
     coef = list(CONVDIFF7[: 5 if len(dims) == 2 else 7])
     n = int(np.prod(dims))
@@ -161,15 +162,12 @@ def test_stencil_kernel_variants_agree(lk, ctx, oracle, kind, dims):
     xh = randn(np.random.default_rng(2), n, dt)
     x = lk.Vector(ctx, kind, n).put(xh)
     tol = dict(rtol=1e-5, atol=1e-5) if kind == "s" else dict(rtol=1e-13, atol=1e-13)
-    try:
-        for v in (0, 1, 3, 4):
-            ctx.set_option("stencil_variant", v)
-            y = lk.Vector(ctx, kind, n).put(np.full(n, np.nan, dtype=dt)); z = lk.Vector(ctx, kind, n).put(np.full(n, np.nan, dtype=dt))
-            A.matvec(x, y); A.rmatvec(x, z)
-            np.testing.assert_allclose(y.get(), Ao.apply(xh), **tol)
-            np.testing.assert_allclose(z.get(), Ao.apply(xh, trans=True), **tol)
-    finally:
-        ctx.set_option("stencil_variant", -1)
+    y = lk.Vector(ctx, kind, n).put(np.full(n, np.nan, dtype=dt)); z = lk.Vector(ctx, kind, n).put(np.full(n, np.nan, dtype=dt))
+    A.matvec(x, y); A.rmatvec(x, z)
+    np.testing.assert_allclose(y.get(), Ao.apply(xh), **tol)
+    np.testing.assert_allclose(z.get(), Ao.apply(xh, trans=True), **tol)
+    with pytest.raises(lk.LkbError, match="unknown option stencil_variant"):
+        ctx.set_option("stencil_variant", 0)
 
 
 @pytest.mark.parametrize("kind", KINDS)
@@ -911,22 +909,21 @@ def test_basis_level_helpers(lk, ctx, oracle, kind):
 
 
 @pytest.mark.parametrize("kind", ["z", "d", "s"])
-def test_csr_l2_blocked_layout_matches_plain(lk, ctx, oracle, kind):
+def test_csr_l2_blocked_slices_vs_plain_and_oracle(lk, ctx, oracle, kind):
     """The L2-blocked CSR layout (column blocks, used when the gathered vector exceeds L2: C5 at BASELINE size) forced on a
-    small matrix: matvec / rmatvec agree with the oracle and with the plain layout, run-to-run bitwise, and a
-    bidiagonalization through it matches the oracle at 1e-10."""
+    small matrix with 8 KB and 64 KB slices: matvec / rmatvec agree with the oracle and with the plain layout, run-to-run
+    bitwise, and a bidiagonalization through it matches the oracle at 1e-10.  There is one blocked SpMV kernel and no option
+    to select another."""
     dt = lk.DTYPES[kind]; m, n, pr = 9001, 7003, 12
     rp, ci, va = oracle.csr_random(kind, m, n, pr, 46)
     Ao = oracle.Op.csr(m, n, rp, ci, va)
     xh = oracle.fill(n, kind, "normal", 3); uh = oracle.fill(m, kind, "normal", 4)
     x = lk.Vector(ctx, kind, n).put(xh); u = lk.Vector(ctx, kind, m).put(uh)
     res = {}
-    for blocked in (4, 3, 2, 1, 0):
-        # blocked = 3 / 4: the kernel variants kept for A/B (CSR-stream; thread-per-row with evict_first streams), 64 KB slices
-        ctx.set_option("csr_blocked_variant", {3: 1, 4: 0}.get(blocked, 2))
+    for blocked in (2, 1, 0):
         # 8 KB slices: 512-2048 columns per block (~1 entry per row and block); 64 KB slices: 2-4 blocks with 3-6 entries per
-        # row and block (runs longer than the staging buffer of the pipelined kernel)
-        ctx.set_option("csr_slice_kb", {4: 64, 3: 64, 2: 64, 1: 8, 0: 0}[blocked])
+        # row and block; 0: plain layout
+        ctx.set_option("csr_slice_kb", {2: 64, 1: 8, 0: 0}[blocked])
         ctx.set_option("csr_block_min_kb", 0)
         A = lk.LinOp.csr(ctx, m, n, rp, ci, va)
         y = lk.Vector(ctx, kind, m).put(np.full(m, np.nan, dtype=dt)); v = lk.Vector(ctx, kind, n).put(np.full(n, np.nan, dtype=dt))
@@ -944,8 +941,10 @@ def test_csr_l2_blocked_layout_matches_plain(lk, ctx, oracle, kind):
             Vo = np.zeros((n, kd + 1), dtype=dt, order="F"); Bo = np.zeros_like(B)
             assert oracle.bidiag(Ao, Uo, Vo, Bo) == 0
             assert rel_normwise(B, Bo) < tol_for(kind)
-    ctx.set_option("csr_slice_kb", 48 * 1024); ctx.set_option("csr_block_min_kb", 96 * 1024); ctx.set_option("csr_blocked_variant", 2)
+    ctx.set_option("csr_slice_kb", 48 * 1024); ctx.set_option("csr_block_min_kb", 96 * 1024)
     tol = dict(rtol=1e-4, atol=1e-4) if kind == "s" else dict(rtol=1e-11, atol=1e-11)
-    for blocked in (4, 3, 2, 1, 0):
+    for blocked in (2, 1, 0):
         np.testing.assert_allclose(res[blocked][0], Ao.apply(xh), **tol)
         np.testing.assert_allclose(res[blocked][1], Ao.apply(uh, trans=True), **tol)
+    with pytest.raises(lk.LkbError, match="unknown option csr_blocked_variant"):
+        ctx.set_option("csr_blocked_variant", 2)
