@@ -152,6 +152,13 @@ int lkb_op_dense_create(lkb_ctx_t ctx, int kind, int64_t m, int64_t n, const voi
 typedef int (*lkb_matvec_fn)(void* user, const void* x_dev, void* y_dev, int32_t trans, void* stream);
 int lkb_op_callback_create(lkb_ctx_t ctx, int kind, int64_t m_local, int64_t n_local, lkb_matvec_fn fn,
                            void* user, int32_t capturable, lkb_op_t* A);
+/* diagonal operator M = diag(d): matvec y = d o x, rmatvec y = conj(d) o x, in place allowed (x may be y).  The values
+ * are copied at creation; M has d's layout (n_local, n_global, row0) and needs no communication at N > 1. */
+int lkb_op_diag_create(lkb_vec_t d, lkb_op_t* M);
+/* Jacobi preconditioner M = diag(A)^-1 as a diagonal operator, built on the device.  A: stencil, CSR (plain, L2-blocked,
+ * or row-sharded with equal row and column slabs on this rank), dense or diagonal.  LKB_ERR_ARG for a callback or non-square
+ * A, and for a zero or non-finite diagonal entry (lkb_last_error names its global row). */
+int lkb_op_jacobi_create(lkb_op_t A, lkb_op_t* M);
 int lkb_op_destroy(lkb_op_t A);
 int lkb_op_matvec(lkb_op_t A, lkb_vec_t x, lkb_vec_t y);    /* apply_matvec  :391-407 (bumps counter) */
 int lkb_op_rmatvec(lkb_op_t A, lkb_vec_t x, lkb_vec_t y);   /* apply_rmatvec :409-424 */
@@ -193,6 +200,10 @@ typedef int (*lkb_precond_fn)(void* user, void* vec_dev, int64_t n_local, int32_
                               double target_residual, void* stream);
 int lkb_gmres_precond(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double rtol, double atol,
                       int32_t transpose, lkb_gmres_io* io, lkb_precond_fn precond, void* user);
+/* right preconditioner given as an operator M (wrk = M V(k), w = A wrk; dx <- M dx): the restart cycle stays one device
+ * graph with one host sync.  M's matvec counter counts its applications. */
+int lkb_gmres_precond_op(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double rtol, double atol,
+                         int32_t transpose, lkb_gmres_io* io, lkb_op_t M);
 /* fgmres(A, b, x, info, rtol, atol, preconditioner, options, transpose, meta)  GMRES/fgmres.fypp:65-260:
  * flexible GMRES, the preconditioned vectors Z(k) are stored; options / metadata as gmres. */
 int lkb_fgmres(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double rtol, double atol,
@@ -206,6 +217,11 @@ typedef struct {            /* cg_dp_opts / cg_dp_metadata : IterativeSolvers.fy
 int lkb_cg(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double rtol, double atol, lkb_cg_io* io);
 int lkb_cg_precond(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double rtol, double atol, lkb_cg_io* io,
                    lkb_precond_fn precond, void* user);
+/* preconditioner given as an operator M (z = M r): the iteration stays on the device (chunks of 16 iterations, one graph
+ * each when A and M are capturable).  A diagonal M (lkb_op_diag_create / lkb_op_jacobi_create) is fused into the CG vector
+ * kernels.  Residual = sqrt(|r^H z|); M's matvec counter grows by n_iter + 1. */
+int lkb_cg_precond_op(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double rtol, double atol,
+                      lkb_cg_io* io, lkb_op_t M);
 /* eigs(A, X, eigvals, residuals, info, x0, kdim, tolerance, transpose)  IterativeSolvers.fypp:972-1143
  *   X: nev columns (out); eigvals: nev complex (double[2] each); residuals: nev doubles.
  *   x0 may be NULL (random start); kdim <= 0 = 4*nev; tolerance < 0 = rtol_kind. */

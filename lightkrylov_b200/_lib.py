@@ -95,6 +95,8 @@ SIGNATURES = {
     "lkb_op_csr_create_dist_device": (_i, [_vp, _i, _i64, _i64, _i64, _i64, _i64, _i64, _vp, _vp, _vp, _i32, _P(_vp)]),
     "lkb_op_dense_create": (_i, [_vp, _i, _i64, _i64, _vp, _P(_vp)]),
     "lkb_op_callback_create": (_i, [_vp, _i, _i64, _i64, MATVEC_FN, _vp, _i32, _P(_vp)]),
+    "lkb_op_diag_create": (_i, [_vp, _P(_vp)]),
+    "lkb_op_jacobi_create": (_i, [_vp, _P(_vp)]),
     "lkb_op_destroy": (_i, [_vp]),
     "lkb_op_matvec": (_i, [_vp, _vp, _vp]),
     "lkb_op_rmatvec": (_i, [_vp, _vp, _vp]),
@@ -109,6 +111,8 @@ SIGNATURES = {
     "lkb_gmres_precond": (_i, [_vp, _vp, _vp, _P(_i32), _d, _d, _i32, _P(GmresIO), PRECOND_FN, _vp]),
     "lkb_fgmres": (_i, [_vp, _vp, _vp, _P(_i32), _d, _d, _i32, _P(GmresIO), PRECOND_FN, _vp]),
     "lkb_cg_precond": (_i, [_vp, _vp, _vp, _P(_i32), _d, _d, _P(CgIO), PRECOND_FN, _vp]),
+    "lkb_gmres_precond_op": (_i, [_vp, _vp, _vp, _P(_i32), _d, _d, _i32, _P(GmresIO), _vp]),
+    "lkb_cg_precond_op": (_i, [_vp, _vp, _vp, _P(_i32), _d, _d, _P(CgIO), _vp]),
     "lkb_eigs": (_i, [_vp, _vp, _i, _P(_d), _P(_d), _P(_i32), _vp, _i32, _d, _i32]),
     "lkb_eighs": (_i, [_vp, _vp, _i, _P(_d), _P(_d), _P(_i32), _vp, _i32, _d]),
     "lkb_svds": (_i, [_vp, _vp, _P(_d), _vp, _i, _P(_d), _P(_i32), _vp, _i32, _d]),

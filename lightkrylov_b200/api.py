@@ -427,6 +427,25 @@ class LinOp:
         op.row0, op.n_global = 0, n_local
         return op
 
+    @classmethod
+    def diag(cls, d: Vector) -> "LinOp":
+        """M = diag(d): matvec d * x, rmatvec conj(d) * x, x may be y.  The values of d are copied; M has d's layout."""
+        h = C.c_void_p()
+        check(d.ctx.lib.lkb_op_diag_create(d.h, C.byref(h)), "diag")
+        op = cls(d.ctx, d.kind, h, d.n, d.n)
+        op.row0, op.n_global = d.row0, d.n_global
+        return op
+
+    @classmethod
+    def jacobi(cls, A: "LinOp") -> "LinOp":
+        """Jacobi preconditioner M = diag(A)^-1, built on the device: a diagonal operator with A's row layout."""
+        h = C.c_void_p()
+        check(A.ctx.lib.lkb_op_jacobi_create(A.h, C.byref(h)), "jacobi")
+        op = cls(A.ctx, A.kind, h, A.m, A.m)
+        op.row0 = getattr(A, "out_row0", A.row0)
+        op.n_global = getattr(A, "m_global", A.n_global)
+        return op
+
     def matvec(self, x: Vector, y: Vector):
         check(self.ctx.lib.lkb_op_matvec(self.h, x.h, y.h), "matvec")
 
@@ -518,7 +537,8 @@ def qr_pivoting(Q: Basis, col0: int = 0, p: Optional[int] = None, tol: float = -
 
 
 def _wrap_precond(preconditioner):
-    """preconditioner(vec_ptr, n_local, iter, current_residual, target_residual, stream) -> None/int"""
+    """preconditioner(vec_ptr, n_local, iter, current_residual, target_residual, stream) -> None/int
+    (a host callback; a LinOp preconditioner goes to the *_precond_op entry points instead)"""
     return _lib.PRECOND_FN(lambda user, v, n, it, cur, tgt, stream: int(preconditioner(v, n, it, cur, tgt, stream) or 0))
 
 
@@ -530,6 +550,9 @@ def gmres(A: LinOp, b: Vector, x: Vector, rtol: float = -1.0, atol: float = -1.0
     info = C.c_int32()
     if preconditioner is None:
         check(A.ctx.lib.lkb_gmres(A.h, b.h, x.h, C.byref(info), rtol, atol, int(transpose), C.byref(io)), "gmres")
+    elif isinstance(preconditioner, LinOp):
+        check(A.ctx.lib.lkb_gmres_precond_op(A.h, b.h, x.h, C.byref(info), rtol, atol, int(transpose), C.byref(io),
+                                             preconditioner.h), "gmres")
     else:
         cb = _wrap_precond(preconditioner)
         check(A.ctx.lib.lkb_gmres_precond(A.h, b.h, x.h, C.byref(info), rtol, atol, int(transpose), C.byref(io),
@@ -541,7 +564,10 @@ def gmres(A: LinOp, b: Vector, x: Vector, rtol: float = -1.0, atol: float = -1.0
 
 def fgmres(A: LinOp, b: Vector, x: Vector, rtol: float = -1.0, atol: float = -1.0, kdim: int = 30,
            maxiter: int = 10, transpose: bool = False, preconditioner=None):
-    """Flexible GMRES (GMRES/fgmres.fypp): same options / metadata as gmres."""
+    """Flexible GMRES (GMRES/fgmres.fypp): same options / metadata as gmres.  The preconditioner is a callable: fgmres
+    exists for preconditioners that change between inner steps, and with a fixed operator it is gmres."""
+    if isinstance(preconditioner, LinOp):
+        raise TypeError("fgmres takes a callable preconditioner; pass a LinOp preconditioner to gmres")
     cap = (kdim + 2) * (maxiter + 2) + 8
     res = (C.c_double * cap)()
     io = _lib.GmresIO(kdim=kdim, maxiter=maxiter, res=res, res_cap=cap)
@@ -561,6 +587,8 @@ def cg(A: LinOp, b: Vector, x: Vector, rtol: float = -1.0, atol: float = -1.0, m
     info = C.c_int32()
     if preconditioner is None:
         check(A.ctx.lib.lkb_cg(A.h, b.h, x.h, C.byref(info), rtol, atol, C.byref(io)), "cg")
+    elif isinstance(preconditioner, LinOp):
+        check(A.ctx.lib.lkb_cg_precond_op(A.h, b.h, x.h, C.byref(info), rtol, atol, C.byref(io), preconditioner.h), "cg")
     else:
         cb = _wrap_precond(preconditioner)
         check(A.ctx.lib.lkb_cg_precond(A.h, b.h, x.h, C.byref(info), rtol, atol, C.byref(io), cb, None), "cg")

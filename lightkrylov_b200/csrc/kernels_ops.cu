@@ -484,6 +484,72 @@ void launch_csr_blocked(int kind, cudaStream_t s, const CsrBlocked& b, const voi
 }
 
 // ------------------------------------------------------------------------------------------
+// Jacobi preconditioner (set-up, once per operator): d_r = 1 / A_rr, the diagonal found the way each operator stores it.
+//   stencil       the centre coefficient on every row
+//   csr           the sum of the row's entries at column col0 + r (duplicates summed, as k_csr sums them)
+//   blocked csr   the same, scanning only the column block that holds col0 + r (tab gives the row's range in it)
+//   dense         a[r + rows * r]
+//   diagonal      the operator's own d
+// The diagonal is formed in W precision and inverted there; a zero or non-finite entry lowers *bad_row to its global row.
+LKB_DI bool finite_nonzero(double a) { return isfinite(a) && a != 0.0; }
+LKB_DI bool finite_nonzero(double2 a) { return isfinite(a.x) && isfinite(a.y) && (a.x != 0.0 || a.y != 0.0); }
+LKB_DI double recip_w(double a) { return 1.0 / a; }
+LKB_DI double2 recip_w(double2 a) { const double q = a.x * a.x + a.y * a.y; return make_double2(a.x / q, -a.y / q); }
+
+template <int K, int MODE>
+__global__ void __launch_bounds__(256)
+k_jacobi(const JacobiSrc src, typename Tr<K>::E* __restrict__ d, unsigned long long* __restrict__ bad_row)
+{
+    using E = typename Tr<K>::E;
+    using W = typename Tr<K>::W;
+    const E* val = (const E*)src.val;
+    for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < src.rows; r += (int64_t)gridDim.x * blockDim.x) {
+        W a = zero_v(W());
+        if constexpr (MODE == JAC_STENCIL) {
+            E c; from_scalar(src.c0, c); a = widen(c);
+        } else if constexpr (MODE == JAC_CSR) {
+            const int64_t cr = src.col0 + r;
+            for (int64_t q = src.rowptr[r]; q < src.rowptr[r + 1]; ++q)
+                if (src.col[q] == cr) wadd(a, widen(val[q]));
+        } else if constexpr (MODE == JAC_CSR_BLOCKED) {
+            const int64_t cr = src.col0 + r;
+            const uint32_t* tab = src.blk.tab + (size_t)(cr / src.blk.cw) * (src.rows + 1);
+            const E* bval = (const E*)src.blk.val;
+            for (uint32_t q = tab[r]; q < tab[r + 1]; ++q)
+                if (src.blk.col[q] == cr) wadd(a, widen(bval[q]));
+        } else if constexpr (MODE == JAC_DENSE) {
+            a = widen(((const E*)src.a)[r * (src.rows + 1)]);
+        } else {
+            a = widen(((const E*)src.a)[r]);
+        }
+        if (finite_nonzero(a)) narrow(recip_w(a), d[r]);
+        else atomicMin(bad_row, (unsigned long long)(src.row0 + r));
+    }
+}
+template <int K>
+static void jacobi_t(cudaStream_t s, const JacobiSrc& src, void* d, unsigned long long* bad, int sms) {
+    using E = typename Tr<K>::E;
+    int64_t nb = (src.rows + 255) / 256;
+    if (nb < 1) nb = 1;
+    if (nb > (int64_t)sms * 16) nb = (int64_t)sms * 16;
+    switch (src.mode) {
+        case JAC_STENCIL: k_jacobi<K, JAC_STENCIL><<<(int)nb, 256, 0, s>>>(src, (E*)d, bad); break;
+        case JAC_CSR: k_jacobi<K, JAC_CSR><<<(int)nb, 256, 0, s>>>(src, (E*)d, bad); break;
+        case JAC_CSR_BLOCKED: k_jacobi<K, JAC_CSR_BLOCKED><<<(int)nb, 256, 0, s>>>(src, (E*)d, bad); break;
+        case JAC_DENSE: k_jacobi<K, JAC_DENSE><<<(int)nb, 256, 0, s>>>(src, (E*)d, bad); break;
+        default: k_jacobi<K, JAC_DIAG><<<(int)nb, 256, 0, s>>>(src, (E*)d, bad); break;
+    }
+}
+void launch_jacobi(int kind, cudaStream_t s, const JacobiSrc& src, void* d, unsigned long long* bad_row, int sms) {
+    switch (kind) {
+        case KS: jacobi_t<KS>(s, src, d, bad_row, sms); break;
+        case KD: jacobi_t<KD>(s, src, d, bad_row, sms); break;
+        case KC: jacobi_t<KC>(s, src, d, bad_row, sms); break;
+        default: jacobi_t<KZ>(s, src, d, bad_row, sms); break;
+    }
+}
+
+// ------------------------------------------------------------------------------------------
 // dense_linop (AbstractLinops.fypp:608-671, gemv): only the n = 128 plumbing config uses it.
 template <int K>
 __global__ void k_dense(int64_t m, int64_t n, const typename Tr<K>::E* __restrict__ a,

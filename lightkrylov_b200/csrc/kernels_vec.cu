@@ -244,14 +244,41 @@ LKB_DI double2 as_w2(double2 a) { return a; }
 LKB_DI void from_w2(double2 a, double& o) { o = a.x; }
 LKB_DI void from_w2(double2 a, double2& o) { o = a; }
 
-// x += alpha p ; r -= alpha Ap ; nrm2 = r_new^H r_new   with alpha = rr_old / pAp  (device scalars)
-template <int K>
+// Preconditioned CG (CG.fypp:113-116, 137: z = M r, rz = r^H z, p = z + beta p) runs in the same kernels, selected at
+// compile time by MODE:
+//   CG_PLAIN  no preconditioner: nrm2 = r^H r (the unpreconditioned loop; its code is unchanged by the other modes)
+//   CG_DIAG   M = diag(d): nrm2 = sum conj(r_i) (d_i r_i) in W (complex for c / z, d need not be real), and
+//             k_cg_direction forms p = d o r + beta p.  z is never stored: the mode reads d twice per iteration.
+//   CG_NORED  any other M: only x and r are updated; the caller applies M to r and reduces r^H z with a multi-dot.
+
+// One W per CTA: all threads of the LAST CTA call this after the ticket; the total is returned in thread 0
+// (fixed order, as reduce_scalar_last).
+template <typename W>
+LKB_DI W reduce_w_last(const W* __restrict__ partial, int nb)
+{
+    __shared__ W s_red[32];
+    const int tid = threadIdx.x, nt = blockDim.x;
+    W a = zero_v(W());
+    for (int b = tid; b < nb; b += nt) wadd(a, ldcg_w(&partial[b]));
+    a = warp_sum(a);
+    __syncthreads();
+    if ((tid & 31) == 0) s_red[tid >> 5] = a;
+    __syncthreads();
+    W t = zero_v(W());
+    if (tid == 0)
+        for (int q = 0; q < (nt + 31) / 32; ++q) wadd(t, s_red[q]);
+    return t;
+}
+
+// x += alpha p ; r -= alpha Ap ; nrm2 = r_new^H r_new (CG_DIAG: r_new^H d o r_new)   with alpha = rr_old / pAp  (device scalars)
+template <int K, int MODE>
 __global__ void __launch_bounds__(256, 2)
 k_cg_update(const typename Tr<K>::W* __restrict__ scal, const typename Tr<K>::W* __restrict__ pAp,
             const typename Tr<K>::E* __restrict__ p, const typename Tr<K>::E* __restrict__ Ap,
             typename Tr<K>::E* __restrict__ x, typename Tr<K>::E* __restrict__ r, int64_t n,
             double* __restrict__ partial, typename Tr<K>::W* __restrict__ nrm2_out,
-            unsigned* __restrict__ counter, const int* __restrict__ flags, const P2P p2p)
+            unsigned* __restrict__ counter, const int* __restrict__ flags, const P2P p2p,
+            const typename Tr<K>::E* __restrict__ d)
 {
     using E = typename Tr<K>::E;
     using W = typename Tr<K>::W;
@@ -262,14 +289,18 @@ k_cg_update(const typename Tr<K>::W* __restrict__ scal, const typename Tr<K>::W*
     E alpha; narrow(aw, alpha);
     const int64_t npk = n / EPP;
     double nrm = 0.0;
+    W rz = zero_v(W());
     for (int64_t pk = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; pk < npk; pk += (int64_t)gridDim.x * blockDim.x) {
         const P pv = ld_pack_nc<P>(p + pk * EPP), av = ld_pack_nc<P>(Ap + pk * EPP);
         P xv = ld_pack<P>(x + pk * EPP), rv = ld_pack<P>(r + pk * EPP);
+        P dv;
+        if constexpr (MODE == CG_DIAG) dv = ld_pack_nc<P>(d + pk * EPP);
 #pragma unroll
         for (int e = 0; e < EPP; ++e) {
             fmacc(xv.v[e], pv.v[e], alpha);
             fnma(rv.v[e], av.v[e], alpha);
-            nrm += abs2_w(rv.v[e]);
+            if constexpr (MODE == CG_PLAIN) nrm += abs2_w(rv.v[e]);
+            if constexpr (MODE == CG_DIAG) fma_conj(rz, widen(rv.v[e]), widen(mul_v(dv.v[e], rv.v[e])));
         }
         st_pack(x + pk * EPP, xv);
         st_pack(r + pk * EPP, rv);
@@ -278,8 +309,36 @@ k_cg_update(const typename Tr<K>::W* __restrict__ scal, const typename Tr<K>::W*
         for (int64_t t = npk * EPP; t < n; ++t) {
             E xv = x[t], rv = r[t];
             fmacc(xv, p[t], alpha); fnma(rv, Ap[t], alpha);
-            x[t] = xv; r[t] = rv; nrm += abs2_w(rv);
+            x[t] = xv; r[t] = rv;
+            if constexpr (MODE == CG_PLAIN) nrm += abs2_w(rv);
+            if constexpr (MODE == CG_DIAG) fma_conj(rz, widen(rv), widen(mul_v(d[t], rv)));
         }
+    if constexpr (MODE == CG_NORED) return;
+    if constexpr (MODE == CG_DIAG) {
+        __shared__ W smw[8];
+        __shared__ bool is_last_w;
+        W* pw = reinterpret_cast<W*>(partial);
+        const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+        const W a = warp_sum(rz);
+        if (lane == 0) smw[wid] = a;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            W t = smw[0];
+            for (int q = 1; q < (int)(blockDim.x >> 5); ++q) wadd(t, smw[q]);
+            pw[blockIdx.x] = t;
+            __threadfence();
+            is_last_w = (atomicAdd(counter, 1u) == gridDim.x - 1u);
+        }
+        __syncthreads();
+        if (is_last_w) {
+            __threadfence();
+            const W t = reduce_w_last<W>(pw, (int)gridDim.x);
+            if (threadIdx.x == 0) { nrm2_out[0] = t; *counter = 0u; }
+            __syncthreads();
+            if (p2p.world > 1) p2p_allreduce_cta<W>(p2p, nrm2_out, 1);
+        }
+        return;
+    }
     __shared__ double sm[8];
     __shared__ bool is_last;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -326,11 +385,12 @@ __global__ void k_cg_check(typename Tr<K>::W* __restrict__ scal, const typename 
     if (it >= maxiter) { flags[F_STOP] = 1; flags[F_INFO] = it; }
 }
 
-// p = r + beta p  (beta = scal[1] on the device)
-template <int K>
+// p = r + beta p  (beta = scal[1] on the device);  CG_DIAG: p = d o r + beta p  (r is then the residual, d o r = z)
+template <int K, int MODE>
 __global__ void __launch_bounds__(256)
 k_cg_direction(const typename Tr<K>::W* __restrict__ scal, const typename Tr<K>::E* __restrict__ r,
-               typename Tr<K>::E* __restrict__ p, int64_t n, const int* __restrict__ flags)
+               typename Tr<K>::E* __restrict__ p, int64_t n, const int* __restrict__ flags,
+               const typename Tr<K>::E* __restrict__ d)
 {
     using E = typename Tr<K>::E;
     constexpr int EPP = Tr<K>::EPP;
@@ -339,14 +399,46 @@ k_cg_direction(const typename Tr<K>::W* __restrict__ scal, const typename Tr<K>:
     E beta; narrow(scal[1], beta);
     const int64_t npk = n / EPP;
     for (int64_t pk = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; pk < npk; pk += (int64_t)gridDim.x * blockDim.x) {
-        const P rv = ld_pack_nc<P>(r + pk * EPP);
+        P rv = ld_pack_nc<P>(r + pk * EPP);
+        if constexpr (MODE == CG_DIAG) {
+            const P dv = ld_pack_nc<P>(d + pk * EPP);
+#pragma unroll
+            for (int e = 0; e < EPP; ++e) rv.v[e] = mul_v(dv.v[e], rv.v[e]);
+        }
         P pv = ld_pack<P>(p + pk * EPP);
 #pragma unroll
         for (int e = 0; e < EPP; ++e) pv.v[e] = add_v(rv.v[e], mul_v(beta, pv.v[e]));
         st_pack(p + pk * EPP, pv);
     }
     if (blockIdx.x == 0 && threadIdx.x == 0)
-        for (int64_t t = npk * EPP; t < n; ++t) p[t] = add_v(r[t], mul_v(beta, p[t]));
+        for (int64_t t = npk * EPP; t < n; ++t) {
+            E z = r[t];
+            if constexpr (MODE == CG_DIAG) z = mul_v(d[t], z);
+            p[t] = add_v(z, mul_v(beta, p[t]));
+        }
+}
+
+// y = d o x (matvec of a diagonal operator) or conj(d) o x (rmatvec).  y may be x: every pack is read once, by the
+// thread that then writes it, so the streaming read-only loads stay valid in place.
+template <int K, bool CONJ>
+__global__ void __launch_bounds__(256)
+k_diag(const typename Tr<K>::E* __restrict__ d, const typename Tr<K>::E* x, typename Tr<K>::E* y, int64_t n,
+       const int* __restrict__ flags)
+{
+    using E = typename Tr<K>::E;
+    constexpr int EPP = Tr<K>::EPP;
+    using P = Pack<E, EPP>;
+    if (flags && flags[F_STOP]) return;
+    const int64_t npk = n / EPP;
+    for (int64_t pk = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; pk < npk; pk += (int64_t)gridDim.x * blockDim.x) {
+        const P dv = ld_pack_nc<P>(d + pk * EPP);
+        P xv = ld_pack_nc<P>(x + pk * EPP);
+#pragma unroll
+        for (int e = 0; e < EPP; ++e) xv.v[e] = mul_v(CONJ ? conj_v(dv.v[e]) : dv.v[e], xv.v[e]);
+        st_pack(y + pk * EPP, xv);
+    }
+    if (blockIdx.x == 0 && threadIdx.x == 0)
+        for (int64_t t = npk * EPP; t < n; ++t) y[t] = mul_v(CONJ ? conj_v(d[t]) : d[t], x[t]);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -484,23 +576,33 @@ void launch_update(int kind, cudaStream_t s, const void* c1, const void* c2, int
 }
 void launch_cg_update(int kind, cudaStream_t s, const void* scal, const void* pAp, const void* p, const void* Ap, void* x,
                       void* r, int64_t n, void* partial, void* nrm2_out, unsigned* counter, const int* flags, int sms,
-                      const P2P* p2p) {
+                      const P2P* p2p, int mode, const void* d) {
     const P2P pp = p2p ? *p2p : P2P();
     LKB_DISPATCH(kind, {
         using E = typename Tr<K>::E; using W = typename Tr<K>::W;
         int64_t nb = (n / Tr<K>::EPP + 255) / 256; if (nb < 1) nb = 1; if (nb > 4 * (int64_t)sms) nb = 4 * (int64_t)sms;
         if (nb > MAX_ROWBLOCKS) nb = MAX_ROWBLOCKS;
-        k_cg_update<K><<<(int)nb, 256, 0, s>>>((const W*)scal, (const W*)pAp, (const E*)p, (const E*)Ap, (E*)x, (E*)r, n,
-                                              (double*)partial, (W*)nrm2_out, counter, flags, pp);
+        auto kern = mode == CG_DIAG ? k_cg_update<K, CG_DIAG> : mode == CG_NORED ? k_cg_update<K, CG_NORED> : k_cg_update<K, CG_PLAIN>;
+        kern<<<(int)nb, 256, 0, s>>>((const W*)scal, (const W*)pAp, (const E*)p, (const E*)Ap, (E*)x, (E*)r, n,
+                                     (double*)partial, (W*)nrm2_out, counter, flags, pp, (const E*)d);
     });
 }
 void launch_cg_check(int kind, cudaStream_t s, void* scal, const void* rr_new, double tol, int maxiter, double* res_hist, int* flags) {
     LKB_DISPATCH(kind, { using W = typename Tr<K>::W; k_cg_check<K><<<1, 1, 0, s>>>((W*)scal, (const W*)rr_new, tol, maxiter, res_hist, flags); });
 }
-void launch_cg_direction(int kind, cudaStream_t s, const void* scal, const void* r, void* p, int64_t n, const int* flags, int sms) {
+void launch_cg_direction(int kind, cudaStream_t s, const void* scal, const void* r, void* p, int64_t n, const int* flags, int sms,
+                         const void* d) {
     LKB_DISPATCH(kind, {
         using E = typename Tr<K>::E; using W = typename Tr<K>::W;
-        k_cg_direction<K><<<ew_grid(n / Tr<K>::EPP, sms), 256, 0, s>>>((const W*)scal, (const E*)r, (E*)p, n, flags);
+        auto kern = d ? k_cg_direction<K, CG_DIAG> : k_cg_direction<K, CG_PLAIN>;
+        kern<<<ew_grid(n / Tr<K>::EPP, sms), 256, 0, s>>>((const W*)scal, (const E*)r, (E*)p, n, flags, (const E*)d);
+    });
+}
+void launch_diag(int kind, cudaStream_t s, const void* d, const void* x, void* y, int64_t n, bool conj, const int* flags, int sms) {
+    LKB_DISPATCH(kind, {
+        using E = typename Tr<K>::E;
+        auto kern = conj ? k_diag<K, true> : k_diag<K, false>;
+        kern<<<ew_grid(n / Tr<K>::EPP, sms), 256, 0, s>>>((const E*)d, (const E*)x, (E*)y, n, flags);
     });
 }
 void launch_gmres_update(int kind, cudaStream_t s, const void* c1, const void* c2, int k, const void* nrm2, void* H, int ldh,

@@ -777,6 +777,84 @@ int lkb_op_callback_create(lkb_ctx_t c, int kind, int64_t m_local, int64_t n_loc
     *A = op;
     return 0;
 }
+// Diagonal operator M = diag(d), e.g. the inverse mass matrix of a spectral-element code.  Row-local, so it has
+// the layout of d and needs no communication at N > 1.  Its values are copied: d may be released afterwards.
+static int diag_from_device(lkb_ctx_t c, int kind, int64_t n, int64_t row0, int64_t n_global, lkb_op_s** M) {
+    cudaSetDevice(c->dev);
+    lkb_op_s* op = new lkb_op_s();
+    op->ctx = c; op->type = 4; op->kind = kind; op->m = op->n = n; op->uid = next_uid();
+    op->diag_row0 = row0; op->diag_n_global = n_global;
+    if (cudaMalloc(&op->diag, std::max<size_t>((size_t)n * kind_size(kind), 16)) != cudaSuccess) {
+        cudaGetLastError(); op->diag = nullptr; delete op;
+        set_error("diag: cudaMalloc of %lld entries failed", (long long)n); return LKB_ERR_ALLOC;
+    }
+    *M = op;
+    return 0;
+}
+int lkb_op_diag_create(lkb_vec_t d, lkb_op_t* M) {
+    if (!d || !M) { set_error("diag_create: null argument"); return LKB_ERR_ARG; }
+    lkb_ctx_s* c = d->ctx;
+    lkb_op_s* op = nullptr;
+    LKB_TRY(diag_from_device(c, d->kind, d->n, d->row0, d->n_global, &op));
+    if (cudaMemcpyAsync(op->diag, d->d, (size_t)d->n * kind_size(d->kind), cudaMemcpyDeviceToDevice, c->stream) != cudaSuccess ||
+        cudaStreamSynchronize(c->stream) != cudaSuccess) {
+        set_error("diag_create: copy of d failed: %s", cudaGetErrorString(cudaGetLastError()));
+        lkb_op_destroy(op); return LKB_ERR_CUDA;
+    }
+    *M = op;
+    return 0;
+}
+// Jacobi preconditioner M = diag(A)^-1, found and inverted on the device (k_jacobi).  Not collective: a rank whose slab
+// holds a zero or non-finite diagonal entry reports it, with the first such global row.
+int lkb_op_jacobi_create(lkb_op_t A, lkb_op_t* M) {
+    if (!A || !M) { set_error("jacobi_create: null argument"); return LKB_ERR_ARG; }
+    lkb_ctx_s* c = A->ctx;
+    if (A->type == 9) { set_error("jacobi_create: a callback operator has no diagonal the library can read"); return LKB_ERR_ARG; }
+    if (A->m != A->n) { set_error("jacobi_create: A is not square (%lld x %lld local rows / columns)", (long long)A->m, (long long)A->n); return LKB_ERR_ARG; }
+    JacobiSrc src;
+    src.rows = A->m;
+    int64_t n_global = A->m;
+    if (A->type == 1) {
+        const int64_t plane = A->st.dim == 2 ? A->st.nx : A->st.nx * A->st.ny;
+        src.mode = JAC_STENCIL; src.c0 = A->st.coef[0];
+        src.row0 = A->slow0 * plane; n_global = A->nslow_global * plane;
+    } else if (A->type == 3) {
+        if (A->dist) {
+            const int r = c->rank;
+            if (A->row_off[r] != A->col_off[r] || A->row_cnt[r] != A->col_cnt[r] || A->m_global != A->n_global) {
+                set_error("jacobi_create: row-sharded CSR whose row slab [%lld,+%lld) differs from its column slab [%lld,+%lld) "
+                          "on rank %d (the diagonal is defined only when they agree)", (long long)A->row_off[r], (long long)A->row_cnt[r],
+                          (long long)A->col_off[r], (long long)A->col_cnt[r], r);
+                return LKB_ERR_ARG;
+            }
+            src.row0 = src.col0 = A->row_off[r]; n_global = A->n_global;
+        }
+        if (A->blk.nb > 0) { src.mode = JAC_CSR_BLOCKED; src.blk = A->blk; }
+        else { src.mode = JAC_CSR; src.rowptr = A->rowptr; src.col = A->col; src.val = A->val; }
+    } else if (A->type == 0) {
+        src.mode = JAC_DENSE; src.a = A->a;
+    } else if (A->type == 4) {
+        src.mode = JAC_DIAG; src.a = A->diag; src.row0 = A->diag_row0; n_global = A->diag_n_global;
+    } else {
+        set_error("jacobi_create: unsupported operator type %d", A->type); return LKB_ERR_ARG;
+    }
+    lkb_op_s* op = nullptr;
+    LKB_TRY(diag_from_device(c, A->kind, A->m, src.row0, n_global, &op));
+    unsigned long long* bad = nullptr; unsigned long long hbad = 0;
+    cudaError_t e = cudaMalloc((void**)&bad, sizeof(unsigned long long));
+    if (e == cudaSuccess) e = cudaMemsetAsync(bad, 0xff, sizeof(unsigned long long), c->stream);
+    if (e == cudaSuccess) { launch_jacobi(A->kind, c->stream, src, op->diag, bad, c->sms); e = cudaGetLastError(); }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&hbad, bad, sizeof(hbad), cudaMemcpyDeviceToHost, c->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    if (bad) cudaFree(bad);
+    if (e != cudaSuccess) { set_error("jacobi_create: %s", cudaGetErrorString(e)); lkb_op_destroy(op); return LKB_ERR_CUDA; }
+    if (hbad != ~0ULL) {
+        set_error("jacobi_create: the diagonal entry of global row %llu is zero or not finite", hbad);
+        lkb_op_destroy(op); return LKB_ERR_ARG;
+    }
+    *M = op;
+    return 0;
+}
 int lkb_op_destroy(lkb_op_t A) {
     if (!A) return LKB_ERR_ARG;
     cudaStreamSynchronize(A->ctx->stream);
@@ -784,7 +862,7 @@ int lkb_op_destroy(lkb_op_t A) {
     if (A->hp_lo_map) cudaIpcCloseMemHandle(A->hp_lo_map);
     if (A->hp_hi_map) cudaIpcCloseMemHandle(A->hp_hi_map);
     if (A->hp_active) { cudaFree(A->hp.my_region); cudaFree(A->hp.epoch); }
-    void* bufs[] = { A->halo_lo, A->halo_hi, A->rowptr, A->col, A->val, A->t_rowptr, A->t_col, A->t_val, A->a, A->x_full, A->y_full, A->y_red,
+    void* bufs[] = { A->halo_lo, A->halo_hi, A->rowptr, A->col, A->val, A->t_rowptr, A->t_col, A->t_val, A->a, A->diag, A->x_full, A->y_full, A->y_red,
                      A->blk.tab, A->blk.col, A->blk.val, A->t_blk.tab, A->t_blk.col, A->t_blk.val };
     for (void* b : bufs) if (b) cudaFree(b);
     delete A;
@@ -881,14 +959,18 @@ int op_apply_enqueue(lkb_op_s* A, const void* x, void* y, bool trans, const int*
         }
     } else if (A->type == 0) {
         launch_dense(A->kind, c->stream, A->m, A->n, A->a, x, y, trans, flags);
+    } else if (A->type == 4) {
+        launch_diag(A->kind, c->stream, A->diag, x, y, A->m, trans, flags, c->sms);      // row-local: no exchange at N > 1
     } else {
         int r = A->fn(A->user, x, y, trans ? 1 : 0, (void*)c->stream);
         if (r != 0) { set_error("user matvec callback returned %d", r); return LKB_ERR_ARG; }
         nl = 0;
     }
     // anything but our own plain kernels (NCCL gathers / reductions, device-to-device copies, a user callback) breaks
-    // the programmatic-launch chain: the next PDL-aware kernel is launched normally
-    if (!(A->type == 1 || A->type == 0 || (A->type == 3 && !A->dist))) pdl_rearm();
+    // the programmatic-launch chain: the next PDL-aware kernel is launched normally.  The diagonal operator is one plain
+    // kernel (k_diag, launched without the PDL attribute, like the stencil): a PDL-aware successor waits for its completion
+    // in griddepcontrol.wait, so it keeps the chain.
+    if (!(A->type == 1 || A->type == 0 || A->type == 4 || (A->type == 3 && !A->dist))) pdl_rearm();
     prof_end(c, PC_MATVEC, nl);
     return check_launch(c, "matvec");
 }
@@ -899,7 +981,7 @@ static int op_apply_api(lkb_op_t A, lkb_vec_t x, lkb_vec_t y, bool trans) {
     if (!A || !x || !y) return LKB_ERR_ARG;
     const int64_t nin = trans ? A->m : A->n, nout = trans ? A->n : A->m;
     if (x->n != nin || y->n != nout || x->kind != A->kind || y->kind != A->kind) { set_error("matvec: size/kind mismatch"); return LKB_ERR_ARG; }
-    if (x->d == y->d) { set_error("matvec: vec_out must not alias vec_in"); return LKB_ERR_ARG; }
+    if (x->d == y->d && A->type != 4) { set_error("matvec: vec_out must not alias vec_in"); return LKB_ERR_ARG; }   // (k_diag works in place)
     if (trans) A->n_rmatvec++; else A->n_matvec++;
     return op_apply_enqueue(A, x->d, y->d, trans, nullptr);
 }

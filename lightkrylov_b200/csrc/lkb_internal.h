@@ -84,7 +84,7 @@ struct lkb_basis_s {
     bool owns = true;          // false: lkb_basis_view of a column range of another basis
 };
 struct lkb_op_s {
-    lkb_ctx_s* ctx; int type; int kind;           // type: 0 dense, 1 stencil, 3 csr, 9 callback
+    lkb_ctx_s* ctx; int type; int kind;           // type: 0 dense, 1 stencil, 3 csr, 4 diagonal, 9 callback
     int64_t m, n;                                 // local rows of the output / input vectors
     int64_t n_matvec = 0, n_rmatvec = 0;
     // stencil
@@ -101,6 +101,8 @@ struct lkb_op_s {
     std::vector<int64_t> col_off, col_cnt, row_off, row_cnt;
     // dense
     void* a = nullptr;
+    // diagonal: y = d o x, d laid out like the vectors it applies to (global index of the first row, global length)
+    void* diag = nullptr; int64_t diag_row0 = 0, diag_n_global = 0;
     // callback
     int (*fn)(void*, const void*, void*, int32_t, void*) = nullptr; void* user = nullptr; bool capturable = false;
     uint64_t uid = 0;

@@ -157,12 +157,19 @@ void launch_multiaxpy_fin(int kind, cudaStream_t s, const void* V, int64_t ld, i
 void launch_copy_gated(int kind, cudaStream_t s, const void* src, void* dst, int64_t n, const int* flags, int sms);
 void launch_fill(int kind, cudaStream_t s, void* x, int64_t n, int64_t row0, int dist, uint64_t seed, int sms);
 
-// device-resident CG iteration (kernels_vec.cu): see k_cg_update / k_cg_check / k_cg_direction
+// device-resident CG iteration (kernels_vec.cu): see k_cg_update / k_cg_check / k_cg_direction.
+// mode: CG_PLAIN (no preconditioner), CG_DIAG (M = diag(d) fused into both vector kernels), CG_NORED (any other M:
+// k_cg_update skips its reduction, the caller applies M and reduces r^H z)
+enum { CG_PLAIN = 0, CG_DIAG = 1, CG_NORED = 2 };
 void launch_cg_update(int kind, cudaStream_t s, const void* scal, const void* pAp, const void* p, const void* Ap, void* x,
                       void* r, int64_t n, void* partial, void* nrm2_out, unsigned* counter, const int* flags, int sms,
-                      const P2P* p2p);
+                      const P2P* p2p, int mode = CG_PLAIN, const void* d = nullptr);
 void launch_cg_check(int kind, cudaStream_t s, void* scal, const void* rr_new, double tol, int maxiter, double* res_hist, int* flags);
-void launch_cg_direction(int kind, cudaStream_t s, const void* scal, const void* r, void* p, int64_t n, const int* flags, int sms);
+// p = r + beta p, or with d != nullptr p = d o r + beta p
+void launch_cg_direction(int kind, cudaStream_t s, const void* scal, const void* r, void* p, int64_t n, const int* flags, int sms,
+                         const void* d = nullptr);
+// diagonal operator: y = d o x (conj: y = conj(d) o x); y may alias x
+void launch_diag(int kind, cudaStream_t s, const void* d, const void* x, void* y, int64_t n, bool conj, const int* flags, int sms);
 
 // GMRES column update + Givens + convergence flag on the device (H / e / cs / sn are double2 arrays)
 void launch_gmres_update(int kind, cudaStream_t s, const void* c1, const void* c2, int k, const void* nrm2, void* H, int ldh,
@@ -186,6 +193,19 @@ struct CsrBlocked {
 };
 // y = A x over the blocked layout: one sweep per column block, y accumulated across the blocks
 void launch_csr_blocked(int kind, cudaStream_t s, const CsrBlocked& b, const void* x, void* y, bool conj_vals, const int* flags, int sms);
+// Jacobi preconditioner d = diag(A)^-1 built on the device (kernels_ops.cu: k_jacobi, one instantiation per operator type).
+// Rows whose diagonal entry is zero or not finite leave d unwritten and lower *bad_row (initialised to ~0) to their global row.
+enum { JAC_STENCIL = 0, JAC_CSR = 1, JAC_CSR_BLOCKED = 2, JAC_DENSE = 3, JAC_DIAG = 4 };
+struct JacobiSrc {
+    int mode = JAC_STENCIL;
+    int64_t rows = 0, row0 = 0;       // local rows; global index of the first (error message only)
+    Scalar c0 = {0, 0};               // stencil: the centre coefficient
+    const int64_t* rowptr = nullptr; const int32_t* col = nullptr; const void* val = nullptr;   // plain csr
+    CsrBlocked blk;                   // L2-blocked csr
+    int64_t col0 = 0;                 // csr: the diagonal of local row r is at column col0 + r (row-sharded: global index)
+    const void* a = nullptr;          // dense (column-major rows x rows) or the diagonal operator's d
+};
+void launch_jacobi(int kind, cudaStream_t s, const JacobiSrc& src, void* d, unsigned long long* bad_row, int sms);
 void launch_stencil(int kind, cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans,
                     const int* flags, int sms);
 // CSR SpMV y = A x (vector-per-row); conj_vals: use conj(A) values (for the explicit-transpose rmatvec)

@@ -70,11 +70,13 @@ extern "C" {
 
 // flexible = fgmres (GMRES/fgmres.fypp:65-260): the preconditioned vectors Z(k) are stored and the update is
 // dx = Z(:k) y, so the preconditioner may change from one inner step to the next.
+// M: the right preconditioner as an operator (gmres only): it is enqueued inside the device cycle like A.
 static int gmres_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double rtol, double atol, int32_t transpose,
-                      lkb_gmres_io* io, lkb_precond_fn precond, void* puser, bool flexible = false) {
+                      lkb_gmres_io* io, lkb_precond_fn precond, void* puser, bool flexible = false, lkb_op_t M = nullptr) {
     if (!A || !b || !x || !info) { set_error("gmres: null argument"); return LKB_ERR_ARG; }
     if (b->n != x->n || b->kind != A->kind || x->kind != A->kind || A->m != b->n || A->n != b->n)
         { set_error("gmres: size/kind mismatch"); return LKB_ERR_ARG; }
+    if (M && (M->kind != A->kind || M->m != b->n || M->n != b->n)) { set_error("gmres: preconditioner size/kind mismatch"); return LKB_ERR_ARG; }
     lkb_ctx_s* c = b->ctx;
     const int kind = b->kind;
     const bool cplx = kind_cplx(kind);
@@ -96,7 +98,7 @@ static int gmres_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, doubl
     {
         int ra = lkb_basis_create(c, kind, b->n, b->n_global, b->row0, kdim + 1, &V);
         if (!ra) ra = lkb_vec_create(c, kind, b->n, b->n_global, b->row0, &dx);
-        if (!ra && precond && !flexible) ra = lkb_vec_create(c, kind, b->n, b->n_global, b->row0, &wrk);
+        if (!ra && (precond || M) && !flexible) ra = lkb_vec_create(c, kind, b->n, b->n_global, b->row0, &wrk);
         if (!ra && flexible) ra = lkb_basis_create(c, kind, b->n, b->n_global, b->row0, kdim, &Z);
         if (ra) {      // release whatever was allocated before the failure
             if (V) lkb_basis_destroy(V); if (dx) lkb_vec_destroy(dx); if (wrk) lkb_vec_destroy(wrk); if (Z) lkb_basis_destroy(Z);
@@ -129,7 +131,7 @@ static int gmres_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, doubl
         return check_launch(c, "gmres residual");
     };
 
-    // Without a preconditioner the whole inner cycle runs on the device (graph-captured once per call)
+    // Without a preconditioner callback the whole inner cycle runs on the device (graph-captured once per call)
     const bool device_cycle = !precond && !flexible;
     void* gH = nullptr; void* ge = nullptr; double* gres = nullptr;
     cudaGraphExec_t cycle_exec = nullptr; int64_t cycle_launches = 0;
@@ -141,8 +143,12 @@ static int gmres_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, doubl
         bool pushed = false;
         for (int kk = 1; kk <= kdim; ++kk) {
             void* w = col_ptr(V, kk);
-            LKB_TRY(op_apply_enqueue(A, col_ptr(V, kk - 1), w, trans, c->flags, pushed));
-            const HaloP2P* hp = (kk < kdim) ? op_halo_desc(A) : nullptr;
+            const void* src = col_ptr(V, kk - 1);
+            if (M) { LKB_TRY(op_apply_enqueue(M, src, wrk->d, false, c->flags)); src = wrk->d; }   // wrk = M V(k)  (gmres.fypp:155)
+            LKB_TRY(op_apply_enqueue(A, src, w, trans, c->flags, pushed));
+            // the fused halo push of V(k+1) is right only when V(k+1) is A's next input; with M in between that input is
+            // wrk, and op_apply_enqueue(A, wrk, ...) exchanges its halo itself
+            const HaloP2P* hp = (kk < kdim && !M) ? op_halo_desc(A) : nullptr;
             if (fin_ok) {     // final pass normalises with the predicted norm (mode 4: k_gmres_update does the column)
                 FinArgs fa; fa.mode = 4; fa.tol = tol; fa.kstep = kk; fa.hcol = nullptr; fa.with_c1 = false; fa.hp = hp;
                 LKB_TRY(dgs_enqueue(c, kind, V->d, V->ld, kk, w, b->n, c->flags, false, false, &fa));
@@ -163,7 +169,7 @@ static int gmres_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, doubl
             dev_alloc(c, (void**)&gres, (size_t)(kdim + 2) * 8) != 0) { cleanup_dev(); return cleanup(LKB_ERR_ALLOC); }
         rc = ensure_ws(c, kdim + 1);
         if (rc) { cleanup_dev(); return cleanup(rc); }
-        if (c->graphs && !c->profile && (A->type != 9 || A->capturable)) {
+        if (c->graphs && !c->profile && (A->type != 9 || A->capturable) && (!M || M->type != 9 || M->capturable)) {
             const int64_t l0 = c->launches;
             int r2 = cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess ? 0 : LKB_ERR_CUDA;
             if (r2 == 0) {
@@ -218,6 +224,7 @@ static int gmres_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, doubl
             for (int i = 0; i <= kdim; ++i) e[i] = cd(eh[2 * i], eh[2 * i + 1]);
             for (int i = 1; i <= kdone; ++i) { io->n_iter++; io->n_inner++; push_res(io->res, io->res_cap, &io->res_len, rh[i]); }
             if (trans) A->n_rmatvec += kdone; else A->n_matvec += kdone;
+            if (M) M->n_matvec += kdone;
             if (hf[F_STOP]) io->converged = 1;
             k = hf[F_STOP] ? kdone : kdim + 1;
         } else
@@ -277,7 +284,9 @@ static int gmres_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, doubl
             for (int i = 0; i < k; ++i) store_kind(kind, y[i], &yk[(size_t)i * kind_size(kind)]);
             GM_TRY(lkb_basis_lincomb(flexible ? Z : V, k, yk.data(), dx));         // fgmres: dx = Z(:k) y (fgmres.fypp:207)
             if (precond && !flexible) GM_TRY(apply_precond(dx->d, -1, -1.0, -1.0)); // preconditioner%apply(dx)  (gmres.fypp:202)
-            launch_axpby(kind, c->stream, one, dx->d, one, x->d, x->n, c->sms); c->launches++;
+            const void* upd = dx->d;
+            if (M) { M->n_matvec++; GM_TRY(op_apply_enqueue(M, dx->d, wrk->d, false, nullptr)); upd = wrk->d; }   // dx <- M dx
+            launch_axpby(kind, c->stream, one, upd, one, x->d, x->n, c->sms); c->launches++;
         }
         GM_TRY(residual_into_v1(false));
         GM_TRY(vec_norm_sync(c, kind, col_ptr(V, 0), b->n, &beta));
@@ -306,12 +315,21 @@ int lkb_fgmres(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double rtol,
                lkb_gmres_io* io, lkb_precond_fn precond, void* user) {
     return gmres_impl(A, b, x, info, rtol, atol, transpose, io, precond, user, true);
 }
+int lkb_gmres_precond_op(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double rtol, double atol, int32_t transpose,
+                         lkb_gmres_io* io, lkb_op_t M) {
+    if (!M) { set_error("gmres_precond_op: null preconditioner"); return LKB_ERR_ARG; }
+    return gmres_impl(A, b, x, info, rtol, atol, transpose, io, nullptr, nullptr, false, M);
+}
 
+// The preconditioner is a host callback (precond: host-driven loop below) or an operator M (device-resident loop).
 static int cg_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double rtol, double atol, lkb_cg_io* io,
-                   lkb_precond_fn precond, void* puser) {
+                   lkb_precond_fn precond, void* puser, lkb_op_t M = nullptr) {
     if (!A || !b || !x || !info) { set_error("cg: null argument"); return LKB_ERR_ARG; }
     if (b->n != x->n || b->kind != A->kind || x->kind != A->kind || A->m != b->n || A->n != b->n)
         { set_error("cg: size/kind mismatch"); return LKB_ERR_ARG; }
+    if (M && (M->kind != A->kind || M->m != b->n || M->n != b->n)) { set_error("cg: preconditioner size/kind mismatch"); return LKB_ERR_ARG; }
+    // a diagonal M is fused into k_cg_update / k_cg_direction; any other M is applied to r and reduced by a multi-dot
+    const int mode = !M ? CG_PLAIN : (M->type == 4 ? CG_DIAG : CG_NORED);
     lkb_ctx_s* c = b->ctx;
     const int kind = b->kind;
     lkb_cg_io local; memset(&local, 0, sizeof(local));
@@ -328,7 +346,7 @@ static int cg_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double r
         int ra = lkb_vec_create(c, kind, b->n, b->n_global, b->row0, &r);
         if (!ra) ra = lkb_vec_create(c, kind, b->n, b->n_global, b->row0, &p);
         if (!ra) ra = lkb_vec_create(c, kind, b->n, b->n_global, b->row0, &Ap);
-        if (!ra && precond) ra = lkb_vec_create(c, kind, b->n, b->n_global, b->row0, &z);
+        if (!ra && (precond || mode == CG_NORED)) ra = lkb_vec_create(c, kind, b->n, b->n_global, b->row0, &z);
         if (ra) {
             if (r) lkb_vec_destroy(r); if (p) lkb_vec_destroy(p); if (Ap) lkb_vec_destroy(Ap); if (z) lkb_vec_destroy(z);
             return ra;
@@ -354,6 +372,13 @@ static int cg_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double r
         CG_TRY(make_z());
         launch_axpby(kind, c->stream, one, z->d, zero, p->d, b->n, c->sms); c->launches++;  // p = z
         CG_TRY(vec_dot_sync(c, kind, r->d, z->d, b->n, &rr_old));
+    } else if (M) {
+        // z = M r ; p = z ; rz = r^H z   (a diagonal M writes z straight into p: the loop never stores z)
+        M->n_matvec++;
+        void* z0 = mode == CG_DIAG ? p->d : z->d;
+        CG_TRY(op_apply_enqueue(M, r->d, z0, false, nullptr));
+        if (mode == CG_NORED) { launch_axpby(kind, c->stream, one, z->d, zero, p->d, b->n, c->sms); c->launches++; }
+        CG_TRY(vec_dot_sync(c, kind, r->d, z0, b->n, &rr_old));
     } else {
         launch_axpby(kind, c->stream, one, r->d, zero, p->d, b->n, c->sms); c->launches++;  // p = r
         CG_TRY(vec_dot_sync(c, kind, r->d, r->d, b->n, &rr_old));
@@ -383,18 +408,29 @@ static int cg_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double r
             LKB_TRY(allreduce_w(c, c->tmpw, ndw));
             prof_begin(c, PC_OTHER);
             launch_cg_update(kind, c->stream, scal, c->tmpw, p->d, Ap->d, x->d, r->d, b->n, c->partial, c->nrm2, c->counter,
-                             c->flags, c->sms, c->p2p_arg());
+                             c->flags, c->sms, c->p2p_arg(), mode, mode == CG_DIAG ? M->diag : nullptr);
             prof_end(c, PC_OTHER, 1);
-            LKB_TRY(allreduce_w(c, c->nrm2, 1));
+            const void* rr_new = c->nrm2;
+            if (mode == CG_NORED) {         // z = M r ; rz = r^H z (multi-dot, j = 1: c2[0])
+                LKB_TRY(op_apply_enqueue(M, r->d, z->d, false, c->flags));
+                prof_begin(c, PC_DOT);
+                launch_multidot(kind, c->stream, r->d, b->n, 1, z->d, b->n, c->partial, c->c2, c->counter, c->flags, c->sms, c->p2p_arg());
+                prof_end(c, PC_DOT, 1);
+                LKB_TRY(allreduce_w(c, c->c2, ndw));
+                rr_new = c->c2;
+            } else {
+                LKB_TRY(allreduce_w(c, c->nrm2, mode == CG_DIAG && kind_cplx(kind) ? 2 : 1));
+            }
             prof_begin(c, PC_OTHER);
-            launch_cg_check(kind, c->stream, scal, c->nrm2, tol, maxiter, res_hist, c->flags);
-            launch_cg_direction(kind, c->stream, scal, r->d, p->d, b->n, c->flags, c->sms);
+            launch_cg_check(kind, c->stream, scal, rr_new, tol, maxiter, res_hist, c->flags);
+            launch_cg_direction(kind, c->stream, scal, mode == CG_NORED ? z->d : r->d, p->d, b->n, c->flags, c->sms,
+                                mode == CG_DIAG ? M->diag : nullptr);
             prof_end(c, PC_OTHER, 2);
             return check_launch(c, "cg iteration");
         };
         cudaGraphExec_t exec = nullptr;
         int64_t graph_launches = 0;
-        const bool use_graph = c->graphs && !c->profile && (A->type != 9 || A->capturable);
+        const bool use_graph = c->graphs && !c->profile && (A->type != 9 || A->capturable) && (!M || M->type != 9 || M->capturable);
         if (use_graph) {
             const int64_t l0 = c->launches;
             CG_TRY(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess ? 0 : LKB_ERR_CUDA);
@@ -420,6 +456,7 @@ static int cg_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double r
         if (exec) cudaGraphExecDestroy(exec);
         io->n_iter = hf[5]; io->converged = hf[6];
         A->n_matvec += io->n_iter;
+        if (M) M->n_matvec += io->n_iter;
         std::vector<double> hist((size_t)io->n_iter + 1);
         CG_TRY(cudaMemcpy(hist.data(), res_hist, hist.size() * sizeof(double), cudaMemcpyDeviceToHost) == cudaSuccess ? 0 : LKB_ERR_CUDA);
         for (int i = 1; i <= io->n_iter; ++i) push_res(io->res, io->res_cap, &io->res_len, hist[i]);
@@ -461,6 +498,11 @@ int lkb_cg(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double rtol, dou
 int lkb_cg_precond(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double rtol, double atol, lkb_cg_io* io,
                    lkb_precond_fn precond, void* user) {
     return cg_impl(A, b, x, info, rtol, atol, io, precond, user);
+}
+int lkb_cg_precond_op(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double rtol, double atol, lkb_cg_io* io,
+                      lkb_op_t M) {
+    if (!M) { set_error("cg_precond_op: null preconditioner"); return LKB_ERR_ARG; }
+    return cg_impl(A, b, x, info, rtol, atol, io, nullptr, nullptr, M);
 }
 
 }  // extern "C"
