@@ -211,25 +211,6 @@ int vec_dot_sync(lkb_ctx_s* c, int kind, const void* x, const void* y, int64_t n
 }
 }  // namespace lkb
 
-static Scalar scalar_from(int kind, const void* p) {
-    Scalar s{0, 0};
-    switch (kind) {
-        case KS: s.re = *(const float*)p; break;
-        case KD: s.re = *(const double*)p; break;
-        case KC: s.re = ((const float*)p)[0]; s.im = ((const float*)p)[1]; break;
-        default: s.re = ((const double*)p)[0]; s.im = ((const double*)p)[1]; break;
-    }
-    return s;
-}
-static void scalar_to(int kind, Scalar s, void* p) {
-    switch (kind) {
-        case KS: *(float*)p = (float)s.re; break;
-        case KD: *(double*)p = s.re; break;
-        case KC: ((float*)p)[0] = (float)s.re; ((float*)p)[1] = (float)s.im; break;
-        default: ((double*)p)[0] = s.re; ((double*)p)[1] = s.im; break;
-    }
-}
-
 extern "C" {
 
 const char* lkb_last_error(void) { return g_err; }
@@ -457,14 +438,14 @@ int lkb_vec_rand(lkb_vec_t v, int32_t ifnorm) {
 }
 int lkb_vec_scal(lkb_vec_t v, const void* alpha) {
     prof_begin(v->ctx, PC_OTHER);
-    launch_scal(v->kind, v->ctx->stream, scalar_from(v->kind, alpha), v->d, v->n, v->ctx->sms);
+    launch_scal(v->kind, v->ctx->stream, to_scalar(load_kind(v->kind, alpha, 0)), v->d, v->n, v->ctx->sms);
     prof_end(v->ctx, PC_OTHER, 1);
     return check_launch(v->ctx, "scal");
 }
 int lkb_vec_axpby(const void* alpha, lkb_vec_t x, const void* beta, lkb_vec_t self) {
     if (!x || !self || x->n != self->n || x->kind != self->kind) { set_error("axpby: size/kind mismatch"); return LKB_ERR_ARG; }
     prof_begin(self->ctx, PC_OTHER);
-    launch_axpby(self->kind, self->ctx->stream, scalar_from(self->kind, alpha), x->d, scalar_from(self->kind, beta),
+    launch_axpby(self->kind, self->ctx->stream, to_scalar(load_kind(self->kind, alpha, 0)), x->d, to_scalar(load_kind(self->kind, beta, 0)),
                  self->d, self->n, self->ctx->sms);
     prof_end(self->ctx, PC_OTHER, 1);
     return check_launch(self->ctx, "axpby");
@@ -473,7 +454,7 @@ int lkb_vec_dot(lkb_vec_t self, lkb_vec_t vec, void* out) {
     if (!self || !vec || self->n != vec->n || self->kind != vec->kind) { set_error("dot: size/kind mismatch"); return LKB_ERR_ARG; }
     Scalar s;
     LKB_TRY(vec_dot_sync(self->ctx, self->kind, self->d, vec->d, self->n, &s));
-    scalar_to(self->kind, s, out);
+    store_kind(self->kind, out, 0, cd(s.re, s.im));
     return 0;
 }
 int lkb_vec_norm(lkb_vec_t v, double* out) { return vec_norm_sync(v->ctx, v->kind, v->d, v->n, out); }
@@ -533,7 +514,7 @@ int lkb_basis_axpby(const void* alpha, lkb_basis_t X, int xcol0, const void* bet
     if (!X || !Y || !alpha || !beta || xcol0 < 0 || ycol0 < 0 || ncols < 0 || xcol0 + ncols > X->ncols || ycol0 + ncols > Y->ncols ||
         X->n != Y->n || X->kind != Y->kind) { set_error("basis_axpby: bad arguments"); return LKB_ERR_ARG; }
     lkb_ctx_s* c = Y->ctx;
-    const Scalar a = scalar_from(Y->kind, alpha), bb = scalar_from(Y->kind, beta);
+    const Scalar a = to_scalar(load_kind(Y->kind, alpha, 0)), bb = to_scalar(load_kind(Y->kind, beta, 0));
     for (int q = 0; q < ncols; ++q) {
         launch_axpby(Y->kind, c->stream, a, col_ptr(X, xcol0 + q), bb, col_ptr(Y, ycol0 + q), Y->n, c->sms);
         c->launches++;
@@ -589,14 +570,14 @@ static int stencil_create(lkb_ctx_t c, int kind, int dim, int64_t nx, int64_t ny
     if (slow0 < 0 || nslow_local < 1 || slow0 + nslow_local > nslow) { set_error("stencil: bad slab [%lld,+%lld) of %lld", (long long)slow0, (long long)nslow_local, (long long)nslow); return LKB_ERR_ARG; }
     cudaSetDevice(c->dev);
     lkb_op_s* op = new lkb_op_s();
-    op->ctx = c; op->type = 1; op->kind = kind; op->uid = next_uid();
+    op->ctx = c; op->type = OP_STENCIL; op->kind = kind; op->uid = next_uid();
     op->st.dim = dim; op->st.nx = nx;
     op->st.ny = dim == 2 ? nslow_local : ny;
     op->st.nz = dim == 2 ? 1 : nslow_local;
     op->slow0 = slow0; op->nslow_global = nslow;
     const int ncoef = dim == 2 ? 5 : 7;
     const size_t es = kind_size(kind);
-    for (int q = 0; q < 7; ++q) op->st.coef[q] = q < ncoef ? scalar_from(kind, (const char*)coef + q * es) : Scalar{0, 0};
+    for (int q = 0; q < 7; ++q) op->st.coef[q] = q < ncoef ? to_scalar(load_kind(kind, coef, q)) : Scalar{0, 0};
     op->m = op->n = nx * op->st.ny * op->st.nz;
     op->halo_elems = dim == 2 ? nx : nx * ny;
     op->st.halo_lo = op->st.halo_hi = nullptr;
@@ -727,7 +708,7 @@ int lkb_op_csr_create_dist(lkb_ctx_t c, int kind, int64_t m_global, int64_t n_gl
     if (!c || !A || !rowptr_local || m_local < 0 || n_local < 0 || m_global < 1 || n_global < 1) return LKB_ERR_ARG;
     cudaSetDevice(c->dev);
     lkb_op_s* op = new lkb_op_s();
-    op->ctx = c; op->type = 3; op->kind = kind; op->m = m_local; op->n = n_local; op->uid = next_uid();
+    op->ctx = c; op->type = OP_CSR; op->kind = kind; op->m = m_local; op->n = n_local; op->uid = next_uid();
     op->dist = true; op->m_global = m_global; op->n_global = n_global;
     int r = csr_build(c, op, kind, m_local, n_global, rowptr_local, col_global, val);
     if (r == 0) r = csr_dist_finish(c, op, kind, n_global, row0, m_local, col0, n_local);
@@ -744,7 +725,7 @@ int lkb_op_csr_create_dist_device(lkb_ctx_t c, int kind, int64_t m_global, int64
     if (!adopt) { set_error("csr_create_dist_device: only adopt != 0 is supported"); return LKB_ERR_ARG; }
     cudaSetDevice(c->dev);
     lkb_op_s* op = new lkb_op_s();
-    op->ctx = c; op->type = 3; op->kind = kind; op->m = m_local; op->n = n_local; op->uid = next_uid();
+    op->ctx = c; op->type = OP_CSR; op->kind = kind; op->m = m_local; op->n = n_local; op->uid = next_uid();
     op->dist = true; op->m_global = m_global; op->n_global = n_global;
     op->rowptr = rowptr_dev; op->col = col_dev; op->val = val_dev;
     int r = csr_finish_device(c, op, kind, m_local, n_global);
@@ -762,7 +743,7 @@ int lkb_op_dense_create(lkb_ctx_t c, int kind, int64_t m, int64_t n, const void*
     if (c->world > 1) { set_error("dense operators are single-rank (plumbing config only)"); return LKB_ERR_ARG; }
     cudaSetDevice(c->dev);
     lkb_op_s* op = new lkb_op_s();
-    op->ctx = c; op->type = 0; op->kind = kind; op->m = m; op->n = n; op->uid = next_uid();
+    op->ctx = c; op->type = OP_DENSE; op->kind = kind; op->m = m; op->n = n; op->uid = next_uid();
     LKB_CUDA(cudaMalloc(&op->a, (size_t)m * n * kind_size(kind)));
     LKB_CUDA(cudaMemcpy(op->a, a, (size_t)m * n * kind_size(kind), cudaMemcpyHostToDevice));
     *A = op;
@@ -772,7 +753,7 @@ int lkb_op_callback_create(lkb_ctx_t c, int kind, int64_t m_local, int64_t n_loc
                            int32_t capturable, lkb_op_t* A) {
     if (!c || !A || !fn) return LKB_ERR_ARG;
     lkb_op_s* op = new lkb_op_s();
-    op->ctx = c; op->type = 9; op->kind = kind; op->m = m_local; op->n = n_local; op->uid = next_uid();
+    op->ctx = c; op->type = OP_CALLBACK; op->kind = kind; op->m = m_local; op->n = n_local; op->uid = next_uid();
     op->fn = fn; op->user = user; op->capturable = capturable != 0;
     *A = op;
     return 0;
@@ -782,7 +763,7 @@ int lkb_op_callback_create(lkb_ctx_t c, int kind, int64_t m_local, int64_t n_loc
 static int diag_from_device(lkb_ctx_t c, int kind, int64_t n, int64_t row0, int64_t n_global, lkb_op_s** M) {
     cudaSetDevice(c->dev);
     lkb_op_s* op = new lkb_op_s();
-    op->ctx = c; op->type = 4; op->kind = kind; op->m = op->n = n; op->uid = next_uid();
+    op->ctx = c; op->type = OP_DIAG; op->kind = kind; op->m = op->n = n; op->uid = next_uid();
     op->diag_row0 = row0; op->diag_n_global = n_global;
     if (cudaMalloc(&op->diag, std::max<size_t>((size_t)n * kind_size(kind), 16)) != cudaSuccess) {
         cudaGetLastError(); op->diag = nullptr; delete op;
@@ -809,16 +790,16 @@ int lkb_op_diag_create(lkb_vec_t d, lkb_op_t* M) {
 int lkb_op_jacobi_create(lkb_op_t A, lkb_op_t* M) {
     if (!A || !M) { set_error("jacobi_create: null argument"); return LKB_ERR_ARG; }
     lkb_ctx_s* c = A->ctx;
-    if (A->type == 9) { set_error("jacobi_create: a callback operator has no diagonal the library can read"); return LKB_ERR_ARG; }
+    if (A->type == OP_CALLBACK) { set_error("jacobi_create: a callback operator has no diagonal the library can read"); return LKB_ERR_ARG; }
     if (A->m != A->n) { set_error("jacobi_create: A is not square (%lld x %lld local rows / columns)", (long long)A->m, (long long)A->n); return LKB_ERR_ARG; }
     JacobiSrc src;
     src.rows = A->m;
     int64_t n_global = A->m;
-    if (A->type == 1) {
+    if (A->type == OP_STENCIL) {
         const int64_t plane = A->st.dim == 2 ? A->st.nx : A->st.nx * A->st.ny;
         src.mode = JAC_STENCIL; src.c0 = A->st.coef[0];
         src.row0 = A->slow0 * plane; n_global = A->nslow_global * plane;
-    } else if (A->type == 3) {
+    } else if (A->type == OP_CSR) {
         if (A->dist) {
             const int r = c->rank;
             if (A->row_off[r] != A->col_off[r] || A->row_cnt[r] != A->col_cnt[r] || A->m_global != A->n_global) {
@@ -831,9 +812,9 @@ int lkb_op_jacobi_create(lkb_op_t A, lkb_op_t* M) {
         }
         if (A->blk.nb > 0) { src.mode = JAC_CSR_BLOCKED; src.blk = A->blk; }
         else { src.mode = JAC_CSR; src.rowptr = A->rowptr; src.col = A->col; src.val = A->val; }
-    } else if (A->type == 0) {
+    } else if (A->type == OP_DENSE) {
         src.mode = JAC_DENSE; src.a = A->a;
-    } else if (A->type == 4) {
+    } else if (A->type == OP_DIAG) {
         src.mode = JAC_DIAG; src.a = A->diag; src.row0 = A->diag_row0; n_global = A->diag_n_global;
     } else {
         set_error("jacobi_create: unsupported operator type %d", A->type); return LKB_ERR_ARG;
@@ -880,14 +861,14 @@ int lkb_op_reset_counters(lkb_op_t A) { A->n_matvec = A->n_rmatvec = 0; return 0
 namespace lkb {
 const HaloP2P* op_halo_desc(const lkb_op_s* A) {
     const lkb_ctx_s* c = A->ctx;
-    return (A->type == 1 && c->world > 1 && A->hp_active && c->p2p_active && c->fused_halo && c->fin) ? &A->hp : nullptr;
+    return (A->type == OP_STENCIL && c->world > 1 && A->hp_active && c->p2p_active && c->fused_halo && c->fin) ? &A->hp : nullptr;
 }
 int op_apply_enqueue(lkb_op_s* A, const void* x, void* y, bool trans, const int* flags, bool halo_prepushed) {
     lkb_ctx_s* c = A->ctx;
     const size_t es = kind_size(A->kind);
     int nl = 1;
     prof_begin(c, PC_MATVEC);
-    if (A->type == 1) {
+    if (A->type == OP_STENCIL) {
         if (c->world > 1 && A->hp_active) {
             // halo exchange over NVLink peer memory: pushed by the kernel that finished x, or by k_halo_push
             // (copy + synchronisation in one kernel)
@@ -914,7 +895,7 @@ int op_apply_enqueue(lkb_op_s* A, const void* x, void* y, bool trans, const int*
             pdl_rearm();
         }
         launch_stencil(A->kind, c->stream, A->st, x, y, trans, flags, c->sms);
-    } else if (A->type == 3 && A->dist) {
+    } else if (A->type == OP_CSR && A->dist) {
         const int dt = (A->kind == KS || A->kind == KC) ? 7 : 8;            // ncclFloat32 / ncclFloat64
         const size_t per = kind_cplx(A->kind) ? 2 : 1;
         NcclApi* api = c->world > 1 ? nccl_api() : nullptr;
@@ -949,7 +930,7 @@ int op_apply_enqueue(lkb_op_s* A, const void* x, void* y, bool trans, const int*
                 LKB_CUDA(cudaMemcpyAsync(y, (char*)A->y_full + (size_t)A->col_off[0] * es, (size_t)A->n * es, cudaMemcpyDeviceToDevice, c->stream));
             }
         }
-    } else if (A->type == 3) {
+    } else if (A->type == OP_CSR) {
         if (!trans) {
             if (A->blk.nb > 0) { launch_csr_blocked(A->kind, c->stream, A->blk, x, y, false, flags, c->sms); nl = A->blk.nb; }
             else launch_csr(A->kind, c->stream, A->m, A->rowptr, A->col, A->val, x, y, false, flags, c->sms | (A->lpr << 16));
@@ -957,9 +938,9 @@ int op_apply_enqueue(lkb_op_s* A, const void* x, void* y, bool trans, const int*
             if (A->t_blk.nb > 0) { launch_csr_blocked(A->kind, c->stream, A->t_blk, x, y, true, flags, c->sms); nl = A->t_blk.nb; }
             else launch_csr(A->kind, c->stream, A->n, A->t_rowptr, A->t_col, A->t_val, x, y, true, flags, c->sms | (A->t_lpr << 16));
         }
-    } else if (A->type == 0) {
+    } else if (A->type == OP_DENSE) {
         launch_dense(A->kind, c->stream, A->m, A->n, A->a, x, y, trans, flags);
-    } else if (A->type == 4) {
+    } else if (A->type == OP_DIAG) {
         launch_diag(A->kind, c->stream, A->diag, x, y, A->m, trans, flags, c->sms);      // row-local: no exchange at N > 1
     } else {
         int r = A->fn(A->user, x, y, trans ? 1 : 0, (void*)c->stream);
@@ -970,7 +951,7 @@ int op_apply_enqueue(lkb_op_s* A, const void* x, void* y, bool trans, const int*
     // the programmatic-launch chain: the next PDL-aware kernel is launched normally.  The diagonal operator is one plain
     // kernel (k_diag, launched without the PDL attribute, like the stencil): a PDL-aware successor waits for its completion
     // in griddepcontrol.wait, so it keeps the chain.
-    if (!(A->type == 1 || A->type == 0 || A->type == 4 || (A->type == 3 && !A->dist))) pdl_rearm();
+    if (!(A->type == OP_STENCIL || A->type == OP_DENSE || A->type == OP_DIAG || (A->type == OP_CSR && !A->dist))) pdl_rearm();
     prof_end(c, PC_MATVEC, nl);
     return check_launch(c, "matvec");
 }
@@ -981,7 +962,7 @@ static int op_apply_api(lkb_op_t A, lkb_vec_t x, lkb_vec_t y, bool trans) {
     if (!A || !x || !y) return LKB_ERR_ARG;
     const int64_t nin = trans ? A->m : A->n, nout = trans ? A->n : A->m;
     if (x->n != nin || y->n != nout || x->kind != A->kind || y->kind != A->kind) { set_error("matvec: size/kind mismatch"); return LKB_ERR_ARG; }
-    if (x->d == y->d && A->type != 4) { set_error("matvec: vec_out must not alias vec_in"); return LKB_ERR_ARG; }   // (k_diag works in place)
+    if (x->d == y->d && A->type != OP_DIAG) { set_error("matvec: vec_out must not alias vec_in"); return LKB_ERR_ARG; }   // (k_diag works in place)
     if (trans) A->n_rmatvec++; else A->n_matvec++;
     return op_apply_enqueue(A, x->d, y->d, trans, nullptr);
 }

@@ -320,7 +320,7 @@ int lkb_op_csr_create(lkb_ctx_t c, int kind, int64_t m, int64_t n, const int64_t
     if (c->world > 1) { set_error("lkb_op_csr_create is single-rank; use lkb_op_csr_create_dist for a row-sharded matrix"); return LKB_ERR_ARG; }
     cudaSetDevice(c->dev);
     lkb_op_s* op = new lkb_op_s();
-    op->ctx = c; op->type = 3; op->kind = kind; op->m = m; op->n = n; op->uid = next_uid();
+    op->ctx = c; op->type = OP_CSR; op->kind = kind; op->m = m; op->n = n; op->uid = next_uid();
     int r = csr_build(c, op, kind, m, n, rowptr, col, val);
     if (r) { lkb_op_destroy(op); return r; }
     *A = op;
@@ -333,7 +333,7 @@ int lkb_op_csr_create_device(lkb_ctx_t c, int kind, int64_t m, int64_t n, int64_
     if (c->world > 1) { set_error("lkb_op_csr_create_device is single-rank"); return LKB_ERR_ARG; }
     cudaSetDevice(c->dev);
     lkb_op_s* op = new lkb_op_s();
-    op->ctx = c; op->type = 3; op->kind = kind; op->m = m; op->n = n; op->uid = next_uid();
+    op->ctx = c; op->type = OP_CSR; op->kind = kind; op->m = m; op->n = n; op->uid = next_uid();
     if (adopt) {
         op->rowptr = rowptr_dev; op->col = col_dev; op->val = val_dev;
     } else {

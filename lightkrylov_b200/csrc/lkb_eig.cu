@@ -26,7 +26,6 @@
 #include "lkb_internal.h"
 
 using namespace lkb;
-typedef std::complex<double> cd;
 typedef int lint;   // LP64 LAPACK
 
 namespace {
@@ -91,23 +90,6 @@ int lapack_ready() {
         if (lapack_open(p, "", "_") == 0) return 0;
     set_error("no host LAPACK provider: call lkb_set_lapack(path, prefix, suffix) or set LKB_LAPACK_LIB");
     return LKB_ERR_LAPACK;
-}
-
-cd load_kind(int kind, const void* H, size_t idx) {
-    switch (kind) {
-        case KS: return cd(((const float*)H)[idx], 0.0);
-        case KD: return cd(((const double*)H)[idx], 0.0);
-        case KC: return cd(((const float*)H)[2 * idx], ((const float*)H)[2 * idx + 1]);
-        default: return cd(((const double*)H)[2 * idx], ((const double*)H)[2 * idx + 1]);
-    }
-}
-void store_kind(int kind, void* H, size_t idx, cd v) {
-    switch (kind) {
-        case KS: ((float*)H)[idx] = (float)v.real(); break;
-        case KD: ((double*)H)[idx] = v.real(); break;
-        case KC: ((float*)H)[2 * idx] = (float)v.real(); ((float*)H)[2 * idx + 1] = (float)v.imag(); break;
-        default: ((double*)H)[2 * idx] = v.real(); ((double*)H)[2 * idx + 1] = v.imag(); break;
-    }
 }
 
 // eig(A(:k,:k)) -> vals (complex), vecs in LAPACK layout: for real kinds the REAL-pair convention
@@ -275,19 +257,25 @@ int device_combine(lkb_basis_s* Xw, int k, const std::vector<cd>& Zc, int ldz, i
 }
 
 // Two pinned host slots + events for the "collect step k, enqueue step k+1 speculatively, then run the host LAPACK
-// of step k" pipeline shared by eigs / eighs / svds.
+// of step k" pipeline shared by eigs / eighs / svds.  A speculative step's copy into a slot may still be in flight when
+// the solver returns: the destructor waits for the stream before it frees the slots.
 struct StepSlots {
+    cudaStream_t stream;
     void* slot[2] = {nullptr, nullptr};
     cudaEvent_t ev[2] = {nullptr, nullptr};
+    explicit StepSlots(cudaStream_t s) : stream(s) {}
+    StepSlots(const StepSlots&) = delete;
+    StepSlots& operator=(const StepSlots&) = delete;
+    ~StepSlots() {
+        cudaStreamSynchronize(stream);
+        for (int q = 0; q < 2; ++q) { if (slot[q]) cudaFreeHost(slot[q]); if (ev[q]) cudaEventDestroy(ev[q]); }
+    }
     int init(size_t bytes) {
         for (int q = 0; q < 2; ++q)
             if (cudaMallocHost(&slot[q], bytes) != cudaSuccess || cudaEventCreateWithFlags(&ev[q], cudaEventDisableTiming) != cudaSuccess) {
-                release(); set_error("pinned staging allocation failed"); return LKB_ERR_ALLOC;
+                set_error("pinned staging allocation failed"); return LKB_ERR_ALLOC;
             }
         return 0;
-    }
-    void release() {
-        for (int q = 0; q < 2; ++q) { if (slot[q]) cudaFreeHost(slot[q]); if (ev[q]) cudaEventDestroy(ev[q]); slot[q] = nullptr; ev[q] = nullptr; }
     }
 };
 
@@ -352,20 +340,19 @@ int lkb_krylov_schur(lkb_basis_t X, void* H, int ldh, int kdim, int32_t* nkeep) 
         int64_t chunk = (int64_t)(((size_t)1 << 30) / ((size_t)nk * es));
         chunk = std::max<int64_t>(4096, (chunk / 4096) * 4096);
         chunk = std::min<int64_t>(chunk, ((X->n + 4095) / 4096) * 4096);
-        void* tmp = nullptr;
-        LKB_TRY(dev_alloc(c, &tmp, (size_t)chunk * nk * es));
+        DevBuf tmp(c);
+        LKB_TRY(tmp.alloc((size_t)chunk * nk * es));
         int r = 0;
         for (int64_t r0 = 0; r0 < X->n && r == 0; r0 += chunk) {
             const int64_t rows = std::min<int64_t>(chunk, X->n - r0);
             prof_begin(c, PC_OTHER);
-            launch_basis_gemm(kind, c->stream, (char*)X->d + (size_t)r0 * es, X->ld, k, c->coefd, k, nk, tmp, chunk, rows, c->sms);
+            launch_basis_gemm(kind, c->stream, (char*)X->d + (size_t)r0 * es, X->ld, k, c->coefd, k, nk, tmp.p, chunk, rows, c->sms);
             prof_end(c, PC_OTHER, 1);
             r = check_launch(c, "basis_gemm");
-            if (r == 0 && cudaMemcpy2DAsync((char*)X->d + (size_t)r0 * es, (size_t)X->ld * es, tmp, (size_t)chunk * es,
+            if (r == 0 && cudaMemcpy2DAsync((char*)X->d + (size_t)r0 * es, (size_t)X->ld * es, tmp.p, (size_t)chunk * es,
                                             (size_t)rows * es, nk, cudaMemcpyDeviceToDevice, c->stream) != cudaSuccess) r = LKB_ERR_CUDA;
         }
         cudaStreamSynchronize(c->stream);
-        dev_free(c, tmp);
         if (r) return r;
     }
     LKB_CUDA(cudaMemcpyAsync(col_ptr(X, nk), col_ptr(X, k), (size_t)X->n * es, cudaMemcpyDeviceToDevice, c->stream));
@@ -390,12 +377,9 @@ int lkb_eigs(lkb_op_t A, lkb_basis_t X, int nev, double* eigvals, double* residu
     const size_t es = kind_size(kind);
     const int kd = kdim > 0 ? kdim : 4 * nev;
     const double tol = tolerance >= 0 ? tolerance : rtol_of(kind);
-    lkb_basis_t Xw = nullptr;
-    LKB_TRY(lkb_basis_create(c, kind, X->n, X->n_global, X->row0, kd + 1, &Xw));
-    int rc = 0;
-    auto cleanup = [&](int r) { lkb_basis_destroy(Xw); return r; };
-#define EG_TRY(call) do { rc = (call); if (rc) return cleanup(rc); } while (0)
-    EG_TRY(start_vector(Xw, x0));
+    BasisOwner Xw;
+    LKB_TRY(lkb_basis_create(c, kind, X->n, X->n_global, X->row0, kd + 1, Xw.out()));
+    LKB_TRY(start_vector(Xw, x0));
     const int ldh = kd + 1;
     std::vector<char> H((size_t)ldh * kd * es, 0);
     std::vector<cd> vals, vecs, Hc((size_t)kd * kd);
@@ -411,21 +395,12 @@ int lkb_eigs(lkb_op_t A, lkb_basis_t X, int nev, double* eigvals, double* residu
     // speculative step that turns out to be unnecessary (convergence at k) is simply discarded.
     const bool tr = transpose != 0;
     const double atolk = atol_of(kind);
-    void* slots[2] = {nullptr, nullptr};
-    cudaEvent_t evs[2] = {nullptr, nullptr};
-    const size_t slot_bytes = (size_t)ldh * es + 256;
-    auto free_slots = [&]() { for (int q = 0; q < 2; ++q) { if (slots[q]) cudaFreeHost(slots[q]); if (evs[q]) cudaEventDestroy(evs[q]); } };
-    for (int q = 0; q < 2; ++q) {
-        if (cudaMallocHost(&slots[q], slot_bytes) != cudaSuccess || cudaEventCreateWithFlags(&evs[q], cudaEventDisableTiming) != cudaSuccess) {
-            free_slots(); set_error("eigs: pinned staging allocation failed"); return cleanup(LKB_ERR_ALLOC);
-        }
-    }
-#undef EG_TRY
-#define EG_TRY(call) do { rc = (call); if (rc) { cudaStreamSynchronize(c->stream); free_slots(); return cleanup(rc); } } while (0)
+    StepSlots ss(c->stream);
+    if (ss.init((size_t)ldh * es + 256)) { set_error("eigs: pinned staging allocation failed"); return LKB_ERR_ALLOC; }
     auto enqueue_step = [&](int kk) -> int {
         LKB_TRY(arnoldi_enqueue(A, Xw, kk, kk, atolk, tr));
-        LKB_TRY(arnoldi_fetch_async(Xw, kk, kk, slots[kk & 1]));
-        LKB_CUDA(cudaEventRecord(evs[kk & 1], c->stream));
+        LKB_TRY(arnoldi_fetch_async(Xw, kk, kk, ss.slot[kk & 1]));
+        LKB_CUDA(cudaEventRecord(ss.ev[kk & 1], c->stream));
         return 0;
     };
     int restarts = 0;
@@ -433,12 +408,12 @@ int lkb_eigs(lkb_op_t A, lkb_basis_t X, int nev, double* eigvals, double* residu
         int inflight = 0;                              // highest step already enqueued
         for (k = kstart; k <= kd; ++k) {
             int32_t ainfo = 0;
-            if (inflight < k) { EG_TRY(enqueue_step(k)); inflight = k; }
-            EG_TRY(cudaEventSynchronize(evs[k & 1]) == cudaSuccess ? 0 : LKB_ERR_CUDA);
-            EG_TRY(arnoldi_collect(A, Xw, H.data(), ldh, &ainfo, k, k, tr, slots[k & 1]));
-            if (ainfo == 0 && k < kd) { EG_TRY(enqueue_step(k + 1)); inflight = k + 1; }   // speculative
+            if (inflight < k) { LKB_TRY(enqueue_step(k)); inflight = k; }
+            LKB_CUDA(cudaEventSynchronize(ss.ev[k & 1]));
+            LKB_TRY(arnoldi_collect(A, Xw, H.data(), ldh, &ainfo, k, k, tr, ss.slot[k & 1]));
+            if (ainfo == 0 && k < kd) { LKB_TRY(enqueue_step(k + 1)); inflight = k + 1; }   // speculative
             load_Hc(k);
-            EG_TRY(host_eig(kind, k, Hc, kd, vals, vecs));
+            LKB_TRY(host_eig(kind, k, Hc, kd, vals, vecs));
             const cd beta = load_kind(kind, H.data(), (size_t)k + (size_t)ldh * (k - 1));
             std::fill(res.begin(), res.end(), 0.0);
             for (int i = 0; i < k; ++i) {
@@ -450,7 +425,7 @@ int lkb_eigs(lkb_op_t A, lkb_basis_t X, int nev, double* eigvals, double* residu
                 res[i] = std::abs(beta) * alpha;
             }
             niter++;
-            EG_TRY(bcast_host(c, res.data(), (size_t)k * sizeof(double)));
+            LKB_TRY(bcast_host(c, res.data(), (size_t)k * sizeof(double)));
             conv = 0; for (int i = 0; i < k; ++i) conv += res[i] < tol;
             if (c->write_intermediate) {                          // write_results_c(eigs_output, ...)  (:1091)
                 // LITERAL side effect: write_results sorts its `res` argument IN PLACE (`call sort_index(res, indices)`, intent(inout),
@@ -480,26 +455,23 @@ int lkb_eigs(lkb_op_t A, lkb_basis_t X, int nev, double* eigvals, double* residu
         const int converged_at = conv >= nev ? k : 0;
         if (converged_at && converged_at < kd) {
             // a speculative step k+1 wrote X(k+2); in the reference the columns beyond k+1 are still zero at this point
-            EG_TRY(cudaStreamSynchronize(c->stream) == cudaSuccess ? 0 : LKB_ERR_CUDA);
-            EG_TRY(lkb_basis_zero(Xw, converged_at + 1, kd - converged_at));
+            LKB_CUDA(cudaStreamSynchronize(c->stream));
+            LKB_TRY(lkb_basis_zero(Xw, converged_at + 1, kd - converged_at));
         }
         // Krylov-Schur restart (IterativeSolvers.fypp:1096-1100); note the loop index is kd+1 here unless converged
         int32_t nk = 0;
-        EG_TRY(lkb_krylov_schur(Xw, H.data(), ldh, kd, &nk));
+        LKB_TRY(lkb_krylov_schur(Xw, H.data(), ldh, kd, &nk));
         kstart = nk + 1;
         k = converged_at ? converged_at : kd + 1;
-        if (++restarts > 2000) { set_error("eigs: no convergence after 2000 Krylov-Schur restarts"); EG_TRY(LKB_ERR_ARG); }
+        if (++restarts > 2000) { set_error("eigs: no convergence after 2000 Krylov-Schur restarts"); return LKB_ERR_ARG; }
     }
-    EG_TRY(cudaStreamSynchronize(c->stream) == cudaSuccess ? 0 : LKB_ERR_CUDA);
-    free_slots();
-#undef EG_TRY
-#define EG_TRY(call) do { rc = (call); if (rc) return cleanup(rc); } while (0)
+    LKB_CUDA(cudaStreamSynchronize(c->stream));
     // post-process (:1108-1132)
     k = std::min(k, kd);
     load_Hc(k);
-    EG_TRY(host_eig(kind, k, Hc, kd, vals, vecs));
-    EG_TRY(bcast_host(c, vals.data(), vals.size() * sizeof(cd)));
-    EG_TRY(bcast_host(c, vecs.data(), vecs.size() * sizeof(cd)));
+    LKB_TRY(host_eig(kind, k, Hc, kd, vals, vecs));
+    LKB_TRY(bcast_host(c, vals.data(), vals.size() * sizeof(cd)));
+    LKB_TRY(bcast_host(c, vecs.data(), vecs.size() * sizeof(cd)));
     std::vector<double> av(kd, 0.0);
     for (int i = 0; i < k; ++i) av[i] = std::abs(vals[i]);
     std::vector<int> idx = sort_index_reverse(av);
@@ -511,11 +483,10 @@ int lkb_eigs(lkb_op_t A, lkb_basis_t X, int nev, double* eigvals, double* residu
         residuals[i] = res[s];
         if (s < k) for (int j = 0; j < k; ++j) Y[j + (size_t)k * i] = vecs[j + (size_t)k * s];
     }
-    EG_TRY(device_combine(Xw, k, Y, k, nev, X->d, X->ld));
-    EG_TRY(lkb_sync(c));
+    LKB_TRY(device_combine(Xw, k, Y, k, nev, X->d, X->ld));
+    LKB_TRY(lkb_sync(c));
     *info = niter;
-#undef EG_TRY
-    return cleanup(0);
+    return 0;
 }
 
 int lkb_eighs(lkb_op_t A, lkb_basis_t X, int nev, double* eigvals, double* residuals, int32_t* info, lkb_vec_t x0,
@@ -528,12 +499,9 @@ int lkb_eighs(lkb_op_t A, lkb_basis_t X, int nev, double* eigvals, double* resid
     const size_t es = kind_size(kind);
     const int kd = kdim > 0 ? kdim : 4 * nev;
     const double tol = tolerance >= 0 ? tolerance : rtol_of(kind);
-    lkb_basis_t Xw = nullptr;
-    LKB_TRY(lkb_basis_create(c, kind, X->n, X->n_global, X->row0, kd + 1, &Xw));
-    int rc = 0;
-    auto cleanup = [&](int r) { lkb_basis_destroy(Xw); return r; };
-#define EH_TRY(call) do { rc = (call); if (rc) return cleanup(rc); } while (0)
-    EH_TRY(start_vector(Xw, x0));
+    BasisOwner Xw;
+    LKB_TRY(lkb_basis_create(c, kind, X->n, X->n_global, X->row0, kd + 1, Xw.out()));
+    LKB_TRY(start_vector(Xw, x0));
     const int ldt = kd + 1;
     std::vector<char> T((size_t)ldt * kd * es, 0);
     std::vector<double> ev(kd, 0.0), res(kd, 0.0);
@@ -542,10 +510,8 @@ int lkb_eighs(lkb_op_t A, lkb_basis_t X, int nev, double* eigvals, double* resid
     int k = 1, conv = 0;
     // Host/device overlap as in eigs: step k+1 is enqueued speculatively before the host runs syev / heev on T_k
     // (eighs.fypp:84-100); Xwrk and T are internal work arrays, a speculative step past convergence is discarded.
-    StepSlots ss;
-    EH_TRY(ss.init((size_t)ldt * es + 256));
-#undef EH_TRY
-#define EH_TRY(call) do { rc = (call); if (rc) { cudaStreamSynchronize(c->stream); ss.release(); return cleanup(rc); } } while (0)
+    StepSlots ss(c->stream);
+    LKB_TRY(ss.init((size_t)ldt * es + 256));
     const double atolk = atol_of(kind);
     auto enqueue_step = [&](int kk) -> int {
         LKB_TRY(lanczos_enqueue(A, Xw, kk, kk, atolk));
@@ -556,19 +522,19 @@ int lkb_eighs(lkb_op_t A, lkb_basis_t X, int nev, double* eigvals, double* resid
     int inflight = 0;
     for (k = 1; k <= kd; ++k) {
         int32_t linfo = 0;
-        if (inflight < k) { EH_TRY(enqueue_step(k)); inflight = k; }
-        EH_TRY(cudaEventSynchronize(ss.ev[k & 1]) == cudaSuccess ? 0 : LKB_ERR_CUDA);
-        EH_TRY(lanczos_collect(A, Xw, T.data(), ldt, &linfo, k, k, ss.slot[k & 1]));
-        if (linfo == 0 && k < kd) { EH_TRY(enqueue_step(k + 1)); inflight = k + 1; }      // speculative
+        if (inflight < k) { LKB_TRY(enqueue_step(k)); inflight = k; }
+        LKB_CUDA(cudaEventSynchronize(ss.ev[k & 1]));
+        LKB_TRY(lanczos_collect(A, Xw, T.data(), ldt, &linfo, k, k, ss.slot[k & 1]));
+        if (linfo == 0 && k < kd) { LKB_TRY(enqueue_step(k + 1)); inflight = k + 1; }      // speculative
         std::fill(ev.begin(), ev.end(), 0.0); std::fill(vecs.begin(), vecs.end(), cd(0));
         Tk.assign((size_t)k * k, cd(0));
         for (int j = 0; j < k; ++j) for (int i = 0; i < k; ++i) Tk[i + (size_t)k * j] = load_kind(kind, T.data(), (size_t)i + (size_t)ldt * j);
-        EH_TRY(sp ? host_eigh_t<float>(cplx, k, Tk, ev.data(), vk) : host_eigh_t<double>(cplx, k, Tk, ev.data(), vk));
+        LKB_TRY(sp ? host_eigh_t<float>(cplx, k, Tk, ev.data(), vk) : host_eigh_t<double>(cplx, k, Tk, ev.data(), vk));
         for (int j = 0; j < k; ++j) for (int i = 0; i < k; ++i) vecs[i + (size_t)kd * j] = vk[i + (size_t)k * j];
         const cd beta = load_kind(kind, T.data(), (size_t)k + (size_t)ldt * (k - 1));
         std::fill(res.begin(), res.end(), 0.0);
         for (int i = 0; i < k; ++i) res[i] = std::abs(beta * vecs[(k - 1) + (size_t)kd * i]);
-        EH_TRY(bcast_host(c, res.data(), (size_t)k * sizeof(double)));
+        LKB_TRY(bcast_host(c, res.data(), (size_t)k * sizeof(double)));
         conv = 0; for (int i = 0; i < k; ++i) conv += res[i] < tol;
         if (c->write_intermediate) {                              // write_results_r(eighs_output, ...)  (eighs.fypp:99)
             std::vector<double> rr(res.begin(), res.begin() + k); // sorts the residual table in place, see lkb_eigs
@@ -578,12 +544,9 @@ int lkb_eighs(lkb_op_t A, lkb_basis_t X, int nev, double* eigvals, double* resid
         }
         if (conv >= nev) break;
     }
-    EH_TRY(cudaStreamSynchronize(c->stream) == cudaSuccess ? 0 : LKB_ERR_CUDA);     // a discarded speculative step may still run
-    ss.release();
-#undef EH_TRY
-#define EH_TRY(call) do { rc = (call); if (rc) return cleanup(rc); } while (0)
-    EH_TRY(bcast_host(c, ev.data(), ev.size() * sizeof(double)));
-    EH_TRY(bcast_host(c, vecs.data(), vecs.size() * sizeof(cd)));
+    LKB_CUDA(cudaStreamSynchronize(c->stream));     // a discarded speculative step may still run
+    LKB_TRY(bcast_host(c, ev.data(), ev.size() * sizeof(double)));
+    LKB_TRY(bcast_host(c, vecs.data(), vecs.size() * sizeof(cd)));
     std::vector<int> idx = sort_index_reverse(ev);        // over all kdim_ entries, zero padding included (eighs.fypp:106-107)
     k = std::min(k, kd);
     std::vector<cd> Y((size_t)k * nev, cd(0));
@@ -592,11 +555,10 @@ int lkb_eighs(lkb_op_t A, lkb_basis_t X, int nev, double* eigvals, double* resid
         eigvals[i] = ev[s]; residuals[i] = res[s];
         for (int j = 0; j < k; ++j) Y[j + (size_t)k * i] = vecs[j + (size_t)kd * s];
     }
-    EH_TRY(device_combine(Xw, k, Y, k, nev, X->d, X->ld));
-    EH_TRY(lkb_sync(c));
+    LKB_TRY(device_combine(Xw, k, Y, k, nev, X->d, X->ld));
+    LKB_TRY(lkb_sync(c));
     *info = k;
-#undef EH_TRY
-    return cleanup(0);
+    return 0;
 }
 
 int lkb_svds(lkb_op_t A, lkb_basis_t U, double* S, lkb_basis_t V, int nsv, double* residuals, int32_t* info,
@@ -609,13 +571,10 @@ int lkb_svds(lkb_op_t A, lkb_basis_t U, double* S, lkb_basis_t V, int nsv, doubl
     const size_t es = kind_size(kind);
     const int kd = kdim > 0 ? kdim : 4 * nsv;
     const double tol = tolerance >= 0 ? tolerance : rtol_of(kind);
-    lkb_basis_t Uw = nullptr, Vw = nullptr;
-    LKB_TRY(lkb_basis_create(c, kind, U->n, U->n_global, U->row0, kd + 1, &Uw));
-    int rc = lkb_basis_create(c, kind, V->n, V->n_global, V->row0, kd + 1, &Vw);
-    if (rc) { lkb_basis_destroy(Uw); return rc; }
-    auto cleanup = [&](int r) { lkb_basis_destroy(Uw); lkb_basis_destroy(Vw); return r; };
-#define SV_TRY(call) do { rc = (call); if (rc) return cleanup(rc); } while (0)
-    SV_TRY(start_vector(Uw, u0));
+    BasisOwner Uw, Vw;
+    LKB_TRY(lkb_basis_create(c, kind, U->n, U->n_global, U->row0, kd + 1, Uw.out()));
+    LKB_TRY(lkb_basis_create(c, kind, V->n, V->n_global, V->row0, kd + 1, Vw.out()));
+    LKB_TRY(start_vector(Uw, u0));
     const int ldb = kd + 1;
     std::vector<char> B((size_t)ldb * kd * es, 0);
     std::vector<double> sv(kd, 0.0), res(kd, 0.0);
@@ -624,10 +583,8 @@ int lkb_svds(lkb_op_t A, lkb_basis_t U, double* S, lkb_basis_t V, int nsv, doubl
     *info = 0;
     int k = 1, conv = 0;
     // speculative step k+1 overlapped with the host gesdd of B_k (svd_solvers.fypp:85-101), as in eigs / eighs
-    StepSlots ss;
-    SV_TRY(ss.init((size_t)ldb * es + 256));
-#undef SV_TRY
-#define SV_TRY(call) do { rc = (call); if (rc) { cudaStreamSynchronize(c->stream); ss.release(); return cleanup(rc); } } while (0)
+    StepSlots ss(c->stream);
+    LKB_TRY(ss.init((size_t)ldb * es + 256));
     auto enqueue_step = [&](int kk) -> int {
         LKB_TRY(bidiag_enqueue(A, Uw, Vw, kk, kk, tol));                    // tol = solver tolerance (svd_solvers.fypp:82)
         LKB_TRY(krylov_fetch_async(c, kind, ldb, kk, kk, ss.slot[kk & 1]));
@@ -637,15 +594,15 @@ int lkb_svds(lkb_op_t A, lkb_basis_t U, double* S, lkb_basis_t V, int nsv, doubl
     int inflight = 0;
     for (k = 1; k <= kd; ++k) {
         int32_t binfo = 0;
-        if (inflight < k) { SV_TRY(enqueue_step(k)); inflight = k; }
-        SV_TRY(cudaEventSynchronize(ss.ev[k & 1]) == cudaSuccess ? 0 : LKB_ERR_CUDA);
-        SV_TRY(bidiag_collect(A, Uw, B.data(), ldb, &binfo, k, k, ss.slot[k & 1]));
-        if (binfo == 0 && k < kd) { SV_TRY(enqueue_step(k + 1)); inflight = k + 1; }      // speculative
+        if (inflight < k) { LKB_TRY(enqueue_step(k)); inflight = k; }
+        LKB_CUDA(cudaEventSynchronize(ss.ev[k & 1]));
+        LKB_TRY(bidiag_collect(A, Uw, B.data(), ldb, &binfo, k, k, ss.slot[k & 1]));
+        if (binfo == 0 && k < kd) { LKB_TRY(enqueue_step(k + 1)); inflight = k + 1; }      // speculative
         std::fill(sv.begin(), sv.end(), 0.0);
         std::fill(umat.begin(), umat.end(), cd(0)); std::fill(vmat.begin(), vmat.end(), cd(0));
         Bk.assign((size_t)k * k, cd(0));
         for (int j = 0; j < k; ++j) for (int i = 0; i < k; ++i) Bk[i + (size_t)k * j] = load_kind(kind, B.data(), (size_t)i + (size_t)ldb * j);
-        SV_TRY(sp ? host_svd_t<float>(cplx, k, Bk, sv.data(), uk, vk) : host_svd_t<double>(cplx, k, Bk, sv.data(), uk, vk));
+        LKB_TRY(sp ? host_svd_t<float>(cplx, k, Bk, sv.data(), uk, vk) : host_svd_t<double>(cplx, k, Bk, sv.data(), uk, vk));
         for (int j = 0; j < k; ++j) for (int i = 0; i < k; ++i) {
             umat[i + (size_t)kd * j] = uk[i + (size_t)k * j];
             vmat[i + (size_t)kd * j] = vk[i + (size_t)k * j];
@@ -653,7 +610,7 @@ int lkb_svds(lkb_op_t A, lkb_basis_t U, double* S, lkb_basis_t V, int nsv, doubl
         const cd beta = load_kind(kind, B.data(), (size_t)k + (size_t)ldb * (k - 1));
         std::fill(res.begin(), res.end(), 0.0);
         for (int i = 0; i < k; ++i) res[i] = std::abs(beta * vmat[(k - 1) + (size_t)kd * i]);
-        SV_TRY(bcast_host(c, res.data(), (size_t)k * sizeof(double)));
+        LKB_TRY(bcast_host(c, res.data(), (size_t)k * sizeof(double)));
         conv = 0; for (int i = 0; i < k; ++i) conv += res[i] < tol;
         if (c->write_intermediate) {                              // write_results_r(svds_output, ...)  (svd_solvers.fypp:100)
             std::vector<double> rr(res.begin(), res.begin() + k); // sorts the residual table in place, see lkb_eigs
@@ -663,13 +620,10 @@ int lkb_svds(lkb_op_t A, lkb_basis_t U, double* S, lkb_basis_t V, int nsv, doubl
         }
         if (conv >= nsv) break;
     }
-    SV_TRY(cudaStreamSynchronize(c->stream) == cudaSuccess ? 0 : LKB_ERR_CUDA);
-    ss.release();
-#undef SV_TRY
-#define SV_TRY(call) do { rc = (call); if (rc) return cleanup(rc); } while (0)
-    SV_TRY(bcast_host(c, sv.data(), sv.size() * sizeof(double)));
-    SV_TRY(bcast_host(c, umat.data(), umat.size() * sizeof(cd)));
-    SV_TRY(bcast_host(c, vmat.data(), vmat.size() * sizeof(cd)));
+    LKB_CUDA(cudaStreamSynchronize(c->stream));
+    LKB_TRY(bcast_host(c, sv.data(), sv.size() * sizeof(double)));
+    LKB_TRY(bcast_host(c, umat.data(), umat.size() * sizeof(cd)));
+    LKB_TRY(bcast_host(c, vmat.data(), vmat.size() * sizeof(cd)));
     for (int i = 0; i < nsv; ++i) { S[i] = sv[i]; residuals[i] = res[i]; }
     k = std::min(k, kd);
     *info = k;
@@ -678,11 +632,10 @@ int lkb_svds(lkb_op_t A, lkb_basis_t U, double* S, lkb_basis_t V, int nsv, doubl
         Yu[j + (size_t)k * i] = umat[j + (size_t)kd * i];
         Yv[j + (size_t)k * i] = vmat[j + (size_t)kd * i];
     }
-    SV_TRY(device_combine(Uw, k, Yu, k, nsv, U->d, U->ld));
-    SV_TRY(device_combine(Vw, k, Yv, k, nsv, V->d, V->ld));
-    SV_TRY(lkb_sync(c));
-#undef SV_TRY
-    return cleanup(0);
+    LKB_TRY(device_combine(Uw, k, Yu, k, nsv, U->d, U->ld));
+    LKB_TRY(device_combine(Vw, k, Yv, k, nsv, V->d, V->ld));
+    LKB_TRY(lkb_sync(c));
+    return 0;
 }
 
 }  // extern "C"

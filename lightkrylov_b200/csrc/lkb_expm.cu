@@ -19,7 +19,6 @@
 #include "lkb_internal.h"
 
 using namespace lkb;
-typedef std::complex<double> cd;
 
 namespace {
 
@@ -84,23 +83,6 @@ bool dense_expm(int n, const std::vector<cd>& Ain, std::vector<cd>& E) {
     return true;
 }
 
-cd load_kind(int kind, const void* H, size_t idx) {
-    switch (kind) {
-        case KS: return cd(((const float*)H)[idx], 0.0);
-        case KD: return cd(((const double*)H)[idx], 0.0);
-        case KC: return cd(((const float*)H)[2 * idx], ((const float*)H)[2 * idx + 1]);
-        default: return cd(((const double*)H)[2 * idx], ((const double*)H)[2 * idx + 1]);
-    }
-}
-void store_kind(int kind, void* H, size_t idx, cd v) {
-    switch (kind) {
-        case KS: ((float*)H)[idx] = (float)v.real(); break;
-        case KD: ((double*)H)[idx] = v.real(); break;
-        case KC: ((float*)H)[2 * idx] = (float)v.real(); ((float*)H)[2 * idx + 1] = (float)v.imag(); break;
-        default: ((double*)H)[2 * idx] = v.real(); ((double*)H)[2 * idx + 1] = v.imag(); break;
-    }
-}
-
 // Fortran edit descriptor E16.9: 0.ddddddddd E+ee right-justified in 16 columns
 std::string fortran_e16_9(double v) {
     char buf[64];
@@ -141,14 +123,11 @@ int lkb_kexpm_vec(lkb_vec_t cvec, lkb_op_t A, lkb_vec_t b, double tau, double to
         *info = 1;
         return 0;
     }
-    lkb_basis_t X = nullptr;
-    LKB_TRY(lkb_basis_create(c, kind, b->n, b->n_global, b->row0, nk + 1, &X));
-    int rc = 0;
-    auto cleanup = [&](int r) { lkb_basis_destroy(X); return r; };
-#define KX_TRY(call) do { rc = (call); if (rc) return cleanup(rc); } while (0)
+    BasisOwner X;
+    LKB_TRY(lkb_basis_create(c, kind, b->n, b->n_global, b->row0, nk + 1, X.out()));
     launch_axpby(kind, c->stream, Scalar{1.0 / beta, 0.0}, b->d, Scalar{0, 0}, X->d, b->n, c->sms);     // X(1) = b / beta
     c->launches++;
-    KX_TRY(check_launch(c, "kexpm start"));
+    LKB_TRY(check_launch(c, "kexpm start"));
     const int ldh = nk + 1;
     std::vector<char> H((size_t)ldh * (nk + 1) * es, 0);          // (nk+1) x (nk+1) as in the reference (:170)
     std::vector<cd> Hk, E;
@@ -157,31 +136,30 @@ int lkb_kexpm_vec(lkb_vec_t cvec, lkb_op_t A, lkb_vec_t b, double tau, double to
     for (int k = 1; k <= nk; ++k) {
         kp = k + 1;
         int32_t ainfo = 0;
-        KX_TRY(lkb_arnoldi(A, X, H.data(), ldh, &ainfo, k, k, -1.0, trans, 1));
+        LKB_TRY(lkb_arnoldi(A, X, H.data(), ldh, &ainfo, k, k, -1.0, trans, 1));
         const bool breakdown = (ainfo == k);
         if (breakdown) kp = k;                                     // do not consider the extended matrix (:199-203)
         Hk.assign((size_t)kp * kp, cd(0));
         for (int j = 0; j < kp; ++j)
             for (int i = 0; i < kp; ++i) Hk[i + (size_t)kp * j] = tau * load_kind(kind, H.data(), (size_t)i + (size_t)ldh * j);
-        if (!dense_expm(kp, Hk, E)) { set_error("kexpm_vec: singular Pade denominator"); return cleanup(LKB_ERR_LAPACK); }
+        if (!dense_expm(kp, Hk, E)) { set_error("kexpm_vec: singular Pade denominator"); return LKB_ERR_LAPACK; }
         // |E(kp,1) beta| (:213).  The reference writes merge(0, abs(E(kp,1)*beta), info == k), but `info` was overwritten with -2
         // three lines earlier when the breakdown was detected (:201), so the estimate is NOT zeroed on breakdown: the loop goes
         // on with the refilled vector and stops two steps later, where E(kp,1) is exactly zero (H(k+1,k) = 0 decouples the
         // blocks).  Reproduced literally: info = k + 2 after a breakdown at step k unless |E(k,1) beta| <= tol already.
         err_est = std::abs(E[(size_t)(kp - 1)] * beta);
-        KX_TRY(bcast_host(c, &err_est, sizeof(double)));
+        LKB_TRY(bcast_host(c, &err_est, sizeof(double)));
         if (err_est <= tol || k == nk) {
             // c = beta * X(:kp) E(:kp,1)   (:209-210; the reference forms it every step, only the last one survives)
             std::vector<char> coef((size_t)kp * es);
-            for (int i = 0; i < kp; ++i) store_kind(kind, coef.data(), (size_t)i, beta * E[(size_t)i]);
-            KX_TRY(lkb_basis_lincomb(X, kp, coef.data(), cvec));
+            for (int i = 0; i < kp; ++i) store_kind(kind, coef.data(), i, beta * E[(size_t)i]);
+            LKB_TRY(lkb_basis_lincomb(X, kp, coef.data(), cvec));
             if (err_est <= tol) break;
         }
     }
-    KX_TRY(lkb_sync(c));
+    LKB_TRY(lkb_sync(c));
     *info = (err_est <= tol) ? kp : -1;
-#undef KX_TRY
-    return cleanup(0);
+    return 0;
 }
 
 // kexpm_mat(C, A, B, tau, tol, info, trans, kdim)       src/Expm/ExpmLib.fypp:234-362
@@ -204,20 +182,17 @@ int lkb_kexpm_mat(lkb_basis_t Cb, lkb_op_t A, lkb_basis_t B, int p, double tau, 
     const int nsteps = kdim > 0 ? kdim : 100;
     const int nk = nsteps * p;
     *info = 0;
-    lkb_basis_t Xwrk = nullptr, X = nullptr;
-    int rc = 0;
-    auto cleanup = [&](int r) { if (X) lkb_basis_destroy(X); if (Xwrk) lkb_basis_destroy(Xwrk); return r; };
-#define KM_TRY(call) do { rc = (call); if (rc) return cleanup(rc); } while (0)
-    KM_TRY(lkb_basis_create(c, kind, B->n, B->n_global, B->row0, p, &Xwrk));
+    BasisOwner Xwrk, X;
+    LKB_TRY(lkb_basis_create(c, kind, B->n, B->n_global, B->row0, p, Xwrk.out()));
     const double one_d[2] = {1.0, 0.0}, zero_d[2] = {0.0, 0.0};
     const float one_f[2] = {1.f, 0.f}, zero_f[2] = {0.f, 0.f};
     const bool sp = (kind == KS || kind == KC);
-    KM_TRY(lkb_basis_axpby(sp ? (const void*)one_f : (const void*)one_d, B, 0, sp ? (const void*)zero_f : (const void*)zero_d, Xwrk, 0, p));
+    LKB_TRY(lkb_basis_axpby(sp ? (const void*)one_f : (const void*)one_d, B, 0, sp ? (const void*)zero_f : (const void*)zero_d, Xwrk, 0, p));
     // B = Q R P^T : pivoting QR, then permcols(R, invperm(perm))   (:295)
     std::vector<char> Rp((size_t)p * p * es, 0);
     std::vector<int32_t> perm(p, 0), invp(p, 0);
     int32_t qinfo = 0;
-    KM_TRY(lkb_qr_pivoting(Xwrk, 0, p, Rp.data(), p, perm.data(), -1.0, &qinfo));
+    LKB_TRY(lkb_qr_pivoting(Xwrk, 0, p, Rp.data(), p, perm.data(), -1.0, &qinfo));
     for (int i = 0; i < p; ++i) invp[perm[i] - 1] = i;
     std::vector<cd> R((size_t)p * p);
     double fro2 = 0.0;
@@ -229,11 +204,11 @@ int lkb_kexpm_mat(lkb_basis_t Cb, lkb_op_t A, lkb_basis_t B, int p, double tau, 
     double err_est = 0.0;
     int kpp = p;
     if (fro2 == 0.0) {                                             // input is zero => output is zero (:297-300)
-        KM_TRY(lkb_basis_zero(Cb, 0, p));
+        LKB_TRY(lkb_basis_zero(Cb, 0, p));
     } else {
         int cap = std::min(nk, 8);                                 // block steps the basis / H currently have room for
-        KM_TRY(lkb_basis_create(c, kind, B->n, B->n_global, B->row0, p * (cap + 1), &X));
-        KM_TRY(lkb_initialize_krylov_subspace(X, Xwrk, 0, p));
+        LKB_TRY(lkb_basis_create(c, kind, B->n, B->n_global, B->row0, p * (cap + 1), X.out()));
+        LKB_TRY(lkb_initialize_krylov_subspace(X, Xwrk, 0, p));
         int ldh = p * (cap + 1);
         std::vector<char> H((size_t)ldh * ldh * es, 0);
         std::vector<cd> Hk, E, M;
@@ -243,12 +218,10 @@ int lkb_kexpm_mat(lkb_basis_t Cb, lkb_op_t A, lkb_basis_t B, int p, double tau, 
         for (int k = 1; k <= nk; ++k) {
             if (k > cap) {                                         // double the room: copy the basis and re-lay H
                 const int cap2 = std::min(nk, 2 * cap), ld2 = p * (cap2 + 1);
-                lkb_basis_t X2 = nullptr;
-                KM_TRY(lkb_basis_create(c, kind, B->n, B->n_global, B->row0, p * (cap2 + 1), &X2));
-                rc = lkb_basis_axpby(one, X, 0, zero, X2, 0, p * (cap + 1));
-                if (rc) { lkb_basis_destroy(X2); return cleanup(rc); }
-                lkb_basis_destroy(X);
-                X = X2;
+                BasisOwner X2;
+                LKB_TRY(lkb_basis_create(c, kind, B->n, B->n_global, B->row0, p * (cap2 + 1), X2.out()));
+                LKB_TRY(lkb_basis_axpby(one, X, 0, zero, X2, 0, p * (cap + 1)));
+                std::swap(X, X2);                                  // the old basis goes with X2
                 std::vector<char> H2((size_t)ld2 * ld2 * es, 0);
                 for (int j = 0; j < ldh; ++j) memcpy(&H2[(size_t)j * ld2 * es], &H[(size_t)j * ldh * es], (size_t)ldh * es);
                 H.swap(H2);
@@ -257,12 +230,12 @@ int lkb_kexpm_mat(lkb_basis_t Cb, lkb_op_t A, lkb_basis_t B, int p, double tau, 
             const int kp = k * p;
             kpp = kp + p;
             int32_t ainfo = 0;
-            KM_TRY(lkb_arnoldi(A, X, H.data(), ldh, &ainfo, k, k, -1.0, trans, p));
+            LKB_TRY(lkb_arnoldi(A, X, H.data(), ldh, &ainfo, k, k, -1.0, trans, p));
             if (ainfo == kp) kpp = kp;                             // breakdown: do not consider the extended matrix (:314-318)
             Hk.assign((size_t)kpp * kpp, cd(0));
             for (int j = 0; j < kpp; ++j)
                 for (int i = 0; i < kpp; ++i) Hk[i + (size_t)kpp * j] = tau * load_kind(kind, H.data(), (size_t)i + (size_t)ldh * j);
-            if (!dense_expm(kpp, Hk, E)) { set_error("kexpm_mat: singular Pade denominator"); return cleanup(LKB_ERR_LAPACK); }
+            if (!dense_expm(kpp, Hk, E)) { set_error("kexpm_mat: singular Pade denominator"); return LKB_ERR_LAPACK; }
             // M = E(:kpp, :p) R ; err_est = || M(kp+1:kpp, :) ||_F   (:338-346; the section is empty after a breakdown)
             M.assign((size_t)kpp * p, cd(0));
             for (int q = 0; q < p; ++q)
@@ -274,25 +247,22 @@ int lkb_kexpm_mat(lkb_basis_t Cb, lkb_op_t A, lkb_basis_t B, int p, double tau, 
             double e2 = 0.0;
             for (int q = 0; q < p; ++q) for (int i = kp; i < kpp; ++i) e2 += std::norm(M[i + (size_t)kpp * q]);
             err_est = sqrt(e2);
-            KM_TRY(bcast_host(c, &err_est, sizeof(double)));
+            LKB_TRY(bcast_host(c, &err_est, sizeof(double)));
             if (err_est <= tol || k == nk) {
                 coef.resize((size_t)kpp * es);
                 for (int q = 0; q < p; ++q) {
-                    for (int i = 0; i < kpp; ++i) store_kind(kind, coef.data(), (size_t)i, M[i + (size_t)kpp * q]);
-                    lkb_vec_t cq = nullptr;
-                    KM_TRY(lkb_basis_col(Cb, q, &cq));
-                    rc = lkb_basis_lincomb(X, kpp, coef.data(), cq);
-                    lkb_vec_destroy(cq);
-                    if (rc) return cleanup(rc);
+                    for (int i = 0; i < kpp; ++i) store_kind(kind, coef.data(), i, M[i + (size_t)kpp * q]);
+                    VecOwner cq;
+                    LKB_TRY(lkb_basis_col(Cb, q, cq.out()));
+                    LKB_TRY(lkb_basis_lincomb(X, kpp, coef.data(), cq));
                 }
                 if (err_est <= tol) break;
             }
         }
     }
-    KM_TRY(lkb_sync(c));
+    LKB_TRY(lkb_sync(c));
     *info = (err_est <= tol) ? kpp : -1;
-#undef KM_TRY
-    return cleanup(0);
+    return 0;
 }
 
 // krylov_exptA(vec_out, A, vec_in, tau, info, trans)    src/Expm/ExpmLib.fypp:364-392: the wrapper that conforms to the

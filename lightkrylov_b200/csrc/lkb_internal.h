@@ -2,10 +2,14 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <complex>
+#include <functional>
 #include <map>
 #include <string>
 #include <tuple>
+#include <utility>
 #include <vector>
+#include "../../include/lkb.h"
 #include "lkb_kernels.h"
 
 namespace lkb {
@@ -32,6 +36,8 @@ struct NcclApi {
 NcclApi* nccl_api();   // nullptr (+ error set) when libnccl cannot be loaded
 
 enum ProfClass { PC_MATVEC = 0, PC_DOT = 1, PC_AXPY = 2, PC_OTHER = 3, PC_FUSED = 4, PC_COUNT = 8 };
+// lkb_op_s::type.  The values are printed by lkb_op_jacobi_create's error message.
+enum OpType { OP_DENSE = 0, OP_STENCIL = 1, OP_CSR = 3, OP_DIAG = 4, OP_CALLBACK = 9 };
 
 }  // namespace lkb
 
@@ -84,7 +90,7 @@ struct lkb_basis_s {
     bool owns = true;          // false: lkb_basis_view of a column range of another basis
 };
 struct lkb_op_s {
-    lkb_ctx_s* ctx; int type; int kind;           // type: 0 dense, 1 stencil, 3 csr, 4 diagonal, 9 callback
+    lkb_ctx_s* ctx; int type; int kind;           // type: lkb::OpType
     int64_t m, n;                                 // local rows of the output / input vectors
     int64_t n_matvec = 0, n_rmatvec = 0;
     // stencil
@@ -163,4 +169,67 @@ int lanczos_enqueue(lkb_op_s* A, lkb_basis_s* X, int kstart, int kend, double to
 int lanczos_collect(lkb_op_s* A, lkb_basis_s* X, void* T, int ldt, int32_t* info, int kstart, int kend, const void* pinned_host);
 int bidiag_enqueue(lkb_op_s* A, lkb_basis_s* U, lkb_basis_s* V, int kstart, int kend, double tol);
 int bidiag_collect(lkb_op_s* A, lkb_basis_s* U, void* B, int ldb, int32_t* info, int kstart, int kend, const void* pinned_host);
+// a callback operator may be captured into a CUDA graph only when its creator declared it capturable
+inline bool op_capturable(const lkb_op_s* A) { return A->type != OP_CALLBACK || A->capturable; }
+
+// One element of a host array of `kind` as a complex double, and back (the single precisions round on the way in)
+typedef std::complex<double> cd;
+inline cd load_kind(int kind, const void* base, size_t idx) {
+    switch (kind) {
+        case KS: return cd(((const float*)base)[idx], 0.0);
+        case KD: return cd(((const double*)base)[idx], 0.0);
+        case KC: return cd(((const float*)base)[2 * idx], ((const float*)base)[2 * idx + 1]);
+        default: return cd(((const double*)base)[2 * idx], ((const double*)base)[2 * idx + 1]);
+    }
+}
+inline void store_kind(int kind, void* base, size_t idx, cd v) {
+    switch (kind) {
+        case KS: ((float*)base)[idx] = (float)v.real(); break;
+        case KD: ((double*)base)[idx] = v.real(); break;
+        case KC: ((float*)base)[2 * idx] = (float)v.real(); ((float*)base)[2 * idx + 1] = (float)v.imag(); break;
+        default: ((double*)base)[2 * idx] = v.real(); ((double*)base)[2 * idx + 1] = v.imag(); break;
+    }
+}
+inline Scalar to_scalar(cd v) { return Scalar{v.real(), v.imag()}; }
+
+// ---- scope owners of a solver's work space: every return path releases it, in reverse order of declaration ----
+// (The host-shell test mocks replace lkb_basis_destroy, lkb_vec_destroy and dev_free; an owner whose release calls the CUDA
+// runtime directly is defined in its .cu file.)
+template <class T, int (*Destroy)(T)> class Owner {
+  public:
+    Owner() = default;
+    Owner(Owner&& o) noexcept : p_(o.p_) { o.p_ = nullptr; }
+    Owner& operator=(Owner&& o) noexcept { std::swap(p_, o.p_); return *this; }
+    Owner(const Owner&) = delete;
+    Owner& operator=(const Owner&) = delete;
+    ~Owner() { if (p_) Destroy(p_); }
+    T* out() { return &p_; }                   // for the create call that fills an empty owner
+    operator T() const { return p_; }
+    T operator->() const { return p_; }
+  private:
+    T p_ = nullptr;
+};
+typedef Owner<lkb_basis_t, lkb_basis_destroy> BasisOwner;
+typedef Owner<lkb_vec_t, lkb_vec_destroy> VecOwner;
+// a dev_alloc buffer
+struct DevBuf {
+    lkb_ctx_s* c; void* p = nullptr;
+    explicit DevBuf(lkb_ctx_s* ctx) : c(ctx) {}
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    ~DevBuf() { dev_free(c, p); }
+    int alloc(size_t bytes) { return dev_alloc(c, &p, bytes); }
+};
+// an instantiated CUDA graph and the kernel launches one replay stands for (destructor in lkb_krylov.cu)
+struct GraphExec {
+    cudaGraphExec_t exec = nullptr;
+    int64_t launches = 0;
+    GraphExec() = default;
+    GraphExec(const GraphExec&) = delete;
+    GraphExec& operator=(const GraphExec&) = delete;
+    ~GraphExec();
+};
+// Run `body` (which only enqueues work on c->stream) under stream capture with c->capturing set, and instantiate the graph.
+// The launches the body counted go to *launches, not to c->launches.  `what` prefixes the error messages ("gmres: ").
+int capture_graph(lkb_ctx_s* c, const char* what, const std::function<int()>& body, cudaGraphExec_t* exec, int64_t* launches);
 }  // namespace lkb

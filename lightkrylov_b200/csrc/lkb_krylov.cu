@@ -9,7 +9,6 @@
 // kstart..kend factorisation is a single graph launch with one host sync at the end.
 #include <stdio.h>
 #include <string.h>
-#include <functional>
 #include <vector>
 #include "../../include/lkb.h"
 #include "lkb_internal.h"
@@ -102,25 +101,32 @@ int step_tail_enqueue(lkb_ctx_s* c, int kind, const void* V, int64_t ld, int j, 
     return check_launch(c, "step tail");
 }
 
+GraphExec::~GraphExec() { if (exec) cudaGraphExecDestroy(exec); }
+
+int capture_graph(lkb_ctx_s* c, const char* what, const std::function<int()>& body, cudaGraphExec_t* exec, int64_t* launches) {
+    const int64_t l0 = c->launches;
+    cudaError_t e = cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal);
+    if (e != cudaSuccess) { set_error("%sgraph capture failed: %s", what, cudaGetErrorString(e)); return LKB_ERR_CUDA; }
+    c->capturing = true;
+    int r = body();
+    c->capturing = false;
+    cudaGraph_t g = nullptr;
+    e = cudaStreamEndCapture(c->stream, &g);
+    *launches = c->launches - l0;
+    c->launches = l0;
+    if (r == 0 && e != cudaSuccess) { set_error("%sgraph capture failed: %s", what, cudaGetErrorString(e)); r = LKB_ERR_CUDA; }
+    if (r == 0 && cudaGraphInstantiate(exec, g, 0) != cudaSuccess) { set_error("%sgraph instantiate failed", what); r = LKB_ERR_CUDA; }
+    if (g) cudaGraphDestroy(g);
+    return r;
+}
+
 // Run `body` (which only enqueues work on c->stream) either directly or through a cached CUDA graph.
 static int run_maybe_graph(lkb_ctx_s* c, bool allow_graph, const std::string& key, const std::function<int()>& body) {
     if (!(c->graphs && allow_graph) || c->profile) return body();
     auto it = c->graph_cache.find(key);
     if (it == c->graph_cache.end()) {
-        const int64_t l0 = c->launches;
-        LKB_CUDA(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
-        c->capturing = true;
-        int r = body();
-        c->capturing = false;
-        cudaGraph_t g = nullptr;
-        cudaError_t e = cudaStreamEndCapture(c->stream, &g);
-        if (r != 0) { if (g) cudaGraphDestroy(g); return r; }
-        if (e != cudaSuccess) { set_error("graph capture failed: %s", cudaGetErrorString(e)); return LKB_ERR_CUDA; }
-        cudaGraphExec_t exec = nullptr;
-        LKB_CUDA(cudaGraphInstantiate(&exec, g, 0));
-        cudaGraphDestroy(g);
-        lkb_ctx_s::GraphEntry ent{exec, c->launches - l0};
-        c->launches = l0;
+        lkb_ctx_s::GraphEntry ent{nullptr, 0};
+        LKB_TRY(capture_graph(c, "", body, &ent.exec, &ent.launches));
         if (c->graph_cache.size() > 4096) {   // bound the cache
             for (auto& kv : c->graph_cache) cudaGraphExecDestroy(kv.second.exec);
             c->graph_cache.clear();
@@ -131,8 +137,6 @@ static int run_maybe_graph(lkb_ctx_s* c, bool allow_graph, const std::string& ke
     c->launches += it->second.launches;
     return 0;
 }
-
-static bool op_capturable(const lkb_op_s* A) { return A->type != 9 || A->capturable; }
 
 static std::string make_key(const char* tag, const lkb_op_s* A, const lkb_basis_s* X, const lkb_basis_s* Y,
                             int kstart, int kend, double tol, int trans) {
@@ -181,24 +185,6 @@ static int fetch_coeffs(lkb_ctx_s* c, int kind, int j, bool two, std::vector<Sca
     if (flags) memcpy(flags, tail + 16, F_COUNT * sizeof(int));
     return 0;
 }
-static void scalar_store(int kind, Scalar s, void* p) {
-    switch (kind) {
-        case KS: *(float*)p = (float)s.re; break;
-        case KD: *(double*)p = s.re; break;
-        case KC: ((float*)p)[0] = (float)s.re; ((float*)p)[1] = (float)s.im; break;
-        default: ((double*)p)[0] = s.re; ((double*)p)[1] = s.im; break;
-    }
-}
-static Scalar scalar_load(int kind, const void* p) {
-    Scalar s{0, 0};
-    switch (kind) {
-        case KS: s.re = *(const float*)p; break;
-        case KD: s.re = *(const double*)p; break;
-        case KC: s.re = ((const float*)p)[0]; s.im = ((const float*)p)[1]; break;
-        default: s.re = ((const double*)p)[0]; s.im = ((const double*)p)[1]; break;
-    }
-    return s;
-}
 // upload host coefficients (kind elements, length len) as W type into c->coefd, scaled by sgn
 static int upload_coef(lkb_ctx_s* c, int kind, const void* coef, int len, double sgn) {
     const size_t wsz = kind_cplx(kind) ? 16 : 8;
@@ -206,9 +192,9 @@ static int upload_coef(lkb_ctx_s* c, int kind, const void* coef, int len, double
     LKB_TRY(ensure_coefd(c, std::max((size_t)len * 16, (size_t)4096)));
     LKB_CUDA(cudaStreamSynchronize(c->stream));   // hstage may still be in flight
     for (int i = 0; i < len; ++i) {
-        Scalar s = scalar_load(kind, (const char*)coef + (size_t)i * kind_size(kind));
+        const cd s = load_kind(kind, coef, i);
         double* d = (double*)((char*)c->hstage + (size_t)i * wsz);
-        d[0] = sgn * s.re; if (kind_cplx(kind)) d[1] = sgn * s.im;
+        d[0] = sgn * s.real(); if (kind_cplx(kind)) d[1] = sgn * s.imag();
     }
     LKB_CUDA(cudaMemcpyAsync(c->coefd, c->hstage, (size_t)len * wsz, cudaMemcpyHostToDevice, c->stream));
     return 0;
@@ -260,7 +246,7 @@ int lkb_basis_innerprod(lkb_basis_t X, int j, lkb_basis_t W, int wcol0, int p, v
         LKB_TRY(allreduce_w(c, c->c1, (size_t)(j + 1) * (kind_cplx(X->kind) ? 2 : 1)));
         LKB_TRY(fetch_coeffs(c, X->kind, j, false, col, nullptr, nullptr));
         for (int i = 0; i < j; ++i)
-            scalar_store(X->kind, col[i], (char*)out + ((size_t)i + (size_t)ldout * q) * kind_size(X->kind));
+            store_kind(X->kind, out, (size_t)i + (size_t)ldout * q, cd(col[i].re, col[i].im));
     }
     return 0;
 }
@@ -326,7 +312,7 @@ static int gs_common(lkb_basis_t X, int j, lkb_basis_t W, int wcol0, int p, int3
         if (hf[F_GSINFO]) *info = q + 1;
         if (beta)
             for (int i = 0; i < j; ++i)
-                scalar_store(X->kind, col[i], (char*)beta + ((size_t)i + (size_t)ldbeta * q) * kind_size(X->kind));
+                store_kind(X->kind, beta, (size_t)i + (size_t)ldbeta * q, cd(col[i].re, col[i].im));
     }
     return 0;
 }
@@ -358,7 +344,7 @@ int lkb_qr(lkb_basis_t Q, int col0, int p, void* R, int ldr, double tol, int32_t
         LKB_TRY(fetch_coeffs(c, kind, j, true, col, &nrm2, hf));
         if (j > 0) {
             *info = hf[F_GSINFO] ? 1 : 0;
-            for (int i = 0; i < j; ++i) scalar_store(kind, col[i], (char*)R + ((size_t)i + (size_t)ldr * j) * es);
+            for (int i = 0; i < j; ++i) store_kind(kind, R, (size_t)i + (size_t)ldr * j, cd(col[i].re, col[i].im));
         }
         double beta = sqrt(fabs(nrm2));
         if (beta != beta) { set_error("|beta| = NaN detected! Abort"); return LKB_ERR_NAN; }
@@ -372,8 +358,7 @@ int lkb_qr(lkb_basis_t Q, int col0, int p, void* R, int ldr, double tol, int32_t
             if (j > 0) *info = hf[F_GSINFO] ? 1 : 0;
             beta = sqrt(fabs(nrm2));
         } else {
-            Scalar b{beta, 0};
-            scalar_store(kind, b, (char*)R + ((size_t)j + (size_t)ldr * j) * es);
+            store_kind(kind, R, (size_t)j + (size_t)ldr * j, beta);
         }
         launch_scal(kind, c->stream, Scalar{1.0 / beta, 0.0}, q, Q->n, c->sms);
         c->launches++;
@@ -406,7 +391,7 @@ int lkb_qr_pivoting(lkb_basis_t Q, int col0, int p, void* R, int ldr, int32_t* p
         LKB_TRY(vec_dot_sync(c, kind, qcol(i), qcol(i), Q->n, &Rii[i]));
         Rii[i] = round_kind(Rii[i]);
     }
-    struct Tmp { lkb_ctx_s* c; void* d; ~Tmp() { if (d) dev_free(c, d); } } tmp{c, nullptr};
+    DevBuf tmp(c);
     // Q(i) <- rand ; double_gram_schmidt_step(Q(i), Q(:i-1)) ; returns the step's info and the norm afterwards
     auto refill = [&](int i, int32_t* ginfo, double* beta) -> int {
         launch_fill(kind, c->stream, qcol(i), Q->n, Q->row0, LKB_DIST_NORMAL, next_seed(c), c->sms);
@@ -436,11 +421,11 @@ int lkb_qr_pivoting(lkb_basis_t Q, int col0, int p, void* R, int ldr, int32_t* p
         // swap_columns(Q, R, Rii, perm, j, idx)
         if (idx != j) {
             const size_t bytes = (size_t)Q->n * es;
-            if (!tmp.d && bytes) LKB_TRY(dev_alloc(c, &tmp.d, bytes));
+            if (!tmp.p && bytes) LKB_TRY(tmp.alloc(bytes));
             if (bytes) {
-                LKB_CUDA(cudaMemcpyAsync(tmp.d, qcol(j), bytes, cudaMemcpyDeviceToDevice, c->stream));
+                LKB_CUDA(cudaMemcpyAsync(tmp.p, qcol(j), bytes, cudaMemcpyDeviceToDevice, c->stream));
                 LKB_CUDA(cudaMemcpyAsync(qcol(j), qcol(idx), bytes, cudaMemcpyDeviceToDevice, c->stream));
-                LKB_CUDA(cudaMemcpyAsync(qcol(idx), tmp.d, bytes, cudaMemcpyDeviceToDevice, c->stream));
+                LKB_CUDA(cudaMemcpyAsync(qcol(idx), tmp.p, bytes, cudaMemcpyDeviceToDevice, c->stream));
             }
             std::swap(Rii[j], Rii[idx]);
             std::swap(perm[j], perm[idx]);
@@ -455,7 +440,7 @@ int lkb_qr_pivoting(lkb_basis_t Q, int col0, int p, void* R, int ldr, int32_t* p
             LKB_TRY(refill(j, &g, &beta));
             *info = g;                                                      // `info = j` is overwritten by the DGS call
         } else {
-            scalar_store(kind, Scalar{beta, 0.0}, Rat(j, j));
+            store_kind(kind, R, (size_t)j + (size_t)ldr * j, beta);
         }
         launch_scal(kind, c->stream, Scalar{1.0 / beta, 0.0}, qcol(j), Q->n, c->sms);
         c->launches++;
@@ -465,7 +450,7 @@ int lkb_qr_pivoting(lkb_basis_t Q, int col0, int p, void* R, int ldr, int32_t* p
             b = round_kind(b);
             launch_axpby(kind, c->stream, Scalar{-b.re, -b.im}, qcol(j), Scalar{1.0, 0.0}, qcol(i), Q->n, c->sms);
             c->launches++;
-            scalar_store(kind, b, Rat(j, i));
+            store_kind(kind, R, (size_t)j + (size_t)ldr * i, cd(b.re, b.im));
             Rii[i] = round_kind(Scalar{Rii[i].re - (b.re * b.re - b.im * b.im), Rii[i].im - 2.0 * b.re * b.im});
         }
         LKB_TRY(check_launch(c, "qr_pivoting"));
@@ -649,15 +634,14 @@ static int arnoldi_block(lkb_op_t A, lkb_basis_t X, void* H, int ldh, int32_t* i
                     for (int r = 0; r < kp; ++r) {
                         const double* a = (const double*)(hs + ((size_t)q * jp + r) * wsz);
                         const double* b = (const double*)(hs + (2 * (size_t)jp + (size_t)q * jp + r) * wsz);
-                        Scalar v{a[0] + b[0], kind_cplx(kind) ? a[1] + b[1] : 0.0};
-                        scalar_store(kind, v, (char*)H + ((size_t)r + (size_t)ldh * (kpm + i + q)) * es);
+                        store_kind(kind, H, (size_t)r + (size_t)ldh * (kpm + i + q), cd(a[0] + b[0], kind_cplx(kind) ? a[1] + b[1] : 0.0));
                     }
                 continue;
             }
             LKB_TRY(dgs_enqueue(c, kind, X->d, X->ld, kp, col_ptr(X, kp + i), X->n, c->flags, false, true));
             LKB_TRY(fetch_coeffs(c, kind, kp, true, col, nullptr, hf));
             for (int r = 0; r < kp; ++r)
-                scalar_store(kind, col[r], (char*)H + ((size_t)r + (size_t)ldh * (kpm + i)) * es);
+                store_kind(kind, H, (size_t)r + (size_t)ldh * (kpm + i), cd(col[r].re, col[r].im));
         }
         int32_t qinfo = 0;
         LKB_TRY(lkb_qr(X, kp, p, R.data(), p, -1.0, &qinfo));

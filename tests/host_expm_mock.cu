@@ -58,10 +58,12 @@ int lkb_basis_axpby(const void* alpha, lkb_basis_t X, int xcol0, const void* bet
 }
 int lkb_basis_col(lkb_basis_t b, int i0, lkb_vec_t* view) {
     if (!b || i0 < 0 || i0 >= b->ncols) return LKB_ERR_ARG;
+    if (alloc_fails()) return LKB_ERR_ALLOC;
     *view = new lkb_vec_s{b->ctx, b->kind, b->n, b->n_global, b->row0, col_ptr(b, i0), false};
+    g_live[LIVE_VECS]++;
     return 0;
 }
-int lkb_vec_destroy(lkb_vec_t v) { if (!v) return LKB_ERR_ARG; if (v->owns) free(v->d); delete v; return 0; }
+int lkb_vec_destroy(lkb_vec_t v) { if (!v) return LKB_ERR_ARG; if (v->owns) free(v->d); delete v; g_live[LIVE_VECS]--; return 0; }
 int lkb_vec_zero(lkb_vec_t v) { memset(v->d, 0, (size_t)v->n * kind_size(v->kind)); return 0; }
 // y = X(:, :j) coef
 int lkb_basis_lincomb(lkb_basis_t X, int j, const void* coef, lkb_vec_t y) {

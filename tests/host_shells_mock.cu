@@ -19,13 +19,14 @@
 #include "lkb_internal.h"
 
 // ---- CUDA runtime calls made directly by lkb_eig.cu -> host ----------------------------------------------------------------
-static cudaError_t mock_malloc_host(void** p, size_t n) { *p = calloc(1, n ? n : 1); return *p ? cudaSuccess : cudaErrorMemoryAllocation; }
+cudaError_t mock_malloc_host(void** p, size_t n);      // (host_mock_common.inc: counted, can be made to fail)
+cudaError_t mock_free_host(void* p);
 static cudaError_t mock_memcpy2d(void* dst, size_t dpitch, const void* src, size_t spitch, size_t width, size_t height) {
     for (size_t r = 0; r < height; ++r) memcpy((char*)dst + r * dpitch, (const char*)src + r * spitch, width);
     return cudaSuccess;
 }
 #define cudaMallocHost(p, n) mock_malloc_host((void**)(p), (n))
-#define cudaFreeHost(p) (free(p), cudaSuccess)
+#define cudaFreeHost(p) mock_free_host(p)
 #define cudaEventCreateWithFlags(e, f) (*(e) = (cudaEvent_t)(uintptr_t)1, cudaSuccess)
 #define cudaEventDestroy(e) ((void)(e), cudaSuccess)
 #define cudaEventRecord(e, s) ((void)(e), (void)(s), cudaSuccess)
@@ -37,6 +38,14 @@ static cudaError_t mock_memcpy2d(void* dst, size_t dpitch, const void* src, size
 #include "lkb_eig.cu"        // the product's host shells, verbatim
 
 #include "host_mock_common.inc"
+
+cudaError_t mock_malloc_host(void** p, size_t n) {
+    *p = alloc_fails() ? nullptr : calloc(1, n ? n : 1);
+    if (!*p) return cudaErrorMemoryAllocation;
+    g_live[LIVE_PINNED]++;
+    return cudaSuccess;
+}
+cudaError_t mock_free_host(void* p) { free(p); g_live[LIVE_PINNED]--; return cudaSuccess; }
 
 namespace {
 std::vector<char> g_col;          // the H / T / B column of the step enqueued last (one step is in flight at a time)

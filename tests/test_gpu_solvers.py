@@ -347,3 +347,54 @@ def test_write_intermediate_sorts_the_residual_table(lk, ctx, oracle, tmp_path):
     assert len(lines) == info1 + 1 and lines[0].split() == ["Iter", "value", "residual", "conv"]
     glines = open(tmp_path / "eigs_output.txt").read().splitlines()
     assert glines[0].split() == ["Iter", "Re", "Im", "modulus", "residual", "conv"] and len(glines) >= 2
+
+
+def _solve_with_failing_callback(lk, ctx, case, fail_at):
+    """One small solve whose user callback returns 5 on its `fail_at`-th call (0: never): a host preconditioner (identity) for
+    the *_precond cases, a capturable callback operator that applies the 2-D Laplacian for the *_device cases."""
+    import ctypes as C
+    nx, ny = 48, 40
+    n = nx * ny
+    S = lk.LinOp.stencil5(ctx, "d", nx, ny, (4.0, -1.0, -1.0, -1.0, -1.0))
+    calls = [0]
+
+    def result():
+        calls[0] += 1
+        return 5 if calls[0] == fail_at else 0
+
+    def wrap(ptr):
+        h = C.c_void_p()
+        assert ctx.lib.lkb_vec_wrap(ctx.h, lk.KINDS["d"], n, n, 0, ptr, C.byref(h)) == 0
+        return lk.Vector(ctx, "d", n, _handle=h)
+
+    def matvec(xp, yp, trans, stream):
+        S.matvec(wrap(xp), wrap(yp))
+        return result()
+    solver, path = case.split("_")
+    A, pre = (S, lambda v, nloc, it, cur, tgt, stream: result()) if path == "precond" else \
+             (lk.LinOp.callback(ctx, "d", n, n, matvec, capturable=True), None)
+    b = lk.Vector(ctx, "d", n).put(np.random.default_rng(40).standard_normal(n))
+    x = lk.Vector(ctx, "d", n)
+    kw = dict(maxiter=300) if solver == "cg" else dict(kdim=20, maxiter=20)
+    info, meta = getattr(lk, solver)(A, b, x, preconditioner=pre, **kw)
+    return info, meta["res"], x.get()
+
+
+@pytest.mark.parametrize("graphs", [True, False])
+def test_failing_callback_releases_the_solver_and_leaves_the_context_usable(lk, ctx, graphs):
+    """A host preconditioner that fails on its 3rd call (gmres, fgmres, cg) and a capturable callback operator that fails on its
+    2nd call (the device GMRES cycle and the device CG loop: inside the graph capture when graphs are on): each solve raises
+    LkbError naming the callback, and a clean solve on the same context afterwards is bitwise equal to one on a fresh context."""
+    fresh = lk.Context(0)
+    try:
+        for c in (ctx, fresh):
+            c.set_graphs(graphs)
+        for case, fail_at in [("gmres_precond", 3), ("fgmres_precond", 3), ("cg_precond", 3), ("gmres_device", 2), ("cg_device", 2)]:
+            with pytest.raises(lk.LkbError, match="callback returned 5"):
+                _solve_with_failing_callback(lk, ctx, case, fail_at)
+            info, res, x = _solve_with_failing_callback(lk, ctx, case, 0)
+            info0, res0, x0 = _solve_with_failing_callback(lk, fresh, case, 0)
+            assert info == info0 != 0 and res == res0 and np.array_equal(x, x0), case
+    finally:
+        ctx.set_graphs(True)
+        fresh.close()

@@ -32,6 +32,39 @@ def oracle():
     return lk_oracle
 
 
+def _declare_alloc_hooks(lib):
+    lib.mock_fail_at.argtypes = [C.c_int64]
+    lib.mock_allocs.restype = C.c_int64
+    lib.mock_live.argtypes = [C.c_void_p]
+
+
+def _live(lib):
+    out = (C.c_int64 * 4)()                                      # bases, vectors, pinned blocks, device buffers
+    lib.mock_live(out)
+    return list(out)
+
+
+LKB_ERR_ALLOC = -6
+
+
+def _fail_each_allocation(lib, call):
+    """`call()` runs one solver and returns its code.  Counts the N allocations a successful call makes, then fails the n-th one
+    for every n = 1..N: the call must return LKB_ERR_ALLOC and leave no basis, vector, pinned block or device buffer behind."""
+    lib.mock_fail_at(0)
+    before = _live(lib)
+    assert call() == 0, lib.mock_last_error()
+    nalloc = lib.mock_allocs()
+    assert nalloc > 0 and _live(lib) == before
+    try:
+        for n in range(1, nalloc + 1):
+            lib.mock_fail_at(n)
+            rc = call()
+            assert (rc, _live(lib)) == (LKB_ERR_ALLOC, before), (n, nalloc)
+    finally:
+        lib.mock_fail_at(0)
+    return nalloc
+
+
 @pytest.fixture(scope="module")
 def mock(tmp_path_factory, oracle):
     import scipy
@@ -61,6 +94,7 @@ def mock(tmp_path_factory, oracle):
     lib.lkb_eighs.argtypes = [vp, vp, C.c_int, vp, vp, C.POINTER(i32), vp, i32, dbl]
     lib.lkb_svds.argtypes = [vp, vp, vp, vp, C.c_int, vp, C.POINTER(i32), vp, i32, dbl]
     lib.lkb_krylov_schur.argtypes = [vp, vp, C.c_int, C.c_int, C.POINTER(i32)]
+    _declare_alloc_hooks(lib)
     blas = glob.glob(os.path.join(os.path.dirname(os.path.dirname(scipy.__file__)), "scipy.libs", "libscipy_openblas*.so"))[0]
     assert lib.lkb_set_lapack(blas.encode(), b"scipy_", b"_") == 0, lib.mock_last_error()
     return lib
@@ -320,6 +354,7 @@ def expm_mock(tmp_path_factory, oracle):
     lib.lkb_kexpm_vec.argtypes = [vp, vp, vp, dbl, dbl, C.POINTER(i32), i32, i32]
     lib.lkb_kexpm_mat.argtypes = [vp, vp, vp, C.c_int, dbl, dbl, C.POINTER(i32), i32, i32]
     lib.lkb_krylov_expta.argtypes = [vp, vp, vp, dbl, C.POINTER(i32), i32]
+    _declare_alloc_hooks(lib)
     dts = {0: np.float32, 1: np.float64, 2: np.complex64, 3: np.complex128}
 
     def qr_pivoting(kind, n, p, Qp, ld, Rp, ldr, permp, tol, infop):          # lkb_qr_pivoting -> oracle.qr_with_pivoting, in place
@@ -429,6 +464,61 @@ def test_kexpm_mat_shell_matches_oracle_shell(expm_mock, oracle, kind, p):
         assert binfo == 4 == oracle.kexpm_mat(oracle.Op.dense(D), Bh, 0.2, 1e-12)[1]
         assert np.linalg.norm(Cb - exact) < 1e-12 * np.linalg.norm(exact)
     sh.close()
+
+
+def test_eig_shells_release_everything_when_an_allocation_fails(mock, oracle):
+    """eigs (with Krylov-Schur restarts: a device buffer per restart), eighs and svds: every allocation, work bases and pinned
+    step slots included, may fail; each failure is reported as LKB_ERR_ALLOC with nothing left allocated.  A clean call afterwards
+    still matches the oracle."""
+    i32 = C.c_int32
+    nev = 8
+    Ah = _toeplitz(N, -0.5, 1.0, 0.5, np.float64)
+    x0 = randn(np.random.default_rng(21), N, np.float64)
+    sh = Shells(mock, "d")
+    A = sh.op(oracle.Op.dense(Ah)); X = sh.basis(N, nev); v0 = sh.vec(x0)
+    ev, res, info = np.zeros(2 * nev), np.zeros(nev), i32()
+    n_eigs = _fail_each_allocation(mock, lambda: mock.lkb_eigs(A, X, nev, ev.ctypes.data, res.ctypes.data, C.byref(info), v0,
+                                                               4 * nev, -1.0, 0))
+    assert n_eigs > 4                                                          # Xwrk, two pinned slots, restarts
+    D = np.diag(np.concatenate([np.linspace(0, 1, N - 4), [2.0, 2.5, 3.0, 4.0]]))
+    Ahs = np.asfortranarray(D)
+    As = sh.op(oracle.Op.dense(Ahs)); Xs = sh.basis(N, 4)
+    evs, ress = np.zeros(4), np.zeros(4)
+    assert _fail_each_allocation(mock, lambda: mock.lkb_eighs(As, Xs, 4, evs.ctypes.data, ress.ctypes.data, C.byref(info), v0,
+                                                              40, -1.0)) == 3
+    m, n, nsv = 90, 70, 3
+    M = np.asfortranarray(randn(np.random.default_rng(26), (m, n), np.float64)); u0 = sh.vec(randn(np.random.default_rng(27), m, np.float64))
+    Am = sh.op(oracle.Op.dense(M)); U = sh.basis(m, nsv); V = sh.basis(n, nsv)
+    S, sres = np.zeros(nsv), np.zeros(nsv)
+    assert _fail_each_allocation(mock, lambda: mock.lkb_svds(Am, U, S.ctypes.data, V, nsv, sres.ctypes.data, C.byref(info), u0,
+                                                             30, -1.0)) == 4
+    ev1, _, X1, info1 = sh.eigs(A, N, nev, x0, kdim=4 * nev)
+    sh.close()
+    evo, _, Xo, infoo = oracle.eigs(oracle.Op.dense(Ah), N, nev, x0, kdim=4 * nev)
+    assert info1 == infoo and np.abs(ev1 - evo).max() < _tol("d") * np.abs(evo).max()
+    assert _aligned(X1, Xo, ev1, "d") < 1e-8
+
+
+def test_expm_shells_release_everything_when_an_allocation_fails(expm_mock, oracle):
+    """kexpm_vec and kexpm_mat (p = 3, through the growth of the work basis and the per-column views of C): each allocation fails
+    in turn with LKB_ERR_ALLOC and nothing left allocated; a clean call afterwards still matches the oracle."""
+    n, p, tol = 480, 3, 1e-10
+    Ao = oracle.Op.stencil("d", (24, 20), (-4.0, 1.0, 0.8, 1.0, 1.2))
+    b = oracle.fill(n, "d", "uniform", 3)
+    B = np.asfortranarray(np.stack([oracle.fill(n, "d", "uniform", 5 + i) for i in range(p)], axis=1))
+    sh = ExpmShells(expm_mock, "d")
+    A = sh.op(Ao); cv = sh.vec(np.zeros(n)); bv = sh.vec(b); hB = sh.basis(n, p, B); hC = sh.basis(n, p)
+    info = C.c_int32()
+    assert _fail_each_allocation(expm_mock, lambda: expm_mock.lkb_kexpm_vec(cv, A, bv, 0.1, tol, C.byref(info), 0, 0)) == 1
+    n_mat = _fail_each_allocation(expm_mock, lambda: expm_mock.lkb_kexpm_mat(hC, A, hB, p, 0.1, tol, C.byref(info), 0, 15))
+    c, cinfo = sh.kexpm(A, b, 0.1, tol)
+    Cm, minfo = sh.kexpm_mat(A, B, 0.1, tol, kdim=15)
+    assert minfo // p - 1 > 8 and n_mat == 3 + p                               # Xwrk, X, the doubled X, one view per column
+    sh.close()
+    co, coinfo = oracle.kexpm_vec(Ao, b, 0.1, tol)
+    Co, moinfo = oracle.kexpm_mat(Ao, B, 0.1, tol, kdim=15)
+    assert cinfo == coinfo and np.linalg.norm(c - co) < 1e-12 * np.linalg.norm(co)
+    assert minfo == moinfo and np.linalg.norm(Cm - Co) < 1e-11 * np.linalg.norm(Co)
 
 
 # ------------------------------------------------------------------------------------------------------------------------------
