@@ -6,6 +6,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <algorithm>
+#include <memory>
 #include "../../include/lkb.h"
 #include "lkb_internal.h"
 
@@ -35,6 +36,10 @@ NcclApi* nccl_api() {
 #undef LKB_SYM
     g_nccl.handle = h;
     return &g_nccl;
+}
+int comm_destroy(void* comm) {
+    NcclApi* api = nccl_api();
+    return api ? api->CommDestroy(comm) : LKB_ERR_NCCL;
 }
 #define LKB_NCCL(call) do { int r_ = (call); if (r_ != 0) { \
     lkb::set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #call, nccl_api()->GetErrorString(r_)); return LKB_ERR_NCCL; } } while (0)
@@ -73,52 +78,49 @@ int prof_collect(lkb_ctx_s* c) {
 // Captured graphs hold raw pointers into the context workspaces and into bases / operators: whenever
 // one of those allocations goes away the cached executables that may reference it are dropped.
 void invalidate_graphs(lkb_ctx_s* c, uint64_t uid) {
-    if (uid == 0) {
-        for (auto& kv : c->graph_cache) cudaGraphExecDestroy(kv.second.exec);
-        c->graph_cache.clear();
-        return;
-    }
+    if (uid == 0) { c->graph_cache.clear(); return; }
     char tag[40]; snprintf(tag, sizeof(tag), ":%llu:", (unsigned long long)uid);
     for (auto it = c->graph_cache.begin(); it != c->graph_cache.end();) {
-        if (it->first.find(tag) != std::string::npos) { cudaGraphExecDestroy(it->second.exec); it = c->graph_cache.erase(it); }
+        if (it->first.find(tag) != std::string::npos) it = c->graph_cache.erase(it);
         else ++it;
     }
 }
-static int grow(lkb_ctx_s* c, void** p, size_t* cur, size_t need) {
+static int grow(lkb_ctx_s* c, CudaPtr<void>& p, size_t* cur, size_t need) {
     if (*cur >= need) return 0;
     cudaStreamSynchronize(c->stream);
     invalidate_graphs(c, 0);
-    if (*p) cudaFree(*p);
-    *p = nullptr; *cur = 0;
-    LKB_CUDA(cudaMalloc(p, need));
+    p.reset(); *cur = 0;
+    LKB_TRY(cuda_alloc(p, need));
     *cur = need;
     return 0;
 }
 int ensure_ws(lkb_ctx_s* c, int jp) {
     if (c->capturing) return 0;   // sized before capture begins
     const size_t need = (size_t)MAX_ROWBLOCKS * (size_t)jp * 16;
-    LKB_TRY(grow(c, &c->partial, &c->partial_bytes, std::max(need, (size_t)MAX_ROWBLOCKS * 16 * 8)));
+    LKB_TRY(grow(c, c->partial, &c->partial_bytes, std::max(need, (size_t)MAX_ROWBLOCKS * 16 * 8)));
     if (c->cbuf_len < (size_t)jp) {
         size_t len = std::max((size_t)jp, (size_t)272);
         cudaStreamSynchronize(c->stream);
         invalidate_graphs(c, 0);
-        if (c->c1) cudaFree(c->c1); if (c->c2) cudaFree(c->c2); if (c->tmpw) cudaFree(c->tmpw);
-        c->c1 = c->c2 = c->tmpw = nullptr; c->cbuf_len = 0;
-        LKB_CUDA(cudaMalloc(&c->c1, len * 16)); LKB_CUDA(cudaMalloc(&c->c2, len * 16)); LKB_CUDA(cudaMalloc(&c->tmpw, len * 16));
+        c->c1.reset(); c->c2.reset(); c->tmpw.reset(); c->cbuf_len = 0;
+        LKB_TRY(cuda_alloc(c->c1, len * 16)); LKB_TRY(cuda_alloc(c->c2, len * 16)); LKB_TRY(cuda_alloc(c->tmpw, len * 16));
         c->cbuf_len = len;
     }
     return 0;
 }
 int ensure_hstage(lkb_ctx_s* c, size_t bytes) {
     if (c->hstage_bytes >= bytes) return 0;
-    if (c->hstage) cudaFreeHost(c->hstage);
-    c->hstage = nullptr; c->hstage_bytes = 0;
-    LKB_CUDA(cudaMallocHost(&c->hstage, bytes));
-    c->hstage_bytes = bytes;
+    c->hstage = nullptr; c->hstage_mem.reset(); c->hstage_bytes = 0;
+    LKB_TRY(cuda_alloc(c->hstage_mem, bytes));
+    c->hstage = c->hstage_mem; c->hstage_bytes = bytes;
     return 0;
 }
-int ensure_Hd(lkb_ctx_s* c, size_t bytes) { return grow(c, &c->Hd, &c->Hd_bytes, bytes); }
-int ensure_coefd(lkb_ctx_s* c, size_t bytes) { return grow(c, &c->coefd, &c->coefd_bytes, bytes); }
+int ensure_Hd(lkb_ctx_s* c, size_t bytes) { return grow(c, c->Hd, &c->Hd_bytes, bytes); }
+int ensure_coefd(lkb_ctx_s* c, size_t bytes) {
+    const int r = grow(c, c->coefd_mem, &c->coefd_bytes, bytes);
+    c->coefd = c->coefd_mem;
+    return r;
+}
 
 int allreduce_w(lkb_ctx_s* c, void* buf, size_t ndoubles) {
     if (c->world == 1 || c->p2p_active) return 0;      // p2p: already reduced inside the producing kernel
@@ -215,45 +217,7 @@ extern "C" {
 
 const char* lkb_last_error(void) { return g_err; }
 
-static int ctx_common(int device, lkb_ctx_s* c) {
-    int ndev = 0;
-    cudaError_t e = cudaGetDeviceCount(&ndev);
-    if (e != cudaSuccess || ndev == 0) {
-        set_error("no CUDA device available (%s): liblkb has no CPU fallback", cudaGetErrorString(e));
-        return LKB_ERR_CUDA;
-    }
-    LKB_CUDA(cudaSetDevice(device));
-    c->dev = device;
-    LKB_CUDA(cudaDeviceGetAttribute(&c->sms, cudaDevAttrMultiProcessorCount, device));
-    LKB_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
-    {   // keep freed blocks in the default pool (see dev_alloc)
-        cudaMemPool_t pool = nullptr;
-        if (cudaDeviceGetDefaultMemPool(&pool, device) == cudaSuccess && pool) {
-            unsigned long long thr = ~0ULL;
-            cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &thr);
-        }
-        cudaGetLastError();
-    }
-    LKB_CUDA(cudaMalloc(&c->nrm2, 64));
-    LKB_CUDA(cudaMalloc((void**)&c->inv, 64));
-    LKB_CUDA(cudaMalloc((void**)&c->flags, F_COUNT * sizeof(int)));
-    LKB_CUDA(cudaMalloc((void**)&c->counter, 1024));      // global ticket + one per group of the reduction tree
-    LKB_CUDA(cudaMemset(c->flags, 0, F_COUNT * sizeof(int)));
-    LKB_CUDA(cudaMemset(c->counter, 0, 1024));
-    LKB_CUDA(cudaMemset(c->nrm2, 0, 64));
-    LKB_TRY(ensure_ws(c, 272));
-    LKB_TRY(ensure_hstage(c, 1 << 20));
-    return 0;
-}
-
-int lkb_init(int device, lkb_ctx_t* ctx) {
-    if (!ctx) return LKB_ERR_ARG;
-    lkb_ctx_s* c = new lkb_ctx_s();
-    int r = ctx_common(device, c);
-    if (r) { delete c; return r; }
-    *ctx = c;
-    return 0;
-}
+int lkb_init(int device, lkb_ctx_t* ctx) { return lkb_init_dist(device, 0, 1, nullptr, ctx); }
 int lkb_nccl_unique_id(void* id128) {
     NcclApi* api = nccl_api();
     if (!api) return LKB_ERR_NCCL;
@@ -262,40 +226,54 @@ int lkb_nccl_unique_id(void* id128) {
 }
 int lkb_init_dist(int device, int rank, int world, const void* id128, lkb_ctx_t* ctx) {
     if (!ctx || world < 1 || rank < 0 || rank >= world) return LKB_ERR_ARG;
-    lkb_ctx_s* c = new lkb_ctx_s();
-    int r = ctx_common(device, c);
-    if (r) { delete c; return r; }
-    c->rank = rank; c->world = world;
+    int ndev = 0;
+    cudaError_t e = cudaGetDeviceCount(&ndev);
+    if (e != cudaSuccess || ndev == 0) {
+        set_error("no CUDA device available (%s): liblkb has no CPU fallback", cudaGetErrorString(e));
+        return LKB_ERR_CUDA;
+    }
+    LKB_CUDA(cudaSetDevice(device));
+    std::unique_ptr<lkb_ctx_s> c(new lkb_ctx_s());      // a failure below releases what was built so far
+    c->dev = device; c->rank = rank; c->world = world;
+    LKB_CUDA(cudaDeviceGetAttribute(&c->sms, cudaDevAttrMultiProcessorCount, device));
+    LKB_CUDA(cudaStreamCreateWithFlags(c->stream.out(), cudaStreamNonBlocking));
+    {   // keep freed blocks in the default pool (see dev_alloc)
+        cudaMemPool_t pool = nullptr;
+        if (cudaDeviceGetDefaultMemPool(&pool, device) == cudaSuccess && pool) {
+            unsigned long long thr = ~0ULL;
+            cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &thr);
+        }
+        cudaGetLastError();
+    }
+    LKB_TRY(cuda_alloc(c->nrm2, 64));
+    LKB_TRY(cuda_alloc(c->inv, 64));
+    LKB_TRY(cuda_alloc(c->flags, F_COUNT * sizeof(int)));
+    LKB_TRY(cuda_alloc(c->counter, 1024));      // global ticket + one per group of the reduction tree
+    LKB_CUDA(cudaMemset(c->flags, 0, F_COUNT * sizeof(int)));
+    LKB_CUDA(cudaMemset(c->counter, 0, 1024));
+    LKB_CUDA(cudaMemset(c->nrm2, 0, 64));
+    LKB_TRY(ensure_ws(c.get(), 272));
+    LKB_TRY(ensure_hstage(c.get(), 1 << 20));
     if (world > 1) {
         NcclApi* api = nccl_api();
-        if (!api) { delete c; return LKB_ERR_NCCL; }
+        if (!api) return LKB_ERR_NCCL;
         NcclId id; memcpy(&id, id128, sizeof(id));
-        LKB_NCCL(api->CommInitRank(&c->comm, world, id, rank));
+        LKB_NCCL(api->CommInitRank(c->comm.out(), world, id, rank));
     }
-    *ctx = c;
+    *ctx = c.release();
     return 0;
 }
 int lkb_finalize(lkb_ctx_t c) {
     if (!c) return LKB_ERR_ARG;
-    cudaSetDevice(c->dev);
+    const int dev = c->dev;
+    cudaSetDevice(dev);
     cudaStreamSynchronize(c->stream);
-    for (auto& kv : c->graph_cache) cudaGraphExecDestroy(kv.second.exec);
-    if (c->comm && nccl_api()) nccl_api()->CommDestroy(c->comm);
-    for (int r = 0; r < c->p2p.world; ++r) if (r != c->rank && c->p2p.peer[r]) cudaIpcCloseMemHandle(c->p2p.peer[r]);
-    if (c->p2p_region) cudaFree(c->p2p_region);
-    if (c->p2p.epoch) cudaFree(c->p2p.epoch);
-    if (c->p2p.dbg) cudaFree(c->p2p.dbg);
-    void* bufs[] = { c->partial, c->c1, c->c2, c->tmpw, c->nrm2, c->inv, c->flags, c->counter, c->Hd, c->coefd };
-    for (void* b : bufs) if (b) cudaFree(b);
-    if (c->hstage) cudaFreeHost(c->hstage);
-    cudaStreamSynchronize(c->stream);
+    delete c;
     {
         cudaMemPool_t pool = nullptr;
-        if (cudaDeviceGetDefaultMemPool(&pool, c->dev) == cudaSuccess && pool) cudaMemPoolTrimTo(pool, 0);
+        if (cudaDeviceGetDefaultMemPool(&pool, dev) == cudaSuccess && pool) cudaMemPoolTrimTo(pool, 0);
         cudaGetLastError();
     }
-    cudaStreamDestroy(c->stream);
-    delete c;
     return 0;
 }
 int lkb_sync(lkb_ctx_t c) { LKB_CUDA(cudaStreamSynchronize(c->stream)); return 0; }
@@ -323,9 +301,10 @@ int lkb_p2p_export(lkb_ctx_t c, void* handle64) {
     if (!c || !handle64) return LKB_ERR_ARG;
     cudaSetDevice(c->dev);
     if (!c->p2p_region) {
-        LKB_CUDA(cudaMalloc(&c->p2p_region, p2p_region_bytes()));
+        LKB_TRY(cuda_alloc(c->p2p_region, p2p_region_bytes()));
         LKB_CUDA(cudaMemset(c->p2p_region, 0, p2p_region_bytes()));
-        LKB_CUDA(cudaMalloc((void**)&c->p2p.epoch, 64));
+        LKB_TRY(cuda_alloc(c->p2p_epoch, 64));
+        c->p2p.epoch = c->p2p_epoch;
         LKB_CUDA(cudaMemset(c->p2p.epoch, 0, 64));
         LKB_CUDA(cudaDeviceSynchronize());
     }
@@ -341,12 +320,11 @@ int lkb_p2p_attach(lkb_ctx_t c, const void* handles) {
     cudaSetDevice(c->dev);
     c->p2p.world = c->world; c->p2p.rank = c->rank;
     for (int r = 0; r < c->world; ++r) {
-        if (r == c->rank) { c->p2p.peer[r] = (char*)c->p2p_region; continue; }
+        if (r == c->rank) { c->p2p.peer[r] = (char*)c->p2p_region.get(); continue; }
         cudaIpcMemHandle_t h; memcpy(&h, (const char*)handles + 64 * (size_t)r, 64);
-        void* ptr = nullptr;
-        cudaError_t e = cudaIpcOpenMemHandle(&ptr, h, cudaIpcMemLazyEnablePeerAccess);
+        cudaError_t e = cudaIpcOpenMemHandle(c->peer_map[r].out(), h, cudaIpcMemLazyEnablePeerAccess);
         if (e != cudaSuccess) { set_error("cudaIpcOpenMemHandle(rank %d) failed: %s", r, cudaGetErrorString(e)); cudaGetLastError(); return LKB_ERR_CUDA; }
-        c->p2p.peer[r] = (char*)ptr;
+        c->p2p.peer[r] = (char*)c->peer_map[r].get();
     }
     c->p2p_active = true;
     return 0;
@@ -372,10 +350,11 @@ int lkb_debug_ktime(lkb_ctx_t c, int enable) {
     cudaStreamSynchronize(c->stream);
     invalidate_graphs(c, 0);
     if (enable) {
-        if (!c->p2p.dbg) LKB_CUDA(cudaMalloc((void**)&c->p2p.dbg, KT_WORDS * sizeof(unsigned long long)));
+        if (!c->ktime) LKB_TRY(cuda_alloc(c->ktime, KT_WORDS * sizeof(unsigned long long)));
+        c->p2p.dbg = c->ktime;
         LKB_CUDA(cudaMemset(c->p2p.dbg, 0, KT_WORDS * sizeof(unsigned long long)));
-    } else if (!enable && c->p2p.dbg) {
-        cudaFree(c->p2p.dbg); c->p2p.dbg = nullptr;
+    } else {
+        c->ktime.reset(); c->p2p.dbg = nullptr;
     }
     return 0;
 }
@@ -569,7 +548,7 @@ static int stencil_create(lkb_ctx_t c, int kind, int dim, int64_t nx, int64_t ny
     const int64_t nslow = dim == 2 ? ny : nz;
     if (slow0 < 0 || nslow_local < 1 || slow0 + nslow_local > nslow) { set_error("stencil: bad slab [%lld,+%lld) of %lld", (long long)slow0, (long long)nslow_local, (long long)nslow); return LKB_ERR_ARG; }
     cudaSetDevice(c->dev);
-    lkb_op_s* op = new lkb_op_s();
+    OpOwner op(new lkb_op_s());
     op->ctx = c; op->type = OP_STENCIL; op->kind = kind; op->uid = next_uid();
     op->st.dim = dim; op->st.nx = nx;
     op->st.ny = dim == 2 ? nslow_local : ny;
@@ -582,11 +561,9 @@ static int stencil_create(lkb_ctx_t c, int kind, int dim, int64_t nx, int64_t ny
     op->halo_elems = dim == 2 ? nx : nx * ny;
     op->st.halo_lo = op->st.halo_hi = nullptr;
     if (c->world > 1) {
-        if (cudaMalloc(&op->halo_lo, op->halo_elems * es) != cudaSuccess || cudaMalloc(&op->halo_hi, op->halo_elems * es) != cudaSuccess) {
-            // (NCCL-halo fallback buffers; a failure here is local, but nothing collective has been issued yet)
-            set_error("stencil: cudaMalloc of the halo buffers failed"); cudaGetLastError();
-            lkb_op_destroy(op); return LKB_ERR_ALLOC;
-        }
+        // (NCCL-halo fallback buffers; a failure here is local, but nothing collective has been issued yet)
+        LKB_TRY(cuda_alloc(op->halo_lo, op->halo_elems * es));
+        LKB_TRY(cuda_alloc(op->halo_hi, op->halo_elems * es));
         if (slow0 > 0) op->st.halo_lo = op->halo_lo;
         if (slow0 + nslow_local < nslow) op->st.halo_hi = op->halo_hi;
         if (c->p2p_active) {
@@ -595,33 +572,33 @@ static int stencil_create(lkb_ctx_t c, int kind, int dim, int64_t nx, int64_t ny
             NcclApi* api = nccl_api();
             const size_t side = (((size_t)op->halo_elems * es) + 255) & ~(size_t)255;
             const size_t region = 256 + 4 * side;
-            void* reg = nullptr; void* hbuf = nullptr; unsigned* ctr = nullptr;
-            bool ok = api && cudaMalloc(&reg, region) == cudaSuccess && cudaMemset(reg, 0, region) == cudaSuccess &&
-                      cudaMalloc(&hbuf, 64 * (size_t)(c->world + 1)) == cudaSuccess &&
-                      cudaMalloc((void**)&ctr, 128) == cudaSuccess && cudaMemset(ctr, 0, 128) == cudaSuccess;
+            CudaPtr<void> reg, hbuf; CudaPtr<unsigned> ctr; IpcMap lo_map, hi_map;     // installed in op only when every rank succeeded
+            bool ok = api && cuda_alloc(reg, region) == 0 && cudaMemset(reg, 0, region) == cudaSuccess &&
+                      cuda_alloc(hbuf, 64 * (size_t)(c->world + 1)) == 0 &&
+                      cuda_alloc(ctr, 128) == 0 && cudaMemset(ctr, 0, 128) == cudaSuccess;
             std::vector<char> all(64 * (size_t)c->world);
             if (ok) {
                 cudaIpcMemHandle_t hnd;
                 ok = cudaIpcGetMemHandle(&hnd, reg) == cudaSuccess &&
-                     cudaMemcpy((char*)hbuf + 64 * (size_t)c->world, &hnd, 64, cudaMemcpyHostToDevice) == cudaSuccess;
+                     cudaMemcpy((char*)hbuf.get() + 64 * (size_t)c->world, &hnd, 64, cudaMemcpyHostToDevice) == cudaSuccess;
             }
             // the all-gather is issued unconditionally so that the ranks stay in step even if one failed locally
             int okflag = ok ? 1 : 0;
             if (api && hbuf) {
-                if (api->AllGather((char*)hbuf + 64 * (size_t)c->world, hbuf, 64, /*ncclInt8*/ 0, c->comm, c->stream) != 0) okflag = 0;
+                if (api->AllGather((char*)hbuf.get() + 64 * (size_t)c->world, hbuf, 64, /*ncclInt8*/ 0, c->comm, c->stream) != 0) okflag = 0;
                 if (cudaMemcpyAsync(all.data(), hbuf, all.size(), cudaMemcpyDeviceToHost, c->stream) != cudaSuccess) okflag = 0;
                 if (cudaStreamSynchronize(c->stream) != cudaSuccess) okflag = 0;
             } else okflag = 0;
             const bool has_lo = slow0 > 0, has_hi = slow0 + nslow_local < nslow;
             if (okflag && has_lo) {
                 cudaIpcMemHandle_t hnd; memcpy(&hnd, &all[64 * (size_t)(c->rank - 1)], 64);
-                if (cudaIpcOpenMemHandle(&op->hp_lo_map, hnd, cudaIpcMemLazyEnablePeerAccess) != cudaSuccess) { okflag = 0; cudaGetLastError(); }
+                if (cudaIpcOpenMemHandle(lo_map.out(), hnd, cudaIpcMemLazyEnablePeerAccess) != cudaSuccess) { okflag = 0; cudaGetLastError(); }
             }
             if (okflag && has_hi) {
                 cudaIpcMemHandle_t hnd; memcpy(&hnd, &all[64 * (size_t)(c->rank + 1)], 64);
-                if (cudaIpcOpenMemHandle(&op->hp_hi_map, hnd, cudaIpcMemLazyEnablePeerAccess) != cudaSuccess) { okflag = 0; cudaGetLastError(); }
+                if (cudaIpcOpenMemHandle(hi_map.out(), hnd, cudaIpcMemLazyEnablePeerAccess) != cudaSuccess) { okflag = 0; cudaGetLastError(); }
             }
-            if (hbuf) cudaFree(hbuf);
+            hbuf.reset();
             // every rank must take the same path: agree through one more (tiny) all-reduce-like exchange
             if (ensure_ws(c, 2) != 0) okflag = 0;     // (never return before the agreement step: the ranks would desynchronise)
             {
@@ -633,28 +610,23 @@ static int stencil_create(lkb_ctx_t c, int kind, int dim, int64_t nx, int64_t ny
                 if (v != 0.0) okflag = 0;
             }
             if (okflag) {
-                op->hp.my_region = (char*)reg; op->hp.lo_region = (char*)op->hp_lo_map; op->hp.hi_region = (char*)op->hp_hi_map;
-                op->hp.epoch = ctr; op->hp.ticket = ctr + 16; op->hp.he = op->halo_elems;
+                op->hp.my_region = (char*)reg.get(); op->hp.lo_region = (char*)lo_map.get(); op->hp.hi_region = (char*)hi_map.get();
+                op->hp.epoch = ctr; op->hp.ticket = ctr.get() + 16; op->hp.he = op->halo_elems;
                 op->hp.data_off = 256; op->hp.side_bytes = side;
                 op->hp_active = true;
-                if (has_lo) op->st.halo_lo = (char*)reg + 256;              // parity 0, side 0
-                if (has_hi) op->st.halo_hi = (char*)reg + 256 + side;       // parity 0, side 1
+                if (has_lo) op->st.halo_lo = (char*)reg.get() + 256;              // parity 0, side 0
+                if (has_hi) op->st.halo_hi = (char*)reg.get() + 256 + side;       // parity 0, side 1
                 op->st.halo_epoch = ctr;
                 op->st.halo_parity_stride = (int64_t)(2 * side / es);
-                op->st.flag_lo = (const unsigned*)reg;                      // "lower neighbour pushed epoch e"
-                op->st.flag_hi = (const unsigned*)((char*)reg + 128);       // "upper neighbour pushed epoch e"
-            } else {
-                if (op->hp_lo_map) cudaIpcCloseMemHandle(op->hp_lo_map);
-                if (op->hp_hi_map) cudaIpcCloseMemHandle(op->hp_hi_map);
-                op->hp_lo_map = op->hp_hi_map = nullptr;
-                if (reg) cudaFree(reg);
-                if (ctr) cudaFree(ctr);
+                op->st.flag_lo = (const unsigned*)reg.get();                      // "lower neighbour pushed epoch e"
+                op->st.flag_hi = (const unsigned*)((char*)reg.get() + 128);       // "upper neighbour pushed epoch e"
+                op->hp_region = std::move(reg); op->hp_ctr = std::move(ctr); op->hp_lo_map = std::move(lo_map); op->hp_hi_map = std::move(hi_map);
             }
         }
     }
     const int64_t gy = ((op->st.ny + 7) / 8) * op->st.nz * (nx / 128 + 1);     // upper bound on the 1-D grid of the stencil kernels
-    if (gy > 2147483647LL) { lkb_op_destroy(op); set_error("stencil: grid too large for this kernel (%lld CTAs)", (long long)gy); return LKB_ERR_ARG; }
-    *A = op;
+    if (gy > 2147483647LL) { set_error("stencil: grid too large for this kernel (%lld CTAs)", (long long)gy); return LKB_ERR_ARG; }
+    *A = op.release();
     return 0;
 }
 int lkb_op_stencil5_create(lkb_ctx_t c, int kind, int64_t nx, int64_t ny, const void* coef5, int64_t slow0,
@@ -682,38 +654,32 @@ static int csr_dist_finish(lkb_ctx_t c, lkb_op_s* op, int kind, int64_t n_global
     } else {
         NcclApi* api = nccl_api();
         if (!api) return LKB_ERR_NCCL;
-        void* dbuf = nullptr;
         const int64_t mine[4] = {col0, n_local, row0, m_local};
         std::vector<int64_t> all(4 * (size_t)W);
-        bool ok = cudaMalloc(&dbuf, 32 * (size_t)(W + 1)) == cudaSuccess &&
-                  cudaMemcpy((char*)dbuf + 32 * (size_t)W, mine, 32, cudaMemcpyHostToDevice) == cudaSuccess &&
-                  api->AllGather((char*)dbuf + 32 * (size_t)W, dbuf, 32, /*ncclInt8*/ 0, c->comm, c->stream) == 0 &&
+        CudaPtr<char> dbuf;
+        LKB_TRY(cuda_alloc(dbuf, 32 * (size_t)(W + 1)));
+        bool ok = cudaMemcpy(dbuf.get() + 32 * (size_t)W, mine, 32, cudaMemcpyHostToDevice) == cudaSuccess &&
+                  api->AllGather(dbuf.get() + 32 * (size_t)W, dbuf, 32, /*ncclInt8*/ 0, c->comm, c->stream) == 0 &&
                   cudaMemcpyAsync(all.data(), dbuf, 32 * (size_t)W, cudaMemcpyDeviceToHost, c->stream) == cudaSuccess &&
                   cudaStreamSynchronize(c->stream) == cudaSuccess;
-        if (dbuf) cudaFree(dbuf);
         if (!ok) { set_error("csr_create_dist: slab exchange failed"); return LKB_ERR_NCCL; }
         for (int q = 0; q < W; ++q) { op->col_off[q] = all[4 * q]; op->col_cnt[q] = all[4 * q + 1]; op->row_off[q] = all[4 * q + 2]; op->row_cnt[q] = all[4 * q + 3]; }
     }
-    if (cudaMalloc(&op->x_full, std::max<size_t>((size_t)n_global * es, 16)) != cudaSuccess ||
-        cudaMalloc(&op->y_full, std::max<size_t>((size_t)n_global * es, 16)) != cudaSuccess ||
-        cudaMalloc(&op->y_red, std::max<size_t>((size_t)n_local * es, 16)) != cudaSuccess) {
-        set_error("csr_create_dist: cudaMalloc of the gather / reduce buffers failed"); cudaGetLastError();
-        return LKB_ERR_ALLOC;
-    }
-    return 0;
+    LKB_TRY(cuda_alloc(op->x_full, std::max<size_t>((size_t)n_global * es, 16)));
+    LKB_TRY(cuda_alloc(op->y_full, std::max<size_t>((size_t)n_global * es, 16)));
+    return cuda_alloc(op->y_red, std::max<size_t>((size_t)n_local * es, 16));
 }
 int lkb_op_csr_create_dist(lkb_ctx_t c, int kind, int64_t m_global, int64_t n_global, int64_t row0, int64_t m_local,
                            int64_t col0, int64_t n_local, const int64_t* rowptr_local, const int32_t* col_global,
                            const void* val, lkb_op_t* A) {
     if (!c || !A || !rowptr_local || m_local < 0 || n_local < 0 || m_global < 1 || n_global < 1) return LKB_ERR_ARG;
     cudaSetDevice(c->dev);
-    lkb_op_s* op = new lkb_op_s();
+    OpOwner op(new lkb_op_s());
     op->ctx = c; op->type = OP_CSR; op->kind = kind; op->m = m_local; op->n = n_local; op->uid = next_uid();
     op->dist = true; op->m_global = m_global; op->n_global = n_global;
-    int r = csr_build(c, op, kind, m_local, n_global, rowptr_local, col_global, val);
-    if (r == 0) r = csr_dist_finish(c, op, kind, n_global, row0, m_local, col0, n_local);
-    if (r) { lkb_op_destroy(op); return r; }
-    *A = op;
+    LKB_TRY(csr_dist_finish(c, op, kind, n_global, row0, m_local, col0, n_local));
+    LKB_TRY(csr_build(c, op, kind, m_local, n_global, rowptr_local, col_global, val));
+    *A = op.release();
     return 0;
 }
 // The same from local CSR arrays that already live on this GPU (e.g. lkb_csr_random_device); adopt as in lkb_op_csr_create_device.
@@ -724,29 +690,28 @@ int lkb_op_csr_create_dist_device(lkb_ctx_t c, int kind, int64_t m_global, int64
         { set_error("csr_create_dist_device: bad arguments"); return LKB_ERR_ARG; }
     if (!adopt) { set_error("csr_create_dist_device: only adopt != 0 is supported"); return LKB_ERR_ARG; }
     cudaSetDevice(c->dev);
-    lkb_op_s* op = new lkb_op_s();
+    OpOwner op(new lkb_op_s());
     op->ctx = c; op->type = OP_CSR; op->kind = kind; op->m = m_local; op->n = n_local; op->uid = next_uid();
     op->dist = true; op->m_global = m_global; op->n_global = n_global;
-    op->rowptr = rowptr_dev; op->col = col_dev; op->val = val_dev;
-    int r = csr_finish_device(c, op, kind, m_local, n_global);
-    if (r == 0) r = csr_dist_finish(c, op, kind, n_global, row0, m_local, col0, n_local);
-    if (r) {
-        op->rowptr = nullptr; op->col = nullptr; op->val = nullptr;      // the caller keeps ownership on failure
-        lkb_op_destroy(op);
+    // the slab exchange comes first: once csr_finish_device has succeeded, the adopted arrays may have been released
+    LKB_TRY(csr_dist_finish(c, op, kind, n_global, row0, m_local, col0, n_local));
+    op->rowptr.reset(rowptr_dev); op->col.reset(col_dev); op->val.reset(val_dev);
+    if (int r = csr_finish_device(c, op, kind, m_local, n_global)) {
+        op->rowptr.release(); op->col.release(); op->val.release();      // the caller keeps ownership on failure
         return r;
     }
-    *A = op;
+    *A = op.release();
     return 0;
 }
 int lkb_op_dense_create(lkb_ctx_t c, int kind, int64_t m, int64_t n, const void* a, lkb_op_t* A) {
     if (!c || !A || !a || m < 1 || n < 1) return LKB_ERR_ARG;
     if (c->world > 1) { set_error("dense operators are single-rank (plumbing config only)"); return LKB_ERR_ARG; }
     cudaSetDevice(c->dev);
-    lkb_op_s* op = new lkb_op_s();
+    OpOwner op(new lkb_op_s());
     op->ctx = c; op->type = OP_DENSE; op->kind = kind; op->m = m; op->n = n; op->uid = next_uid();
-    LKB_CUDA(cudaMalloc(&op->a, (size_t)m * n * kind_size(kind)));
+    LKB_TRY(cuda_alloc(op->a, (size_t)m * n * kind_size(kind)));
     LKB_CUDA(cudaMemcpy(op->a, a, (size_t)m * n * kind_size(kind), cudaMemcpyHostToDevice));
-    *A = op;
+    *A = op.release();
     return 0;
 }
 int lkb_op_callback_create(lkb_ctx_t c, int kind, int64_t m_local, int64_t n_local, lkb_matvec_fn fn, void* user,
@@ -760,29 +725,24 @@ int lkb_op_callback_create(lkb_ctx_t c, int kind, int64_t m_local, int64_t n_loc
 }
 // Diagonal operator M = diag(d), e.g. the inverse mass matrix of a spectral-element code.  Row-local, so it has
 // the layout of d and needs no communication at N > 1.  Its values are copied: d may be released afterwards.
-static int diag_from_device(lkb_ctx_t c, int kind, int64_t n, int64_t row0, int64_t n_global, lkb_op_s** M) {
+static int diag_from_device(lkb_ctx_t c, int kind, int64_t n, int64_t row0, int64_t n_global, OpOwner& op) {
     cudaSetDevice(c->dev);
-    lkb_op_s* op = new lkb_op_s();
+    op.reset(new lkb_op_s());
     op->ctx = c; op->type = OP_DIAG; op->kind = kind; op->m = op->n = n; op->uid = next_uid();
     op->diag_row0 = row0; op->diag_n_global = n_global;
-    if (cudaMalloc(&op->diag, std::max<size_t>((size_t)n * kind_size(kind), 16)) != cudaSuccess) {
-        cudaGetLastError(); op->diag = nullptr; delete op;
-        set_error("diag: cudaMalloc of %lld entries failed", (long long)n); return LKB_ERR_ALLOC;
-    }
-    *M = op;
-    return 0;
+    return cuda_alloc(op->diag, std::max<size_t>((size_t)n * kind_size(kind), 16));
 }
 int lkb_op_diag_create(lkb_vec_t d, lkb_op_t* M) {
     if (!d || !M) { set_error("diag_create: null argument"); return LKB_ERR_ARG; }
     lkb_ctx_s* c = d->ctx;
-    lkb_op_s* op = nullptr;
-    LKB_TRY(diag_from_device(c, d->kind, d->n, d->row0, d->n_global, &op));
+    OpOwner op;
+    LKB_TRY(diag_from_device(c, d->kind, d->n, d->row0, d->n_global, op));
     if (cudaMemcpyAsync(op->diag, d->d, (size_t)d->n * kind_size(d->kind), cudaMemcpyDeviceToDevice, c->stream) != cudaSuccess ||
         cudaStreamSynchronize(c->stream) != cudaSuccess) {
         set_error("diag_create: copy of d failed: %s", cudaGetErrorString(cudaGetLastError()));
-        lkb_op_destroy(op); return LKB_ERR_CUDA;
+        return LKB_ERR_CUDA;
     }
-    *M = op;
+    *M = op.release();
     return 0;
 }
 // Jacobi preconditioner M = diag(A)^-1, found and inverted on the device (k_jacobi).  Not collective: a rank whose slab
@@ -819,33 +779,26 @@ int lkb_op_jacobi_create(lkb_op_t A, lkb_op_t* M) {
     } else {
         set_error("jacobi_create: unsupported operator type %d", A->type); return LKB_ERR_ARG;
     }
-    lkb_op_s* op = nullptr;
-    LKB_TRY(diag_from_device(c, A->kind, A->m, src.row0, n_global, &op));
-    unsigned long long* bad = nullptr; unsigned long long hbad = 0;
-    cudaError_t e = cudaMalloc((void**)&bad, sizeof(unsigned long long));
-    if (e == cudaSuccess) e = cudaMemsetAsync(bad, 0xff, sizeof(unsigned long long), c->stream);
-    if (e == cudaSuccess) { launch_jacobi(A->kind, c->stream, src, op->diag, bad, c->sms); e = cudaGetLastError(); }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(&hbad, bad, sizeof(hbad), cudaMemcpyDeviceToHost, c->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    if (bad) cudaFree(bad);
-    if (e != cudaSuccess) { set_error("jacobi_create: %s", cudaGetErrorString(e)); lkb_op_destroy(op); return LKB_ERR_CUDA; }
+    OpOwner op;
+    LKB_TRY(diag_from_device(c, A->kind, A->m, src.row0, n_global, op));
+    CudaPtr<unsigned long long> bad; unsigned long long hbad = 0;
+    LKB_TRY(cuda_alloc(bad, sizeof(unsigned long long)));
+    LKB_CUDA(cudaMemsetAsync(bad, 0xff, sizeof(unsigned long long), c->stream));
+    launch_jacobi(A->kind, c->stream, src, op->diag, bad, c->sms);
+    LKB_TRY(check_launch(c, "jacobi"));
+    LKB_CUDA(cudaMemcpyAsync(&hbad, bad, sizeof(hbad), cudaMemcpyDeviceToHost, c->stream));
+    LKB_CUDA(cudaStreamSynchronize(c->stream));
     if (hbad != ~0ULL) {
         set_error("jacobi_create: the diagonal entry of global row %llu is zero or not finite", hbad);
-        lkb_op_destroy(op); return LKB_ERR_ARG;
+        return LKB_ERR_ARG;
     }
-    *M = op;
+    *M = op.release();
     return 0;
 }
 int lkb_op_destroy(lkb_op_t A) {
     if (!A) return LKB_ERR_ARG;
     cudaStreamSynchronize(A->ctx->stream);
     invalidate_graphs(A->ctx, A->uid);
-    if (A->hp_lo_map) cudaIpcCloseMemHandle(A->hp_lo_map);
-    if (A->hp_hi_map) cudaIpcCloseMemHandle(A->hp_hi_map);
-    if (A->hp_active) { cudaFree(A->hp.my_region); cudaFree(A->hp.epoch); }
-    void* bufs[] = { A->halo_lo, A->halo_hi, A->rowptr, A->col, A->val, A->t_rowptr, A->t_col, A->t_val, A->a, A->diag, A->x_full, A->y_full, A->y_red,
-                     A->blk.tab, A->blk.col, A->blk.val, A->t_blk.tab, A->t_blk.col, A->t_blk.val };
-    for (void* b : bufs) if (b) cudaFree(b);
     delete A;
     return 0;
 }
@@ -905,12 +858,12 @@ int op_apply_enqueue(lkb_op_s* A, const void* x, void* y, bool trans, const int*
             if (c->world > 1) {
                 LKB_NCCL(api->GroupStart());
                 for (int q = 0; q < c->world; ++q) {
-                    void* dst = (char*)A->x_full + (size_t)A->col_off[q] * es;
+                    void* dst = (char*)A->x_full.get() + (size_t)A->col_off[q] * es;
                     LKB_NCCL(api->Broadcast(q == c->rank ? x : dst, dst, (size_t)A->col_cnt[q] * per, dt, q, c->comm, c->stream));
                 }
                 LKB_NCCL(api->GroupEnd());
             } else {
-                LKB_CUDA(cudaMemcpyAsync((char*)A->x_full + (size_t)A->col_off[0] * es, x, (size_t)A->n * es, cudaMemcpyDeviceToDevice, c->stream));
+                LKB_CUDA(cudaMemcpyAsync((char*)A->x_full.get() + (size_t)A->col_off[0] * es, x, (size_t)A->n * es, cudaMemcpyDeviceToDevice, c->stream));
             }
             if (A->blk.nb > 0) { launch_csr_blocked(A->kind, c->stream, A->blk, A->x_full, y, false, flags, c->sms); nl = A->blk.nb; }
             else launch_csr(A->kind, c->stream, A->m, A->rowptr, A->col, A->val, A->x_full, y, false, flags, c->sms | (A->lpr << 16));
@@ -922,12 +875,12 @@ int op_apply_enqueue(lkb_op_s* A, const void* x, void* y, bool trans, const int*
                 // reduce into a scratch slab, then a flags-gated copy: after a device-side stop the reference leaves the
                 // later basis columns untouched, so stale reductions must not land in y
                 for (int q = 0; q < c->world; ++q)
-                    LKB_NCCL(api->Reduce((char*)A->y_full + (size_t)A->col_off[q] * es, A->y_red, (size_t)A->col_cnt[q] * per, dt, /*ncclSum*/ 0, q, c->comm, c->stream));
+                    LKB_NCCL(api->Reduce((char*)A->y_full.get() + (size_t)A->col_off[q] * es, A->y_red, (size_t)A->col_cnt[q] * per, dt, /*ncclSum*/ 0, q, c->comm, c->stream));
                 LKB_NCCL(api->GroupEnd());
                 launch_copy_gated(A->kind, c->stream, A->y_red, y, A->n, flags, c->sms);
                 nl = 2;
             } else {
-                LKB_CUDA(cudaMemcpyAsync(y, (char*)A->y_full + (size_t)A->col_off[0] * es, (size_t)A->n * es, cudaMemcpyDeviceToDevice, c->stream));
+                LKB_CUDA(cudaMemcpyAsync(y, (char*)A->y_full.get() + (size_t)A->col_off[0] * es, (size_t)A->n * es, cudaMemcpyDeviceToDevice, c->stream));
             }
         }
     } else if (A->type == OP_CSR) {

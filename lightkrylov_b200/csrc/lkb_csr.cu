@@ -162,27 +162,27 @@ int pick_lpr(int64_t nnz, int64_t rows) {
 
 namespace lkb {
 
-int csr_block_device(lkb_ctx_s* c, int kind, int64_t rows, int64_t ncols, int64_t** rowptr, int32_t** col, void** val, CsrBlocked* blk);
+void csr_block_device(lkb_ctx_s* c, int kind, int64_t rows, int64_t ncols, int64_t nnz, CudaPtr<int64_t>& rowptr, CudaPtr<int32_t>& col,
+                      CudaPtr<void>& val, CsrBlocked* blk, CsrBlockedMem* mem);
 
 // Validate (rowptr, col) ON THE DEVICE and build the explicit transpose.  `rows` = local rows, `ncols_index` =
 // size of the column index space (global n for a row-sharded operator).  op->rowptr / col / val must already
-// point at device arrays owned by the operator.
+// point at device arrays owned by the operator.  Nothing can fail once the L2 blocking may have released them.
 int csr_finish_device(lkb_ctx_s* c, lkb_op_s* op, int kind, int64_t rows, int64_t ncols_index) {
     const size_t es = kind_size(kind);
     int64_t nnz = 0;
-    LKB_CUDA(cudaMemcpy(&nnz, op->rowptr + rows, sizeof(int64_t), cudaMemcpyDeviceToHost));
+    LKB_CUDA(cudaMemcpy(&nnz, op->rowptr.get() + rows, sizeof(int64_t), cudaMemcpyDeviceToHost));
     if (nnz < 0 || nnz >= (int64_t)0xffffffffLL) { set_error("csr: nnz = %lld is outside [0, 2^32-1)", (long long)nnz); return LKB_ERR_ARG; }
     if (rows > 2147483647LL || ncols_index > 2147483647LL) { set_error("csr: more than 2^31-1 rows / columns per rank"); return LKB_ERR_ARG; }
     // ---- validation: rowptr[0] == 0, rowptr non-decreasing, 0 <= col < ncols_index (ADVICE r01: an out-of-range
     // index, e.g. 1-based Fortran indices, must be an LKB_ERR_ARG, not heap corruption) ----
-    int* derr = nullptr;
-    LKB_CUDA(cudaMalloc((void**)&derr, sizeof(int)));
+    CudaPtr<int> derr;
+    LKB_TRY(cuda_alloc(derr, sizeof(int)));
     LKB_CUDA(cudaMemsetAsync(derr, 0, sizeof(int), c->stream));
     k_csr_validate<<<grid_for(std::max(rows, nnz), c->sms), 256, 0, c->stream>>>(rows, ncols_index, nnz, op->rowptr, op->col, derr);
     int herr = 0;
     LKB_CUDA(cudaMemcpyAsync(&herr, derr, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     LKB_CUDA(cudaStreamSynchronize(c->stream));
-    cudaFree(derr);
     if (herr) {
         static const char* what[] = {"", "rowptr[0] != 0", "rowptr is not non-decreasing", "column index out of range (indices are 0-based)",
                                      "rowptr[rows] != nnz"};
@@ -192,103 +192,95 @@ int csr_finish_device(lkb_ctx_s* c, lkb_op_s* op, int kind, int64_t rows, int64_
     op->lpr = pick_lpr(nnz, rows); op->t_lpr = pick_lpr(nnz, ncols_index);
     // ---- transpose: stable radix sort of (col, position) ----
     const int64_t nn = std::max<int64_t>(nnz, 1);
-    uint32_t *keys_out = nullptr, *perm_in = nullptr, *perm_out = nullptr; void* tmp = nullptr;
-    auto free_tmp = [&]() { if (keys_out) cudaFree(keys_out); if (perm_in) cudaFree(perm_in); if (perm_out) cudaFree(perm_out); if (tmp) cudaFree(tmp); };
-#define CSR_CUDA(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { free_tmp(); \
-        set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_)); return e_ == cudaErrorMemoryAllocation ? LKB_ERR_ALLOC : LKB_ERR_CUDA; } } while (0)
-    CSR_CUDA(cudaMalloc((void**)&keys_out, nn * sizeof(uint32_t)));
-    CSR_CUDA(cudaMalloc((void**)&perm_in, nn * sizeof(uint32_t)));
-    CSR_CUDA(cudaMalloc((void**)&perm_out, nn * sizeof(uint32_t)));
+    CudaPtr<uint32_t> keys_out, perm_in, perm_out; CudaPtr<void> tmp;
+    LKB_TRY(cuda_alloc(keys_out, nn * sizeof(uint32_t)));
+    LKB_TRY(cuda_alloc(perm_in, nn * sizeof(uint32_t)));
+    LKB_TRY(cuda_alloc(perm_out, nn * sizeof(uint32_t)));
     k_iota_u32<<<grid_for(nnz, c->sms), 256, 0, c->stream>>>(perm_in, nnz);
     int end_bit = 1;
     while (end_bit < 32 && ((int64_t)1 << end_bit) < ncols_index) ++end_bit;
     size_t tmp_bytes = 0;
-    CSR_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, (const uint32_t*)op->col, keys_out, perm_in, perm_out, nnz, 0, end_bit, c->stream));
-    CSR_CUDA(cudaMalloc(&tmp, std::max<size_t>(tmp_bytes, 16)));
-    CSR_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, (const uint32_t*)op->col, keys_out, perm_in, perm_out, nnz, 0, end_bit, c->stream));
-    CSR_CUDA(cudaMalloc((void**)&op->t_rowptr, (ncols_index + 1) * sizeof(int64_t)));
-    CSR_CUDA(cudaMalloc((void**)&op->t_col, nn * sizeof(int32_t)));
-    CSR_CUDA(cudaMalloc(&op->t_val, nn * es));
+    LKB_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, (const uint32_t*)op->col.get(), keys_out.get(), perm_in.get(), perm_out.get(), nnz, 0, end_bit, c->stream));
+    LKB_TRY(cuda_alloc(tmp, std::max<size_t>(tmp_bytes, 16)));
+    LKB_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, (const uint32_t*)op->col.get(), keys_out.get(), perm_in.get(), perm_out.get(), nnz, 0, end_bit, c->stream));
+    LKB_TRY(cuda_alloc(op->t_rowptr, (ncols_index + 1) * sizeof(int64_t)));
+    LKB_TRY(cuda_alloc(op->t_col, nn * sizeof(int32_t)));
+    LKB_TRY(cuda_alloc(op->t_val, nn * es));
     k_csr_trowptr<<<grid_for(nnz + 1, c->sms), 256, 0, c->stream>>>(nnz, ncols_index, keys_out, op->t_rowptr);
     const int g = grid_for(nnz, c->sms);
     switch (kind) {
-        case KS: k_csr_tfill<float><<<g, 256, 0, c->stream>>>(nnz, rows, op->rowptr, perm_out, (const float*)op->val, op->t_col, (float*)op->t_val); break;
-        case KD: k_csr_tfill<double><<<g, 256, 0, c->stream>>>(nnz, rows, op->rowptr, perm_out, (const double*)op->val, op->t_col, (double*)op->t_val); break;
-        case KC: k_csr_tfill<float2><<<g, 256, 0, c->stream>>>(nnz, rows, op->rowptr, perm_out, (const float2*)op->val, op->t_col, (float2*)op->t_val); break;
-        default: k_csr_tfill<double2><<<g, 256, 0, c->stream>>>(nnz, rows, op->rowptr, perm_out, (const double2*)op->val, op->t_col, (double2*)op->t_val); break;
+        case KS: k_csr_tfill<float><<<g, 256, 0, c->stream>>>(nnz, rows, op->rowptr, perm_out, (const float*)op->val.get(), op->t_col, (float*)op->t_val.get()); break;
+        case KD: k_csr_tfill<double><<<g, 256, 0, c->stream>>>(nnz, rows, op->rowptr, perm_out, (const double*)op->val.get(), op->t_col, (double*)op->t_val.get()); break;
+        case KC: k_csr_tfill<float2><<<g, 256, 0, c->stream>>>(nnz, rows, op->rowptr, perm_out, (const float2*)op->val.get(), op->t_col, (float2*)op->t_val.get()); break;
+        default: k_csr_tfill<double2><<<g, 256, 0, c->stream>>>(nnz, rows, op->rowptr, perm_out, (const double2*)op->val.get(), op->t_col, (double2*)op->t_val.get()); break;
     }
-    CSR_CUDA(cudaGetLastError());
-    CSR_CUDA(cudaStreamSynchronize(c->stream));
-#undef CSR_CUDA
-    free_tmp();
+    LKB_CUDA(cudaGetLastError());
+    LKB_CUDA(cudaStreamSynchronize(c->stream));
+    keys_out.reset(); perm_in.reset(); perm_out.reset(); tmp.reset();
     // L2 blocking when the gathered vector exceeds L2 (no-op otherwise).  Row-sharded operator: only the forward
     // orientation (it gathers from the full-length x_full; the transposed one gathers from this rank's slab of u)
-    LKB_TRY(csr_block_device(c, kind, rows, ncols_index, &op->rowptr, &op->col, &op->val, &op->blk));
-    if (!op->dist) LKB_TRY(csr_block_device(c, kind, ncols_index, rows, &op->t_rowptr, &op->t_col, &op->t_val, &op->t_blk));
+    csr_block_device(c, kind, rows, ncols_index, nnz, op->rowptr, op->col, op->val, &op->blk, &op->blk_mem);
+    if (!op->dist) csr_block_device(c, kind, ncols_index, rows, nnz, op->t_rowptr, op->t_col, op->t_val, &op->t_blk, &op->t_blk_mem);
     return 0;
 }
 
-// Build the L2-blocked copy of a CSR matrix (rows x ncols) when the gathered vector is too large for L2; the plain
-// arrays are released afterwards (`*rowptr / *col / *val` become null).  blk.nb == 0 afterwards: not blocked.
-int csr_block_device(lkb_ctx_s* c, int kind, int64_t rows, int64_t ncols, int64_t** rowptr, int32_t** col, void** val, CsrBlocked* blk) {
+// The L2-blocked copy of a CSR matrix in nb column blocks of width cw.  On success it replaces the plain arrays (they are
+// released) and blk views mem.
+static int csr_blocked_copy(lkb_ctx_s* c, int kind, int64_t rows, int64_t nnz, int nb, int64_t cw, CudaPtr<int64_t>& rowptr,
+                            CudaPtr<int32_t>& col, CudaPtr<void>& val, CsrBlocked* blk, CsrBlockedMem* mem) {
+    const size_t es = kind_size(kind);
+    CudaPtr<uint8_t> keys, keys_out; CudaPtr<uint32_t> iota, perm, brow; CudaPtr<void> tmp;
+    CsrBlockedMem b;
+    LKB_TRY(cuda_alloc(keys, nnz)); LKB_TRY(cuda_alloc(keys_out, nnz));
+    LKB_TRY(cuda_alloc(iota, nnz * sizeof(uint32_t))); LKB_TRY(cuda_alloc(perm, nnz * sizeof(uint32_t)));
+    k_blk_keys<<<grid_for(nnz, c->sms), 256, 0, c->stream>>>(nnz, cw, col, keys, iota);
+    int end_bit = 1; while ((1 << end_bit) < nb) ++end_bit;
+    size_t tmp_bytes = 0;
+    LKB_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, keys.get(), keys_out.get(), iota.get(), perm.get(), nnz, 0, end_bit, c->stream));
+    LKB_TRY(cuda_alloc(tmp, std::max<size_t>(tmp_bytes, 16)));
+    LKB_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, keys.get(), keys_out.get(), iota.get(), perm.get(), nnz, 0, end_bit, c->stream));
+    LKB_CUDA(cudaStreamSynchronize(c->stream));
+    keys.reset(); iota.reset(); tmp.reset();
+    LKB_TRY(cuda_alloc(brow, nnz * sizeof(uint32_t)));
+    LKB_TRY(cuda_alloc(b.col, nnz * sizeof(int32_t)));
+    LKB_TRY(cuda_alloc(b.val, nnz * es));
+    const int g = grid_for(nnz, c->sms);
+    switch (kind) {
+        case KS: k_blk_gather<float><<<g, 256, 0, c->stream>>>(nnz, rows, rowptr, perm, col, (const float*)val.get(), b.col, (float*)b.val.get(), brow); break;
+        case KD: k_blk_gather<double><<<g, 256, 0, c->stream>>>(nnz, rows, rowptr, perm, col, (const double*)val.get(), b.col, (double*)b.val.get(), brow); break;
+        case KC: k_blk_gather<float2><<<g, 256, 0, c->stream>>>(nnz, rows, rowptr, perm, col, (const float2*)val.get(), b.col, (float2*)b.val.get(), brow); break;
+        default: k_blk_gather<double2><<<g, 256, 0, c->stream>>>(nnz, rows, rowptr, perm, col, (const double2*)val.get(), b.col, (double2*)b.val.get(), brow); break;
+    }
+    LKB_CUDA(cudaGetLastError());
+    LKB_CUDA(cudaStreamSynchronize(c->stream));
+    perm.reset();
+    LKB_TRY(cuda_alloc(b.tab, (size_t)nb * (rows + 1) * sizeof(uint32_t)));
+    k_blk_table<<<grid_for(nnz + 1, c->sms), 256, 0, c->stream>>>(nnz, rows, nb, keys_out, brow, b.tab);
+    LKB_CUDA(cudaGetLastError());
+    LKB_CUDA(cudaStreamSynchronize(c->stream));
+    rowptr.reset(); col.reset(); val.reset();
+    blk->nb = nb; blk->cw = cw; blk->rows = rows; blk->nnz = nnz; blk->tab = b.tab; blk->col = b.col; blk->val = b.val;
+    *mem = std::move(b);
+    return 0;
+}
+
+// Build the L2-blocked copy of a CSR matrix (rows x ncols, nnz entries) when the gathered vector is too large for L2.
+// blk.nb == 0 afterwards: not blocked.  A failure here (in practice: not enough memory for the second copy) is not fatal:
+// the plain arrays are only released after everything else succeeded, so the matrix simply stays unblocked.
+void csr_block_device(lkb_ctx_s* c, int kind, int64_t rows, int64_t ncols, int64_t nnz, CudaPtr<int64_t>& rowptr, CudaPtr<int32_t>& col,
+                      CudaPtr<void>& val, CsrBlocked* blk, CsrBlockedMem* mem) {
     blk->nb = 0;
     const size_t es = kind_size(kind);
     // slice / threshold: lkb_set_option(ctx, "csr_slice_kb" | "csr_block_min_kb", v); defaults 48 MB / 96 MB
     const int64_t slice_b = (int64_t)c->csr_slice_kb * 1024, min_b = (int64_t)c->csr_block_min_kb * 1024;
-    if (slice_b <= 0 || (int64_t)ncols * (int64_t)es < min_b) return 0;                 // x (nearly) fits in L2: plain CSR
-    int64_t nnz = 0;
-    LKB_CUDA(cudaMemcpy(&nnz, *rowptr + rows, sizeof(int64_t), cudaMemcpyDeviceToHost));
-    if (nnz < 1) return 0;
+    if (slice_b <= 0 || (int64_t)ncols * (int64_t)es < min_b) return;                 // x (nearly) fits in L2: plain CSR
+    if (nnz < 1) return;
     int64_t cw = (slice_b / (int64_t)es + 1023) / 1024 * 1024;
     int nb = (int)((ncols + cw - 1) / cw);
     if (nb > 255) { nb = 255; cw = ((ncols + nb - 1) / nb + 1023) / 1024 * 1024; nb = (int)((ncols + cw - 1) / cw); }
-    if (nb < 2) return 0;
-    if ((int64_t)nb * (rows + 1) >= (int64_t)1 << 40) return 0;
-    uint8_t *keys = nullptr, *keys_out = nullptr; uint32_t *iota = nullptr, *perm = nullptr, *brow = nullptr; void* tmp = nullptr;
-    int32_t* bcol = nullptr; void* bval = nullptr; uint32_t* tab = nullptr;
-    auto free_tmp = [&]() { for (void* p : {(void*)keys, (void*)keys_out, (void*)iota, (void*)perm, (void*)brow, tmp}) if (p) cudaFree(p); };
-    // a failure here (in practice: not enough memory for the second copy) is not fatal: the plain CSR arrays are only
-    // released after everything else succeeded, so the operator simply stays unblocked
-    auto fail = [&](const char*, cudaError_t) {
-        free_tmp(); if (bcol) cudaFree(bcol); if (bval) cudaFree(bval); if (tab) cudaFree(tab);
-        cudaGetLastError();
-        return 0;
-    };
-#define BLK_CUDA(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return fail(#call, e_); } while (0)
-    BLK_CUDA(cudaMalloc((void**)&keys, nnz)); BLK_CUDA(cudaMalloc((void**)&keys_out, nnz));
-    BLK_CUDA(cudaMalloc((void**)&iota, nnz * sizeof(uint32_t))); BLK_CUDA(cudaMalloc((void**)&perm, nnz * sizeof(uint32_t)));
-    k_blk_keys<<<grid_for(nnz, c->sms), 256, 0, c->stream>>>(nnz, cw, *col, keys, iota);
-    int end_bit = 1; while ((1 << end_bit) < nb) ++end_bit;
-    size_t tmp_bytes = 0;
-    BLK_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, keys, keys_out, iota, perm, nnz, 0, end_bit, c->stream));
-    BLK_CUDA(cudaMalloc(&tmp, std::max<size_t>(tmp_bytes, 16)));
-    BLK_CUDA(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, keys, keys_out, iota, perm, nnz, 0, end_bit, c->stream));
-    BLK_CUDA(cudaStreamSynchronize(c->stream));
-    cudaFree(keys); keys = nullptr; cudaFree(iota); iota = nullptr; cudaFree(tmp); tmp = nullptr;
-    BLK_CUDA(cudaMalloc((void**)&brow, nnz * sizeof(uint32_t)));
-    BLK_CUDA(cudaMalloc((void**)&bcol, nnz * sizeof(int32_t)));
-    BLK_CUDA(cudaMalloc(&bval, nnz * es));
-    const int g = grid_for(nnz, c->sms);
-    switch (kind) {
-        case KS: k_blk_gather<float><<<g, 256, 0, c->stream>>>(nnz, rows, *rowptr, perm, *col, (const float*)*val, bcol, (float*)bval, brow); break;
-        case KD: k_blk_gather<double><<<g, 256, 0, c->stream>>>(nnz, rows, *rowptr, perm, *col, (const double*)*val, bcol, (double*)bval, brow); break;
-        case KC: k_blk_gather<float2><<<g, 256, 0, c->stream>>>(nnz, rows, *rowptr, perm, *col, (const float2*)*val, bcol, (float2*)bval, brow); break;
-        default: k_blk_gather<double2><<<g, 256, 0, c->stream>>>(nnz, rows, *rowptr, perm, *col, (const double2*)*val, bcol, (double2*)bval, brow); break;
-    }
-    BLK_CUDA(cudaGetLastError());
-    BLK_CUDA(cudaStreamSynchronize(c->stream));
-    cudaFree(perm); perm = nullptr;
-    BLK_CUDA(cudaMalloc((void**)&tab, (size_t)nb * (rows + 1) * sizeof(uint32_t)));
-    k_blk_table<<<grid_for(nnz + 1, c->sms), 256, 0, c->stream>>>(nnz, rows, nb, keys_out, brow, tab);
-    BLK_CUDA(cudaGetLastError());
-    BLK_CUDA(cudaStreamSynchronize(c->stream));
-#undef BLK_CUDA
-    free_tmp();
-    // the blocked copy replaces the plain arrays
-    cudaFree(*rowptr); cudaFree(*col); cudaFree(*val);
-    *rowptr = nullptr; *col = nullptr; *val = nullptr;
-    blk->nb = nb; blk->cw = cw; blk->rows = rows; blk->nnz = nnz; blk->tab = tab; blk->col = bcol; blk->val = bval;
-    return 0;
+    if (nb < 2) return;
+    if ((int64_t)nb * (rows + 1) >= (int64_t)1 << 40) return;
+    if (csr_blocked_copy(c, kind, rows, nnz, nb, cw, rowptr, col, val, blk, mem) != 0) cudaGetLastError();
 }
 
 // host arrays -> device copies owned by the operator, then the common device set-up
@@ -299,9 +291,9 @@ int csr_build(lkb_ctx_s* c, lkb_op_s* op, int kind, int64_t rows, int64_t ncols_
     if (nnz < 0) { set_error("csr: rowptr[rows] = %lld < 0", (long long)nnz); return LKB_ERR_ARG; }
     if (nnz > 0 && (!col || !val)) { set_error("csr: col / val are null with nnz = %lld", (long long)nnz); return LKB_ERR_ARG; }
     const size_t es = kind_size(kind);
-    LKB_CUDA(cudaMalloc((void**)&op->rowptr, (rows + 1) * sizeof(int64_t)));
-    LKB_CUDA(cudaMalloc((void**)&op->col, std::max<int64_t>(nnz, 1) * sizeof(int32_t)));
-    LKB_CUDA(cudaMalloc(&op->val, std::max<int64_t>(nnz, 1) * es));
+    LKB_TRY(cuda_alloc(op->rowptr, (rows + 1) * sizeof(int64_t)));
+    LKB_TRY(cuda_alloc(op->col, std::max<int64_t>(nnz, 1) * sizeof(int32_t)));
+    LKB_TRY(cuda_alloc(op->val, std::max<int64_t>(nnz, 1) * es));
     LKB_CUDA(cudaMemcpy(op->rowptr, rowptr, (rows + 1) * sizeof(int64_t), cudaMemcpyHostToDevice));
     if (nnz > 0) {
         LKB_CUDA(cudaMemcpy(op->col, col, nnz * sizeof(int32_t), cudaMemcpyHostToDevice));
@@ -319,11 +311,10 @@ int lkb_op_csr_create(lkb_ctx_t c, int kind, int64_t m, int64_t n, const int64_t
     if (!c || !A || !rowptr || m < 1 || n < 1 || kind < 0 || kind > 3) { set_error("csr_create: bad arguments"); return LKB_ERR_ARG; }
     if (c->world > 1) { set_error("lkb_op_csr_create is single-rank; use lkb_op_csr_create_dist for a row-sharded matrix"); return LKB_ERR_ARG; }
     cudaSetDevice(c->dev);
-    lkb_op_s* op = new lkb_op_s();
+    OpOwner op(new lkb_op_s());
     op->ctx = c; op->type = OP_CSR; op->kind = kind; op->m = m; op->n = n; op->uid = next_uid();
-    int r = csr_build(c, op, kind, m, n, rowptr, col, val);
-    if (r) { lkb_op_destroy(op); return r; }
-    *A = op;
+    LKB_TRY(csr_build(c, op, kind, m, n, rowptr, col, val));
+    *A = op.release();
     return 0;
 }
 
@@ -332,30 +323,29 @@ int lkb_op_csr_create_device(lkb_ctx_t c, int kind, int64_t m, int64_t n, int64_
     if (!c || !A || !rowptr_dev || !col_dev || !val_dev || m < 1 || n < 1 || kind < 0 || kind > 3) { set_error("csr_create_device: bad arguments"); return LKB_ERR_ARG; }
     if (c->world > 1) { set_error("lkb_op_csr_create_device is single-rank"); return LKB_ERR_ARG; }
     cudaSetDevice(c->dev);
-    lkb_op_s* op = new lkb_op_s();
+    OpOwner op(new lkb_op_s());
     op->ctx = c; op->type = OP_CSR; op->kind = kind; op->m = m; op->n = n; op->uid = next_uid();
     if (adopt) {
-        op->rowptr = rowptr_dev; op->col = col_dev; op->val = val_dev;
+        op->rowptr.reset(rowptr_dev); op->col.reset(col_dev); op->val.reset(val_dev);
     } else {
-        int64_t nnz = 0;
-        cudaError_t e = cudaMemcpy(&nnz, rowptr_dev + m, sizeof(int64_t), cudaMemcpyDeviceToHost);
+        int64_t nnz = 0;            // (a negative nnz is rejected by csr_finish_device)
+        LKB_CUDA(cudaMemcpy(&nnz, rowptr_dev + m, sizeof(int64_t), cudaMemcpyDeviceToHost));
         const size_t es = kind_size(kind);
         const int64_t nn = std::max<int64_t>(nnz, 1);
-        if (e == cudaSuccess && nnz >= 0) e = cudaMalloc((void**)&op->rowptr, (m + 1) * sizeof(int64_t));
-        if (e == cudaSuccess) e = cudaMalloc((void**)&op->col, nn * sizeof(int32_t));
-        if (e == cudaSuccess) e = cudaMalloc(&op->val, nn * es);
-        if (e == cudaSuccess) e = cudaMemcpy(op->rowptr, rowptr_dev, (m + 1) * sizeof(int64_t), cudaMemcpyDeviceToDevice);
-        if (e == cudaSuccess && nnz > 0) e = cudaMemcpy(op->col, col_dev, nnz * sizeof(int32_t), cudaMemcpyDeviceToDevice);
-        if (e == cudaSuccess && nnz > 0) e = cudaMemcpy(op->val, val_dev, nnz * es, cudaMemcpyDeviceToDevice);
-        if (e != cudaSuccess || nnz < 0) { set_error("csr_create_device: copy failed: %s", cudaGetErrorString(e)); lkb_op_destroy(op); return LKB_ERR_CUDA; }
+        LKB_TRY(cuda_alloc(op->rowptr, (m + 1) * sizeof(int64_t)));
+        LKB_TRY(cuda_alloc(op->col, nn * sizeof(int32_t)));
+        LKB_TRY(cuda_alloc(op->val, nn * es));
+        LKB_CUDA(cudaMemcpy(op->rowptr, rowptr_dev, (m + 1) * sizeof(int64_t), cudaMemcpyDeviceToDevice));
+        if (nnz > 0) {
+            LKB_CUDA(cudaMemcpy(op->col, col_dev, nnz * sizeof(int32_t), cudaMemcpyDeviceToDevice));
+            LKB_CUDA(cudaMemcpy(op->val, val_dev, nnz * es, cudaMemcpyDeviceToDevice));
+        }
     }
-    int r = csr_finish_device(c, op, kind, m, n);
-    if (r) {
-        if (adopt) { op->rowptr = nullptr; op->col = nullptr; op->val = nullptr; }    // the caller keeps ownership on failure
-        lkb_op_destroy(op);
+    if (int r = csr_finish_device(c, op, kind, m, n)) {
+        if (adopt) { op->rowptr.release(); op->col.release(); op->val.release(); }    // the caller keeps ownership on failure
         return r;
     }
-    *A = op;
+    *A = op.release();
     return 0;
 }
 
@@ -366,26 +356,21 @@ int lkb_csr_random_device(lkb_ctx_t c, int kind, int64_t m_local, int64_t row0, 
     cudaSetDevice(c->dev);
     const int64_t nnz = m_local * per_row;
     const size_t es = kind_size(kind);
-    int64_t* rp = nullptr; int32_t* ci = nullptr; void* va = nullptr;
-    cudaError_t e = cudaMalloc((void**)&rp, (m_local + 1) * sizeof(int64_t));
-    if (e == cudaSuccess) e = cudaMalloc((void**)&ci, nnz * sizeof(int32_t));
-    if (e == cudaSuccess) e = cudaMalloc(&va, nnz * es);
-    if (e != cudaSuccess) {
-        if (rp) cudaFree(rp); if (ci) cudaFree(ci); if (va) cudaFree(va);
-        set_error("csr_random: cudaMalloc failed: %s", cudaGetErrorString(e));
-        return LKB_ERR_ALLOC;
-    }
+    CudaPtr<int64_t> rp; CudaPtr<int32_t> ci; CudaPtr<void> va;
+    LKB_TRY(cuda_alloc(rp, (m_local + 1) * sizeof(int64_t)));
+    LKB_TRY(cuda_alloc(ci, nnz * sizeof(int32_t)));
+    LKB_TRY(cuda_alloc(va, nnz * es));
     const uint64_t sc = mix64(seed), sv = mix64(seed + 1);
     const int g = grid_for(m_local + 1, c->sms);
     switch (kind) {
-        case KS: k_csr_random<float, false><<<g, 256, 0, c->stream>>>(m_local, row0, n, per_row, sc, sv, rp, ci, (float*)va); break;
-        case KD: k_csr_random<double, false><<<g, 256, 0, c->stream>>>(m_local, row0, n, per_row, sc, sv, rp, ci, (double*)va); break;
-        case KC: k_csr_random<float2, true><<<g, 256, 0, c->stream>>>(m_local, row0, n, per_row, sc, sv, rp, ci, (float2*)va); break;
-        default: k_csr_random<double2, true><<<g, 256, 0, c->stream>>>(m_local, row0, n, per_row, sc, sv, rp, ci, (double2*)va); break;
+        case KS: k_csr_random<float, false><<<g, 256, 0, c->stream>>>(m_local, row0, n, per_row, sc, sv, rp, ci, (float*)va.get()); break;
+        case KD: k_csr_random<double, false><<<g, 256, 0, c->stream>>>(m_local, row0, n, per_row, sc, sv, rp, ci, (double*)va.get()); break;
+        case KC: k_csr_random<float2, true><<<g, 256, 0, c->stream>>>(m_local, row0, n, per_row, sc, sv, rp, ci, (float2*)va.get()); break;
+        default: k_csr_random<double2, true><<<g, 256, 0, c->stream>>>(m_local, row0, n, per_row, sc, sv, rp, ci, (double2*)va.get()); break;
     }
     LKB_TRY(check_launch(c, "csr_random"));
     LKB_CUDA(cudaStreamSynchronize(c->stream));
-    *rowptr_dev = rp; *col_dev = ci; *val_dev = va;
+    *rowptr_dev = rp.release(); *col_dev = ci.release(); *val_dev = va.release();
     return 0;
 }
 

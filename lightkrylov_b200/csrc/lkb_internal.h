@@ -39,24 +39,61 @@ enum ProfClass { PC_MATVEC = 0, PC_DOT = 1, PC_AXPY = 2, PC_OTHER = 3, PC_FUSED 
 // lkb_op_s::type.  The values are printed by lkb_op_jacobi_create's error message.
 enum OpType { OP_DENSE = 0, OP_STENCIL = 1, OP_CSR = 3, OP_DIAG = 4, OP_CALLBACK = 9 };
 
+// ---- owners: every raw CUDA resource and every solver work object has exactly one, and goes with it ------------------
+// Members and locals are released in reverse order of declaration.  (The host-shell test mocks replace lkb_basis_destroy,
+// lkb_vec_destroy and dev_free.)
+template <class T, auto Release> class Owner {
+  public:
+    Owner() = default;
+    explicit Owner(T p) : p_(p) {}
+    Owner(Owner&& o) noexcept : p_(o.release()) {}
+    Owner& operator=(Owner&& o) noexcept { reset(o.release()); return *this; }
+    Owner(const Owner&) = delete;
+    Owner& operator=(const Owner&) = delete;
+    ~Owner() { reset(); }
+    void reset(T p = nullptr) { T old = p_; p_ = p; if (old) Release(old); }
+    T release() { T p = p_; p_ = nullptr; return p; }   // hand the resource to a caller, or back to one on failure
+    T* out() { return &p_; }                   // for the create call that fills an empty owner
+    T get() const { return p_; }
+    operator T() const { return p_; }
+    T operator->() const { return p_; }
+  private:
+    T p_ = nullptr;
+};
+int comm_destroy(void* comm);                  // ncclCommDestroy through nccl_api()
+template <class T> using CudaPtr = Owner<T*, cudaFree>;     // cudaMalloc memory (operator and context buffers)
+typedef Owner<void*, cudaFreeHost> PinnedPtr;
+typedef Owner<void*, cudaIpcCloseMemHandle> IpcMap;         // a peer's region mapped with cudaIpcOpenMemHandle
+typedef Owner<cudaStream_t, cudaStreamDestroy> StreamOwner;
+typedef Owner<void*, comm_destroy> CommOwner;
+typedef Owner<lkb_basis_t, lkb_basis_destroy> BasisOwner;
+typedef Owner<lkb_vec_t, lkb_vec_destroy> VecOwner;
+typedef Owner<lkb_op_t, lkb_op_destroy> OpOwner;           // an operator until its creator hands it out
+// an instantiated CUDA graph and the kernel launches one replay stands for
+struct GraphExec { Owner<cudaGraphExec_t, cudaGraphExecDestroy> exec; int64_t launches = 0; };
+// the arrays an L2-blocked CsrBlocked views
+struct CsrBlockedMem { CudaPtr<uint32_t> tab; CudaPtr<int32_t> col; CudaPtr<void> val; };
 }  // namespace lkb
 
 struct lkb_ctx_s {
     int dev = 0, sms = 148;
     int rank = 0, world = 1;
-    void* comm = nullptr;
-    cudaStream_t stream = nullptr;
+    // The owners below go in reverse order: cached graphs, the communicator, the peer mappings, the buffers, the stream.
+    lkb::StreamOwner stream;
     // device workspace
-    void* partial = nullptr; size_t partial_bytes = 0;
-    void* c1 = nullptr; void* c2 = nullptr; void* tmpw = nullptr; size_t cbuf_len = 0;   // W elements
-    void* nrm2 = nullptr;       // one W
-    double* inv = nullptr;      // one double
-    int* flags = nullptr;       // F_COUNT ints
-    unsigned* counter = nullptr;
-    void* Hd = nullptr; size_t Hd_bytes = 0;
+    lkb::CudaPtr<void> partial; size_t partial_bytes = 0;
+    lkb::CudaPtr<void> c1, c2, tmpw; size_t cbuf_len = 0;   // W elements
+    lkb::CudaPtr<void> nrm2;       // one W
+    lkb::CudaPtr<double> inv;      // one double
+    lkb::CudaPtr<int> flags;       // F_COUNT ints
+    lkb::CudaPtr<unsigned> counter;
+    lkb::CudaPtr<void> Hd; size_t Hd_bytes = 0;
+    // coefd and hstage are views of the two owners below.  (The host-shell test mocks point them at host memory that they
+    // allocate and free themselves, and leave the owners empty.)
     void* coefd = nullptr; size_t coefd_bytes = 0;
-    // pinned host staging
-    void* hstage = nullptr; size_t hstage_bytes = 0;
+    void* hstage = nullptr; size_t hstage_bytes = 0;     // pinned host staging
+    lkb::CudaPtr<void> coefd_mem;
+    lkb::PinnedPtr hstage_mem;
     uint64_t seed = 0x1234abcdULL, seed_calls = 0;
     bool graphs = true;
     bool fused = true;
@@ -68,8 +105,12 @@ struct lkb_ctx_s {
     bool fused_halo = true;     // P2P halo push fused into the kernel that finishes the next matvec input
     // in-kernel NVLink allreduce (CUDA IPC peer buffers); falls back to NCCL when not attached
     bool p2p_active = false;
-    lkb::P2P p2p;
-    void* p2p_region = nullptr;
+    lkb::P2P p2p;               // kernel view of the four owners below
+    lkb::CudaPtr<void> p2p_region;
+    lkb::CudaPtr<unsigned> p2p_epoch;
+    lkb::CudaPtr<unsigned long long> ktime;      // lkb_debug_ktime
+    lkb::IpcMap peer_map[lkb::P2P_MAXW];
+    lkb::CommOwner comm;
     const lkb::P2P* p2p_arg() const { return (p2p_active || p2p.dbg) ? &p2p : nullptr; }
     bool capturing = false;
     bool profile = false;
@@ -78,8 +119,7 @@ struct lkb_ctx_s {
     int64_t prof_n[lkb::PC_COUNT] = {0, 0, 0, 0, 0, 0, 0, 0};
     struct ProfEv { int cls; cudaEvent_t a, b; };
     std::vector<ProfEv> prof_evs;
-    struct GraphEntry { cudaGraphExec_t exec; int64_t launches; };
-    std::map<std::string, GraphEntry> graph_cache;
+    std::map<std::string, lkb::GraphExec> graph_cache;
 };
 
 struct lkb_vec_s {
@@ -95,20 +135,23 @@ struct lkb_op_s {
     int64_t n_matvec = 0, n_rmatvec = 0;
     // stencil
     lkb::StencilArgs st; int64_t slow0 = 0, nslow_global = 0;
-    void* halo_lo = nullptr; void* halo_hi = nullptr; int64_t halo_elems = 0;
-    lkb::HaloP2P hp; bool hp_active = false; void* hp_lo_map = nullptr; void* hp_hi_map = nullptr;
+    lkb::CudaPtr<void> halo_lo, halo_hi; int64_t halo_elems = 0;
+    // P2P halo exchange: hp views this rank's halo region, its counters and the neighbours' regions mapped into this process
+    lkb::HaloP2P hp; bool hp_active = false;
+    lkb::CudaPtr<void> hp_region; lkb::CudaPtr<unsigned> hp_ctr; lkb::IpcMap hp_lo_map, hp_hi_map;
     // csr (+ explicit transpose for rmatvec)
-    int64_t* rowptr = nullptr; int32_t* col = nullptr; void* val = nullptr; int lpr = 8;
-    int64_t* t_rowptr = nullptr; int32_t* t_col = nullptr; void* t_val = nullptr; int t_lpr = 8;
+    lkb::CudaPtr<int64_t> rowptr; lkb::CudaPtr<int32_t> col; lkb::CudaPtr<void> val; int lpr = 8;
+    lkb::CudaPtr<int64_t> t_rowptr; lkb::CudaPtr<int32_t> t_col; lkb::CudaPtr<void> t_val; int t_lpr = 8;
     lkb::CsrBlocked blk, t_blk;                   // L2-blocked layouts (nb > 0: they replace the plain arrays above)
+    lkb::CsrBlockedMem blk_mem, t_blk_mem;
     // row-sharded csr: full-length gather / scatter buffers and every rank's (offset, count) of the column and row spaces
     bool dist = false; int64_t m_global = 0, n_global = 0;
-    void* x_full = nullptr; void* y_full = nullptr; void* y_red = nullptr;
+    lkb::CudaPtr<void> x_full, y_full, y_red;
     std::vector<int64_t> col_off, col_cnt, row_off, row_cnt;
     // dense
-    void* a = nullptr;
+    lkb::CudaPtr<void> a;
     // diagonal: y = d o x, d laid out like the vectors it applies to (global index of the first row, global length)
-    void* diag = nullptr; int64_t diag_row0 = 0, diag_n_global = 0;
+    lkb::CudaPtr<void> diag; int64_t diag_row0 = 0, diag_n_global = 0;
     // callback
     int (*fn)(void*, const void*, void*, int32_t, void*) = nullptr; void* user = nullptr; bool capturable = false;
     uint64_t uid = 0;
@@ -122,6 +165,20 @@ namespace lkb {
 
 int dev_alloc(lkb_ctx_s* c, void** p, size_t bytes);   // stream-ordered, pooled (vectors, bases, solver work space)
 void dev_free(lkb_ctx_s* c, void* p);
+// Fill an owner with `bytes` of cudaMalloc memory (of pinned host memory for a PinnedPtr).  A failure clears the runtime's
+// last error, so that it is not reported again by the next launch check.
+template <class T, auto Release> int cuda_alloc(Owner<T, Release>& o, size_t bytes) {
+    constexpr bool host = Release == cudaFreeHost;
+    void* p = nullptr;
+    const cudaError_t e = host ? cudaMallocHost(&p, bytes) : cudaMalloc(&p, bytes);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        set_error("%s(%zu) failed: %s", host ? "cudaMallocHost" : "cudaMalloc", bytes, cudaGetErrorString(e));
+        return LKB_ERR_ALLOC;
+    }
+    o.reset((T)p);
+    return 0;
+}
 int ensure_ws(lkb_ctx_s* c, int jp);                 // grow partial / c1 / c2 for jp = j+1 coefficients
 int ensure_hstage(lkb_ctx_s* c, size_t bytes);
 int ensure_Hd(lkb_ctx_s* c, size_t bytes);
@@ -192,25 +249,6 @@ inline void store_kind(int kind, void* base, size_t idx, cd v) {
 }
 inline Scalar to_scalar(cd v) { return Scalar{v.real(), v.imag()}; }
 
-// ---- scope owners of a solver's work space: every return path releases it, in reverse order of declaration ----
-// (The host-shell test mocks replace lkb_basis_destroy, lkb_vec_destroy and dev_free; an owner whose release calls the CUDA
-// runtime directly is defined in its .cu file.)
-template <class T, int (*Destroy)(T)> class Owner {
-  public:
-    Owner() = default;
-    Owner(Owner&& o) noexcept : p_(o.p_) { o.p_ = nullptr; }
-    Owner& operator=(Owner&& o) noexcept { std::swap(p_, o.p_); return *this; }
-    Owner(const Owner&) = delete;
-    Owner& operator=(const Owner&) = delete;
-    ~Owner() { if (p_) Destroy(p_); }
-    T* out() { return &p_; }                   // for the create call that fills an empty owner
-    operator T() const { return p_; }
-    T operator->() const { return p_; }
-  private:
-    T p_ = nullptr;
-};
-typedef Owner<lkb_basis_t, lkb_basis_destroy> BasisOwner;
-typedef Owner<lkb_vec_t, lkb_vec_destroy> VecOwner;
 // a dev_alloc buffer
 struct DevBuf {
     lkb_ctx_s* c; void* p = nullptr;
@@ -220,16 +258,7 @@ struct DevBuf {
     ~DevBuf() { dev_free(c, p); }
     int alloc(size_t bytes) { return dev_alloc(c, &p, bytes); }
 };
-// an instantiated CUDA graph and the kernel launches one replay stands for (destructor in lkb_krylov.cu)
-struct GraphExec {
-    cudaGraphExec_t exec = nullptr;
-    int64_t launches = 0;
-    GraphExec() = default;
-    GraphExec(const GraphExec&) = delete;
-    GraphExec& operator=(const GraphExec&) = delete;
-    ~GraphExec();
-};
 // Run `body` (which only enqueues work on c->stream) under stream capture with c->capturing set, and instantiate the graph.
-// The launches the body counted go to *launches, not to c->launches.  `what` prefixes the error messages ("gmres: ").
-int capture_graph(lkb_ctx_s* c, const char* what, const std::function<int()>& body, cudaGraphExec_t* exec, int64_t* launches);
+// The launches the body counted go to g->launches, not to c->launches.  `what` prefixes the error messages ("gmres: ").
+int capture_graph(lkb_ctx_s* c, const char* what, const std::function<int()>& body, GraphExec* g);
 }  // namespace lkb

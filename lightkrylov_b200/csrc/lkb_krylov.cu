@@ -56,14 +56,14 @@ int dgs_enqueue(lkb_ctx_s* c, int kind, const void* V, int64_t ld, int j, void* 
     }
     LKB_TRY(allreduce_w(c, c->c2, nd));
     if (want_gsinfo) {
-        launch_gsinfo(c->stream, (char*)c->c2 + (size_t)j * wsz, kind_cplx(kind), atol_of(kind), c->flags);
+        launch_gsinfo(c->stream, (char*)c->c2.get() + (size_t)j * wsz, kind_cplx(kind), atol_of(kind), c->flags);
         c->launches++;
     }
     if (fin) {
         // pass-2 update + predicted-norm normalisation + H/T/B column + (optional) halo push in ONE kernel
         prof_begin(c, PC_AXPY);
         SweepDir sd(d0);
-        launch_multiaxpy_fin(kind, c->stream, V, ld, j, fin->with_c1 ? c->c1 : nullptr, c->c2, w, n, c->partial, c->nrm2, c->counter,
+        launch_multiaxpy_fin(kind, c->stream, V, ld, j, fin->with_c1 ? c->c1.get() : nullptr, c->c2, w, n, c->partial, c->nrm2, c->counter,
                              fin->hcol, fin->tol, atol_of(kind), c->inv, flags, fin->kstep, fin->mode, c->sms, c->p2p_arg(), fin->hp);
         prof_end(c, PC_AXPY, 1);
         return check_launch(c, "multiaxpy_fin");
@@ -91,7 +91,7 @@ int step_tail_enqueue(lkb_ctx_s* c, int kind, const void* V, int64_t ld, int j, 
     } else {
         LKB_TRY(dgs_enqueue(c, kind, V, ld, j, w, n, c->flags, true, false));
         prof_begin(c, PC_OTHER);
-        launch_update(kind, c->stream, mode == 0 ? c->c1 : nullptr, mode == 0 ? c->c2 : nullptr, j, c->nrm2, hcol, tol,
+        launch_update(kind, c->stream, mode == 0 ? c->c1.get() : nullptr, mode == 0 ? c->c2.get() : nullptr, j, c->nrm2, hcol, tol,
                       atol_of(kind), c->inv, c->flags, kstep, mode);
         prof_end(c, PC_OTHER, 1);
     }
@@ -101,9 +101,7 @@ int step_tail_enqueue(lkb_ctx_s* c, int kind, const void* V, int64_t ld, int j, 
     return check_launch(c, "step tail");
 }
 
-GraphExec::~GraphExec() { if (exec) cudaGraphExecDestroy(exec); }
-
-int capture_graph(lkb_ctx_s* c, const char* what, const std::function<int()>& body, cudaGraphExec_t* exec, int64_t* launches) {
+int capture_graph(lkb_ctx_s* c, const char* what, const std::function<int()>& body, GraphExec* ge) {
     const int64_t l0 = c->launches;
     cudaError_t e = cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal);
     if (e != cudaSuccess) { set_error("%sgraph capture failed: %s", what, cudaGetErrorString(e)); return LKB_ERR_CUDA; }
@@ -112,10 +110,10 @@ int capture_graph(lkb_ctx_s* c, const char* what, const std::function<int()>& bo
     c->capturing = false;
     cudaGraph_t g = nullptr;
     e = cudaStreamEndCapture(c->stream, &g);
-    *launches = c->launches - l0;
+    ge->launches = c->launches - l0;
     c->launches = l0;
     if (r == 0 && e != cudaSuccess) { set_error("%sgraph capture failed: %s", what, cudaGetErrorString(e)); r = LKB_ERR_CUDA; }
-    if (r == 0 && cudaGraphInstantiate(exec, g, 0) != cudaSuccess) { set_error("%sgraph instantiate failed", what); r = LKB_ERR_CUDA; }
+    if (r == 0 && cudaGraphInstantiate(ge->exec.out(), g, 0) != cudaSuccess) { set_error("%sgraph instantiate failed", what); r = LKB_ERR_CUDA; }
     if (g) cudaGraphDestroy(g);
     return r;
 }
@@ -125,13 +123,10 @@ static int run_maybe_graph(lkb_ctx_s* c, bool allow_graph, const std::string& ke
     if (!(c->graphs && allow_graph) || c->profile) return body();
     auto it = c->graph_cache.find(key);
     if (it == c->graph_cache.end()) {
-        lkb_ctx_s::GraphEntry ent{nullptr, 0};
-        LKB_TRY(capture_graph(c, "", body, &ent.exec, &ent.launches));
-        if (c->graph_cache.size() > 4096) {   // bound the cache
-            for (auto& kv : c->graph_cache) cudaGraphExecDestroy(kv.second.exec);
-            c->graph_cache.clear();
-        }
-        it = c->graph_cache.emplace(key, ent).first;
+        GraphExec ge;
+        LKB_TRY(capture_graph(c, "", body, &ge));
+        if (c->graph_cache.size() > 4096) c->graph_cache.clear();   // bound the cache
+        it = c->graph_cache.emplace(key, std::move(ge)).first;
     }
     LKB_CUDA(cudaGraphLaunch(it->second.exec, c->stream));
     c->launches += it->second.launches;
@@ -302,7 +297,7 @@ static int gs_common(lkb_basis_t X, int j, lkb_basis_t W, int wcol0, int p, int3
             launch_multidot(X->kind, c->stream, X->d, X->ld, j, w, X->n, c->partial, c->c1, c->counter, nullptr, c->sms, c->p2p_arg());
             prof_end(c, PC_DOT, 1);
             LKB_TRY(allreduce_w(c, c->c1, (size_t)(j + 1) * (kind_cplx(X->kind) ? 2 : 1)));
-            launch_gsinfo(c->stream, (char*)c->c1 + (size_t)j * (kind_cplx(X->kind) ? 16 : 8), 0, atol_of(X->kind), c->flags);
+            launch_gsinfo(c->stream, (char*)c->c1.get() + (size_t)j * (kind_cplx(X->kind) ? 16 : 8), 0, atol_of(X->kind), c->flags);
             prof_begin(c, PC_AXPY);
             launch_multiaxpy(X->kind, c->stream, X->d, X->ld, j, c->c1, w, X->n, false, c->partial, c->nrm2, c->counter, nullptr, c->sms, c->p2p_arg());
             prof_end(c, PC_AXPY, 1);
@@ -540,7 +535,7 @@ int arnoldi_enqueue(lkb_op_s* A, lkb_basis_s* X, int kstart, int kend, double to
             LKB_TRY(op_apply_enqueue(A, col_ptr(X, k - 1), w, tr, c->flags, pushed));
             // the kernel that finishes X(k) also pushes its halo rows for the next step's matvec
             const HaloP2P* hp = (k < kend) ? op_halo_desc(A) : nullptr;
-            LKB_TRY(step_tail_enqueue(c, kind, X->d, X->ld, k, w, X->n, 0, tol, k, (char*)c->Hd + (size_t)ldhd * (k - 1) * es, hp));
+            LKB_TRY(step_tail_enqueue(c, kind, X->d, X->ld, k, w, X->n, 0, tol, k, (char*)c->Hd.get() + (size_t)ldhd * (k - 1) * es, hp));
             pushed = hp != nullptr;
         }
         return 0;
@@ -696,7 +691,7 @@ int lanczos_enqueue(lkb_op_s* A, lkb_basis_s* X, int kstart, int kend, double to
         bool pushed = false;
         for (int k = kstart; k <= kend; ++k) {
             void* w = col_ptr(X, k);
-            char* tcol = (char*)c->Hd + (size_t)ldtd * (k - 1) * es;
+            char* tcol = (char*)c->Hd.get() + (size_t)ldtd * (k - 1) * es;
             LKB_TRY(op_apply_enqueue(A, col_ptr(X, k - 1), w, false, c->flags, pushed));
             for (int i = (k - 1 > 1 ? k - 1 : 1); i <= k; ++i) {        // update_tridiag_matrix :57-59
                 void* xi = col_ptr(X, i - 1);
@@ -722,7 +717,7 @@ int krylov_fetch_async(lkb_ctx_s* c, int kind, int ldd, int kstart, int kend, vo
     const size_t es = kind_size(kind);
     const int ncol = kend - kstart + 1;
     char* hs = (char*)host;
-    LKB_CUDA(cudaMemcpyAsync(hs, (char*)c->Hd + (size_t)ldd * (kstart - 1) * es, (size_t)ldd * ncol * es, cudaMemcpyDeviceToHost, c->stream));
+    LKB_CUDA(cudaMemcpyAsync(hs, (char*)c->Hd.get() + (size_t)ldd * (kstart - 1) * es, (size_t)ldd * ncol * es, cudaMemcpyDeviceToHost, c->stream));
     LKB_CUDA(cudaMemcpyAsync(hs + (size_t)ldd * ncol * es, c->flags, F_COUNT * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     return 0;
 }
@@ -783,7 +778,7 @@ int bidiag_enqueue(lkb_op_s* A, lkb_basis_s* U, lkb_basis_s* V, int kstart, int 
         LKB_TRY(reset_flags(c));
         PdlScope pdl(c->pdl && !c->profile);
         for (int k = kstart; k <= kend; ++k) {
-            char* bcol = (char*)c->Hd + (size_t)ldbd * (k - 1) * es;
+            char* bcol = (char*)c->Hd.get() + (size_t)ldbd * (k - 1) * es;
             void* vk = col_ptr(V, k - 1);
             LKB_TRY(op_apply_enqueue(A, col_ptr(U, k - 1), vk, true, c->flags));
             LKB_TRY(step_tail_enqueue(c, kind, V->d, V->ld, k - 1, vk, V->n, 2, tol, 2 * k - 1, bcol, nullptr));

@@ -156,7 +156,7 @@ static int gmres_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, doubl
         LKB_TRY(gres.alloc((size_t)(kdim + 2) * 8));
         LKB_TRY(ensure_ws(c, kdim + 1));
         if (c->graphs && !c->profile && op_capturable(A) && (!M || op_capturable(M)))
-            LKB_TRY(capture_graph(c, "gmres: ", enqueue_cycle, &cycle.exec, &cycle.launches));
+            LKB_TRY(capture_graph(c, "gmres: ", enqueue_cycle, &cycle));
     }
     while (!io->converged && io->n_outer <= maxiter) {
         std::fill(H.begin(), H.end(), cd(0));
@@ -367,7 +367,7 @@ static int cg_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double r
             LKB_TRY(allreduce_w(c, c->tmpw, ndw));
             prof_begin(c, PC_OTHER);
             launch_cg_update(kind, c->stream, scal.p, c->tmpw, p->d, Ap->d, x->d, r->d, b->n, c->partial, c->nrm2, c->counter,
-                             c->flags, c->sms, c->p2p_arg(), mode, mode == CG_DIAG ? M->diag : nullptr);
+                             c->flags, c->sms, c->p2p_arg(), mode, mode == CG_DIAG ? M->diag.get() : nullptr);
             prof_end(c, PC_OTHER, 1);
             const void* rr_new = c->nrm2;
             if (mode == CG_NORED) {         // z = M r ; rz = r^H z (multi-dot, j = 1: c2[0])
@@ -383,7 +383,7 @@ static int cg_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double r
             prof_begin(c, PC_OTHER);
             launch_cg_check(kind, c->stream, scal.p, rr_new, tol, maxiter, (double*)res_hist.p, c->flags);
             launch_cg_direction(kind, c->stream, scal.p, mode == CG_NORED ? z->d : r->d, p->d, b->n, c->flags, c->sms,
-                                mode == CG_DIAG ? M->diag : nullptr);
+                                mode == CG_DIAG ? M->diag.get() : nullptr);
             prof_end(c, PC_OTHER, 2);
             return check_launch(c, "cg iteration");
         };
@@ -392,7 +392,7 @@ static int cg_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double r
             return 0;
         };
         if (c->graphs && !c->profile && op_capturable(A) && (!M || op_capturable(M)))
-            LKB_TRY(capture_graph(c, "cg: ", one_chunk, &chunk.exec, &chunk.launches));
+            LKB_TRY(capture_graph(c, "cg: ", one_chunk, &chunk));
         int hf[F_COUNT] = {0};
         while (true) {
             if (chunk.exec) { LKB_CUDA(cudaGraphLaunch(chunk.exec, c->stream)); c->launches += chunk.launches; }
