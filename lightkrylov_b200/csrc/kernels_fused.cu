@@ -317,39 +317,44 @@ static PFN_tmapEncodeTiled get_encode() {
 }
 
 template <int K>
+static bool axpy_dot_ok(const void* V, int64_t ld, int j, const void* w, int64_t n) {
+    constexpr int EPP = Tr<K>::EPP;
+    const size_t es = sizeof(typename Tr<K>::E);
+    const int eltsz = (K == KS) ? 4 : 8;                           // tensor described in 4- or 8-byte words
+    if (j < 1 || j > FZ_NW * FZ_CB) return false;                 // one 16-column chunk per warp
+    if (n % EPP != 0 || n < 32 * EPP) return false;
+    if (((uintptr_t)V & 15) || ((uintptr_t)w & 15) || ((size_t)ld * es) % 16) return false;
+    return get_encode() && (int64_t)n * (int64_t)es / eltsz < ((int64_t)1 << 31);
+}
+
+template <int K>
 static bool axpy_dot_t(cudaStream_t s, const void* V, int64_t ld, int j, const void* c1, void* w, int64_t n,
                        void* partial, void* out, unsigned* counter, const int* flags, int sms, const P2P* p2p) {
     using E = typename Tr<K>::E; using W = typename Tr<K>::W;
     constexpr int EPP = Tr<K>::EPP;
     const size_t es = sizeof(E);
-    if (j < 1 || j > FZ_NW * FZ_CB) return false;                 // one 16-column chunk per warp
-    if (n % EPP != 0 || n < 32 * EPP) return false;
-    if (((uintptr_t)V & 15) || ((uintptr_t)w & 15) || ((size_t)ld * es) % 16) return false;
-    PFN_tmapEncodeTiled enc = get_encode();
-    if (!enc) return false;
     const int jc = (j + FZ_CB - 1) & ~(FZ_CB - 1);
     // rows per tile: stage = jc * tp * 16 B <= 64 KB; few columns -> taller tiles, so the per-tile
     // synchronisation cost (~1500 clk) stays small against the tile's HBM time (TMA box rows <= 256 words)
     const int tp = jc > 64 ? 32 : ((jc > 32 || K == KS) ? 64 : 128);
     const int eltsz = (K == KS) ? 4 : 8;                           // tensor described in 4- or 8-byte words
     const int elt_per_pack = 16 / eltsz;
-    if ((int64_t)n * (int64_t)es / eltsz >= ((int64_t)1 << 31)) return false;
     CUtensorMap tmap;
     cuuint64_t gdim[2] = {(cuuint64_t)((size_t)n * es / eltsz), (cuuint64_t)j};
     cuuint64_t gstr[1] = {(cuuint64_t)((size_t)ld * es)};
     cuuint32_t box[2] = {(cuuint32_t)(tp * elt_per_pack), (cuuint32_t)jc};   // one box = the whole tile
     cuuint32_t estr[2] = {1, 1};
-    CUresult r = enc(&tmap, eltsz == 4 ? CU_TENSOR_MAP_DATA_TYPE_UINT32 : CU_TENSOR_MAP_DATA_TYPE_UINT64, 2,
-                     const_cast<void*>(V), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    CUresult r = get_encode()(&tmap, eltsz == 4 ? CU_TENSOR_MAP_DATA_TYPE_UINT32 : CU_TENSOR_MAP_DATA_TYPE_UINT64, 2,
+                              const_cast<void*>(V), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                              CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return false;
     // as many stages as fit: the ring must keep >= ~100 KB in flight per SM to cover the ~2 us loaded
-    // TMA latency at 23 B/clk/SM (measured: 3 x 40 KB stages ran latency-bound at 5.0 TB/s)
+    // TMA latency at 23 B/clk/SM (measured: 3 x 40 KB stages ran latency-bound at 5.0 TB/s).  Any j <= 128 leaves room
+    // for at least 3 stages of <= 66 KB.
     const size_t budget = 222 * 1024;
     const size_t fixed = (size_t)(FZ_NW + 1) * tp * 16 + 128;
     int nst = (int)((budget - fixed) / ((size_t)jc * tp * 16 + (size_t)tp * 16 + 16));
     if (nst > FZ_MAXSTAGES) nst = FZ_MAXSTAGES;
-    if (nst < 2) return false;
     const size_t sh = (size_t)nst * jc * tp * 16 + (size_t)(FZ_NW + 1 + nst) * tp * 16 + 16 * nst + 64;
     static const SmemAttrOnce attr((const void*)k_axpy_dot<K>, 224 * 1024);
     attr.ensure();
@@ -362,6 +367,14 @@ static bool axpy_dot_t(cudaStream_t s, const void* V, int64_t ld, int j, const v
     return true;
 }
 
+bool axpy_dot_supported(int kind, const void* V, int64_t ld, int j, const void* w, int64_t n) {
+    switch (kind) {
+        case KS: return axpy_dot_ok<KS>(V, ld, j, w, n);
+        case KD: return axpy_dot_ok<KD>(V, ld, j, w, n);
+        case KC: return axpy_dot_ok<KC>(V, ld, j, w, n);
+        default: return axpy_dot_ok<KZ>(V, ld, j, w, n);
+    }
+}
 bool launch_axpy_dot(int kind, cudaStream_t s, const void* V, int64_t ld, int j, const void* c1, void* w, int64_t n,
                      void* partial, void* out, unsigned* counter, const int* flags, int sms, const P2P* p2p) {
     switch (kind) {

@@ -214,14 +214,6 @@ __global__ void k_gsinfo(const double* __restrict__ ww, double atol, int* __rest
 }
 
 template <int K>
-__global__ void k_wadd(const typename Tr<K>::W* a, const typename Tr<K>::W* b, typename Tr<K>::W* out, int n,
-                       const int* flags) {
-    if (flags && flags[F_STOP]) return;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        typename Tr<K>::W t = a[i]; wadd(t, b[i]); out[i] = t;
-    }
-}
-template <int K>
 __global__ void k_narrow(const typename Tr<K>::W* src, typename Tr<K>::E* dst, int n, const int* flags) {
     if (flags && flags[F_STOP]) return;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) narrow(src[i], dst[i]);
@@ -615,12 +607,6 @@ void launch_gmres_update(int kind, cudaStream_t s, const void* c1, const void* c
 }
 void launch_gsinfo(cudaStream_t s, const void* ww, int, double atol, int* flags) {
     k_gsinfo<<<1, 1, 0, s>>>((const double*)ww, atol, flags);
-}
-void launch_wadd(int kind, cudaStream_t s, const void* a, const void* b, void* out, int n, const int* flags) {
-    LKB_DISPATCH(kind, {
-        using W = typename Tr<K>::W;
-        k_wadd<K><<<1, 256, 0, s>>>((const W*)a, (const W*)b, (W*)out, n, flags);
-    });
 }
 void launch_narrow(int kind, cudaStream_t s, const void* src, void* dst, int n, const int* flags) {
     LKB_DISPATCH(kind, {

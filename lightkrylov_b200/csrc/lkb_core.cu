@@ -183,11 +183,7 @@ int fetch_flags(lkb_ctx_s* c, int* host_flags) {
 
 int norm2_enqueue(lkb_ctx_s* c, int kind, const void* w, int64_t n, const int* flags) {
     LKB_TRY(ensure_ws(c, 1));
-    prof_begin(c, PC_DOT);
-    launch_multidot(kind, c->stream, w, n, 0, w, n, c->partial, c->nrm2, c->counter, flags, c->sms, c->p2p_arg());
-    prof_end(c, PC_DOT, 1);
-    LKB_TRY(check_launch(c, "norm2"));
-    return allreduce_w(c, c->nrm2, 1);
+    return dot_reduce(c, kind, w, n, 0, w, n, c->nrm2, flags);
 }
 int vec_norm_sync(lkb_ctx_s* c, int kind, const void* w, int64_t n, double* out) {
     LKB_TRY(norm2_enqueue(c, kind, w, n, nullptr));
@@ -199,11 +195,7 @@ int vec_norm_sync(lkb_ctx_s* c, int kind, const void* w, int64_t n, double* out)
 }
 int vec_dot_sync(lkb_ctx_s* c, int kind, const void* x, const void* y, int64_t n, Scalar* out) {
     LKB_TRY(ensure_ws(c, 2));
-    prof_begin(c, PC_DOT);
-    launch_multidot(kind, c->stream, x, n, 1, y, n, c->partial, c->tmpw, c->counter, nullptr, c->sms, c->p2p_arg());
-    prof_end(c, PC_DOT, 1);
-    LKB_TRY(check_launch(c, "dot"));
-    LKB_TRY(allreduce_w(c, c->tmpw, kind_cplx(kind) ? 2 : 1));
+    LKB_TRY(dot_reduce(c, kind, x, n, 1, y, n, c->tmpw, nullptr));
     LKB_TRY(ensure_hstage(c, 4096));
     LKB_CUDA(cudaMemcpyAsync(c->hstage, c->tmpw, 16, cudaMemcpyDeviceToHost, c->stream));
     LKB_CUDA(cudaStreamSynchronize(c->stream));
@@ -398,9 +390,7 @@ int lkb_vec_zero(lkb_vec_t v) {
     return 0;
 }
 int lkb_vec_fill_random(lkb_vec_t v, int dist, uint64_t seed) {
-    prof_begin(v->ctx, PC_OTHER);
-    launch_fill(v->kind, v->ctx->stream, v->d, v->n, v->row0, dist, seed, v->ctx->sms);
-    prof_end(v->ctx, PC_OTHER, 1);
+    prof_launch(v->ctx, PC_OTHER, 1, [&] { launch_fill(v->kind, v->ctx->stream, v->d, v->n, v->row0, dist, seed, v->ctx->sms); });
     return check_launch(v->ctx, "fill");
 }
 int lkb_vec_rand(lkb_vec_t v, int32_t ifnorm) {
@@ -408,25 +398,21 @@ int lkb_vec_rand(lkb_vec_t v, int32_t ifnorm) {
     if (ifnorm) {
         double nrm = 0;
         LKB_TRY(vec_norm_sync(v->ctx, v->kind, v->d, v->n, &nrm));
-        Scalar a{1.0 / nrm, 0.0};
-        launch_scal(v->kind, v->ctx->stream, a, v->d, v->n, v->ctx->sms);
-        v->ctx->launches++;
+        prof_launch(v->ctx, PC_OTHER, 1, [&] { launch_scal(v->kind, v->ctx->stream, Scalar{1.0 / nrm, 0.0}, v->d, v->n, v->ctx->sms); });
         return check_launch(v->ctx, "scal");
     }
     return 0;
 }
 int lkb_vec_scal(lkb_vec_t v, const void* alpha) {
-    prof_begin(v->ctx, PC_OTHER);
-    launch_scal(v->kind, v->ctx->stream, to_scalar(load_kind(v->kind, alpha, 0)), v->d, v->n, v->ctx->sms);
-    prof_end(v->ctx, PC_OTHER, 1);
+    prof_launch(v->ctx, PC_OTHER, 1, [&] { launch_scal(v->kind, v->ctx->stream, to_scalar(load_kind(v->kind, alpha, 0)), v->d, v->n, v->ctx->sms); });
     return check_launch(v->ctx, "scal");
 }
 int lkb_vec_axpby(const void* alpha, lkb_vec_t x, const void* beta, lkb_vec_t self) {
     if (!x || !self || x->n != self->n || x->kind != self->kind) { set_error("axpby: size/kind mismatch"); return LKB_ERR_ARG; }
-    prof_begin(self->ctx, PC_OTHER);
-    launch_axpby(self->kind, self->ctx->stream, to_scalar(load_kind(self->kind, alpha, 0)), x->d, to_scalar(load_kind(self->kind, beta, 0)),
-                 self->d, self->n, self->ctx->sms);
-    prof_end(self->ctx, PC_OTHER, 1);
+    prof_launch(self->ctx, PC_OTHER, 1, [&] {
+        launch_axpby(self->kind, self->ctx->stream, to_scalar(load_kind(self->kind, alpha, 0)), x->d, to_scalar(load_kind(self->kind, beta, 0)),
+                     self->d, self->n, self->ctx->sms);
+    });
     return check_launch(self->ctx, "axpby");
 }
 int lkb_vec_dot(lkb_vec_t self, lkb_vec_t vec, void* out) {
@@ -494,10 +480,8 @@ int lkb_basis_axpby(const void* alpha, lkb_basis_t X, int xcol0, const void* bet
         X->n != Y->n || X->kind != Y->kind) { set_error("basis_axpby: bad arguments"); return LKB_ERR_ARG; }
     lkb_ctx_s* c = Y->ctx;
     const Scalar a = to_scalar(load_kind(Y->kind, alpha, 0)), bb = to_scalar(load_kind(Y->kind, beta, 0));
-    for (int q = 0; q < ncols; ++q) {
-        launch_axpby(Y->kind, c->stream, a, col_ptr(X, xcol0 + q), bb, col_ptr(Y, ycol0 + q), Y->n, c->sms);
-        c->launches++;
-    }
+    for (int q = 0; q < ncols; ++q)
+        prof_launch(c, PC_OTHER, 1, [&] { launch_axpby(Y->kind, c->stream, a, col_ptr(X, xcol0 + q), bb, col_ptr(Y, ycol0 + q), Y->n, c->sms); });
     return check_launch(c, "basis_axpby");
 }
 // rand_basis (AbstractVectors.fypp:725-730)
@@ -506,13 +490,11 @@ int lkb_basis_rand(lkb_basis_t b, int col0, int ncols, int32_t ifnorm) {
     lkb_ctx_s* c = b->ctx;
     for (int q = 0; q < ncols; ++q) {
         void* w = col_ptr(b, col0 + q);
-        launch_fill(b->kind, c->stream, w, b->n, b->row0, LKB_DIST_NORMAL, next_seed(c), c->sms);
-        c->launches++;
+        prof_launch(c, PC_OTHER, 1, [&] { launch_fill(b->kind, c->stream, w, b->n, b->row0, LKB_DIST_NORMAL, next_seed(c), c->sms); });
         if (ifnorm) {
             double nrm = 0;
             LKB_TRY(vec_norm_sync(c, b->kind, w, b->n, &nrm));
-            launch_scal(b->kind, c->stream, Scalar{1.0 / nrm, 0.0}, w, b->n, c->sms);
-            c->launches++;
+            prof_launch(c, PC_OTHER, 1, [&] { launch_scal(b->kind, c->stream, Scalar{1.0 / nrm, 0.0}, w, b->n, c->sms); });
         }
     }
     return check_launch(c, "basis_rand");
@@ -812,9 +794,9 @@ int lkb_op_reset_counters(lkb_op_t A) { A->n_matvec = A->n_rmatvec = 0; return 0
 }  // extern "C"
 
 namespace lkb {
-const HaloP2P* op_halo_desc(const lkb_op_s* A) {
+const HaloP2P* op_halo_desc(const lkb_op_s* A, int j) {
     const lkb_ctx_s* c = A->ctx;
-    return (A->type == OP_STENCIL && c->world > 1 && A->hp_active && c->p2p_active && c->fused_halo && c->fin) ? &A->hp : nullptr;
+    return (A->type == OP_STENCIL && c->world > 1 && A->hp_active && c->fused_halo && fin_usable(c, j)) ? &A->hp : nullptr;
 }
 int op_apply_enqueue(lkb_op_s* A, const void* x, void* y, bool trans, const int* flags, bool halo_prepushed) {
     lkb_ctx_s* c = A->ctx;

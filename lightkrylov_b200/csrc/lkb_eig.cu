@@ -250,9 +250,7 @@ int device_combine(lkb_basis_s* Xw, int k, const std::vector<cd>& Zc, int ldz, i
     LKB_CUDA(cudaStreamSynchronize(c->stream));
     for (int q = 0; q < p; ++q) for (int i = 0; i < k; ++i) store_kind(kind, c->hstage, (size_t)i + (size_t)k * q, Zc[i + (size_t)ldz * q]);
     LKB_CUDA(cudaMemcpyAsync(c->coefd, c->hstage, (size_t)k * p * es, cudaMemcpyHostToDevice, c->stream));
-    prof_begin(c, PC_OTHER);
-    launch_basis_gemm(kind, c->stream, Xw->d, Xw->ld, k, c->coefd, k, p, Yd, ldy, Xw->n, c->sms);
-    prof_end(c, PC_OTHER, 1);
+    prof_launch(c, PC_OTHER, 1, [&] { launch_basis_gemm(kind, c->stream, Xw->d, Xw->ld, k, c->coefd, k, p, Yd, ldy, Xw->n, c->sms); });
     return check_launch(c, "basis_gemm");
 }
 
@@ -285,16 +283,13 @@ int start_vector(lkb_basis_s* Xw, lkb_vec_t x0) {
     LKB_TRY(lkb_basis_zero(Xw, 0, Xw->ncols));
     if (x0) {
         if (x0->n != Xw->n || x0->kind != kind) { set_error("x0: size/kind mismatch"); return LKB_ERR_ARG; }
-        launch_axpby(kind, c->stream, Scalar{1, 0}, x0->d, Scalar{0, 0}, Xw->d, Xw->n, c->sms);   // copy(Xwrk(1), x0)
-        c->launches++;
+        prof_launch(c, PC_OTHER, 1, [&] { launch_axpby(kind, c->stream, Scalar{1, 0}, x0->d, Scalar{0, 0}, Xw->d, Xw->n, c->sms); });   // copy(Xwrk(1), x0)
     } else {
-        launch_fill(kind, c->stream, Xw->d, Xw->n, Xw->row0, LKB_DIST_NORMAL, next_seed(c), c->sms);   // rand(.true.)
-        c->launches++;
+        prof_launch(c, PC_OTHER, 1, [&] { launch_fill(kind, c->stream, Xw->d, Xw->n, Xw->row0, LKB_DIST_NORMAL, next_seed(c), c->sms); });   // rand(.true.)
     }
     double nrm = 0;
     LKB_TRY(vec_norm_sync(c, kind, Xw->d, Xw->n, &nrm));
-    launch_scal(kind, c->stream, Scalar{1.0 / nrm, 0}, Xw->d, Xw->n, c->sms);
-    c->launches++;
+    prof_launch(c, PC_OTHER, 1, [&] { launch_scal(kind, c->stream, Scalar{1.0 / nrm, 0}, Xw->d, Xw->n, c->sms); });
     return check_launch(c, "start vector");
 }
 
@@ -345,9 +340,7 @@ int lkb_krylov_schur(lkb_basis_t X, void* H, int ldh, int kdim, int32_t* nkeep) 
         int r = 0;
         for (int64_t r0 = 0; r0 < X->n && r == 0; r0 += chunk) {
             const int64_t rows = std::min<int64_t>(chunk, X->n - r0);
-            prof_begin(c, PC_OTHER);
-            launch_basis_gemm(kind, c->stream, (char*)X->d + (size_t)r0 * es, X->ld, k, c->coefd, k, nk, tmp.p, chunk, rows, c->sms);
-            prof_end(c, PC_OTHER, 1);
+            prof_launch(c, PC_OTHER, 1, [&] { launch_basis_gemm(kind, c->stream, (char*)X->d + (size_t)r0 * es, X->ld, k, c->coefd, k, nk, tmp.p, chunk, rows, c->sms); });
             r = check_launch(c, "basis_gemm");
             if (r == 0 && cudaMemcpy2DAsync((char*)X->d + (size_t)r0 * es, (size_t)X->ld * es, tmp.p, (size_t)chunk * es,
                                             (size_t)rows * es, nk, cudaMemcpyDeviceToDevice, c->stream) != cudaSuccess) r = LKB_ERR_CUDA;
@@ -399,7 +392,7 @@ int lkb_eigs(lkb_op_t A, lkb_basis_t X, int nev, double* eigvals, double* residu
     if (ss.init((size_t)ldh * es + 256)) { set_error("eigs: pinned staging allocation failed"); return LKB_ERR_ALLOC; }
     auto enqueue_step = [&](int kk) -> int {
         LKB_TRY(arnoldi_enqueue(A, Xw, kk, kk, atolk, tr));
-        LKB_TRY(arnoldi_fetch_async(Xw, kk, kk, ss.slot[kk & 1]));
+        LKB_TRY(krylov_fetch_async(c, kind, Xw->ncols, kk, kk, ss.slot[kk & 1]));
         LKB_CUDA(cudaEventRecord(ss.ev[kk & 1], c->stream));
         return 0;
     };

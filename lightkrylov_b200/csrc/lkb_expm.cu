@@ -125,8 +125,7 @@ int lkb_kexpm_vec(lkb_vec_t cvec, lkb_op_t A, lkb_vec_t b, double tau, double to
     }
     BasisOwner X;
     LKB_TRY(lkb_basis_create(c, kind, b->n, b->n_global, b->row0, nk + 1, X.out()));
-    launch_axpby(kind, c->stream, Scalar{1.0 / beta, 0.0}, b->d, Scalar{0, 0}, X->d, b->n, c->sms);     // X(1) = b / beta
-    c->launches++;
+    prof_launch(c, PC_OTHER, 1, [&] { launch_axpby(kind, c->stream, Scalar{1.0 / beta, 0.0}, b->d, Scalar{0, 0}, X->d, b->n, c->sms); });   // X(1) = b / beta
     LKB_TRY(check_launch(c, "kexpm start"));
     const int ldh = nk + 1;
     std::vector<char> H((size_t)ldh * (nk + 1) * es, 0);          // (nk+1) x (nk+1) as in the reference (:170)

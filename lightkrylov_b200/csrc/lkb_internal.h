@@ -187,8 +187,11 @@ int allreduce_w(lkb_ctx_s* c, void* buf, size_t ndoubles);
 // make rank 0's copy of a small HOST array authoritative on every rank (k x k host-LAPACK results)
 int bcast_host(lkb_ctx_s* c, void* host_buf, size_t bytes);   // in-place sum over ranks (no-op when world == 1)
 int check_launch(lkb_ctx_s* c, const char* what);
+// The profile bracket: prof_end counts the launches in c->launches and, with lkb_set_profile, times them under class
+// `cls`.  Every kernel launch of the library goes through it exactly once (graph replays add their recorded count).
 void prof_begin(lkb_ctx_s* c, int cls);
 void prof_end(lkb_ctx_s* c, int cls, int nlaunch);
+template <class F> void prof_launch(lkb_ctx_s* c, int cls, int nlaunch, F&& launch) { prof_begin(c, cls); launch(); prof_end(c, cls, nlaunch); }
 int prof_collect(lkb_ctx_s* c);
 inline void* col_ptr(const lkb_basis_s* b, int i) { return (char*)b->d + (size_t)i * (size_t)b->ld * kind_size(b->kind); }
 inline double atol_of(int kind) { return (kind == KS || kind == KC) ? 1e-6 : 1e-15; }   // Constants.f90:18-37
@@ -197,13 +200,25 @@ inline double rtol_of(int kind) { return (kind == KS || kind == KC) ? 1e-3 : 3.1
 // halo_prepushed: x's boundary rows were already stored into the neighbours' halo buffers by the kernel that
 // finished x (k_multiaxpy_fin / k_scale_dev with a HaloP2P descriptor): skip the k_halo_push kernel.
 int op_apply_enqueue(lkb_op_s* A, const void* x, void* y, bool trans, const int* flags, bool halo_prepushed = false);
-// descriptor for a fused halo push of this operator's next input vector, or nullptr (single GPU / NCCL halos / not a stencil)
-const lkb::HaloP2P* op_halo_desc(const lkb_op_s* A);
+// The final CGS2 pass of a step against V(:, 0:j) may be k_multiaxpy_fin, which normalises with the predicted norm: not for
+// j = 0, not with option "fin" = 0, and not when the reductions go through ncclAllReduce (the predicted norm must not be
+// summed over ranks).
+inline bool fin_usable(const lkb_ctx_s* c, int j) { return c->fin && j > 0 && (c->world == 1 || c->p2p_active); }
+// descriptor for a fused halo push of this operator's next input vector by the final pass of a step against V(:, 0:j), or
+// nullptr (single GPU / NCCL halos / not a stencil / no k_multiaxpy_fin)
+const lkb::HaloP2P* op_halo_desc(const lkb_op_s* A, int j);
 // final-pass description of a CGS2 step that ends in k_multiaxpy_fin (see step_tail_enqueue)
 struct FinArgs { int mode; double tol; int kstep; void* hcol; bool with_c1; const lkb::HaloP2P* hp; };
+// multi-dot out(0:j) = V(:, 0:j)^H w, out(j) = w^H w, summed over the ranks
+int dot_reduce(lkb_ctx_s* c, int kind, const void* V, int64_t ld, int j, const void* w, int64_t n, void* out, const int* flags);
+// multi-axpy w -= V(:, 0:j) coef; with want_norm, nrm2 = ||w||^2 summed over the ranks
+int axpy_sub(lkb_ctx_s* c, int kind, const void* V, int64_t ld, int j, const void* coef, void* w, int64_t n, bool want_norm,
+             const int* flags);
 // enqueue one double Gram-Schmidt step of w against V(:, 0:j); leaves c1, c2 (and nrm2 if asked) in the workspace
 int dgs_enqueue(lkb_ctx_s* c, int kind, const void* V, int64_t ld, int j, void* w, int64_t n, int* flags,
                 bool want_norm, bool want_gsinfo, const FinArgs* fin = nullptr);
+// Read c1 + c2 (first j entries; only c1 unless `two`) and, optionally, nrm2 and the flags to the host (one sync)
+int fetch_coeffs(lkb_ctx_s* c, int kind, int j, bool two, std::vector<Scalar>& out, double* nrm2, int* flags);
 int step_tail_enqueue(lkb_ctx_s* c, int kind, const void* V, int64_t ld, int j, void* w, int64_t n, int mode, double tol,
                       int kstep, void* hcol, const lkb::HaloP2P* hp);
 int norm2_enqueue(lkb_ctx_s* c, int kind, const void* w, int64_t n, const int* flags);  // nrm2 <- ||w||^2
@@ -218,7 +233,6 @@ int csr_finish_device(lkb_ctx_s* c, lkb_op_s* op, int kind, int64_t rows, int64_
 uint64_t next_uid();
 void invalidate_graphs(lkb_ctx_s* c, uint64_t uid);   // uid == 0: all
 int arnoldi_enqueue(lkb_op_s* A, lkb_basis_s* X, int kstart, int kend, double tol, bool tr);
-int arnoldi_fetch_async(lkb_basis_s* X, int kstart, int kend, void* pinned_host);
 int arnoldi_collect(lkb_op_s* A, lkb_basis_s* X, void* H, int ldh, int32_t* info, int kstart, int kend, bool tr,
                     const void* pinned_host);
 int krylov_fetch_async(lkb_ctx_s* c, int kind, int ldd, int kstart, int kend, void* pinned_host);

@@ -134,8 +134,10 @@ void launch_multidot2(int kind, cudaStream_t s, const void* V, int64_t ld, int j
 void launch_multiaxpy2(int kind, cudaStream_t s, const void* V, int64_t ld, int j, const void* c, void* w0, void* w1,
                        int64_t n, const int* flags, int sms);
 // Fused pass-1 multi-axpy + pass-2 multi-dot (TMA + mbarrier pipeline, kernels_fused.cu):
-//   w -= V c1 ; out[0..j) = V^H w_new ; out[j] = w_new^H w_new.   Returns false when the shape is not
-//   supported (j > 128, ragged n, unaligned) -- the caller then runs the two separate kernels.
+//   w -= V c1 ; out[0..j) = V^H w_new ; out[j] = w_new^H w_new.   axpy_dot_supported is false when the shape is not
+//   supported (j > 128, ragged n, unaligned, no tensor-map encoder) -- the caller then runs the two separate kernels.
+//   launch_axpy_dot returns false, without launching, only when the driver rejects the tensor map: the same fallback.
+bool axpy_dot_supported(int kind, const void* V, int64_t ld, int j, const void* w, int64_t n);
 bool launch_axpy_dot(int kind, cudaStream_t s, const void* V, int64_t ld, int j, const void* c1, void* w, int64_t n,
                      void* partial, void* out, unsigned* counter, const int* flags, int sms, const P2P* p2p = nullptr);
 // y = alpha*x + beta*y  (beta == 0: y is overwritten without being read)
@@ -181,8 +183,6 @@ void launch_update(int kind, cudaStream_t s, const void* c1, const void* c2, int
                    double tol, double atol, void* inv_dev, int* flags, int kstep, int mode);
 // gs_info: flags[F_GSINFO] = (sqrt(|ww|) < atol)
 void launch_gsinfo(cudaStream_t s, const void* ww, int is_cplx, double atol, int* flags);
-// out[i] = a[i] + b[i] (W type, i < n) -- combine the two CGS passes
-void launch_wadd(int kind, cudaStream_t s, const void* a, const void* b, void* out, int n, const int* flags);
 // dst (E type) = src (W type) narrowed, length n
 void launch_narrow(int kind, cudaStream_t s, const void* src, void* dst, int n, const int* flags);
 

@@ -17,6 +17,20 @@ using namespace lkb;
 
 namespace lkb {
 
+int dot_reduce(lkb_ctx_s* c, int kind, const void* V, int64_t ld, int j, const void* w, int64_t n, void* out, const int* flags) {
+    prof_launch(c, PC_DOT, 1, [&] { launch_multidot(kind, c->stream, V, ld, j, w, n, c->partial, out, c->counter, flags, c->sms, c->p2p_arg()); });
+    LKB_TRY(check_launch(c, "multidot"));
+    return allreduce_w(c, out, (size_t)(j + 1) * (kind_cplx(kind) ? 2 : 1));
+}
+int axpy_sub(lkb_ctx_s* c, int kind, const void* V, int64_t ld, int j, const void* coef, void* w, int64_t n, bool want_norm,
+             const int* flags) {
+    prof_launch(c, PC_AXPY, 1, [&] {
+        launch_multiaxpy(kind, c->stream, V, ld, j, coef, w, n, want_norm, c->partial, c->nrm2, c->counter, flags, c->sms, c->p2p_arg());
+    });
+    LKB_TRY(check_launch(c, "multiaxpy"));
+    return want_norm ? allreduce_w(c, c->nrm2, 1) : 0;
+}
+
 int dgs_enqueue(lkb_ctx_s* c, int kind, const void* V, int64_t ld, int j, void* w, int64_t n, int* flags,
                 bool want_norm, bool want_gsinfo, const FinArgs* fin) {
     if (j <= 0) {
@@ -24,80 +38,60 @@ int dgs_enqueue(lkb_ctx_s* c, int kind, const void* V, int64_t ld, int j, void* 
         return 0;
     }
     LKB_TRY(ensure_ws(c, j + 1));
-    const size_t nd = (size_t)(j + 1) * (kind_cplx(kind) ? 2 : 1);
-    const size_t wsz = kind_cplx(kind) ? 16 : 8;
     // serpentine sweeps: pass-1 dot, fused middle and final update walk the rows in alternating directions, and the
     // first direction alternates with the step index (the previous step's final update ended where this one starts)
     const int d0 = (c->serpentine && fin) ? (fin->kstep & 1) : 0;
     const int d1 = (c->serpentine && fin) ? 1 - d0 : 0;
     // pass 1 coefficients
-    prof_begin(c, PC_DOT);
-    { SweepDir sd(d0); launch_multidot(kind, c->stream, V, ld, j, w, n, c->partial, c->c1, c->counter, flags, c->sms, c->p2p_arg()); }
-    prof_end(c, PC_DOT, 1);
-    LKB_TRY(check_launch(c, "multidot"));
-    LKB_TRY(allreduce_w(c, c->c1, nd));
+    { SweepDir sd(d0); LKB_TRY(dot_reduce(c, kind, V, ld, j, w, n, c->c1, flags)); }
     // pass-1 update fused with the pass-2 coefficients (V read once for both) when the shape allows
     bool fused = false;
-    if (c->fused) {
+    if (c->fused && axpy_dot_supported(kind, V, ld, j, w, n)) {
         prof_begin(c, PC_FUSED);
         { SweepDir sd(d1); fused = launch_axpy_dot(kind, c->stream, V, ld, j, c->c1, w, n, c->partial, c->c2, c->counter, flags, c->sms, c->p2p_arg()); }
-        prof_end(c, PC_FUSED, fused ? 1 : 0);
-        if (!fused && c->profile && !c->capturing) { cudaEventDestroy(c->prof_evs.back().a); cudaEventDestroy(c->prof_evs.back().b); c->prof_evs.pop_back(); }
+        prof_end(c, PC_FUSED, fused ? 1 : 0);       // (not launched only when the driver rejected the tensor map)
         LKB_TRY(check_launch(c, "axpy_dot"));
     }
-    if (!fused) {
-        prof_begin(c, PC_AXPY);
-        launch_multiaxpy(kind, c->stream, V, ld, j, c->c1, w, n, false, c->partial, c->nrm2, c->counter, flags, c->sms, c->p2p_arg());
-        prof_end(c, PC_AXPY, 1);
-        prof_begin(c, PC_DOT);
-        launch_multidot(kind, c->stream, V, ld, j, w, n, c->partial, c->c2, c->counter, flags, c->sms, c->p2p_arg());
-        prof_end(c, PC_DOT, 1);
-        LKB_TRY(check_launch(c, "multidot"));
+    if (fused) {
+        LKB_TRY(allreduce_w(c, c->c2, (size_t)(j + 1) * (kind_cplx(kind) ? 2 : 1)));
+    } else {
+        LKB_TRY(axpy_sub(c, kind, V, ld, j, c->c1, w, n, false, flags));
+        LKB_TRY(dot_reduce(c, kind, V, ld, j, w, n, c->c2, flags));
     }
-    LKB_TRY(allreduce_w(c, c->c2, nd));
-    if (want_gsinfo) {
-        launch_gsinfo(c->stream, (char*)c->c2.get() + (size_t)j * wsz, kind_cplx(kind), atol_of(kind), c->flags);
-        c->launches++;
-    }
+    if (want_gsinfo)
+        prof_launch(c, PC_OTHER, 1, [&] {
+            launch_gsinfo(c->stream, (char*)c->c2.get() + (size_t)j * (kind_cplx(kind) ? 16 : 8), kind_cplx(kind), atol_of(kind), c->flags);
+        });
     if (fin) {
         // pass-2 update + predicted-norm normalisation + H/T/B column + (optional) halo push in ONE kernel
-        prof_begin(c, PC_AXPY);
         SweepDir sd(d0);
-        launch_multiaxpy_fin(kind, c->stream, V, ld, j, fin->with_c1 ? c->c1.get() : nullptr, c->c2, w, n, c->partial, c->nrm2, c->counter,
-                             fin->hcol, fin->tol, atol_of(kind), c->inv, flags, fin->kstep, fin->mode, c->sms, c->p2p_arg(), fin->hp);
-        prof_end(c, PC_AXPY, 1);
+        prof_launch(c, PC_AXPY, 1, [&] {
+            launch_multiaxpy_fin(kind, c->stream, V, ld, j, fin->with_c1 ? c->c1.get() : nullptr, c->c2, w, n, c->partial, c->nrm2, c->counter,
+                                 fin->hcol, fin->tol, atol_of(kind), c->inv, flags, fin->kstep, fin->mode, c->sms, c->p2p_arg(), fin->hp);
+        });
         return check_launch(c, "multiaxpy_fin");
     }
-    prof_begin(c, PC_AXPY);
-    launch_multiaxpy(kind, c->stream, V, ld, j, c->c2, w, n, want_norm, c->partial, c->nrm2, c->counter, flags, c->sms, c->p2p_arg());
-    prof_end(c, PC_AXPY, 1);
-    LKB_TRY(check_launch(c, "multiaxpy"));
-    if (want_norm) LKB_TRY(allreduce_w(c, c->nrm2, 1));
-    return 0;
+    return axpy_sub(c, kind, V, ld, j, c->c2, w, n, want_norm, flags);
 }
 
 // Orthogonalisation + normalisation + column update of ONE Krylov step (everything after the matvec):
 //   CGS2 of w against V(:, 0:j), beta = ||w||, column of H / T / B, breakdown decision, w /= beta.
 // mode 0 arnoldi (hcol(0:j) = c1 + c2), 1 lanczos, 2 bidiag (only hcol(j) = beta is written).
-// Default: the final pass is k_multiaxpy_fin (3 kernels + 1 empty launch per step, 2 reductions).  Falls back to
-// the round-1 sequence (multi-axpy with norm, allreduce, k_update, k_scale_dev) for j = 0, when the reductions
-// go through ncclAllReduce (the predicted norm must not be summed over ranks), or with option "fin" = 0.
+// Default: the final pass is k_multiaxpy_fin (3 kernels + 1 empty launch per step, 2 reductions).  Where fin_usable
+// rules it out: the round-1 sequence (multi-axpy with norm, allreduce, k_update, k_scale_dev).
 int step_tail_enqueue(lkb_ctx_s* c, int kind, const void* V, int64_t ld, int j, void* w, int64_t n, int mode, double tol,
                       int kstep, void* hcol, const HaloP2P* hp) {
-    const bool fin_ok = c->fin && j > 0 && (c->world == 1 || c->p2p_active);
-    if (fin_ok) {
-        FinArgs fa; fa.mode = mode; fa.tol = tol; fa.kstep = kstep; fa.hcol = hcol; fa.with_c1 = (mode == 0); fa.hp = hp;
+    if (fin_usable(c, j)) {
+        const FinArgs fa{mode, tol, kstep, hcol, mode == 0, hp};
         LKB_TRY(dgs_enqueue(c, kind, V, ld, j, w, n, c->flags, false, false, &fa));
     } else {
         LKB_TRY(dgs_enqueue(c, kind, V, ld, j, w, n, c->flags, true, false));
-        prof_begin(c, PC_OTHER);
-        launch_update(kind, c->stream, mode == 0 ? c->c1.get() : nullptr, mode == 0 ? c->c2.get() : nullptr, j, c->nrm2, hcol, tol,
-                      atol_of(kind), c->inv, c->flags, kstep, mode);
-        prof_end(c, PC_OTHER, 1);
+        prof_launch(c, PC_OTHER, 1, [&] {
+            launch_update(kind, c->stream, mode == 0 ? c->c1.get() : nullptr, mode == 0 ? c->c2.get() : nullptr, j, c->nrm2, hcol, tol,
+                          atol_of(kind), c->inv, c->flags, kstep, mode);
+        });
     }
-    prof_begin(c, PC_OTHER);
-    launch_scale_dev(kind, c->stream, w, n, c->inv, c->flags, kstep, c->sms, hp);
-    prof_end(c, PC_OTHER, 1);
+    prof_launch(c, PC_OTHER, 1, [&] { launch_scale_dev(kind, c->stream, w, n, c->inv, c->flags, kstep, c->sms, hp); });
     return check_launch(c, "step tail");
 }
 
@@ -154,8 +148,7 @@ static double host_abs(int kind, const void* p) {
     }
 }
 
-// Read c1 + c2 (first j entries) and, optionally, nrm2 to the host (one sync).
-static int fetch_coeffs(lkb_ctx_s* c, int kind, int j, bool two, std::vector<Scalar>& out, double* nrm2, int* flags) {
+int fetch_coeffs(lkb_ctx_s* c, int kind, int j, bool two, std::vector<Scalar>& out, double* nrm2, int* flags) {
     const size_t wsz = kind_cplx(kind) ? 16 : 8;
     LKB_TRY(ensure_hstage(c, 2 * (size_t)(j + 1) * 16 + 4096));
     char* hs = (char*)c->hstage;
@@ -200,6 +193,38 @@ static int reset_flags(lkb_ctx_s* c) {
     return 0;
 }
 
+// ---- the frame shared by arnoldi (p = 1), lanczos and bidiagonalization -------------------------------------------------
+// X (U for bidiag) holds kdim + 1 columns; the device H / T / B has leading dimension kdim + 1.
+// Enqueue `steps` kstart..kend after the shared prologue, directly or through the graph cached under (tag, A, X, Y, ...).
+static int krylov_run(const char* tag, lkb_op_s* A, const lkb_basis_s* X, const lkb_basis_s* Y, int kstart, int kend, double tol,
+                      bool tr, const std::function<int()>& steps) {
+    lkb_ctx_s* c = X->ctx;
+    LKB_TRY(ensure_Hd(c, (size_t)X->ncols * (X->ncols - 1) * kind_size(X->kind)));
+    LKB_TRY(ensure_ws(c, kend + 1));
+    auto body = [&]() -> int {
+        LKB_TRY(reset_flags(c));
+        PdlScope pdl(c->pdl && !c->profile);      // the kernels of the step loop overlap their heads with the predecessors' tails
+        return steps();
+    };
+    return run_maybe_graph(c, op_capturable(A), make_key(tag, A, X, Y, kstart, kend, tol, tr), body);
+}
+// The synchronous entry points: enqueue, copy the new columns and the flags to the staging buffer, wait, collect from it.
+static int krylov_sync(const lkb_basis_s* X, int kstart, int kend, const std::function<int()>& enqueue,
+                       const std::function<int(const void*)>& collect) {
+    lkb_ctx_s* c = X->ctx;
+    LKB_TRY(ensure_hstage(c, (size_t)X->ncols * (kend - kstart + 1) * kind_size(X->kind) + 4096));
+    LKB_TRY(enqueue());
+    LKB_TRY(krylov_fetch_async(c, X->kind, X->ncols, kstart, kend, c->hstage));
+    LKB_CUDA(cudaStreamSynchronize(c->stream));
+    return collect(c->hstage);
+}
+// The flags krylov_fetch_async staged behind the ncol columns; a NaN norm is an error with message `nan_msg`.
+static int staged_flags(const lkb_basis_s* X, int ncol, const void* host, int* hf, const char* nan_msg) {
+    memcpy(hf, (const char*)host + (size_t)X->ncols * ncol * kind_size(X->kind), F_COUNT * sizeof(int));
+    if (hf[F_NAN]) { set_error("%s", nan_msg); return LKB_ERR_NAN; }
+    return 0;
+}
+
 // is_orthonormal (src/Krylov/utilities.fypp:90-98): mnorm(Gram(X) - I, "Fro") > rtol_sp (hard-wired, all kinds) => not orthonormal
 static int check_orthonormal(lkb_basis_s* X, int j, bool* ok) {
     lkb_ctx_s* c = X->ctx;
@@ -209,10 +234,7 @@ static int check_orthonormal(lkb_basis_s* X, int j, bool* ok) {
     const double lim2 = 1e-3 * 1e-3;                           // rtol_sp = sqrt(atol_sp) = 1e-3
     for (int q = 0; q < j && fro2 <= lim2; ++q) {
         LKB_TRY(ensure_ws(c, j + 1));
-        launch_multidot(X->kind, c->stream, X->d, X->ld, j, col_ptr(X, q), X->n, c->partial, c->c1, c->counter, nullptr, c->sms, c->p2p_arg());
-        c->launches++;
-        LKB_TRY(check_launch(c, "gram"));
-        LKB_TRY(allreduce_w(c, c->c1, (size_t)(j + 1) * (kind_cplx(X->kind) ? 2 : 1)));
+        LKB_TRY(dot_reduce(c, X->kind, X->d, X->ld, j, col_ptr(X, q), X->n, c->c1, nullptr));
         LKB_TRY(fetch_coeffs(c, X->kind, j, false, col, nullptr, nullptr));
         for (int i = 0; i < j; ++i) {
             const double re = col[i].re - (i == q ? 1.0 : 0.0);
@@ -234,11 +256,7 @@ int lkb_basis_innerprod(lkb_basis_t X, int j, lkb_basis_t W, int wcol0, int p, v
     std::vector<Scalar> col;
     for (int q = 0; q < p; ++q) {
         LKB_TRY(ensure_ws(c, j + 1));
-        prof_begin(c, PC_DOT);
-        launch_multidot(X->kind, c->stream, X->d, X->ld, j, col_ptr(W, wcol0 + q), X->n, c->partial, c->c1, c->counter, nullptr, c->sms, c->p2p_arg());
-        prof_end(c, PC_DOT, 1);
-        LKB_TRY(check_launch(c, "innerprod"));
-        LKB_TRY(allreduce_w(c, c->c1, (size_t)(j + 1) * (kind_cplx(X->kind) ? 2 : 1)));
+        LKB_TRY(dot_reduce(c, X->kind, X->d, X->ld, j, col_ptr(W, wcol0 + q), X->n, c->c1, nullptr));
         LKB_TRY(fetch_coeffs(c, X->kind, j, false, col, nullptr, nullptr));
         for (int i = 0; i < j; ++i)
             store_kind(X->kind, out, (size_t)i + (size_t)ldout * q, cd(col[i].re, col[i].im));
@@ -252,10 +270,7 @@ int lkb_basis_lincomb_sub(lkb_basis_t X, int j, const void* coef, int ldcoef, lk
     lkb_ctx_s* c = X->ctx;
     for (int q = 0; q < p; ++q) {
         LKB_TRY(upload_coef(c, X->kind, (const char*)coef + (size_t)ldcoef * q * kind_size(X->kind), j, 1.0));
-        prof_begin(c, PC_AXPY);
-        launch_multiaxpy(X->kind, c->stream, X->d, X->ld, j, c->coefd, col_ptr(W, wcol0 + q), X->n, false, c->partial, c->nrm2, c->counter, nullptr, c->sms, c->p2p_arg());
-        prof_end(c, PC_AXPY, 1);
-        LKB_TRY(check_launch(c, "lincomb_sub"));
+        LKB_TRY(axpy_sub(c, X->kind, X->d, X->ld, j, c->coefd, col_ptr(W, wcol0 + q), X->n, false, nullptr));
     }
     return 0;
 }
@@ -266,10 +281,7 @@ int lkb_basis_lincomb(lkb_basis_t X, int j, const void* coef, lkb_vec_t y) {
     lkb_ctx_s* c = X->ctx;
     LKB_TRY(upload_coef(c, X->kind, coef, j, -1.0));
     LKB_TRY(lkb_vec_zero(y));
-    prof_begin(c, PC_AXPY);
-    launch_multiaxpy(X->kind, c->stream, X->d, X->ld, j, c->coefd, y->d, X->n, false, c->partial, c->nrm2, c->counter, nullptr, c->sms, c->p2p_arg());
-    prof_end(c, PC_AXPY, 1);
-    return check_launch(c, "lincomb");
+    return axpy_sub(c, X->kind, X->d, X->ld, j, c->coefd, y->d, X->n, false, nullptr);
 }
 
 static int gs_common(lkb_basis_t X, int j, lkb_basis_t W, int wcol0, int p, int32_t chk, void* beta, int ldbeta,
@@ -293,15 +305,11 @@ static int gs_common(lkb_basis_t X, int j, lkb_basis_t W, int wcol0, int p, int3
             LKB_TRY(dgs_enqueue(c, X->kind, X->d, X->ld, j, w, X->n, c->flags, false, true));
         } else {
             LKB_TRY(ensure_ws(c, j + 1));
-            prof_begin(c, PC_DOT);
-            launch_multidot(X->kind, c->stream, X->d, X->ld, j, w, X->n, c->partial, c->c1, c->counter, nullptr, c->sms, c->p2p_arg());
-            prof_end(c, PC_DOT, 1);
-            LKB_TRY(allreduce_w(c, c->c1, (size_t)(j + 1) * (kind_cplx(X->kind) ? 2 : 1)));
-            launch_gsinfo(c->stream, (char*)c->c1.get() + (size_t)j * (kind_cplx(X->kind) ? 16 : 8), 0, atol_of(X->kind), c->flags);
-            prof_begin(c, PC_AXPY);
-            launch_multiaxpy(X->kind, c->stream, X->d, X->ld, j, c->c1, w, X->n, false, c->partial, c->nrm2, c->counter, nullptr, c->sms, c->p2p_arg());
-            prof_end(c, PC_AXPY, 1);
-            LKB_TRY(check_launch(c, "orthogonalize"));
+            LKB_TRY(dot_reduce(c, X->kind, X->d, X->ld, j, w, X->n, c->c1, nullptr));
+            prof_launch(c, PC_OTHER, 1, [&] {
+                launch_gsinfo(c->stream, (char*)c->c1.get() + (size_t)j * (kind_cplx(X->kind) ? 16 : 8), 0, atol_of(X->kind), c->flags);
+            });
+            LKB_TRY(axpy_sub(c, X->kind, X->d, X->ld, j, c->c1, w, X->n, false, nullptr));
         }
         LKB_TRY(fetch_coeffs(c, X->kind, j, two_pass, col, nullptr, hf));
         if (hf[F_GSINFO]) *info = q + 1;
@@ -345,8 +353,7 @@ int lkb_qr(lkb_basis_t Q, int col0, int p, void* R, int ldr, double tol, int32_t
         if (beta != beta) { set_error("|beta| = NaN detected! Abort"); return LKB_ERR_NAN; }
         if (beta < tol) {
             if (!flag) { flag = true; *info = j + 1; }
-            launch_fill(kind, c->stream, q, Q->n, Q->row0, LKB_DIST_NORMAL, next_seed(c), c->sms);
-            c->launches++;
+            prof_launch(c, PC_OTHER, 1, [&] { launch_fill(kind, c->stream, q, Q->n, Q->row0, LKB_DIST_NORMAL, next_seed(c), c->sms); });
             LKB_TRY(reset_flags(c));
             LKB_TRY(dgs_enqueue(c, kind, col_ptr(Q, col0), Q->ld, j, q, Q->n, c->flags, true, true));
             LKB_TRY(fetch_coeffs(c, kind, j, true, col, &nrm2, hf));
@@ -355,8 +362,7 @@ int lkb_qr(lkb_basis_t Q, int col0, int p, void* R, int ldr, double tol, int32_t
         } else {
             store_kind(kind, R, (size_t)j + (size_t)ldr * j, beta);
         }
-        launch_scal(kind, c->stream, Scalar{1.0 / beta, 0.0}, q, Q->n, c->sms);
-        c->launches++;
+        prof_launch(c, PC_OTHER, 1, [&] { launch_scal(kind, c->stream, Scalar{1.0 / beta, 0.0}, q, Q->n, c->sms); });
         LKB_TRY(check_launch(c, "qr scal"));
     }
     return 0;
@@ -389,8 +395,7 @@ int lkb_qr_pivoting(lkb_basis_t Q, int col0, int p, void* R, int ldr, int32_t* p
     DevBuf tmp(c);
     // Q(i) <- rand ; double_gram_schmidt_step(Q(i), Q(:i-1)) ; returns the step's info and the norm afterwards
     auto refill = [&](int i, int32_t* ginfo, double* beta) -> int {
-        launch_fill(kind, c->stream, qcol(i), Q->n, Q->row0, LKB_DIST_NORMAL, next_seed(c), c->sms);
-        c->launches++;
+        prof_launch(c, PC_OTHER, 1, [&] { launch_fill(kind, c->stream, qcol(i), Q->n, Q->row0, LKB_DIST_NORMAL, next_seed(c), c->sms); });
         double nrm2 = 0;
         LKB_TRY(reset_flags(c));
         LKB_TRY(dgs_enqueue(c, kind, qcol(0), Q->ld, i, qcol(i), Q->n, c->flags, true, true));
@@ -406,8 +411,7 @@ int lkb_qr_pivoting(lkb_basis_t Q, int col0, int p, void* R, int ldr, int32_t* p
             for (int i = j; i < p; ++i) {
                 int32_t g = 0; double beta = 0;
                 LKB_TRY(refill(i, &g, &beta));
-                launch_scal(kind, c->stream, Scalar{1.0 / beta, 0.0}, qcol(i), Q->n, c->sms);
-                c->launches++;
+                prof_launch(c, PC_OTHER, 1, [&] { launch_scal(kind, c->stream, Scalar{1.0 / beta, 0.0}, qcol(i), Q->n, c->sms); });
                 LKB_TRY(check_launch(c, "qr_pivoting completion"));
             }
             *info = j + 1;
@@ -437,14 +441,12 @@ int lkb_qr_pivoting(lkb_basis_t Q, int col0, int p, void* R, int ldr, int32_t* p
         } else {
             store_kind(kind, R, (size_t)j + (size_t)ldr * j, beta);
         }
-        launch_scal(kind, c->stream, Scalar{1.0 / beta, 0.0}, qcol(j), Q->n, c->sms);
-        c->launches++;
+        prof_launch(c, PC_OTHER, 1, [&] { launch_scal(kind, c->stream, Scalar{1.0 / beta, 0.0}, qcol(j), Q->n, c->sms); });
         for (int i = j + 1; i < p; ++i) {                                   // orthogonalise the trailing columns (:93-97)
             Scalar b{0, 0};
             LKB_TRY(vec_dot_sync(c, kind, qcol(j), qcol(i), Q->n, &b));
             b = round_kind(b);
-            launch_axpby(kind, c->stream, Scalar{-b.re, -b.im}, qcol(j), Scalar{1.0, 0.0}, qcol(i), Q->n, c->sms);
-            c->launches++;
+            prof_launch(c, PC_OTHER, 1, [&] { launch_axpby(kind, c->stream, Scalar{-b.re, -b.im}, qcol(j), Scalar{1.0, 0.0}, qcol(i), Q->n, c->sms); });
             store_kind(kind, R, (size_t)j + (size_t)ldr * i, cd(b.re, b.im));
             Rii[i] = round_kind(Scalar{Rii[i].re - (b.re * b.re - b.im * b.im), Rii[i].im - 2.0 * b.re * b.im});
         }
@@ -498,19 +500,13 @@ int lkb_arnoldi(lkb_op_t A, lkb_basis_t X, void* H, int ldh, int32_t* info, int3
     if (kend <= 0) kend = kdim;
     if (kstart > kend || kend > kdim || ldh < (kend + 1) * p || A->kind != X->kind || A->m != X->n || A->n != X->n)
         { set_error("arnoldi: inconsistent sizes (kdim=%d kstart=%d kend=%d ldh=%d)", kdim, kstart, kend, ldh); return LKB_ERR_ARG; }
-    lkb_ctx_s* c = X->ctx;
-    const int kind = X->kind;
-    const size_t es = kind_size(kind);
-    if (tol < 0) tol = atol_of(kind);
+    if (tol < 0) tol = atol_of(X->kind);
     *info = 0;
     if (p > 1) return arnoldi_block(A, X, H, ldh, info, kstart, kend, tol, transpose != 0, p);
 
     const bool tr = transpose != 0;
-    LKB_TRY(ensure_hstage(c, (size_t)(kdim + 1) * (kend - kstart + 1) * es + 4096));
-    LKB_TRY(arnoldi_enqueue(A, X, kstart, kend, tol, tr));
-    LKB_TRY(arnoldi_fetch_async(X, kstart, kend, c->hstage));
-    LKB_CUDA(cudaStreamSynchronize(c->stream));
-    return arnoldi_collect(A, X, H, ldh, info, kstart, kend, tr, c->hstage);
+    return krylov_sync(X, kstart, kend, [&] { return arnoldi_enqueue(A, X, kstart, kend, tol, tr); },
+                       [&](const void* hs) { return arnoldi_collect(A, X, H, ldh, info, kstart, kend, tr, hs); });
 }
 
 }  // extern "C"
@@ -520,44 +516,29 @@ namespace lkb {
 // step k with the device work of step k+1 (SURVEY 8f rank 3).
 int arnoldi_enqueue(lkb_op_s* A, lkb_basis_s* X, int kstart, int kend, double tol, bool tr) {
     lkb_ctx_s* c = X->ctx;
-    const int kind = X->kind;
-    const size_t es = kind_size(kind);
-    const int kdim = X->ncols - 1;
-    const int ldhd = kdim + 1;
-    LKB_TRY(ensure_Hd(c, (size_t)ldhd * kdim * es));
-    LKB_TRY(ensure_ws(c, kend + 1));
-    auto body = [&]() -> int {
-        LKB_TRY(reset_flags(c));
-        PdlScope pdl(c->pdl && !c->profile);      // the kernels of the step loop overlap their heads with the predecessors' tails
+    const size_t es = kind_size(X->kind);
+    return krylov_run("arn", A, X, nullptr, kstart, kend, tol, tr, [&]() -> int {
         bool pushed = false;       // X(k-1)'s boundary rows already sit in the neighbours' halo buffers
         for (int k = kstart; k <= kend; ++k) {
             void* w = col_ptr(X, k);
             LKB_TRY(op_apply_enqueue(A, col_ptr(X, k - 1), w, tr, c->flags, pushed));
             // the kernel that finishes X(k) also pushes its halo rows for the next step's matvec
-            const HaloP2P* hp = (k < kend) ? op_halo_desc(A) : nullptr;
-            LKB_TRY(step_tail_enqueue(c, kind, X->d, X->ld, k, w, X->n, 0, tol, k, (char*)c->Hd.get() + (size_t)ldhd * (k - 1) * es, hp));
+            const HaloP2P* hp = (k < kend) ? op_halo_desc(A, k) : nullptr;
+            LKB_TRY(step_tail_enqueue(c, X->kind, X->d, X->ld, k, w, X->n, 0, tol, k, (char*)c->Hd.get() + (size_t)X->ncols * (k - 1) * es, hp));
             pushed = hp != nullptr;
         }
         return 0;
-    };
-    return run_maybe_graph(c, op_capturable(A), make_key("arn", A, X, nullptr, kstart, kend, tol, tr), body);
-}
-// D2H of the freshly written Hessenberg columns + flags into `host` (pinned), no sync
-int arnoldi_fetch_async(lkb_basis_s* X, int kstart, int kend, void* host) {
-    return krylov_fetch_async(X->ctx, X->kind, X->ncols, kstart, kend, host);
+    });
 }
 // after the stream reached the fetch: scatter the columns into the caller's H, set info, refill on breakdown
 int arnoldi_collect(lkb_op_s* A, lkb_basis_s* X, void* H, int ldh, int32_t* info, int kstart, int kend, bool tr,
                     const void* host) {
     lkb_ctx_s* c = X->ctx;
     const int kind = X->kind;
-    const size_t es = kind_size(kind);
     const int ldhd = X->ncols;
-    const int ncol = kend - kstart + 1;
     const char* hs = (const char*)host;
     int hf[F_COUNT];
-    memcpy(hf, hs + (size_t)ldhd * ncol * es, sizeof(hf));
-    if (hf[F_NAN]) { set_error("|beta| = NaN detected! Abort"); return LKB_ERR_NAN; }
+    LKB_TRY(staged_flags(X, kend - kstart + 1, host, hf, "|beta| = NaN detected! Abort"));
     const int kdone = hf[F_STOP] ? hf[F_INFO] : kend;
     for (int k = kstart; k <= kdone; ++k)
         for (int i = 0; i <= k; ++i)
@@ -569,12 +550,10 @@ int arnoldi_collect(lkb_op_s* A, lkb_basis_s* X, void* H, int ldh, int32_t* info
         if (hf[F_REFILL]) {
             // qr.fypp:153-158 : the numerically-zero vector is replaced by a normalised random one
             void* w = col_ptr(X, kdone);
-            launch_fill(kind, c->stream, w, X->n, X->row0, LKB_DIST_NORMAL, next_seed(c), c->sms);
-            c->launches++;
+            prof_launch(c, PC_OTHER, 1, [&] { launch_fill(kind, c->stream, w, X->n, X->row0, LKB_DIST_NORMAL, next_seed(c), c->sms); });
             double nrm = 0;
             LKB_TRY(vec_norm_sync(c, kind, w, X->n, &nrm));
-            launch_scal(kind, c->stream, Scalar{1.0 / nrm, 0.0}, w, X->n, c->sms);
-            c->launches++;
+            prof_launch(c, PC_OTHER, 1, [&] { launch_scal(kind, c->stream, Scalar{1.0 / nrm, 0.0}, w, X->n, c->sms); });
             LKB_TRY(check_launch(c, "refill"));
         }
     }
@@ -661,14 +640,10 @@ int lkb_lanczos(lkb_op_t A, lkb_basis_t X, void* T, int ldt, int32_t* info, int3
     if (kend <= 0) kend = kdim;
     if (kstart > kend || kend > kdim || ldt < kend + 1 || A->kind != X->kind || A->m != X->n || A->n != X->n)
         { set_error("lanczos: inconsistent sizes"); return LKB_ERR_ARG; }
-    lkb_ctx_s* c = X->ctx;
     if (tol < 0) tol = atol_of(X->kind);
     *info = 0;
-    LKB_TRY(ensure_hstage(c, (size_t)(kdim + 1) * (kend - kstart + 1) * kind_size(X->kind) + 4096));
-    LKB_TRY(lanczos_enqueue(A, X, kstart, kend, tol));
-    LKB_TRY(krylov_fetch_async(X->ctx, X->kind, kdim + 1, kstart, kend, c->hstage));
-    LKB_CUDA(cudaStreamSynchronize(c->stream));
-    return lanczos_collect(A, X, T, ldt, info, kstart, kend, c->hstage);
+    return krylov_sync(X, kstart, kend, [&] { return lanczos_enqueue(A, X, kstart, kend, tol); },
+                       [&](const void* hs) { return lanczos_collect(A, X, T, ldt, info, kstart, kend, hs); });
 }
 
 }  // extern "C"
@@ -680,37 +655,26 @@ int lanczos_enqueue(lkb_op_s* A, lkb_basis_s* X, int kstart, int kend, double to
     lkb_ctx_s* c = X->ctx;
     const int kind = X->kind;
     const size_t es = kind_size(kind);
-    const int kdim = X->ncols - 1;
-    const int ldtd = kdim + 1;
-    LKB_TRY(ensure_Hd(c, (size_t)ldtd * kdim * es));
-    LKB_TRY(ensure_ws(c, kend + 1));
-    const size_t ndw = 2 * (size_t)(kind_cplx(kind) ? 2 : 1);
-    auto body = [&]() -> int {
-        LKB_TRY(reset_flags(c));
-        PdlScope pdl(c->pdl && !c->profile);
+    return krylov_run("lan", A, X, nullptr, kstart, kend, tol, false, [&]() -> int {
         bool pushed = false;
         for (int k = kstart; k <= kend; ++k) {
             void* w = col_ptr(X, k);
-            char* tcol = (char*)c->Hd.get() + (size_t)ldtd * (k - 1) * es;
+            char* tcol = (char*)c->Hd.get() + (size_t)X->ncols * (k - 1) * es;
             LKB_TRY(op_apply_enqueue(A, col_ptr(X, k - 1), w, false, c->flags, pushed));
             for (int i = (k - 1 > 1 ? k - 1 : 1); i <= k; ++i) {        // update_tridiag_matrix :57-59
                 void* xi = col_ptr(X, i - 1);
-                prof_begin(c, PC_DOT);
-                launch_multidot(kind, c->stream, xi, X->ld, 1, w, X->n, c->partial, c->tmpw, c->counter, c->flags, c->sms, c->p2p_arg());
-                prof_end(c, PC_DOT, 1);
-                LKB_TRY(allreduce_w(c, c->tmpw, ndw));
-                prof_begin(c, PC_OTHER);
-                launch_narrow(kind, c->stream, c->tmpw, tcol + (size_t)(i - 1) * es, 1, c->flags);
-                launch_axpy_dev(kind, c->stream, c->tmpw, -1.0, xi, w, X->n, c->flags, c->sms);
-                prof_end(c, PC_OTHER, 2);
+                LKB_TRY(dot_reduce(c, kind, xi, X->ld, 1, w, X->n, c->tmpw, c->flags));
+                prof_launch(c, PC_OTHER, 2, [&] {
+                    launch_narrow(kind, c->stream, c->tmpw, tcol + (size_t)(i - 1) * es, 1, c->flags);
+                    launch_axpy_dev(kind, c->stream, c->tmpw, -1.0, xi, w, X->n, c->flags, c->sms);
+                });
             }
-            const HaloP2P* hp = (k < kend) ? op_halo_desc(A) : nullptr;
+            const HaloP2P* hp = (k < kend) ? op_halo_desc(A, k) : nullptr;
             LKB_TRY(step_tail_enqueue(c, kind, X->d, X->ld, k, w, X->n, 1, tol, k, tcol, hp));
             pushed = hp != nullptr;
         }
         return 0;
-    };
-    return run_maybe_graph(c, op_capturable(A), make_key("lan", A, X, nullptr, kstart, kend, tol, 0), body);
+    });
 }
 // D2H of the freshly written columns of the device-side H / T / B (leading dimension ldd) + flags, no sync
 int krylov_fetch_async(lkb_ctx_s* c, int kind, int ldd, int kstart, int kend, void* host) {
@@ -723,13 +687,10 @@ int krylov_fetch_async(lkb_ctx_s* c, int kind, int ldd, int kstart, int kend, vo
 }
 int lanczos_collect(lkb_op_s* A, lkb_basis_s* X, void* T, int ldt, int32_t* info, int kstart, int kend, const void* host) {
     const int kind = X->kind;
-    const size_t es = kind_size(kind);
     const int ldtd = X->ncols;
-    const int ncol = kend - kstart + 1;
     const char* hs = (const char*)host;
     int hf[F_COUNT];
-    memcpy(hf, hs + (size_t)ldtd * ncol * es, sizeof(hf));
-    if (hf[F_NAN]) { set_error("lanczos: NaN norm"); return LKB_ERR_NAN; }
+    LKB_TRY(staged_flags(X, kend - kstart + 1, host, hf, "lanczos: NaN norm"));
     const int kdone = hf[F_STOP] ? hf[F_INFO] : kend;
     for (int k = kstart; k <= kdone; ++k)
         for (int i = (k - 1 > 1 ? k - 1 : 1); i <= k + 1; ++i)
@@ -753,14 +714,10 @@ int lkb_bidiag(lkb_op_t A, lkb_basis_t U, lkb_basis_t V, void* B, int ldb, int32
     if (kend <= 0) kend = kdim;
     if (kstart > kend || kend > kdim || V->ncols < kend || ldb < kend + 1 || A->kind != U->kind || A->kind != V->kind ||
         A->m != U->n || A->n != V->n) { set_error("bidiag: inconsistent sizes"); return LKB_ERR_ARG; }
-    lkb_ctx_s* c = U->ctx;
     if (tol < 0) tol = atol_of(U->kind);
     *info = 0;
-    LKB_TRY(ensure_hstage(c, (size_t)(kdim + 1) * (kend - kstart + 1) * kind_size(U->kind) + 4096));
-    LKB_TRY(bidiag_enqueue(A, U, V, kstart, kend, tol));
-    LKB_TRY(krylov_fetch_async(c, U->kind, kdim + 1, kstart, kend, c->hstage));
-    LKB_CUDA(cudaStreamSynchronize(c->stream));
-    return bidiag_collect(A, U, B, ldb, info, kstart, kend, c->hstage);
+    return krylov_sync(U, kstart, kend, [&] { return bidiag_enqueue(A, U, V, kstart, kend, tol); },
+                       [&](const void* hs) { return bidiag_collect(A, U, B, ldb, info, kstart, kend, hs); });
 }
 
 }  // extern "C"
@@ -770,15 +727,9 @@ int bidiag_enqueue(lkb_op_s* A, lkb_basis_s* U, lkb_basis_s* V, int kstart, int 
     lkb_ctx_s* c = U->ctx;
     const int kind = U->kind;
     const size_t es = kind_size(kind);
-    const int kdim = U->ncols - 1;
-    const int ldbd = kdim + 1;
-    LKB_TRY(ensure_Hd(c, (size_t)ldbd * kdim * es));
-    LKB_TRY(ensure_ws(c, kend + 1));
-    auto body = [&]() -> int {
-        LKB_TRY(reset_flags(c));
-        PdlScope pdl(c->pdl && !c->profile);
+    return krylov_run("bid", A, U, V, kstart, kend, tol, false, [&]() -> int {
         for (int k = kstart; k <= kend; ++k) {
-            char* bcol = (char*)c->Hd.get() + (size_t)ldbd * (k - 1) * es;
+            char* bcol = (char*)c->Hd.get() + (size_t)U->ncols * (k - 1) * es;
             void* vk = col_ptr(V, k - 1);
             LKB_TRY(op_apply_enqueue(A, col_ptr(U, k - 1), vk, true, c->flags));
             LKB_TRY(step_tail_enqueue(c, kind, V->d, V->ld, k - 1, vk, V->n, 2, tol, 2 * k - 1, bcol, nullptr));
@@ -787,18 +738,14 @@ int bidiag_enqueue(lkb_op_s* A, lkb_basis_s* U, lkb_basis_s* V, int kstart, int 
             LKB_TRY(step_tail_enqueue(c, kind, U->d, U->ld, k, uk1, U->n, 2, tol, 2 * k, bcol, nullptr));
         }
         return 0;
-    };
-    return run_maybe_graph(c, op_capturable(A), make_key("bid", A, U, V, kstart, kend, tol, 0), body);
+    });
 }
 int bidiag_collect(lkb_op_s* A, lkb_basis_s* U, void* B, int ldb, int32_t* info, int kstart, int kend, const void* host) {
     const int kind = U->kind;
-    const size_t es = kind_size(kind);
     const int ldbd = U->ncols;
-    const int ncol = kend - kstart + 1;
     const char* hs = (const char*)host;
     int hf[F_COUNT];
-    memcpy(hf, hs + (size_t)ldbd * ncol * es, sizeof(hf));
-    if (hf[F_NAN]) { set_error("bidiag: NaN norm"); return LKB_ERR_NAN; }
+    LKB_TRY(staged_flags(U, kend - kstart + 1, host, hf, "bidiag: NaN norm"));
     const int stage = hf[F_STOP] ? hf[F_INFO] : 2 * kend;
     const int kdone = (stage + 1) / 2;
     for (int k = kstart; k <= kdone; ++k) {

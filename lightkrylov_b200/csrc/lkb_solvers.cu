@@ -95,6 +95,7 @@ static int gmres_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, doubl
     if ((precond || M) && !flexible) LKB_TRY(lkb_vec_create(c, kind, b->n, b->n_global, b->row0, wrk.out()));
     if (flexible) LKB_TRY(lkb_basis_create(c, kind, b->n, b->n_global, b->row0, kdim, Z.out()));
     std::vector<cd> H((size_t)(kdim + 1) * kdim), e(kdim + 1), cs(kdim), sn(kdim), y(kdim);
+    std::vector<Scalar> col;
     const Scalar one{1, 0}, mone{-1, 0};
     int hf[F_COUNT];
     auto apply_precond = [&](void* v, int iter, double cur, double target) -> int {
@@ -111,8 +112,7 @@ static int gmres_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, doubl
             if (trans) A->n_rmatvec++; else A->n_matvec++;
             LKB_TRY(op_apply_enqueue(A, x->d, col_ptr(V, 0), trans, nullptr));
         }
-        launch_axpby(kind, c->stream, one, b->d, mone, col_ptr(V, 0), b->n, c->sms);   // sub(b); chsgn()
-        c->launches++;
+        prof_launch(c, PC_OTHER, 1, [&] { launch_axpby(kind, c->stream, one, b->d, mone, col_ptr(V, 0), b->n, c->sms); });   // sub(b); chsgn()
         return check_launch(c, "gmres residual");
     };
 
@@ -124,7 +124,6 @@ static int gmres_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, doubl
     StreamSync sync{c->stream};
     auto enqueue_cycle = [&]() -> int {
         char* gcs = (char*)ge.p + (size_t)(kdim + 1) * 16; char* gsn = gcs + (size_t)kdim * 16;
-        const bool fin_ok = c->fin && (c->world == 1 || c->p2p_active);
         PdlScope pdl(c->pdl && !c->profile);
         bool pushed = false;
         for (int kk = 1; kk <= kdim; ++kk) {
@@ -134,18 +133,18 @@ static int gmres_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, doubl
             LKB_TRY(op_apply_enqueue(A, src, w, trans, c->flags, pushed));
             // the fused halo push of V(k+1) is right only when V(k+1) is A's next input; with M in between that input is
             // wrk, and op_apply_enqueue(A, wrk, ...) exchanges its halo itself
-            const HaloP2P* hp = (kk < kdim && !M) ? op_halo_desc(A) : nullptr;
-            if (fin_ok) {     // final pass normalises with the predicted norm (mode 4: k_gmres_update does the column)
-                FinArgs fa; fa.mode = 4; fa.tol = tol; fa.kstep = kk; fa.hcol = nullptr; fa.with_c1 = false; fa.hp = hp;
+            const HaloP2P* hp = (kk < kdim && !M) ? op_halo_desc(A, kk) : nullptr;
+            if (fin_usable(c, kk)) {     // final pass normalises with the predicted norm (mode 4: k_gmres_update does the column)
+                const FinArgs fa{4, tol, kk, nullptr, false, hp};
                 LKB_TRY(dgs_enqueue(c, kind, V->d, V->ld, kk, w, b->n, c->flags, false, false, &fa));
             } else {
                 LKB_TRY(dgs_enqueue(c, kind, V->d, V->ld, kk, w, b->n, c->flags, true, false));
             }
-            pushed = fin_ok && hp != nullptr;
-            prof_begin(c, PC_OTHER);
-            launch_gmres_update(kind, c->stream, c->c1, c->c2, kk, c->nrm2, gH.p, kdim + 1, ge.p, gcs, gsn, tol, c->inv, c->flags, (double*)gres.p);
-            launch_scale_dev(kind, c->stream, w, b->n, c->inv, c->flags, kk, c->sms, fin_ok ? hp : nullptr);
-            prof_end(c, PC_OTHER, 2);
+            pushed = hp != nullptr;
+            prof_launch(c, PC_OTHER, 2, [&] {
+                launch_gmres_update(kind, c->stream, c->c1, c->c2, kk, c->nrm2, gH.p, kdim + 1, ge.p, gcs, gsn, tol, c->inv, c->flags, (double*)gres.p);
+                launch_scale_dev(kind, c->stream, w, b->n, c->inv, c->flags, kk, c->sms, hp);
+            });
             LKB_TRY(check_launch(c, "gmres update"));
         }
         return 0;
@@ -166,7 +165,7 @@ static int gmres_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, doubl
         double beta = 0;
         LKB_TRY(vec_norm_sync(c, kind, col_ptr(V, 0), b->n, &beta));
         e[0] = round_kind(kind, beta);
-        launch_scal(kind, c->stream, Scalar{1.0 / beta, 0}, col_ptr(V, 0), b->n, c->sms); c->launches++;
+        prof_launch(c, PC_OTHER, 1, [&] { launch_scal(kind, c->stream, Scalar{1.0 / beta, 0}, col_ptr(V, 0), b->n, c->sms); });
         std::fill(cs.begin(), cs.end(), cd(0)); std::fill(sn.begin(), sn.end(), cd(0));
         if (io->n_outer == 0) push_res(io->res, io->res_cap, &io->res_len, fabs(beta));
         int k = 1;
@@ -205,11 +204,11 @@ static int gmres_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, doubl
             if (trans) A->n_rmatvec++; else A->n_matvec++;
             const void* src = col_ptr(V, k - 1);
             if (flexible) {     // copy(Z(k), V(k)) ; preconditioner%apply(Z(k), k, beta, tol)   (fgmres.fypp:160-161)
-                launch_axpby(kind, c->stream, one, col_ptr(V, k - 1), Scalar{0, 0}, col_ptr(Z, k - 1), b->n, c->sms); c->launches++;
+                prof_launch(c, PC_OTHER, 1, [&] { launch_axpby(kind, c->stream, one, col_ptr(V, k - 1), Scalar{0, 0}, col_ptr(Z, k - 1), b->n, c->sms); });
                 if (precond) LKB_TRY(apply_precond(col_ptr(Z, k - 1), k, beta, tol));
                 src = col_ptr(Z, k - 1);
             } else if (precond) {      // wrk = V(k) ; preconditioner%apply(wrk, k, beta, tol)   (gmres.fypp:155)
-                launch_axpby(kind, c->stream, one, col_ptr(V, k - 1), Scalar{0, 0}, wrk->d, b->n, c->sms); c->launches++;
+                prof_launch(c, PC_OTHER, 1, [&] { launch_axpby(kind, c->stream, one, col_ptr(V, k - 1), Scalar{0, 0}, wrk->d, b->n, c->sms); });
                 LKB_TRY(apply_precond(wrk->d, k, beta, tol));
                 src = wrk->d;
             }
@@ -217,23 +216,12 @@ static int gmres_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, doubl
             LKB_CUDA(cudaMemsetAsync(c->flags, 0, F_COUNT * sizeof(int), c->stream));
             LKB_TRY(dgs_enqueue(c, kind, V->d, V->ld, k, w, b->n, c->flags, true, false));
             // H(:k, k) = c1 + c2 ; H(k+1, k) = ||V(k+1)||
-            {
-                const size_t wsz = cplx ? 16 : 8;
-                LKB_TRY(ensure_hstage(c, 2 * (size_t)(k + 1) * 16 + 4096));
-                char* hs = (char*)c->hstage;
-                cudaMemcpyAsync(hs, c->c1, (size_t)k * wsz, cudaMemcpyDeviceToHost, c->stream);
-                cudaMemcpyAsync(hs + (size_t)k * wsz, c->c2, (size_t)k * wsz, cudaMemcpyDeviceToHost, c->stream);
-                cudaMemcpyAsync(hs + 2 * (size_t)k * wsz, c->nrm2, 16, cudaMemcpyDeviceToHost, c->stream);
-                LKB_CUDA(cudaStreamSynchronize(c->stream));
-                for (int i = 0; i < k; ++i) {
-                    const double* a = (const double*)(hs + (size_t)i * wsz);
-                    const double* bb = (const double*)(hs + (size_t)(k + i) * wsz);
-                    H[i + (size_t)(kdim + 1) * (k - 1)] = round_kind(kind, cd(a[0] + bb[0], cplx ? a[1] + bb[1] : 0.0));
-                }
-                const double hk = sqrt(fabs(*(const double*)(hs + 2 * (size_t)k * wsz)));
-                H[k + (size_t)(kdim + 1) * (k - 1)] = round_kind(kind, hk);
-                if (hk > tol) { launch_scal(kind, c->stream, Scalar{1.0 / hk, 0}, w, b->n, c->sms); c->launches++; }
-            }
+            double nrm2 = 0;
+            LKB_TRY(fetch_coeffs(c, kind, k, true, col, &nrm2, nullptr));
+            for (int i = 0; i < k; ++i) H[i + (size_t)(kdim + 1) * (k - 1)] = round_kind(kind, cd(col[i].re, col[i].im));
+            const double hk = sqrt(fabs(nrm2));
+            H[k + (size_t)(kdim + 1) * (k - 1)] = round_kind(kind, hk);
+            if (hk > tol) prof_launch(c, PC_OTHER, 1, [&] { launch_scal(kind, c->stream, Scalar{1.0 / hk, 0}, w, b->n, c->sms); });
             cd* hcol = &H[(size_t)(kdim + 1) * (k - 1)];
             if (cplx) givens_cplx(hcol, cs.data(), sn.data(), k); else givens_real(hcol, cs.data(), sn.data(), k);
             for (int i = 0; i <= k; ++i) hcol[i] = round_kind(kind, hcol[i]);
@@ -258,11 +246,11 @@ static int gmres_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, doubl
             if (precond && !flexible) LKB_TRY(apply_precond(dx->d, -1, -1.0, -1.0)); // preconditioner%apply(dx)  (gmres.fypp:202)
             const void* upd = dx->d;
             if (M) { M->n_matvec++; LKB_TRY(op_apply_enqueue(M, dx->d, wrk->d, false, nullptr)); upd = wrk->d; }   // dx <- M dx
-            launch_axpby(kind, c->stream, one, upd, one, x->d, x->n, c->sms); c->launches++;
+            prof_launch(c, PC_OTHER, 1, [&] { launch_axpby(kind, c->stream, one, upd, one, x->d, x->n, c->sms); });
         }
         LKB_TRY(residual_into_v1(false));
         LKB_TRY(vec_norm_sync(c, kind, col_ptr(V, 0), b->n, &beta));
-        if (fabs(beta) > 0.0) { launch_scal(kind, c->stream, Scalar{1.0 / beta, 0}, col_ptr(V, 0), b->n, c->sms); c->launches++; }
+        if (fabs(beta) > 0.0) prof_launch(c, PC_OTHER, 1, [&] { launch_scal(kind, c->stream, Scalar{1.0 / beta, 0}, col_ptr(V, 0), b->n, c->sms); });
         io->n_iter++; io->n_outer++;
         push_res(io->res, io->res_cap, &io->res_len, fabs(beta));
         if (fabs(beta) < tol) { io->converged = 1; break; }
@@ -317,7 +305,7 @@ static int cg_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double r
     if (precond || mode == CG_NORED) LKB_TRY(lkb_vec_create(c, kind, b->n, b->n_global, b->row0, z.out()));
     // z = r ; preconditioner%apply(z)   (CG.fypp:113-114, 137)
     auto make_z = [&]() -> int {
-        launch_axpby(kind, c->stream, Scalar{1, 0}, r->d, Scalar{0, 0}, z->d, b->n, c->sms); c->launches++;
+        prof_launch(c, PC_OTHER, 1, [&] { launch_axpby(kind, c->stream, Scalar{1, 0}, r->d, Scalar{0, 0}, z->d, b->n, c->sms); });
         int pr = precond(puser, z->d, b->n, -1, -1.0, -1.0, (void*)c->stream);
         if (pr != 0) { set_error("preconditioner callback returned %d", pr); return LKB_ERR_ARG; }
         return 0;
@@ -326,21 +314,21 @@ static int cg_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double r
     double xn = 0;
     LKB_TRY(vec_norm_sync(c, kind, x->d, x->n, &xn));
     if (xn > 0) { A->n_matvec++; LKB_TRY(op_apply_enqueue(A, x->d, r->d, false, nullptr)); }
-    launch_axpby(kind, c->stream, one, b->d, mone, r->d, b->n, c->sms); c->launches++;      // r = b - A x
+    prof_launch(c, PC_OTHER, 1, [&] { launch_axpby(kind, c->stream, one, b->d, mone, r->d, b->n, c->sms); });      // r = b - A x
     Scalar rr_old;
     if (precond) {
         LKB_TRY(make_z());
-        launch_axpby(kind, c->stream, one, z->d, zero, p->d, b->n, c->sms); c->launches++;  // p = z
+        prof_launch(c, PC_OTHER, 1, [&] { launch_axpby(kind, c->stream, one, z->d, zero, p->d, b->n, c->sms); });  // p = z
         LKB_TRY(vec_dot_sync(c, kind, r->d, z->d, b->n, &rr_old));
     } else if (M) {
         // z = M r ; p = z ; rz = r^H z   (a diagonal M writes z straight into p: the loop never stores z)
         M->n_matvec++;
         void* z0 = mode == CG_DIAG ? p->d : z->d;
         LKB_TRY(op_apply_enqueue(M, r->d, z0, false, nullptr));
-        if (mode == CG_NORED) { launch_axpby(kind, c->stream, one, z->d, zero, p->d, b->n, c->sms); c->launches++; }
+        if (mode == CG_NORED) prof_launch(c, PC_OTHER, 1, [&] { launch_axpby(kind, c->stream, one, z->d, zero, p->d, b->n, c->sms); });
         LKB_TRY(vec_dot_sync(c, kind, r->d, z0, b->n, &rr_old));
     } else {
-        launch_axpby(kind, c->stream, one, r->d, zero, p->d, b->n, c->sms); c->launches++;  // p = r
+        prof_launch(c, PC_OTHER, 1, [&] { launch_axpby(kind, c->stream, one, r->d, zero, p->d, b->n, c->sms); });  // p = r
         LKB_TRY(vec_dot_sync(c, kind, r->d, r->d, b->n, &rr_old));
     }
     push_res(io->res, io->res_cap, &io->res_len, sqrt(hypot(rr_old.re, rr_old.im)));
@@ -358,33 +346,26 @@ static int cg_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double r
         cudaMemsetAsync(scal.p, 0, 64, c->stream);
         cudaMemcpyAsync(scal.p, c->tmpw, wsz, cudaMemcpyDeviceToDevice, c->stream);     // r_dot_r_old (just reduced)
         cudaMemsetAsync(c->flags, 0, F_COUNT * sizeof(int), c->stream);
-        const size_t ndw = 2 * (size_t)(kind_cplx(kind) ? 2 : 1);
         auto one_iteration = [&]() -> int {
             LKB_TRY(op_apply_enqueue(A, p->d, Ap->d, false, c->flags));
-            prof_begin(c, PC_DOT);
-            launch_multidot(kind, c->stream, p->d, b->n, 1, Ap->d, b->n, c->partial, c->tmpw, c->counter, c->flags, c->sms, c->p2p_arg());
-            prof_end(c, PC_DOT, 1);
-            LKB_TRY(allreduce_w(c, c->tmpw, ndw));
-            prof_begin(c, PC_OTHER);
-            launch_cg_update(kind, c->stream, scal.p, c->tmpw, p->d, Ap->d, x->d, r->d, b->n, c->partial, c->nrm2, c->counter,
-                             c->flags, c->sms, c->p2p_arg(), mode, mode == CG_DIAG ? M->diag.get() : nullptr);
-            prof_end(c, PC_OTHER, 1);
+            LKB_TRY(dot_reduce(c, kind, p->d, b->n, 1, Ap->d, b->n, c->tmpw, c->flags));
+            prof_launch(c, PC_OTHER, 1, [&] {
+                launch_cg_update(kind, c->stream, scal.p, c->tmpw, p->d, Ap->d, x->d, r->d, b->n, c->partial, c->nrm2, c->counter,
+                                 c->flags, c->sms, c->p2p_arg(), mode, mode == CG_DIAG ? M->diag.get() : nullptr);
+            });
             const void* rr_new = c->nrm2;
             if (mode == CG_NORED) {         // z = M r ; rz = r^H z (multi-dot, j = 1: c2[0])
                 LKB_TRY(op_apply_enqueue(M, r->d, z->d, false, c->flags));
-                prof_begin(c, PC_DOT);
-                launch_multidot(kind, c->stream, r->d, b->n, 1, z->d, b->n, c->partial, c->c2, c->counter, c->flags, c->sms, c->p2p_arg());
-                prof_end(c, PC_DOT, 1);
-                LKB_TRY(allreduce_w(c, c->c2, ndw));
+                LKB_TRY(dot_reduce(c, kind, r->d, b->n, 1, z->d, b->n, c->c2, c->flags));
                 rr_new = c->c2;
             } else {
                 LKB_TRY(allreduce_w(c, c->nrm2, mode == CG_DIAG && kind_cplx(kind) ? 2 : 1));
             }
-            prof_begin(c, PC_OTHER);
-            launch_cg_check(kind, c->stream, scal.p, rr_new, tol, maxiter, (double*)res_hist.p, c->flags);
-            launch_cg_direction(kind, c->stream, scal.p, mode == CG_NORED ? z->d : r->d, p->d, b->n, c->flags, c->sms,
-                                mode == CG_DIAG ? M->diag.get() : nullptr);
-            prof_end(c, PC_OTHER, 2);
+            prof_launch(c, PC_OTHER, 2, [&] {
+                launch_cg_check(kind, c->stream, scal.p, rr_new, tol, maxiter, (double*)res_hist.p, c->flags);
+                launch_cg_direction(kind, c->stream, scal.p, mode == CG_NORED ? z->d : r->d, p->d, b->n, c->flags, c->sms,
+                                    mode == CG_DIAG ? M->diag.get() : nullptr);
+            });
             return check_launch(c, "cg iteration");
         };
         auto one_chunk = [&]() -> int {
@@ -416,9 +397,10 @@ static int cg_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double r
         Scalar pAp;
         LKB_TRY(vec_dot_sync(c, kind, p->d, Ap->d, b->n, &pAp));
         const cd alpha = round_kind(kind, cd(rr_old.re, rr_old.im) / cd(pAp.re, pAp.im));
-        launch_axpby(kind, c->stream, to_scalar(alpha), p->d, one, x->d, b->n, c->sms);      // x += alpha p
-        launch_axpby(kind, c->stream, to_scalar(-alpha), Ap->d, one, r->d, b->n, c->sms);    // r -= alpha Ap
-        c->launches += 2;
+        prof_launch(c, PC_OTHER, 2, [&] {
+            launch_axpby(kind, c->stream, to_scalar(alpha), p->d, one, x->d, b->n, c->sms);      // x += alpha p
+            launch_axpby(kind, c->stream, to_scalar(-alpha), Ap->d, one, r->d, b->n, c->sms);    // r -= alpha Ap
+        });
         Scalar rr_new;
         LKB_TRY(make_z()); LKB_TRY(vec_dot_sync(c, kind, r->d, z->d, b->n, &rr_new));
         const double residual = sqrt(hypot(rr_new.re, rr_new.im));
@@ -426,8 +408,7 @@ static int cg_impl(lkb_op_t A, lkb_vec_t b, lkb_vec_t x, int32_t* info, double r
         push_res(io->res, io->res_cap, &io->res_len, residual);
         if (residual < tol) { io->converged = 1; break; }
         const cd beta = round_kind(kind, cd(rr_new.re, rr_new.im) / cd(rr_old.re, rr_old.im));
-        launch_axpby(kind, c->stream, one, z->d, to_scalar(beta), p->d, b->n, c->sms);       // p = z + beta p
-        c->launches++;
+        prof_launch(c, PC_OTHER, 1, [&] { launch_axpby(kind, c->stream, one, z->d, to_scalar(beta), p->d, b->n, c->sms); });   // p = z + beta p
         rr_old = rr_new;
     }
     *info = io->converged ? io->n_iter : -io->n_iter;

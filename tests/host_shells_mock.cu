@@ -96,7 +96,6 @@ static void collect_from(const void* slot, void* M, int ld, int k, size_t es, in
     memcpy((char*)M + (size_t)ld * (k - 1) * es, slot, (size_t)std::min(ld, k + 1) * es);       // rows 0..k of column k
     int v; memcpy(&v, (const char*)slot + (size_t)ld * es, sizeof(int)); *info = v;
 }
-int arnoldi_fetch_async(lkb_basis_s* X, int, int, void* slot) { fetch_into(slot, X->ncols, kind_size(X->kind)); return 0; }
 int arnoldi_collect(lkb_op_s* A, lkb_basis_s* X, void* H, int ldh, int32_t* info, int kstart, int, bool tr, const void* slot) {
     if (ldh != X->ncols) { set_error("mock: ldh"); return LKB_ERR_ARG; }
     collect_from(slot, H, ldh, kstart, kind_size(X->kind), info);
