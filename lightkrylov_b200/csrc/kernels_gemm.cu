@@ -191,25 +191,44 @@ static bool gemm_dmma(cudaStream_t s, const void* X, int64_t ldx, int k, const v
     return true;
 }
 
+template <int K> static constexpr int gemm_pb() { return Tr<K>::cplx ? 8 : 16; }
+template <int K> static const SmemAttrOnce& gemm_attr() {
+    static const SmemAttrOnce a((const void*)k_basis_gemm<K, gemm_pb<K>()>, 160 * 1024);
+    return a;
+}
+template <int K> static bool gemm_fits_t(int k, SmemFit* f) {
+    const size_t per = (size_t)gemm_pb<K>() * sizeof(typename Tr<K>::E);
+    return smem_fit(gemm_attr<K>(), (size_t)k * per, per, 0, f);
+}
+bool basis_gemm_fits(int kind, int k, SmemFit* f) {
+    switch (kind) {
+        case KS: return gemm_fits_t<KS>(k, f);
+        case KD: return gemm_fits_t<KD>(k, f);
+        case KC: return gemm_fits_t<KC>(k, f);
+        default: return gemm_fits_t<KZ>(k, f);
+    }
+}
+
 template <int K>
 static void gemm_t(cudaStream_t s, const void* X, int64_t ldx, int k, const void* Z, int ldz, int p, void* Y,
                    int64_t ldy, int64_t n, int sms) {
     using E = typename Tr<K>::E;
     // output columns per sweep of X: 16 for the real kinds (2 * 16 FMA per 16-byte pack = 26 TFLOP/s fp64 at
     // full HBM speed, ~70 % of the B200 fp64 pipe), 8 for the complex kinds (4 FMA per complex multiply-add)
-    constexpr int PB = Tr<K>::cplx ? 8 : 16;
+    constexpr int PB = gemm_pb<K>();
     const int64_t npk = n / Tr<K>::EPP;
     int64_t nb = (npk + 255) / 256;
     if (nb < 1) nb = 1;
     if (nb > 4 * (int64_t)sms) nb = 4 * (int64_t)sms;
     dim3 grid((unsigned)nb, (unsigned)((p + PB - 1) / PB));
     const size_t sh = (size_t)k * PB * sizeof(E);
-    static const SmemAttrOnce attr((const void*)k_basis_gemm<K, PB>, 160 * 1024);
-    attr.ensure();
+    gemm_attr<K>().ensure(sh);
     k_basis_gemm<K, PB><<<grid, 256, sh, s>>>((const E*)X, ldx, k, (const E*)Z, ldz, p, (E*)Y, ldy, n);
 }
 void launch_basis_gemm(int kind, cudaStream_t s, const void* X, int64_t ldx, int k, const void* Z, int ldz, int p,
                        void* Y, int64_t ldy, int64_t n, int sms) {
+    SmemFit f;
+    if (!basis_gemm_fits(kind, k, &f)) { refuse_launch("basis_gemm", "k", k, f); return; }
     if (kind == KD && p >= 8 && gemm_dmma(s, X, ldx, k, Z, ldz, p, Y, ldy, n)) return;      // fp64 tensor cores
     switch (kind) {
         case KS: gemm_t<KS>(s, X, ldx, k, Z, ldz, p, Y, ldy, n, sms); break;

@@ -722,6 +722,29 @@ k_multiaxpy_fin(const typename Tr<K>::E* __restrict__ V, int64_t ld, int j,
 }
 
 // ------------------------------------------------------------------------------------------
+// Dynamic shared memory of each launcher, and the attribute it runs with (SmemAttrOnce): launches that fit the fixed
+// value keep it, larger ones raise it up to the device's limit.
+template <int K> static size_t multidot_smem(int j) { return (size_t)(MD_THREADS / 32) * (size_t)(j + 1) * sizeof(typename Tr<K>::W); }
+template <int K> static size_t multidot2_smem(int j) { return (size_t)(MD_THREADS / 32) * 2 * (size_t)(j + 1) * sizeof(typename Tr<K>::W); }
+template <int K> static size_t multiaxpy_smem(int j) { return (size_t)(j > 0 ? j : 1) * sizeof(typename Tr<K>::E); }
+template <int K> static const SmemAttrOnce& multidot_attr() { static const SmemAttrOnce a((const void*)k_multidot<K>, 160 * 1024); return a; }
+template <int K> static const SmemAttrOnce& multidot2_attr() { static const SmemAttrOnce a((const void*)k_multidot2<K, 1, 2>, 100 * 1024); return a; }
+template <int K, bool NORM> static const SmemAttrOnce& multiaxpy_attr() { static const SmemAttrOnce a((const void*)k_multiaxpy<K, NORM>, 0); return a; }
+template <int K> static const SmemAttrOnce& multiaxpy_fin_attr() { static const SmemAttrOnce a((const void*)k_multiaxpy_fin<K>, 0); return a; }
+
+template <int K> static bool multidot_fits_t(int j, SmemFit* f) {
+    const size_t w = (MD_THREADS / 32) * sizeof(typename Tr<K>::W);
+    return smem_fit(multidot_attr<K>(), multidot_smem<K>(j), w, w, f);
+}
+template <int K> static bool multidot2_fits_t(int j, SmemFit* f) {
+    const size_t w = (MD_THREADS / 32) * 2 * sizeof(typename Tr<K>::W);
+    return smem_fit(multidot2_attr<K>(), multidot2_smem<K>(j), w, w, f);
+}
+template <int K> static bool multiaxpy_fits_t(int j, bool fin, SmemFit* f) {
+    // k_multiaxpy<K, true> holds the norm's reduction in static shared memory: its (lower) limit stands for both variants
+    const SmemAttrOnce& a = fin ? multiaxpy_fin_attr<K>() : multiaxpy_attr<K, true>();
+    return smem_fit(a, multiaxpy_smem<K>(j), sizeof(typename Tr<K>::E), 0, f);
+}
 template <int K>
 static void multidot_t(cudaStream_t s, const void* V, int64_t ld, int j, const void* w, int64_t n,
                        void* partial, void* out, unsigned* counter, const int* flags, int sms, const P2P* p2p) {
@@ -745,9 +768,8 @@ static void multidot_t(cudaStream_t s, const void* V, int64_t ld, int j, const v
     if (nb > ngroups) nb = ngroups;
     if (nb < 1) nb = 1;
     if (nb > RT_MAXROWS) nb = RT_MAXROWS;
-    const size_t sh = (size_t)(MD_THREADS / 32) * (size_t)(j + 1) * sizeof(W);
-    static const SmemAttrOnce attr((const void*)k_multidot<K>, 160 * 1024);
-    attr.ensure();
+    const size_t sh = multidot_smem<K>(j);
+    multidot_attr<K>().ensure(sh);
     launch_ex(k_multidot<K>, (unsigned)nb, MD_THREADS, sh, s, pdl_take(2), (const E*)V, ld, j, (const E*)w, n, (W*)partial, (W*)out, counter, flags, pp,
               sweep_dir() | (((size_t)n * sizeof(E) <= W_KEEP_BYTES) ? 2 : 0));
 }
@@ -772,8 +794,10 @@ static void multiaxpy_t(cudaStream_t s, const void* V, int64_t ld, int j, const 
     if (nb < 1) nb = 1;
     if (nb > 2 * sms * 2) nb = 2 * sms * 2;
     if (nb > MAX_ROWBLOCKS) nb = MAX_ROWBLOCKS;
-    const size_t sh = (size_t)(j > 0 ? j : 1) * sizeof(E);
+    const size_t sh = multiaxpy_smem<K>(j);
     const bool pdl = pdl_take(8);
+    if (want_norm) multiaxpy_attr<K, true>().ensure(sh);
+    else multiaxpy_attr<K, false>().ensure(sh);
     if (want_norm)
         launch_ex(k_multiaxpy<K, true>, (unsigned)nb, 256, sh, s, pdl, (const E*)V, ld, j, (const W*)c, (E*)w, n, (double*)partial, (W*)nrm2_out, counter, flags, pp);
     else
@@ -800,7 +824,8 @@ static void multiaxpy_fin_t(cudaStream_t s, const void* V, int64_t ld, int j, co
     if (nb < 1) nb = 1;
     if (nb > 2 * sms * 2) nb = 2 * sms * 2;
     if (nb > MAX_ROWBLOCKS) nb = MAX_ROWBLOCKS;
-    const size_t sh = (size_t)(j > 0 ? j : 1) * sizeof(E);
+    const size_t sh = multiaxpy_smem<K>(j);
+    multiaxpy_fin_attr<K>().ensure(sh);
     FinParams fp;
     fp.c1 = c1; fp.hcol = hcol; fp.tol = tol; fp.atol = atol; fp.inv_dev = (double*)inv_dev; fp.flags = flags;
     fp.kstep = kstep; fp.mode = mode;
@@ -830,9 +855,8 @@ static void multidot2_t(cudaStream_t s, const void* V, int64_t ld, int j, const 
     int64_t nb = 2 * (int64_t)sms;
     if (nb > ntiles) nb = ntiles;
     if (nb < 1) nb = 1;
-    const size_t sh = (size_t)(MD_THREADS / 32) * 2 * (size_t)(j + 1) * sizeof(W);
-    static const SmemAttrOnce attr((const void*)k_multidot2<K, 1, 2>, 100 * 1024);
-    attr.ensure();
+    const size_t sh = multidot2_smem<K>(j);
+    multidot2_attr<K>().ensure(sh);
     k_multidot2<K, 1, 2><<<(int)nb, MD_THREADS, sh, s>>>((const E*)V, ld, j, (const E*)w0, (const E*)w1, n, (W*)partial, (W*)out,
                                                          counter, flags, p2p ? *p2p : P2P());
 }
@@ -854,7 +878,7 @@ static void multiaxpy2_t(cudaStream_t s, const void* V, int64_t ld, int j, const
     if (nb > 4 * (int64_t)sms) nb = 4 * (int64_t)sms;
     const size_t sh = (size_t)2 * (j > 0 ? j : 1) * sizeof(E);
     static const SmemAttrOnce attr((const void*)k_multiaxpy2<K>, 160 * 1024);
-    attr.ensure();
+    attr.ensure(sh);
     k_multiaxpy2<K><<<(int)nb, 256, sh, s>>>((const E*)V, ld, j, (const W*)c, (E*)w0, (E*)w1, n, flags);
 }
 void launch_multiaxpy2(int kind, cudaStream_t s, const void* V, int64_t ld, int j, const void* c, void* w0, void* w1,
@@ -864,6 +888,32 @@ void launch_multiaxpy2(int kind, cudaStream_t s, const void* V, int64_t ld, int 
         case KD: multiaxpy2_t<KD>(s, V, ld, j, c, w0, w1, n, flags, sms); break;
         case KC: multiaxpy2_t<KC>(s, V, ld, j, c, w0, w1, n, flags, sms); break;
         default: multiaxpy2_t<KZ>(s, V, ld, j, c, w0, w1, n, flags, sms); break;
+    }
+}
+
+bool multidot_fits(int kind, int j, SmemFit* f) {
+    if (j == 1) { if (f) *f = SmemFit{0, 0, 1}; return true; }     // k_dot2: no dynamic shared memory
+    switch (kind) {
+        case KS: return multidot_fits_t<KS>(j, f);
+        case KD: return multidot_fits_t<KD>(j, f);
+        case KC: return multidot_fits_t<KC>(j, f);
+        default: return multidot_fits_t<KZ>(j, f);
+    }
+}
+bool multidot2_fits(int kind, int j, SmemFit* f) {
+    switch (kind) {
+        case KS: return multidot2_fits_t<KS>(j, f);
+        case KD: return multidot2_fits_t<KD>(j, f);
+        case KC: return multidot2_fits_t<KC>(j, f);
+        default: return multidot2_fits_t<KZ>(j, f);
+    }
+}
+bool multiaxpy_fits(int kind, int j, bool fin, SmemFit* f) {
+    switch (kind) {
+        case KS: return multiaxpy_fits_t<KS>(j, fin, f);
+        case KD: return multiaxpy_fits_t<KD>(j, fin, f);
+        case KC: return multiaxpy_fits_t<KC>(j, fin, f);
+        default: return multiaxpy_fits_t<KZ>(j, fin, f);
     }
 }
 

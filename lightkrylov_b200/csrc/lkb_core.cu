@@ -44,7 +44,19 @@ int comm_destroy(void* comm) {
 #define LKB_NCCL(call) do { int r_ = (call); if (r_ != 0) { \
     lkb::set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #call, nccl_api()->GetErrorString(r_)); return LKB_ERR_NCCL; } } while (0)
 
+int smem_error(const char* what, const char* dim, int value, const SmemFit& f) {
+    set_error("%s: %s = %d needs %zu B of shared memory per block, above this device's limit of %zu B (%s <= %d)",
+              what, dim, value, f.need, f.limit, dim, f.max);
+    return LKB_ERR_ARG;
+}
+static thread_local bool t_refused = false;     // a launcher refused its launch since the last check_launch
+void refuse_launch(const char* what, const char* dim, int value, const SmemFit& f) {
+    smem_error(what, dim, value, f);
+    t_refused = true;
+}
+
 int check_launch(lkb_ctx_s*, const char* what) {
+    if (t_refused) { t_refused = false; return LKB_ERR_ARG; }     // the message is refuse_launch's
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) { set_error("kernel launch failed (%s): %s", what, cudaGetErrorString(e)); return LKB_ERR_CUDA; }
     return 0;

@@ -337,7 +337,7 @@ int lkb_krylov_schur(lkb_basis_t X, void* H, int ldh, int kdim, int32_t* nkeep) 
         chunk = std::min<int64_t>(chunk, ((X->n + 4095) / 4096) * 4096);
         DevBuf tmp(c);
         LKB_TRY(tmp.alloc((size_t)chunk * nk * es));
-        int r = 0;
+        int r = 0;         // a GEMM that does not fit the device is refused at the first chunk: X and H stay unchanged
         for (int64_t r0 = 0; r0 < X->n && r == 0; r0 += chunk) {
             const int64_t rows = std::min<int64_t>(chunk, X->n - r0);
             prof_launch(c, PC_OTHER, 1, [&] { launch_basis_gemm(kind, c->stream, (char*)X->d + (size_t)r0 * es, X->ld, k, c->coefd, k, nk, tmp.p, chunk, rows, c->sms); });

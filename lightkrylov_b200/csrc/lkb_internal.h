@@ -187,6 +187,8 @@ int allreduce_w(lkb_ctx_s* c, void* buf, size_t ndoubles);
 // make rank 0's copy of a small HOST array authoritative on every rank (k x k host-LAPACK results)
 int bcast_host(lkb_ctx_s* c, void* host_buf, size_t bytes);   // in-place sum over ranks (no-op when world == 1)
 int check_launch(lkb_ctx_s* c, const char* what);
+// LKB_ERR_ARG for a launch whose shared memory does not fit the device (lkb_kernels.h: the *_fits checks), naming the limit
+int smem_error(const char* what, const char* dim, int value, const lkb::SmemFit& f);
 // The profile bracket: prof_end counts the launches in c->launches and, with lkb_set_profile, times them under class
 // `cls`.  Every kernel launch of the library goes through it exactly once (graph replays add their recorded count).
 void prof_begin(lkb_ctx_s* c, int cls);

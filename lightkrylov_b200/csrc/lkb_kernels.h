@@ -35,17 +35,43 @@ enum { KT_WORDS = 4 * 1024 + 16 };
 static inline size_t p2p_region_bytes() { return (size_t)P2P_FLAG_BYTES + 2 * (size_t)P2P_MAXW * P2P_SLOT * 16; }
 
 // cudaFuncAttributeMaxDynamicSharedMemorySize is a PER-DEVICE attribute: set it once for every device a kernel is
-// launched on (a process may hold contexts on several GPUs), not once per process.
+// launched on (a process may hold contexts on several GPUs), not once per process.  `bytes` is the attribute every
+// launch that fits in it runs with (0: the runtime's default is left alone); ensure(need) raises the attribute to `need`
+// the first time a launch needs more.  limit() is the most a launch can ask for on this device: the opt-in maximum per
+// block minus the kernel's static shared memory.
 struct SmemAttrOnce {
-    const void* fn; int bytes; mutable unsigned long long done = 0ULL;      // bit d = set on device d
+    const void* fn; int bytes;
+    mutable int cur[64] = {}, lim[64] = {};      // per device: attribute in force, limit() (0 = not yet known)
     SmemAttrOnce(const void* f, int b) : fn(f), bytes(b) {}
-    void ensure() const {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        const unsigned long long bit = 1ULL << (dev & 63);
-        if (!(done & bit)) { cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes); done |= bit; }
+    static int device() { int dev = 0; cudaGetDevice(&dev); return dev; }
+    size_t limit() const {
+        const int dev = device(), d = dev & 63;
+        if (!lim[d]) {
+            int optin = 0;
+            cudaFuncAttributes fa = {};
+            cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+            cudaFuncGetAttributes(&fa, fn);
+            lim[d] = optin - (int)fa.sharedSizeBytes;
+            if (!bytes && !cur[d]) cur[d] = fa.maxDynamicSharedSizeBytes;
+        }
+        return (size_t)lim[d];
+    }
+    void ensure(size_t need = 0) const {
+        const int d = device() & 63;
+        if (!cur[d]) {
+            if (bytes) { cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes); cur[d] = bytes; }
+            else limit();
+        }
+        if ((int64_t)need > cur[d]) { cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need); cur[d] = (int)need; }
     }
 };
+// Whether a launch's dynamic shared memory fits the device (SmemAttrOnce::limit).  `max` is the largest j (or k) that fits.
+struct SmemFit { size_t need = 0, limit = 0; int max = 0; };
+inline bool smem_fit(const SmemAttrOnce& a, size_t need, size_t per, size_t fixed, SmemFit* f) {
+    const size_t lim = a.limit();
+    if (f) { f->need = need; f->limit = lim; f->max = lim >= fixed ? (int)((lim - fixed) / per) : 0; }
+    return need <= lim;
+}
 
 // ---- programmatic dependent launch (PDL) of the step-loop kernels ------------------------------------------
 // The Krylov step loops chain 5 kernels per step whose tails (two-stage reduction, in-kernel allreduce) leave the GPU
@@ -133,6 +159,11 @@ void launch_multidot2(int kind, cudaStream_t s, const void* V, int64_t ld, int j
                       void* partial, void* out, unsigned* counter, const int* flags, int sms, const P2P* p2p = nullptr);
 void launch_multiaxpy2(int kind, cudaStream_t s, const void* V, int64_t ld, int j, const void* c, void* w0, void* w1,
                        int64_t n, const int* flags, int sms);
+// Whether a launch against j basis columns fits the device's shared memory (the per-block accumulators of the
+// multi-dots, the coefficients of the multi-axpys).  A launcher asked for more than fits fails in the runtime.
+bool multidot_fits(int kind, int j, SmemFit* f = nullptr);
+bool multidot2_fits(int kind, int j, SmemFit* f = nullptr);
+bool multiaxpy_fits(int kind, int j, bool fin, SmemFit* f = nullptr);   // fin: k_multiaxpy_fin, else k_multiaxpy
 // Fused pass-1 multi-axpy + pass-2 multi-dot (TMA + mbarrier pipeline, kernels_fused.cu):
 //   w -= V c1 ; out[0..j) = V^H w_new ; out[j] = w_new^H w_new.   axpy_dot_supported is false when the shape is not
 //   supported (j > 128, ragged n, unaligned, no tensor-map encoder) -- the caller then runs the two separate kernels.
@@ -217,5 +248,11 @@ void launch_dense(int kind, cudaStream_t s, int64_t m, int64_t n, const void* a,
 // Y(:, 0:p) = X(:, 0:k) Z(0:k, 0:p)   tall-skinny basis update (Z on device, E type, ldz)
 void launch_basis_gemm(int kind, cudaStream_t s, const void* X, int64_t ldx, int k, const void* Z, int ldz, int p,
                        void* Y, int64_t ldy, int64_t n, int sms);
+// Whether launch_basis_gemm fits for any p: the FMA kernel keeps k x PB coefficients in shared memory (the DMMA kernel
+// declines, in favour of the FMA kernel, any k it has no room for).  launch_basis_gemm refuses a k that does not fit.
+bool basis_gemm_fits(int kind, int k, SmemFit* f = nullptr);
+// A launcher whose shared memory does not fit records the refusal here instead of launching; the check_launch that follows
+// the launch (lkb_core.cu) returns it as LKB_ERR_ARG, with the limit in the message.
+void refuse_launch(const char* what, const char* dim, int value, const SmemFit& f);
 
 }  // namespace lkb

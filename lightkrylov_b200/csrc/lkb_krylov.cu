@@ -18,12 +18,16 @@ using namespace lkb;
 namespace lkb {
 
 int dot_reduce(lkb_ctx_s* c, int kind, const void* V, int64_t ld, int j, const void* w, int64_t n, void* out, const int* flags) {
+    SmemFit f;
+    if (!multidot_fits(kind, j, &f)) return smem_error("multidot", "j", j, f);
     prof_launch(c, PC_DOT, 1, [&] { launch_multidot(kind, c->stream, V, ld, j, w, n, c->partial, out, c->counter, flags, c->sms, c->p2p_arg()); });
     LKB_TRY(check_launch(c, "multidot"));
     return allreduce_w(c, out, (size_t)(j + 1) * (kind_cplx(kind) ? 2 : 1));
 }
 int axpy_sub(lkb_ctx_s* c, int kind, const void* V, int64_t ld, int j, const void* coef, void* w, int64_t n, bool want_norm,
              const int* flags) {
+    SmemFit f;
+    if (!multiaxpy_fits(kind, j, false, &f)) return smem_error("multiaxpy", "j", j, f);
     prof_launch(c, PC_AXPY, 1, [&] {
         launch_multiaxpy(kind, c->stream, V, ld, j, coef, w, n, want_norm, c->partial, c->nrm2, c->counter, flags, c->sms, c->p2p_arg());
     });
@@ -37,6 +41,11 @@ int dgs_enqueue(lkb_ctx_s* c, int kind, const void* V, int64_t ld, int j, void* 
         if (want_norm) return norm2_enqueue(c, kind, w, n, flags);
         return 0;
     }
+    // nothing is enqueued unless every kernel of the step fits
+    SmemFit f;
+    if (!multidot_fits(kind, j, &f)) return smem_error("multidot", "j", j, f);
+    if (!multiaxpy_fits(kind, j, false, &f)) return smem_error("multiaxpy", "j", j, f);
+    if (fin && !multiaxpy_fits(kind, j, true, &f)) return smem_error("multiaxpy_fin", "j", j, f);
     LKB_TRY(ensure_ws(c, j + 1));
     // serpentine sweeps: pass-1 dot, fused middle and final update walk the rows in alternating directions, and the
     // first direction alternates with the step index (the previous step's final update ended where this one starts)
@@ -579,9 +588,12 @@ static int arnoldi_block(lkb_op_t A, lkb_basis_t X, void* H, int ldh, int32_t* i
             LKB_TRY(op_apply_enqueue(A, col_ptr(X, kpm + i), col_ptr(X, kp + i), trans, nullptr));
             if (trans) A->n_rmatvec++; else A->n_matvec++;
         }
-        for (int i = 0; i < p; i += 2) {
+        // a pair of block columns shares one sweep of the basis when k_multidot2's accumulators fit; past that (kp = 1816
+        // real / 908 complex on B200) every column takes the single-vector path
+        const bool pairs = multidot2_fits(kind, kp);
+        for (int i = 0; i < p; i += pairs ? 2 : 1) {
             LKB_TRY(reset_flags(c));
-            if (i + 1 < p) {
+            if (pairs && i + 1 < p) {
                 // two block columns per sweep of the basis (k_multidot2 / k_multiaxpy2): c laid out [2][kp+1]
                 const int jp = kp + 1;
                 const size_t wsz = kind_cplx(kind) ? 16 : 8;
