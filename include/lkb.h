@@ -159,6 +159,23 @@ int lkb_op_diag_create(lkb_vec_t d, lkb_op_t* M);
  * or row-sharded with equal row and column slabs on this rank), dense or diagonal.  LKB_ERR_ARG for a callback or non-square
  * A, and for a zero or non-finite diagonal entry (lkb_last_error names its global row). */
 int lkb_op_jacobi_create(lkb_op_t A, lkb_op_t* M);
+/* Chebyshev polynomial preconditioner M of degree m >= 1, built on A: M r = z_m, the result of m Chebyshev iterations
+ * (Saad, Iterative Methods, Alg. 12.1, true-residual form) on D^-1 A z = D^-1 r from z_0 = 0, D = diag(A), on [a, b] =
+ * [lmin, lmax].  With theta = (b + a)/2, delta = (b - a)/2, sigma = theta/delta, rho_0 = 1/sigma:
+ *     d_0 = D^-1 r / theta ;  z_1 = d_0 ;  for k = 1 .. m-1:  s_k = D^-1 (r - A z_k) ;  rho_k = 1 / (2 sigma - rho_{k-1}) ;
+ *     d_k = rho_k rho_{k-1} d_{k-1} + (2 rho_k / delta) s_k ;  z_{k+1} = z_k + d_k.
+ * m - 1 applications of A and no inner products; m = 1 is D^-1 / theta.  lkb_op_rmatvec applies M^H (A's rmatvec,
+ * conj(D)^-1).  lmax <= 0 selects the Gershgorin bound max_r sum_c |a_rc / a_rr| of D^-1 A (never below its spectral
+ * radius; 2 for the 5- and 7-point Laplacians); lmin <= 0 selects lmax / 100.  lmin >= lmax (after the defaults) is
+ * LKB_ERR_ARG.  For Hermitian A with a positive diagonal and 0 < lmin < lmax, lmax >= lambda_max(D^-1 A), M is Hermitian
+ * positive definite, so CG may use it; an explicit lmax below the spectrum can make M indefinite and break PCG.
+ * A: stencil (every step is one fused stencil kernel), CSR (plain, L2-blocked, or row-sharded with equal row and column
+ * slabs), dense or diagonal; LKB_ERR_ARG for a callback or non-square A and for a zero or non-finite diagonal entry (the
+ * message names its global row).  Collective when A is a row-sharded CSR and lmax <= 0 (the bound is a max over the ranks).
+ * M keeps a pointer to A: lkb_op_destroy(A) returns LKB_ERR_ARG while M is alive.  M's work vectors are allocated here;
+ * M's matvec counter counts applications of M, A's counters are not touched. */
+int lkb_op_chebyshev_create(lkb_op_t A, int32_t degree, double lmin, double lmax, lkb_op_t* M);
+/* LKB_ERR_ARG, and A stays, while a Chebyshev preconditioner built on A is alive */
 int lkb_op_destroy(lkb_op_t A);
 int lkb_op_matvec(lkb_op_t A, lkb_vec_t x, lkb_vec_t y);    /* apply_matvec  :391-407 (bumps counter) */
 int lkb_op_rmatvec(lkb_op_t A, lkb_vec_t x, lkb_vec_t y);   /* apply_rmatvec :409-424 */

@@ -97,6 +97,7 @@ SIGNATURES = {
     "lkb_op_callback_create": (_i, [_vp, _i, _i64, _i64, MATVEC_FN, _vp, _i32, _P(_vp)]),
     "lkb_op_diag_create": (_i, [_vp, _P(_vp)]),
     "lkb_op_jacobi_create": (_i, [_vp, _P(_vp)]),
+    "lkb_op_chebyshev_create": (_i, [_vp, _i32, _d, _d, _P(_vp)]),
     "lkb_op_destroy": (_i, [_vp]),
     "lkb_op_matvec": (_i, [_vp, _vp, _vp]),
     "lkb_op_rmatvec": (_i, [_vp, _vp, _vp]),

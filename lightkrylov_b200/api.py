@@ -446,6 +446,18 @@ class LinOp:
         op.n_global = getattr(A, "m_global", A.n_global)
         return op
 
+    @classmethod
+    def chebyshev(cls, A: "LinOp", degree: int, lmin: Optional[float] = None, lmax: Optional[float] = None) -> "LinOp":
+        """Chebyshev polynomial preconditioner of `degree` on D^-1 A (include/lkb.h: lkb_op_chebyshev_create), built on
+        the device.  lmax None: the Gershgorin bound of D^-1 A; lmin None: lmax / 100.  Keeps A alive."""
+        h = C.c_void_p()
+        check(A.ctx.lib.lkb_op_chebyshev_create(A.h, int(degree), 0.0 if lmin is None else float(lmin),
+                                                0.0 if lmax is None else float(lmax), C.byref(h)), "chebyshev")
+        op = cls(A.ctx, A.kind, h, A.m, A.m, keep=A)
+        op.row0 = getattr(A, "out_row0", A.row0)
+        op.n_global = getattr(A, "m_global", A.n_global)
+        return op
+
     def matvec(self, x: Vector, y: Vector):
         check(self.ctx.lib.lkb_op_matvec(self.h, x.h, y.h), "matvec")
 

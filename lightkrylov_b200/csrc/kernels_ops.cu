@@ -5,6 +5,7 @@
 // homogeneous Dirichlet outside the global grid.  The slowest axis (y in 2-D, z in 3-D) is the
 // row-sharded one: the neighbouring slab's boundary row / plane arrives in halo_lo / halo_hi.
 #include <algorithm>
+#include <type_traits>
 #include "lkb_kernels.h"
 #include "lkb_p2p.cuh"
 
@@ -32,6 +33,14 @@ template <typename E, int PW> struct PackOps {
             for (int e = 0; e < PW; ++e) r.v[e] = __ldcg(p + e);
             return r; }
     }
+    // row-local operands of the Chebyshev epilogue (r, d): streamed, no L1 allocation
+    static LKB_DI P ld_nc(const E* p) {
+        if constexpr (FULL) return ld_pack_nc<P>(p);
+        else { P r;
+#pragma unroll
+            for (int e = 0; e < PW; ++e) r.v[e] = p[e];
+            return r; }
+    }
     static LKB_DI void st(E* p, const P& v) {
         if constexpr (FULL) st_pack(p, v);
         else {
@@ -50,6 +59,38 @@ template <typename E, int PW> struct PackOps {
         return r; }
 };
 
+
+// Store epilogues of the two stencil kernels, chosen at compile time.  StorePlain: y = A x (the matvec).  ChebStep: one
+// step k of the Chebyshev preconditioner (lkb_cheb.cu) on the matvec's output t = (A x)_i and its input x_i = (z_k)_i,
+//     s = invd (r_i - t) ;  d_i <- alpha d_i + beta s ;  y_i = z_{k+1} = z_k + d_i
+// with x = z_k, or on the first step x = r itself (z_1 = d_0 = b0 invd r, so z_1 and A z_1 are b0 invd times x and A x).
+// The last step stores only y.  HBM traffic per step: x, r, d read, d, y written (first step: r read, d, y written).
+struct StorePlain {};
+template <typename E> struct ChebStep {
+    const E* r; E* d;
+    E invd;                                     // D^-1: the scalar 1 / c0 (conjugated for the rmatvec)
+    double alpha, beta, b0;                     // step coefficients (lkb_cheb.cu), rounded to the kind in the kernel
+    int first, last;
+};
+template <typename E, int PW, typename Rl>
+LKB_DI void cheb_store(const ChebStep<E>& c, E* y, int64_t q, const Pack<E, PW>& t, const Pack<E, PW>& x) {
+    using PO = PackOps<E, PW>;
+    using P = Pack<E, PW>;
+    const Rl alpha = (Rl)c.alpha, beta = (Rl)c.beta, b0 = (Rl)c.b0;
+    const P rv = c.first ? x : PO::ld_nc(c.r + q);
+    P dv, zn;
+    if (!c.first) dv = PO::ld_nc(c.d + q);
+#pragma unroll
+    for (int e = 0; e < PW; ++e) {
+        const E zk = c.first ? rscale(mul_v(c.invd, x.v[e]), b0) : x.v[e];
+        const E tk = c.first ? rscale(mul_v(c.invd, t.v[e]), b0) : t.v[e];
+        const E s = mul_v(c.invd, add_v(rv.v[e], rscale(tk, (Rl)-1)));
+        dv.v[e] = add_v(rscale(c.first ? zk : dv.v[e], alpha), rscale(s, beta));
+        zn.v[e] = add_v(zk, dv.v[e]);
+    }
+    if (!c.last) PO::st(c.d + q, dv);
+    PO::st(y + q, zn);
+}
 
 // Both stencil kernels take one CTA per (column block, row block[, plane]) of a 1-D grid, column block fastest
 // (consecutive CTAs stream consecutive segments of the same grid rows).  The row blocks (2-D) / planes (3-D) are rotated
@@ -85,13 +126,13 @@ LKB_DI void halo_wait(const unsigned* halo_epoch, const unsigned* flag_lo, const
 // a deeper plane prefetch thrashed L1).  A z-march with the plane staged in shared memory (two block barriers per
 // plane, round 1) reached 2.8 TB/s.
 // ------------------------------------------------------------------------------------------
-template <int K, int PW>
+template <int K, int PW, class EPI = StorePlain>
 __global__ void __launch_bounds__(256)
 k_stencil(const typename Tr<K>::E* __restrict__ x, typename Tr<K>::E* __restrict__ y,
           int64_t nx, int64_t ny, int64_t nz, Coef7<typename Tr<K>::E> cf,
           const typename Tr<K>::E* __restrict__ halo_lo, const typename Tr<K>::E* __restrict__ halo_hi,
           const unsigned* __restrict__ halo_epoch, int64_t halo_parity_stride, const unsigned* __restrict__ flag_lo,
-          const unsigned* __restrict__ flag_hi, int64_t ncb, const int* __restrict__ flags, const int keep_w)
+          const unsigned* __restrict__ flag_hi, int64_t ncb, const int* __restrict__ flags, const int keep_w, const EPI epi)
 {
     using E = typename Tr<K>::E;
     using PO = PackOps<E, PW>;
@@ -144,7 +185,11 @@ k_stencil(const typename Tr<K>::E* __restrict__ x, typename Tr<K>::E* __restrict
             fmacc(s, up.v[e], cf.c[6]);
             out.v[e] = s;
         }
-        if (active) PO::st_w(y + k * plane + p, out, keep, pol);
+        if constexpr (std::is_same_v<EPI, StorePlain>) {
+            if (active) PO::st_w(y + k * plane + p, out, keep, pol);
+        } else {
+            if (active) cheb_store<E, PW, typename Tr<K>::Rl>(epi, y, k * plane + p, out, center);
+        }
         south = center; center = north;
     }
 }
@@ -169,13 +214,13 @@ template <int BYTES> LKB_DI void cp_async(void* smem_dst, const void* gsrc) {
 }
 LKB_DI void cp_async_wait_all() { asm volatile("cp.async.commit_group;\n\tcp.async.wait_group 0;" ::: "memory"); }
 
-template <int K, int PW>
+template <int K, int PW, class EPI = StorePlain>
 __global__ void __launch_bounds__(ST_TX)
 k_stencil_smem(const typename Tr<K>::E* __restrict__ x, typename Tr<K>::E* __restrict__ y,
                int64_t nx, int64_t ny, int64_t nz, Coef7<typename Tr<K>::E> cf,
                const typename Tr<K>::E* __restrict__ halo_lo, const typename Tr<K>::E* __restrict__ halo_hi,
                const unsigned* __restrict__ halo_epoch, int64_t halo_parity_stride, const unsigned* __restrict__ flag_lo,
-               const unsigned* __restrict__ flag_hi, int64_t ncb, const int* __restrict__ flags, const int keep_w)
+               const unsigned* __restrict__ flag_hi, int64_t ncb, const int* __restrict__ flags, const int keep_w, const EPI epi)
 {
     using E = typename Tr<K>::E;
     using P = Pack<E, PW>;
@@ -244,12 +289,13 @@ k_stencil_smem(const typename Tr<K>::E* __restrict__ x, typename Tr<K>::E* __res
             fmacc(sacc, north.v[e], cf.c[4]);
             out.v[e] = sacc;
         }
-        PackOps<E, PW>::st_w(y + p, out, keep, pol);
+        if constexpr (std::is_same_v<EPI, StorePlain>) PackOps<E, PW>::st_w(y + p, out, keep, pol);
+        else cheb_store<E, PW, typename Tr<K>::Rl>(epi, y, p, out, center);
     }
 }
 
-template <int K, int PW, int DIM>
-static void stencil_launch(cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans, const int* flags) {
+template <int K, int PW, int DIM, class EPI>
+static void stencil_launch(cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans, const int* flags, const EPI& epi) {
     using E = typename Tr<K>::E;
     Coef7<E> cf;
     Scalar c[7];
@@ -266,40 +312,61 @@ static void stencil_launch(cudaStream_t s, const StencilArgs& a, const void* x, 
     auto launch = [&](auto kern, int64_t ncb, unsigned block, size_t smem) {
         const unsigned grid = (unsigned)(nyb * a.nz * ncb);
         launch_ex(kern, grid, block, smem, s, pdl_take(1), (const E*)x, (E*)y, a.nx, a.ny, a.nz, cf,
-                  (const E*)a.halo_lo, (const E*)a.halo_hi, a.halo_epoch, a.halo_parity_stride, a.flag_lo, a.flag_hi, ncb, flags, keep_w);
+                  (const E*)a.halo_lo, (const E*)a.halo_hi, a.halo_epoch, a.halo_parity_stride, a.flag_lo, a.flag_hi, ncb, flags, keep_w, epi);
     };
     if constexpr (DIM == 2) {
-        static const SmemAttrOnce once((const void*)k_stencil_smem<K, PW>, 96 * 1024);
+        static const SmemAttrOnce once((const void*)k_stencil_smem<K, PW, EPI>, 96 * 1024);
         once.ensure();
-        launch(k_stencil_smem<K, PW>, (npk_row + ST_TX - 1) / ST_TX, ST_TX, (size_t)(ST_RY + 2) * ST_TX * sizeof(Pack<E, PW>));
+        launch(k_stencil_smem<K, PW, EPI>, (npk_row + ST_TX - 1) / ST_TX, ST_TX, (size_t)(ST_RY + 2) * ST_TX * sizeof(Pack<E, PW>));
     } else {
         // CTA width: the narrowest multiple of 32 threads that covers a grid row with the same number of CTAs as 256-wide
         // ones would (384^3: 192 packs per row -> 192 threads, no idle lanes; a 256-wide CTA left 25 % of its threads idle:
         // 4.28 TB/s at 384^3 against 5.17 TB/s at 512^3)
         const int64_t ncb = (npk_row + 255) / 256;
-        launch(k_stencil<K, PW>, ncb, (unsigned)std::min<int64_t>(256, ((npk_row + ncb - 1) / ncb + 31) / 32 * 32), 0);
+        launch(k_stencil<K, PW, EPI>, ncb, (unsigned)std::min<int64_t>(256, ((npk_row + ncb - 1) / ncb + 31) / 32 * 32), 0);
     }
 }
 
-template <int K>
-static void stencil_t(cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans, const int* flags) {
+template <int K, class EPI>
+static void stencil_t(cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans, const int* flags, const EPI& epi) {
     constexpr int EPP = Tr<K>::EPP;
     const bool vec = (a.nx % EPP == 0);
     if (a.dim == 2) {
-        if (vec) stencil_launch<K, EPP, 2>(s, a, x, y, trans, flags);
-        else stencil_launch<K, 1, 2>(s, a, x, y, trans, flags);
+        if (vec) stencil_launch<K, EPP, 2>(s, a, x, y, trans, flags, epi);
+        else stencil_launch<K, 1, 2>(s, a, x, y, trans, flags, epi);
     } else {
-        if (vec) stencil_launch<K, EPP, 3>(s, a, x, y, trans, flags);
-        else stencil_launch<K, 1, 3>(s, a, x, y, trans, flags);
+        if (vec) stencil_launch<K, EPP, 3>(s, a, x, y, trans, flags, epi);
+        else stencil_launch<K, 1, 3>(s, a, x, y, trans, flags, epi);
     }
 }
 void launch_stencil(int kind, cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans,
                     const int* flags, int) {
     switch (kind) {
-        case KS: stencil_t<KS>(s, a, x, y, trans, flags); break;
-        case KD: stencil_t<KD>(s, a, x, y, trans, flags); break;
-        case KC: stencil_t<KC>(s, a, x, y, trans, flags); break;
-        default: stencil_t<KZ>(s, a, x, y, trans, flags); break;
+        case KS: stencil_t<KS>(s, a, x, y, trans, flags, StorePlain()); break;
+        case KD: stencil_t<KD>(s, a, x, y, trans, flags, StorePlain()); break;
+        case KC: stencil_t<KC>(s, a, x, y, trans, flags, StorePlain()); break;
+        default: stencil_t<KZ>(s, a, x, y, trans, flags, StorePlain()); break;
+    }
+}
+// One fused Chebyshev step (ChebStep above): y = z_{k+1} from x = z_k (first step: x = r)
+template <int K>
+static void stencil_cheb_t(cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans, const int* flags,
+                           const ChebArgs& ca) {
+    using E = typename Tr<K>::E;
+    ChebStep<E> epi;
+    epi.r = (const E*)ca.r; epi.d = (E*)ca.d;
+    from_scalar(ca.invd, epi.invd);
+    epi.alpha = ca.alpha; epi.beta = ca.beta; epi.b0 = ca.b0;
+    epi.first = ca.first ? 1 : 0; epi.last = ca.last ? 1 : 0;
+    stencil_t<K>(s, a, x, y, trans, flags, epi);
+}
+void launch_stencil_cheb(int kind, cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans, const int* flags,
+                         const ChebArgs& ca) {
+    switch (kind) {
+        case KS: stencil_cheb_t<KS>(s, a, x, y, trans, flags, ca); break;
+        case KD: stencil_cheb_t<KD>(s, a, x, y, trans, flags, ca); break;
+        case KC: stencil_cheb_t<KC>(s, a, x, y, trans, flags, ca); break;
+        default: stencil_cheb_t<KZ>(s, a, x, y, trans, flags, ca); break;
     }
 }
 
@@ -546,6 +613,88 @@ void launch_jacobi(int kind, cudaStream_t s, const JacobiSrc& src, void* d, unsi
         case KD: jacobi_t<KD>(s, src, d, bad_row, sms); break;
         case KC: jacobi_t<KC>(s, src, d, bad_row, sms); break;
         default: jacobi_t<KZ>(s, src, d, bad_row, sms); break;
+    }
+}
+
+// Gershgorin bound of D^-1 A (Chebyshev preconditioner set-up, once per operator): max over the rows of
+// sum_c |a_rc| / |a_rr|, each a_rc the sum of the row's entries at column c (duplicates summed, as the SpMV sums them), in
+// double.  The max of non-negative doubles is exact in any order, so one atomicMax on their bit patterns per warp gives a
+// deterministic result.  Rows whose diagonal entry is zero or not finite are skipped: k_jacobi reports them.
+LKB_DI double abs_w(double a) { return fabs(a); }
+LKB_DI double abs_w(double2 a) { return hypot(a.x, a.y); }
+LKB_DI double2 w2(double a) { return make_double2(a, 0.0); }
+LKB_DI double2 w2(double2 a) { return a; }
+// sum over the distinct columns of entries [q0, q1) of |sum of the entries at that column|; dg = the entry sum at column cr
+template <typename E, typename Q>
+LKB_DI double row_abs_sum(const int32_t* col, const E* val, Q q0, Q q1, int64_t cr, double2& dg) {
+    bool sorted = true;
+    for (Q q = q0 + 1; q < q1; ++q) sorted = sorted && col[q - 1] <= col[q];
+    double sum = 0.0;
+    for (Q q = q0; q < q1;) {
+        const int32_t cq = col[q];
+        auto a = widen(val[q]);
+        Q next = q + 1;
+        if (sorted) {
+            for (; next < q1 && col[next] == cq; ++next) wadd(a, widen(val[next]));
+        } else {
+            bool seen = false;
+            for (Q p = q0; p < q && !seen; ++p) seen = col[p] == cq;
+            if (seen) { q = next; continue; }
+            for (Q p = next; p < q1; ++p) if (col[p] == cq) wadd(a, widen(val[p]));
+        }
+        sum += abs_w(a);
+        if (cq == cr) dg = w2(a);
+        q = next;
+    }
+    return sum;
+}
+template <int K, int MODE>
+__global__ void __launch_bounds__(256)
+k_gershgorin(const JacobiSrc src, unsigned long long* __restrict__ bound_bits)
+{
+    using E = typename Tr<K>::E;
+    double best = 0.0;
+    for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < src.rows; r += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t cr = src.col0 + r;
+        double2 dg = make_double2(0.0, 0.0);
+        double sum = 0.0;
+        if constexpr (MODE == JAC_CSR) {
+            sum = row_abs_sum((const int32_t*)src.col, (const E*)src.val, src.rowptr[r], src.rowptr[r + 1], cr, dg);
+        } else if constexpr (MODE == JAC_CSR_BLOCKED) {
+            for (int b = 0; b < src.blk.nb; ++b) {
+                const uint32_t* tab = src.blk.tab + (size_t)b * (src.rows + 1);
+                sum += row_abs_sum((const int32_t*)src.blk.col, (const E*)src.blk.val, tab[r], tab[r + 1], cr, dg);
+            }
+        } else {      // dense, column-major rows x rows
+            const E* a = (const E*)src.a;
+            for (int64_t c = 0; c < src.rows; ++c) sum += abs_w(widen(a[r + src.rows * c]));
+            dg = w2(widen(a[r * (src.rows + 1)]));
+        }
+        const double ad = hypot(dg.x, dg.y);
+        if (isfinite(ad) && ad != 0.0) best = fmax(best, sum / ad);
+    }
+    unsigned long long bits = (unsigned long long)__double_as_longlong(best);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) bits = max(bits, __shfl_xor_sync(0xffffffffu, bits, o));
+    if ((threadIdx.x & 31) == 0) atomicMax(bound_bits, bits);
+}
+template <int K>
+static void gershgorin_t(cudaStream_t s, const JacobiSrc& src, unsigned long long* bound_bits, int sms) {
+    int64_t nb = (src.rows + 255) / 256;
+    if (nb < 1) nb = 1;
+    if (nb > (int64_t)sms * 16) nb = (int64_t)sms * 16;
+    switch (src.mode) {
+        case JAC_CSR: k_gershgorin<K, JAC_CSR><<<(int)nb, 256, 0, s>>>(src, bound_bits); break;
+        case JAC_CSR_BLOCKED: k_gershgorin<K, JAC_CSR_BLOCKED><<<(int)nb, 256, 0, s>>>(src, bound_bits); break;
+        default: k_gershgorin<K, JAC_DENSE><<<(int)nb, 256, 0, s>>>(src, bound_bits); break;
+    }
+}
+void launch_gershgorin(int kind, cudaStream_t s, const JacobiSrc& src, unsigned long long* bound_bits, int sms) {
+    switch (kind) {
+        case KS: gershgorin_t<KS>(s, src, bound_bits, sms); break;
+        case KD: gershgorin_t<KD>(s, src, bound_bits, sms); break;
+        case KC: gershgorin_t<KC>(s, src, bound_bits, sms); break;
+        default: gershgorin_t<KZ>(s, src, bound_bits, sms); break;
     }
 }
 

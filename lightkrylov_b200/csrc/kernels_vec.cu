@@ -433,6 +433,53 @@ k_diag(const typename Tr<K>::E* __restrict__ d, const typename Tr<K>::E* x, type
         for (int64_t t = npk * EPP; t < n; ++t) y[t] = mul_v(CONJ ? conj_v(d[t]) : d[t], x[t]);
 }
 
+// One step of the Chebyshev preconditioner on an operator without a fused step (lkb_cheb.cu), after t = A z_k:
+//     s = invd o (r - t) ;  d <- alpha d_in + beta s ;  z <- z + d      (d_out: nullptr on the last step)
+// init: t, d_in and z read as zero, so z = beta invd o r = z_1 (beta = 1 / theta).  invd is the vector D^-1 (conj: conj(D)^-1),
+// or the scalar invd_s when it is nullptr.  d_in may be z (first step: d_0 = z_1) and d_out may be d_in: every pack is read
+// by the thread that then writes it, as in k_diag.
+template <int K>
+__global__ void __launch_bounds__(256)
+k_cheb_update(const typename Tr<K>::E* __restrict__ r, const typename Tr<K>::E* __restrict__ invd, typename Tr<K>::E invd_s,
+              const typename Tr<K>::E* __restrict__ t, const typename Tr<K>::E* d_in, typename Tr<K>::E* d_out,
+              typename Tr<K>::E* z, int64_t n, typename Tr<K>::Rl alpha, typename Tr<K>::Rl beta, bool conj, bool init,
+              const int* __restrict__ flags)
+{
+    using E = typename Tr<K>::E;
+    using Rl = typename Tr<K>::Rl;
+    constexpr int EPP = Tr<K>::EPP;
+    using P = Pack<E, EPP>;
+    if (flags && flags[F_STOP]) return;
+    auto step = [&](E rv, E iv, E tv, E dv) -> E {
+        const E s = mul_v(conj ? conj_v(iv) : iv, add_v(rv, rscale(tv, (Rl)-1)));
+        return add_v(rscale(dv, alpha), rscale(s, beta));
+    };
+    const int64_t npk = n / EPP;
+    for (int64_t pk = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; pk < npk; pk += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t o = pk * EPP;
+        const P rv = ld_pack_nc<P>(r + o);
+        P iv, tv, dv, zv;
+#pragma unroll
+        for (int e = 0; e < EPP; ++e) { iv.v[e] = invd_s; tv.v[e] = dv.v[e] = zv.v[e] = zero_v(E()); }
+        if (invd) iv = ld_pack_nc<P>(invd + o);
+        if (!init) { tv = ld_pack_nc<P>(t + o); dv = ld_pack_nc<P>(d_in + o); zv = ld_pack_nc<P>(z + o); }
+#pragma unroll
+        for (int e = 0; e < EPP; ++e) {
+            dv.v[e] = step(rv.v[e], iv.v[e], tv.v[e], dv.v[e]);
+            zv.v[e] = add_v(zv.v[e], dv.v[e]);
+        }
+        if (d_out) st_pack(d_out + o, dv);
+        st_pack(z + o, zv);
+    }
+    if (blockIdx.x == 0 && threadIdx.x == 0)
+        for (int64_t i = npk * EPP; i < n; ++i) {
+            const E zv = init ? zero_v(E()) : z[i];
+            const E dv = step(r[i], invd ? invd[i] : invd_s, init ? zero_v(E()) : t[i], init ? zero_v(E()) : d_in[i]);
+            if (d_out) d_out[i] = dv;
+            z[i] = add_v(zv, dv);
+        }
+}
+
 // ------------------------------------------------------------------------------------------
 // GMRES column update on the device (gmres.fypp:167-194 + submodule_utility_functions.fypp:169-204): after the
 // CGS2 kernels of inner step k this single CTA forms H(:k,k) = c1 + c2 and H(k+1,k) = ||w||, decides the
@@ -595,6 +642,15 @@ void launch_diag(int kind, cudaStream_t s, const void* d, const void* x, void* y
         using E = typename Tr<K>::E;
         auto kern = conj ? k_diag<K, true> : k_diag<K, false>;
         kern<<<ew_grid(n / Tr<K>::EPP, sms), 256, 0, s>>>((const E*)d, (const E*)x, (E*)y, n, flags);
+    });
+}
+void launch_cheb_update(int kind, cudaStream_t s, const void* r, const void* invd, Scalar invd_s, const void* t, const void* d_in,
+                        void* d_out, void* z, int64_t n, double alpha, double beta, bool conj, bool init, const int* flags, int sms) {
+    LKB_DISPATCH(kind, {
+        using E = typename Tr<K>::E; using Rl = typename Tr<K>::Rl;
+        E is; from_scalar(invd_s, is);
+        k_cheb_update<K><<<ew_grid(n / Tr<K>::EPP, sms), 256, 0, s>>>((const E*)r, (const E*)invd, is, (const E*)t, (const E*)d_in,
+                                                                       (E*)d_out, (E*)z, n, (Rl)alpha, (Rl)beta, conj, init, flags);
     });
 }
 void launch_gmres_update(int kind, cudaStream_t s, const void* c1, const void* c2, int k, const void* nrm2, void* H, int ldh,

@@ -744,46 +744,14 @@ int lkb_op_diag_create(lkb_vec_t d, lkb_op_t* M) {
 int lkb_op_jacobi_create(lkb_op_t A, lkb_op_t* M) {
     if (!A || !M) { set_error("jacobi_create: null argument"); return LKB_ERR_ARG; }
     lkb_ctx_s* c = A->ctx;
-    if (A->type == OP_CALLBACK) { set_error("jacobi_create: a callback operator has no diagonal the library can read"); return LKB_ERR_ARG; }
-    if (A->m != A->n) { set_error("jacobi_create: A is not square (%lld x %lld local rows / columns)", (long long)A->m, (long long)A->n); return LKB_ERR_ARG; }
-    JacobiSrc src;
-    src.rows = A->m;
-    int64_t n_global = A->m;
-    if (A->type == OP_STENCIL) {
-        const int64_t plane = A->st.dim == 2 ? A->st.nx : A->st.nx * A->st.ny;
-        src.mode = JAC_STENCIL; src.c0 = A->st.coef[0];
-        src.row0 = A->slow0 * plane; n_global = A->nslow_global * plane;
-    } else if (A->type == OP_CSR) {
-        if (A->dist) {
-            const int r = c->rank;
-            if (A->row_off[r] != A->col_off[r] || A->row_cnt[r] != A->col_cnt[r] || A->m_global != A->n_global) {
-                set_error("jacobi_create: row-sharded CSR whose row slab [%lld,+%lld) differs from its column slab [%lld,+%lld) "
-                          "on rank %d (the diagonal is defined only when they agree)", (long long)A->row_off[r], (long long)A->row_cnt[r],
-                          (long long)A->col_off[r], (long long)A->col_cnt[r], r);
-                return LKB_ERR_ARG;
-            }
-            src.row0 = src.col0 = A->row_off[r]; n_global = A->n_global;
-        }
-        if (A->blk.nb > 0) { src.mode = JAC_CSR_BLOCKED; src.blk = A->blk; }
-        else { src.mode = JAC_CSR; src.rowptr = A->rowptr; src.col = A->col; src.val = A->val; }
-    } else if (A->type == OP_DENSE) {
-        src.mode = JAC_DENSE; src.a = A->a;
-    } else if (A->type == OP_DIAG) {
-        src.mode = JAC_DIAG; src.a = A->diag; src.row0 = A->diag_row0; n_global = A->diag_n_global;
-    } else {
-        set_error("jacobi_create: unsupported operator type %d", A->type); return LKB_ERR_ARG;
-    }
+    JacobiSrc src; int64_t n_global = 0;
+    LKB_TRY(jacobi_source(A, "jacobi_create", &src, &n_global));
     OpOwner op;
     LKB_TRY(diag_from_device(c, A->kind, A->m, src.row0, n_global, op));
-    CudaPtr<unsigned long long> bad; unsigned long long hbad = 0;
-    LKB_TRY(cuda_alloc(bad, sizeof(unsigned long long)));
-    LKB_CUDA(cudaMemsetAsync(bad, 0xff, sizeof(unsigned long long), c->stream));
-    launch_jacobi(A->kind, c->stream, src, op->diag, bad, c->sms);
-    LKB_TRY(check_launch(c, "jacobi"));
-    LKB_CUDA(cudaMemcpyAsync(&hbad, bad, sizeof(hbad), cudaMemcpyDeviceToHost, c->stream));
-    LKB_CUDA(cudaStreamSynchronize(c->stream));
-    if (hbad != ~0ULL) {
-        set_error("jacobi_create: the diagonal entry of global row %llu is zero or not finite", hbad);
+    unsigned long long bad = 0;
+    LKB_TRY(jacobi_build(c, A->kind, src, op->diag, &bad, nullptr));
+    if (bad != ~0ULL) {
+        set_error("jacobi_create: the diagonal entry of global row %llu is zero or not finite", bad);
         return LKB_ERR_ARG;
     }
     *M = op.release();
@@ -791,6 +759,11 @@ int lkb_op_jacobi_create(lkb_op_t A, lkb_op_t* M) {
 }
 int lkb_op_destroy(lkb_op_t A) {
     if (!A) return LKB_ERR_ARG;
+    if (A->cheb_users > 0) {
+        set_error("op_destroy: %d Chebyshev preconditioner(s) built on this operator are still alive (destroy them first)", A->cheb_users);
+        return LKB_ERR_ARG;
+    }
+    if (A->cheb_A) A->cheb_A->cheb_users--;
     cudaStreamSynchronize(A->ctx->stream);
     invalidate_graphs(A->ctx, A->uid);
     delete A;
@@ -806,41 +779,99 @@ int lkb_op_reset_counters(lkb_op_t A) { A->n_matvec = A->n_rmatvec = 0; return 0
 }  // extern "C"
 
 namespace lkb {
+int jacobi_source(const lkb_op_s* A, const char* what, JacobiSrc* out, int64_t* n_global_out) {
+    lkb_ctx_s* c = A->ctx;
+    if (A->type == OP_CALLBACK) { set_error("%s: a callback operator has no diagonal the library can read", what); return LKB_ERR_ARG; }
+    if (A->m != A->n) { set_error("%s: A is not square (%lld x %lld local rows / columns)", what, (long long)A->m, (long long)A->n); return LKB_ERR_ARG; }
+    JacobiSrc src;
+    src.rows = A->m;
+    int64_t n_global = A->m;
+    if (A->type == OP_STENCIL) {
+        const int64_t plane = A->st.dim == 2 ? A->st.nx : A->st.nx * A->st.ny;
+        src.mode = JAC_STENCIL; src.c0 = A->st.coef[0];
+        src.row0 = A->slow0 * plane; n_global = A->nslow_global * plane;
+    } else if (A->type == OP_CSR) {
+        if (A->dist) {
+            const int r = c->rank;
+            if (A->row_off[r] != A->col_off[r] || A->row_cnt[r] != A->col_cnt[r] || A->m_global != A->n_global) {
+                set_error("%s: row-sharded CSR whose row slab [%lld,+%lld) differs from its column slab [%lld,+%lld) "
+                          "on rank %d (the diagonal is defined only when they agree)", what, (long long)A->row_off[r], (long long)A->row_cnt[r],
+                          (long long)A->col_off[r], (long long)A->col_cnt[r], r);
+                return LKB_ERR_ARG;
+            }
+            src.row0 = src.col0 = A->row_off[r]; n_global = A->n_global;
+        }
+        if (A->blk.nb > 0) { src.mode = JAC_CSR_BLOCKED; src.blk = A->blk; }
+        else { src.mode = JAC_CSR; src.rowptr = A->rowptr; src.col = A->col; src.val = A->val; }
+    } else if (A->type == OP_DENSE) {
+        src.mode = JAC_DENSE; src.a = A->a;
+    } else if (A->type == OP_DIAG) {
+        src.mode = JAC_DIAG; src.a = A->diag; src.row0 = A->diag_row0; n_global = A->diag_n_global;
+    } else {
+        set_error("%s: unsupported operator type %d", what, A->type); return LKB_ERR_ARG;
+    }
+    *out = src;
+    *n_global_out = n_global;
+    return 0;
+}
+int jacobi_build(lkb_ctx_s* c, int kind, const JacobiSrc& src, void* d, unsigned long long* bad_row, double* bound) {
+    CudaPtr<unsigned long long> dev;           // [0] the first bad row, [1] the bound's bit pattern
+    unsigned long long h[2] = {~0ULL, 0ULL};
+    LKB_TRY(cuda_alloc(dev, sizeof(h)));
+    LKB_CUDA(cudaMemcpyAsync(dev, h, sizeof(h), cudaMemcpyHostToDevice, c->stream));
+    launch_jacobi(kind, c->stream, src, d, dev, c->sms);
+    if (bound) launch_gershgorin(kind, c->stream, src, dev.get() + 1, c->sms);
+    LKB_TRY(check_launch(c, "jacobi"));
+    LKB_CUDA(cudaMemcpyAsync(h, dev, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
+    LKB_CUDA(cudaStreamSynchronize(c->stream));
+    *bad_row = h[0];
+    if (bound) memcpy(bound, &h[1], sizeof(double));
+    return 0;
+}
+int stencil_halo_exchange(lkb_op_s* A, const void* x, const int* flags, bool halo_prepushed, int* nl) {
+    lkb_ctx_s* c = A->ctx;
+    if (c->world > 1 && A->hp_active) {
+        // halo exchange over NVLink peer memory: pushed by the kernel that finished x, or by k_halo_push
+        // (copy + synchronisation in one kernel)
+        if (!halo_prepushed) { launch_halo_push(A->kind, c->stream, A->hp, x, A->m, flags); *nl += 1; }
+    } else if (c->world > 1) {
+        // halo exchange over NCCL send/recv: my first row/plane -> rank-1's halo_hi, my last -> rank+1's halo_lo
+        NcclApi* api = nccl_api();
+        if (!api) return LKB_ERR_NCCL;
+        const size_t es = kind_size(A->kind);
+        const int64_t he = A->halo_elems;
+        const int64_t nloc = A->m;
+        const size_t cnt = (size_t)he * (kind_cplx(A->kind) ? 2 : 1);
+        const int dt = (A->kind == KS || A->kind == KC) ? 7 : 8;   // ncclFloat32 / ncclFloat64
+        const bool has_lo = A->st.halo_lo != nullptr, has_hi = A->st.halo_hi != nullptr;
+        LKB_NCCL(api->GroupStart());
+        if (has_lo) {
+            LKB_NCCL(api->Send(x, cnt, dt, c->rank - 1, c->comm, c->stream));
+            LKB_NCCL(api->Recv(A->halo_lo, cnt, dt, c->rank - 1, c->comm, c->stream));
+        }
+        if (has_hi) {
+            LKB_NCCL(api->Send((const char*)x + (size_t)(nloc - he) * es, cnt, dt, c->rank + 1, c->comm, c->stream));
+            LKB_NCCL(api->Recv(A->halo_hi, cnt, dt, c->rank + 1, c->comm, c->stream));
+        }
+        LKB_NCCL(api->GroupEnd());
+        pdl_rearm();
+    }
+    return 0;
+}
 const HaloP2P* op_halo_desc(const lkb_op_s* A, int j) {
     const lkb_ctx_s* c = A->ctx;
     return (A->type == OP_STENCIL && c->world > 1 && A->hp_active && c->fused_halo && fin_usable(c, j)) ? &A->hp : nullptr;
 }
 int op_apply_enqueue(lkb_op_s* A, const void* x, void* y, bool trans, const int* flags, bool halo_prepushed) {
+    if (A->type == OP_CHEB) return cheb_apply_enqueue(A, x, y, trans, flags);     // brackets each of its launches itself
     lkb_ctx_s* c = A->ctx;
     const size_t es = kind_size(A->kind);
     int nl = 1;
     prof_begin(c, PC_MATVEC);
     if (A->type == OP_STENCIL) {
-        if (c->world > 1 && A->hp_active) {
-            // halo exchange over NVLink peer memory: pushed by the kernel that finished x, or by k_halo_push
-            // (copy + synchronisation in one kernel)
-            if (!halo_prepushed) { launch_halo_push(A->kind, c->stream, A->hp, x, A->m, flags); nl = 2; }
-        } else if (c->world > 1) {
-            // halo exchange over NCCL send/recv: my first row/plane -> rank-1's halo_hi, my last -> rank+1's halo_lo
-            NcclApi* api = nccl_api();
-            if (!api) return LKB_ERR_NCCL;
-            const int64_t he = A->halo_elems;
-            const int64_t nloc = A->m;
-            const size_t cnt = (size_t)he * (kind_cplx(A->kind) ? 2 : 1);
-            const int dt = (A->kind == KS || A->kind == KC) ? 7 : 8;   // ncclFloat32 / ncclFloat64
-            const bool has_lo = A->st.halo_lo != nullptr, has_hi = A->st.halo_hi != nullptr;
-            LKB_NCCL(api->GroupStart());
-            if (has_lo) {
-                LKB_NCCL(api->Send(x, cnt, dt, c->rank - 1, c->comm, c->stream));
-                LKB_NCCL(api->Recv(A->halo_lo, cnt, dt, c->rank - 1, c->comm, c->stream));
-            }
-            if (has_hi) {
-                LKB_NCCL(api->Send((const char*)x + (size_t)(nloc - he) * es, cnt, dt, c->rank + 1, c->comm, c->stream));
-                LKB_NCCL(api->Recv(A->halo_hi, cnt, dt, c->rank + 1, c->comm, c->stream));
-            }
-            LKB_NCCL(api->GroupEnd());
-            pdl_rearm();
-        }
+        nl = 0;
+        LKB_TRY(stencil_halo_exchange(A, x, flags, halo_prepushed, &nl));
+        nl += 1;
         launch_stencil(A->kind, c->stream, A->st, x, y, trans, flags, c->sms);
     } else if (A->type == OP_CSR && A->dist) {
         const int dt = (A->kind == KS || A->kind == KC) ? 7 : 8;            // ncclFloat32 / ncclFloat64

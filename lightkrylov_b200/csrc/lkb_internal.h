@@ -37,7 +37,7 @@ NcclApi* nccl_api();   // nullptr (+ error set) when libnccl cannot be loaded
 
 enum ProfClass { PC_MATVEC = 0, PC_DOT = 1, PC_AXPY = 2, PC_OTHER = 3, PC_FUSED = 4, PC_COUNT = 8 };
 // lkb_op_s::type.  The values are printed by lkb_op_jacobi_create's error message.
-enum OpType { OP_DENSE = 0, OP_STENCIL = 1, OP_CSR = 3, OP_DIAG = 4, OP_CALLBACK = 9 };
+enum OpType { OP_DENSE = 0, OP_STENCIL = 1, OP_CSR = 3, OP_DIAG = 4, OP_CHEB = 5, OP_CALLBACK = 9 };
 
 // ---- owners: every raw CUDA resource and every solver work object has exactly one, and goes with it ------------------
 // Members and locals are released in reverse order of declaration.  (The host-shell test mocks replace lkb_basis_destroy,
@@ -154,6 +154,13 @@ struct lkb_op_s {
     lkb::CudaPtr<void> diag; int64_t diag_row0 = 0, diag_n_global = 0;
     // callback
     int (*fn)(void*, const void*, void*, int32_t, void*) = nullptr; void* user = nullptr; bool capturable = false;
+    // Chebyshev preconditioner (lkb_cheb.cu) of cheb_A with cheb_m steps.  D^-1 is `diag` above, or the scalar cheb_invd when
+    // cheb_A is a stencil; cheb_b[0] = 1 / theta, and step k = 1 .. m-1 uses cheb_a[k], cheb_b[k].  Work vectors with cheb_A's
+    // local layout: cheb_d (m >= 3), cheb_z (stencil, m >= 3), cheb_t (other operators, m >= 2).
+    lkb_op_s* cheb_A = nullptr; int cheb_m = 0; lkb::Scalar cheb_invd = {0, 0};
+    std::vector<double> cheb_a, cheb_b;
+    lkb::CudaPtr<void> cheb_d, cheb_z, cheb_t;
+    int cheb_users = 0;                           // Chebyshev operators built on this one: lkb_op_destroy refuses while > 0
     uint64_t uid = 0;
 };
 
@@ -202,6 +209,17 @@ inline double rtol_of(int kind) { return (kind == KS || kind == KC) ? 1e-3 : 3.1
 // halo_prepushed: x's boundary rows were already stored into the neighbours' halo buffers by the kernel that
 // finished x (k_multiaxpy_fin / k_scale_dev with a HaloP2P descriptor): skip the k_halo_push kernel.
 int op_apply_enqueue(lkb_op_s* A, const void* x, void* y, bool trans, const int* flags, bool halo_prepushed = false);
+// Exchange the boundary rows / planes of a stencil's input x with the neighbouring slabs (P2P k_halo_push or an NCCL
+// send / recv group; nothing at N = 1).  *nl += the kernels it launched.  The caller brackets it with prof_begin / prof_end.
+int stencil_halo_exchange(lkb_op_s* A, const void* x, const int* flags, bool halo_prepushed, int* nl);
+// y = M r (trans: M^H r) for a Chebyshev operator M (lkb_cheb.cu); op_apply_enqueue dispatches here
+int cheb_apply_enqueue(lkb_op_s* M, const void* r, void* y, bool trans, const int* flags);
+// Jacobi set-up, shared by lkb_op_jacobi_create and lkb_op_chebyshev_create (`what` prefixes the messages): where A keeps
+// its diagonal, for k_jacobi / k_gershgorin; LKB_ERR_ARG for an operator without one (callback, non-square, ...)
+int jacobi_source(const lkb_op_s* A, const char* what, JacobiSrc* src, int64_t* n_global);
+// d = diag(A)^-1 on the device and, with `bound`, this rank's Gershgorin bound of D^-1 A; one host sync.  *bad_row = the
+// first global row whose diagonal entry is zero or not finite, or ~0.
+int jacobi_build(lkb_ctx_s* c, int kind, const JacobiSrc& src, void* d, unsigned long long* bad_row, double* bound);
 // The final CGS2 pass of a step against V(:, 0:j) may be k_multiaxpy_fin, which normalises with the predicted norm: not for
 // j = 0, not with option "fin" = 0, and not when the reductions go through ncclAllReduce (the predicted norm must not be
 // summed over ranks).

@@ -237,6 +237,19 @@ struct JacobiSrc {
     const void* a = nullptr;          // dense (column-major rows x rows) or the diagonal operator's d
 };
 void launch_jacobi(int kind, cudaStream_t s, const JacobiSrc& src, void* d, unsigned long long* bad_row, int sms);
+// Gershgorin bound max_r sum_c |a_rc / a_rr| of D^-1 A for a CSR (plain / blocked) or dense source (kernels_ops.cu:
+// k_gershgorin): *bound_bits (initialised to 0) is raised to the bit pattern of the bound, a non-negative double.
+void launch_gershgorin(int kind, cudaStream_t s, const JacobiSrc& src, unsigned long long* bound_bits, int sms);
+// One step of the Chebyshev preconditioner (lkb_cheb.cu).  Generic (kernels_vec.cu: k_cheb_update), after t = A z:
+// d_out = alpha d_in + beta invd o (r - t), z += d_out; init reads t, d_in and z as zero.  invd: a vector, or nullptr for
+// the scalar invd_s; conj: use conj(invd).  d_out may be nullptr (last step).
+void launch_cheb_update(int kind, cudaStream_t s, const void* r, const void* invd, Scalar invd_s, const void* t, const void* d_in,
+                        void* d_out, void* z, int64_t n, double alpha, double beta, bool conj, bool init, const int* flags, int sms);
+// Fused into the stencil kernels (kernels_ops.cu: ChebStep): y = z_{k+1} from x = z_k (first: x = r, z_1 = b0 D^-1 r),
+// d updated in place unless last.  invd: D^-1 = 1 / c0 of A (trans: conj(D)^-1).
+struct ChebArgs { const void* r; void* d; Scalar invd; double alpha, beta, b0; bool first, last; };
+void launch_stencil_cheb(int kind, cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans, const int* flags,
+                         const ChebArgs& ca);
 void launch_stencil(int kind, cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans,
                     const int* flags, int sms);
 // CSR SpMV y = A x (vector-per-row); conj_vals: use conj(A) values (for the explicit-transpose rmatvec)
