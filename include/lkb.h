@@ -175,7 +175,38 @@ int lkb_op_jacobi_create(lkb_op_t A, lkb_op_t* M);
  * M keeps a pointer to A: lkb_op_destroy(A) returns LKB_ERR_ARG while M is alive.  M's work vectors are allocated here;
  * M's matvec counter counts applications of M, A's counters are not touched. */
 int lkb_op_chebyshev_create(lkb_op_t A, int32_t degree, double lmin, double lmax, lkb_op_t* M);
-/* LKB_ERR_ARG, and A stays, while a Chebyshev preconditioner built on A is alive */
+/* GMRES-polynomial preconditioner M = p(A) (Loe & Morgan, Numer. Linear Algebra Appl. 2022; Trilinos Belos GmresPoly).
+ * With nonzero roots theta_1 .. theta_d, pi(z) = prod_i (1 - z/theta_i) and p(z) = (1 - pi(z))/z (degree d - 1), so
+ * A M = I - pi(A).  M r by the product recurrence, in the order the roots are stored:
+ *     y = r ; z = 0
+ *     root theta (real kinds: real theta; complex kinds: any):  z += y/theta ;  y <- y - A (y/theta)
+ *     pair (theta, conj theta), real kinds only, a = Re theta, q = |theta|^2:
+ *                                   t = A y ;  w = (2a/q) y - t/q ;  z += w ;  y <- y - A w
+ *     return z                      (the last factor's y update is skipped)
+ * d - 1 applications of A and no inner products; d = 1 is r / theta_1.  lkb_op_rmatvec applies M^H = conj(p)(A^H): the
+ * same recurrence with conj(theta_i) and A's rmatvec.  M needs neither spectral bounds nor diag(A), so A may be any square
+ * operator, callbacks included; on a stencil every application of A is one fused stencil kernel.  M is not Hermitian
+ * positive definite in general: it is meant for gmres.  M keeps a pointer to A: lkb_op_destroy(A) returns LKB_ERR_ARG
+ * while M is alive.  M's work vectors (at most three) are allocated here; M's matvec counter counts applications of M,
+ * A's counters are not touched.  M may be captured into a CUDA graph when A may.
+ * roots: nroots (re, im) pairs, applied in the given order.  LKB_ERR_ARG for nroots outside 1 .. 256, a zero or non-finite
+ * root, in a real kind a root with im != 0 not immediately followed by its exact conjugate (the message names its index),
+ * and a non-square A. */
+int lkb_op_poly_create(lkb_op_t A, int32_t nroots, const double* roots, lkb_op_t* M);
+/* The GMRES polynomial of A of the given degree (1 .. 128), collective: `degree` Arnoldi steps (lkb_arnoldi, p = 1,
+ * default tol; A's matvec counter grows by the steps taken) from the normalised lkb_vec_fill_random(normal, seed) vector,
+ * which is the same at any sharding and leaves the context's rand stream alone.  The roots are the harmonic Ritz values,
+ * the eigenvalues of H_k + |h_{k+1,k}|^2 f e_k^T with f = H_k^-H e_k (k = degree, or the step of a breakdown), computed in
+ * double; a root at which pof = prod_{j != i} |1 - theta_i/theta_j| exceeds 1e4 gets ceil((log10 pof - 4)/14) extra copies
+ * (in a real kind its conjugate as many); they are applied in modified Leja order (the largest modulus first, then the
+ * root maximising sum_j log|theta - theta_j| over those already placed, ties to the lowest index; in a real kind a pair
+ * is placed im > 0 first, its conjugate right after).  Rank 0's roots are used on every rank.  LKB_ERR_ARG for a degree
+ * out of range, a singular H_k or a zero / non-finite root; LKB_ERR_LAPACK without a host LAPACK (see lkb_set_lapack). */
+int lkb_op_gmres_poly_create(lkb_op_t A, int32_t degree, uint64_t seed, lkb_op_t* M);
+/* The roots of a polynomial operator in application order: *nroots of them as (re, im) pairs.  LKB_ERR_ARG when M is
+ * not a polynomial operator or cap < *nroots (*nroots is still set).  Feed them to lkb_op_poly_create to rebuild M. */
+int lkb_op_poly_roots(lkb_op_t M, int32_t cap, int32_t* nroots, double* roots);
+/* LKB_ERR_ARG, and A stays, while a Chebyshev or GMRES-polynomial preconditioner built on A is alive */
 int lkb_op_destroy(lkb_op_t A);
 int lkb_op_matvec(lkb_op_t A, lkb_vec_t x, lkb_vec_t y);    /* apply_matvec  :391-407 (bumps counter) */
 int lkb_op_rmatvec(lkb_op_t A, lkb_vec_t x, lkb_vec_t y);   /* apply_rmatvec :409-424 */

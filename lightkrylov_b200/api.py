@@ -458,6 +458,39 @@ class LinOp:
         op.n_global = getattr(A, "m_global", A.n_global)
         return op
 
+    @classmethod
+    def polynomial(cls, A: "LinOp", roots) -> "LinOp":
+        """Polynomial preconditioner M = p(A), p(z) = (1 - prod_i (1 - z / roots[i])) / z, applied in the order of `roots`
+        (a complex array; in a real kind a complex root is immediately followed by its conjugate) (include/lkb.h:
+        lkb_op_poly_create).  Keeps A alive."""
+        th = np.ascontiguousarray(np.asarray(roots, dtype=np.complex128).ravel())
+        ri = np.ascontiguousarray(np.column_stack([th.real, th.imag]).ravel())
+        h = C.c_void_p()
+        check(A.ctx.lib.lkb_op_poly_create(A.h, int(th.size), ri.ctypes.data_as(C.POINTER(C.c_double)), C.byref(h)), "polynomial")
+        return cls._on(A, h)
+
+    @classmethod
+    def gmres_poly(cls, A: "LinOp", degree: int, seed: int = 0) -> "LinOp":
+        """GMRES-polynomial preconditioner of `degree` (include/lkb.h: lkb_op_gmres_poly_create): the roots are the
+        harmonic Ritz values of `degree` Arnoldi steps on A from a seeded random vector.  Collective; keeps A alive."""
+        h = C.c_void_p()
+        check(A.ctx.lib.lkb_op_gmres_poly_create(A.h, int(degree), int(seed), C.byref(h)), "gmres_poly")
+        return cls._on(A, h)
+
+    @classmethod
+    def _on(cls, A: "LinOp", h) -> "LinOp":
+        op = cls(A.ctx, A.kind, h, A.m, A.m, keep=A)
+        op.row0 = getattr(A, "out_row0", A.row0)
+        op.n_global = getattr(A, "m_global", A.n_global)
+        return op
+
+    def poly_roots(self) -> np.ndarray:
+        """The roots of a polynomial operator in application order (complex128)."""
+        n = C.c_int32()
+        buf = np.zeros(2 * 256, dtype=np.float64)
+        check(self.ctx.lib.lkb_op_poly_roots(self.h, 256, C.byref(n), buf.ctypes.data_as(C.POINTER(C.c_double))), "poly_roots")
+        return buf[0:2 * n.value:2] + 1j * buf[1:2 * n.value:2]
+
     def matvec(self, x: Vector, y: Vector):
         check(self.ctx.lib.lkb_op_matvec(self.h, x.h, y.h), "matvec")
 

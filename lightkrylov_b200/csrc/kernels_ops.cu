@@ -91,6 +91,30 @@ LKB_DI void cheb_store(const ChebStep<E>& c, E* y, int64_t q, const Pack<E, PW>&
     if (!c.last) PO::st(c.d + q, dv);
     PO::st(y + q, zn);
 }
+// PolyStep: one step of the GMRES-polynomial preconditioner (lkb_poly.cu) on t = (A x)_i and x_i:
+//     y_i = a . (x, t, v)_i  (y may be nullptr: no output) ;  acc_i = [acc_i] + b . (x, t, v)_i  (acc may be nullptr)
+// v (nullptr: zero) is the held y of a root pair's second half.  HBM traffic: x read, then at most one of (y written,
+// v read) plus acc read and written: at most 4 n s per step.
+template <typename E> struct PolyStep {
+    const E* v; E* acc;
+    PolyCoef<E> c;
+    int acc_read;                               // 0: acc is written, 1: accumulated
+};
+template <typename E, int PW>
+LKB_DI void poly_store(const PolyStep<E>& c, E* y, int64_t q, const Pack<E, PW>& t, const Pack<E, PW>& x) {
+    using PO = PackOps<E, PW>;
+    using P = Pack<E, PW>;
+    P vv = PO::zero(), a = PO::zero(), o;
+    if (c.v) vv = PO::ld_nc(c.v + q);
+    if (c.acc_read) a = PO::ld_nc(c.acc + q);
+#pragma unroll
+    for (int e = 0; e < PW; ++e) {
+        o.v[e] = poly_comb(x.v[e], t.v[e], vv.v[e], c.c.a[0], c.c.a[1], c.c.a[2]);
+        a.v[e] = add_v(a.v[e], poly_comb(x.v[e], t.v[e], vv.v[e], c.c.b[0], c.c.b[1], c.c.b[2]));
+    }
+    if (y) PO::st(y + q, o);
+    if (c.acc) PO::st(c.acc + q, a);
+}
 
 // Both stencil kernels take one CTA per (column block, row block[, plane]) of a 1-D grid, column block fastest
 // (consecutive CTAs stream consecutive segments of the same grid rows).  The row blocks (2-D) / planes (3-D) are rotated
@@ -187,6 +211,8 @@ k_stencil(const typename Tr<K>::E* __restrict__ x, typename Tr<K>::E* __restrict
         }
         if constexpr (std::is_same_v<EPI, StorePlain>) {
             if (active) PO::st_w(y + k * plane + p, out, keep, pol);
+        } else if constexpr (std::is_same_v<EPI, PolyStep<E>>) {
+            if (active) poly_store<E, PW>(epi, y, k * plane + p, out, center);
         } else {
             if (active) cheb_store<E, PW, typename Tr<K>::Rl>(epi, y, k * plane + p, out, center);
         }
@@ -290,6 +316,7 @@ k_stencil_smem(const typename Tr<K>::E* __restrict__ x, typename Tr<K>::E* __res
             out.v[e] = sacc;
         }
         if constexpr (std::is_same_v<EPI, StorePlain>) PackOps<E, PW>::st_w(y + p, out, keep, pol);
+        else if constexpr (std::is_same_v<EPI, PolyStep<E>>) poly_store<E, PW>(epi, y, p, out, center);
         else cheb_store<E, PW, typename Tr<K>::Rl>(epi, y, p, out, center);
     }
 }
@@ -367,6 +394,26 @@ void launch_stencil_cheb(int kind, cudaStream_t s, const StencilArgs& a, const v
         case KD: stencil_cheb_t<KD>(s, a, x, y, trans, flags, ca); break;
         case KC: stencil_cheb_t<KC>(s, a, x, y, trans, flags, ca); break;
         default: stencil_cheb_t<KZ>(s, a, x, y, trans, flags, ca); break;
+    }
+}
+// One fused polynomial step (PolyStep above): y = out (nullptr: none), acc updated, from the stencil input x
+template <int K>
+static void stencil_poly_t(cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans, const int* flags,
+                           const PolyArgs& pa) {
+    using E = typename Tr<K>::E;
+    PolyStep<E> epi;
+    epi.v = (const E*)pa.v; epi.acc = (E*)pa.acc;
+    for (int i = 0; i < 3; ++i) { from_scalar(pa.a[i], epi.c.a[i]); from_scalar(pa.b[i], epi.c.b[i]); }
+    epi.acc_read = pa.acc_read ? 1 : 0;
+    stencil_t<K>(s, a, x, y, trans, flags, epi);
+}
+void launch_stencil_poly(int kind, cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans, const int* flags,
+                         const PolyArgs& pa) {
+    switch (kind) {
+        case KS: stencil_poly_t<KS>(s, a, x, y, trans, flags, pa); break;
+        case KD: stencil_poly_t<KD>(s, a, x, y, trans, flags, pa); break;
+        case KC: stencil_poly_t<KC>(s, a, x, y, trans, flags, pa); break;
+        default: stencil_poly_t<KZ>(s, a, x, y, trans, flags, pa); break;
     }
 }
 

@@ -480,6 +480,51 @@ k_cheb_update(const typename Tr<K>::E* __restrict__ r, const typename Tr<K>::E* 
         }
 }
 
+// One step of the GMRES-polynomial preconditioner on an operator without a fused step (lkb_poly.cu), after t = A x
+// (poly_comb, lkb_types.cuh):  out = a . (x, t, v) ;  acc = [acc] + b . (x, t, v).  t and v may be nullptr (read as zero:
+// t for the degree-1 polynomial, v outside a root pair's second half), out and acc may be nullptr (absent).  out may be t
+// or v (the step's result replaces its own operand): every pack is read by the thread that then writes it, as in k_diag.
+template <int K>
+__global__ void __launch_bounds__(256)
+k_poly_update(const typename Tr<K>::E* __restrict__ x, const typename Tr<K>::E* t, const typename Tr<K>::E* v,
+              typename Tr<K>::E* out, typename Tr<K>::E* __restrict__ acc, int64_t n, const PolyCoef<typename Tr<K>::E> c,
+              int acc_read, const int* __restrict__ flags)
+{
+    using E = typename Tr<K>::E;
+    constexpr int EPP = Tr<K>::EPP;
+    using P = Pack<E, EPP>;
+    if (flags && flags[F_STOP]) return;
+    const int64_t npk = n / EPP;
+    for (int64_t pk = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; pk < npk; pk += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t o = pk * EPP;
+        const P xv = ld_pack_nc<P>(x + o);
+        P tv, vv, av;
+#pragma unroll
+        for (int e = 0; e < EPP; ++e) tv.v[e] = vv.v[e] = av.v[e] = zero_v(E());
+        if (t) tv = ld_pack_nc<P>(t + o);
+        if (v) vv = ld_pack_nc<P>(v + o);
+        if (acc && acc_read) av = ld_pack_nc<P>(acc + o);
+        if (out) {
+            P ov;
+#pragma unroll
+            for (int e = 0; e < EPP; ++e) ov.v[e] = poly_comb(xv.v[e], tv.v[e], vv.v[e], c.a[0], c.a[1], c.a[2]);
+            st_pack(out + o, ov);
+        }
+        if (acc) {
+#pragma unroll
+            for (int e = 0; e < EPP; ++e) av.v[e] = add_v(av.v[e], poly_comb(xv.v[e], tv.v[e], vv.v[e], c.b[0], c.b[1], c.b[2]));
+            st_pack(acc + o, av);
+        }
+    }
+    if (blockIdx.x == 0 && threadIdx.x == 0)
+        for (int64_t i = npk * EPP; i < n; ++i) {
+            const E tv = t ? t[i] : zero_v(E()), vv = v ? v[i] : zero_v(E());
+            const E av = (acc && acc_read) ? acc[i] : zero_v(E());
+            if (out) out[i] = poly_comb(x[i], tv, vv, c.a[0], c.a[1], c.a[2]);
+            if (acc) acc[i] = add_v(av, poly_comb(x[i], tv, vv, c.b[0], c.b[1], c.b[2]));
+        }
+}
+
 // ------------------------------------------------------------------------------------------
 // GMRES column update on the device (gmres.fypp:167-194 + submodule_utility_functions.fypp:169-204): after the
 // CGS2 kernels of inner step k this single CTA forms H(:k,k) = c1 + c2 and H(k+1,k) = ||w||, decides the
@@ -651,6 +696,16 @@ void launch_cheb_update(int kind, cudaStream_t s, const void* r, const void* inv
         E is; from_scalar(invd_s, is);
         k_cheb_update<K><<<ew_grid(n / Tr<K>::EPP, sms), 256, 0, s>>>((const E*)r, (const E*)invd, is, (const E*)t, (const E*)d_in,
                                                                        (E*)d_out, (E*)z, n, (Rl)alpha, (Rl)beta, conj, init, flags);
+    });
+}
+void launch_poly_update(int kind, cudaStream_t s, const void* x, const void* t, void* out, int64_t n, const PolyArgs& pa,
+                        const int* flags, int sms) {
+    LKB_DISPATCH(kind, {
+        using E = typename Tr<K>::E;
+        PolyCoef<E> c;
+        for (int i = 0; i < 3; ++i) { from_scalar(pa.a[i], c.a[i]); from_scalar(pa.b[i], c.b[i]); }
+        k_poly_update<K><<<ew_grid(n / Tr<K>::EPP, sms), 256, 0, s>>>((const E*)x, (const E*)t, (const E*)pa.v, (E*)out,
+                                                                       (E*)pa.acc, n, c, pa.acc_read ? 1 : 0, flags);
     });
 }
 void launch_gmres_update(int kind, cudaStream_t s, const void* c1, const void* c2, int k, const void* nrm2, void* H, int ldh,

@@ -21,7 +21,7 @@ namespace lkb {
 static void* stencil_z(lkb_op_s* M, void* y, int j) { return ((M->cheb_m - j) % 2 == 0) ? y : M->cheb_z.get(); }
 
 int cheb_apply_enqueue(lkb_op_s* M, const void* r, void* y, bool trans, const int* flags) {
-    lkb_op_s* A = M->cheb_A;
+    lkb_op_s* A = M->base;
     lkb_ctx_s* c = M->ctx;
     const int m = M->cheb_m;
     const Scalar invd = M->cheb_invd;       // k_cheb_update conjugates it for trans; the fused step takes conj(D)^-1 itself
@@ -127,8 +127,8 @@ int lkb_op_chebyshev_create(lkb_op_t A, int32_t degree, double lmin, double lmax
     if (degree >= 3) LKB_TRY(cuda_alloc(op->cheb_d, bytes));
     if (degree >= 3 && A->type == OP_STENCIL) LKB_TRY(cuda_alloc(op->cheb_z, bytes));
     if (degree >= 2 && A->type != OP_STENCIL) LKB_TRY(cuda_alloc(op->cheb_t, bytes));
-    op->cheb_A = A;
-    A->cheb_users++;
+    op->base = A;
+    A->users++;
     *M = op.release();
     return 0;
 }

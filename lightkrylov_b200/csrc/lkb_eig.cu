@@ -294,6 +294,13 @@ int start_vector(lkb_basis_s* Xw, lkb_vec_t x0) {
 }
 
 }  // namespace
+namespace lkb {
+int host_eig_double(bool cplx, int k, const std::vector<cd>& A, int lda, std::vector<cd>& vals) {
+    LKB_TRY(lapack_ready());
+    std::vector<cd> vecs;
+    return host_eig_t<double>(cplx, k, A, lda, vals, vecs);
+}
+}  // namespace lkb
 
 extern "C" {
 

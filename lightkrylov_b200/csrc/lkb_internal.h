@@ -37,7 +37,7 @@ NcclApi* nccl_api();   // nullptr (+ error set) when libnccl cannot be loaded
 
 enum ProfClass { PC_MATVEC = 0, PC_DOT = 1, PC_AXPY = 2, PC_OTHER = 3, PC_FUSED = 4, PC_COUNT = 8 };
 // lkb_op_s::type.  The values are printed by lkb_op_jacobi_create's error message.
-enum OpType { OP_DENSE = 0, OP_STENCIL = 1, OP_CSR = 3, OP_DIAG = 4, OP_CHEB = 5, OP_CALLBACK = 9 };
+enum OpType { OP_DENSE = 0, OP_STENCIL = 1, OP_CSR = 3, OP_DIAG = 4, OP_CHEB = 5, OP_POLY = 6, OP_CALLBACK = 9 };
 
 // ---- owners: every raw CUDA resource and every solver work object has exactly one, and goes with it ------------------
 // Members and locals are released in reverse order of declaration.  (The host-shell test mocks replace lkb_basis_destroy,
@@ -73,6 +73,13 @@ typedef Owner<lkb_op_t, lkb_op_destroy> OpOwner;           // an operator until 
 struct GraphExec { Owner<cudaGraphExec_t, cudaGraphExecDestroy> exec; int64_t launches = 0; };
 // the arrays an L2-blocked CsrBlocked views
 struct CsrBlockedMem { CudaPtr<uint32_t> tab; CudaPtr<int32_t> col; CudaPtr<void> val; };
+// One launch (stencil) or matvec + k_poly_update (other operators) of a GMRES-polynomial application (lkb_poly.cu).
+// Buffers: POLY_R = the input r, POLY_NONE = absent, 0..2 = the work vectors poly_w.  x: the matvec input; dst: where the
+// step's out goes (generic path: also the matvec's output, overwritten in place by out); v: the held operand; acc: 0 none,
+// 1 write the output, 2 accumulate into it.  matvec false: no application of A (the degree-1 polynomial).  a, b: the
+// coefficients of (x, t, v) of out and acc (lkb_kernels.h: PolyArgs), conjugated for the rmatvec.
+enum { POLY_NONE = -1, POLY_R = -2 };
+struct PolyStepPlan { int x, dst, v, acc; bool matvec, out; Scalar a[3], b[3]; };
 }  // namespace lkb
 
 struct lkb_ctx_s {
@@ -154,13 +161,20 @@ struct lkb_op_s {
     lkb::CudaPtr<void> diag; int64_t diag_row0 = 0, diag_n_global = 0;
     // callback
     int (*fn)(void*, const void*, void*, int32_t, void*) = nullptr; void* user = nullptr; bool capturable = false;
-    // Chebyshev preconditioner (lkb_cheb.cu) of cheb_A with cheb_m steps.  D^-1 is `diag` above, or the scalar cheb_invd when
-    // cheb_A is a stencil; cheb_b[0] = 1 / theta, and step k = 1 .. m-1 uses cheb_a[k], cheb_b[k].  Work vectors with cheb_A's
+    // polynomial preconditioners (Chebyshev, GMRES polynomial) keep a pointer to the operator they are built on; `users`
+    // counts those built on this one: lkb_op_destroy refuses while > 0
+    lkb_op_s* base = nullptr; int users = 0;
+    // Chebyshev preconditioner (lkb_cheb.cu) of `base` with cheb_m steps.  D^-1 is `diag` above, or the scalar cheb_invd when
+    // base is a stencil; cheb_b[0] = 1 / theta, and step k = 1 .. m-1 uses cheb_a[k], cheb_b[k].  Work vectors with base's
     // local layout: cheb_d (m >= 3), cheb_z (stencil, m >= 3), cheb_t (other operators, m >= 2).
-    lkb_op_s* cheb_A = nullptr; int cheb_m = 0; lkb::Scalar cheb_invd = {0, 0};
+    int cheb_m = 0; lkb::Scalar cheb_invd = {0, 0};
     std::vector<double> cheb_a, cheb_b;
     lkb::CudaPtr<void> cheb_d, cheb_z, cheb_t;
-    int cheb_users = 0;                           // Chebyshev operators built on this one: lkb_op_destroy refuses while > 0
+    // GMRES-polynomial preconditioner (lkb_poly.cu) p(base): its roots in application order, the steps of one application
+    // and up to three work vectors with base's local layout
+    std::vector<lkb::Scalar> poly_roots;
+    std::vector<lkb::PolyStepPlan> poly_plan;
+    lkb::CudaPtr<void> poly_w[3];
     uint64_t uid = 0;
 };
 
@@ -214,6 +228,8 @@ int op_apply_enqueue(lkb_op_s* A, const void* x, void* y, bool trans, const int*
 int stencil_halo_exchange(lkb_op_s* A, const void* x, const int* flags, bool halo_prepushed, int* nl);
 // y = M r (trans: M^H r) for a Chebyshev operator M (lkb_cheb.cu); op_apply_enqueue dispatches here
 int cheb_apply_enqueue(lkb_op_s* M, const void* r, void* y, bool trans, const int* flags);
+// y = M r (trans: M^H r) for a GMRES-polynomial operator M (lkb_poly.cu); op_apply_enqueue dispatches here
+int poly_apply_enqueue(lkb_op_s* M, const void* r, void* y, bool trans, const int* flags);
 // Jacobi set-up, shared by lkb_op_jacobi_create and lkb_op_chebyshev_create (`what` prefixes the messages): where A keeps
 // its diagonal, for k_jacobi / k_gershgorin; LKB_ERR_ARG for an operator without one (callback, non-square, ...)
 int jacobi_source(const lkb_op_s* A, const char* what, JacobiSrc* src, int64_t* n_global);
@@ -261,7 +277,11 @@ int lanczos_collect(lkb_op_s* A, lkb_basis_s* X, void* T, int ldt, int32_t* info
 int bidiag_enqueue(lkb_op_s* A, lkb_basis_s* U, lkb_basis_s* V, int kstart, int kend, double tol);
 int bidiag_collect(lkb_op_s* A, lkb_basis_s* U, void* B, int ldb, int32_t* info, int kstart, int kend, const void* pinned_host);
 // a callback operator may be captured into a CUDA graph only when its creator declared it capturable
-inline bool op_capturable(const lkb_op_s* A) { return A->type != OP_CALLBACK || A->capturable; }
+// (a GMRES-polynomial preconditioner applies its base operator, so it is capturable when that one is)
+inline bool op_capturable(const lkb_op_s* A) {
+    if (A->type == OP_POLY) return op_capturable(A->base);
+    return A->type != OP_CALLBACK || A->capturable;
+}
 
 // One element of a host array of `kind` as a complex double, and back (the single precisions round on the way in)
 typedef std::complex<double> cd;
@@ -282,6 +302,13 @@ inline void store_kind(int kind, void* base, size_t idx, cd v) {
     }
 }
 inline Scalar to_scalar(cd v) { return Scalar{v.real(), v.imag()}; }
+// The roots of the GMRES polynomial of degree k from the Arnoldi relation of A (lkb_poly.cu; host only, in double):
+// H is column-major (k+1) x k with leading dimension ldh.  Harmonic Ritz values of H_k, extra copies of the roots whose
+// product of the other factors exceeds 1e4 at them, modified Leja order (real kinds: conjugate pairs adjacent, im > 0
+// first).  LKB_ERR_ARG for a singular H_k or a zero / non-finite root, LKB_ERR_LAPACK without a LAPACK provider.
+int gmres_poly_roots(int kind, const cd* H, int ldh, int k, std::vector<cd>& roots);
+// eigenvalues of the k x k complex-double matrix A (real when !cplx) by the double-precision geev (lkb_eig.cu)
+int host_eig_double(bool cplx, int k, const std::vector<cd>& A, int lda, std::vector<cd>& vals);
 
 // a dev_alloc buffer
 struct DevBuf {

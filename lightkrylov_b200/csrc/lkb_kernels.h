@@ -250,6 +250,18 @@ void launch_cheb_update(int kind, cudaStream_t s, const void* r, const void* inv
 struct ChebArgs { const void* r; void* d; Scalar invd; double alpha, beta, b0; bool first, last; };
 void launch_stencil_cheb(int kind, cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans, const int* flags,
                          const ChebArgs& ca);
+// One step of the GMRES-polynomial preconditioner (lkb_poly.cu): out = a . (x, t, v), acc = [acc] + b . (x, t, v) with
+// t = A x (poly_comb, lkb_types.cuh).  v / acc nullptr: absent (v read as zero); acc_read: accumulate into acc, else
+// overwrite it.
+struct PolyArgs { const void* v; void* acc; Scalar a[3], b[3]; bool acc_read; };
+// Generic (kernels_vec.cu: k_poly_update), after t = A x into a work vector: t may be nullptr (zero), out may be nullptr
+// (absent) and may be t or v.
+void launch_poly_update(int kind, cudaStream_t s, const void* x, const void* t, void* out, int64_t n, const PolyArgs& pa,
+                        const int* flags, int sms);
+// Fused into the stencil kernels (kernels_ops.cu: PolyStep): t = A x computed in the kernel, y = out (nullptr: none).
+// Neither y, v nor acc may be x.
+void launch_stencil_poly(int kind, cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans, const int* flags,
+                         const PolyArgs& pa);
 void launch_stencil(int kind, cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans,
                     const int* flags, int sms);
 // CSR SpMV y = A x (vector-per-row); conj_vals: use conj(A) values (for the explicit-transpose rmatvec)

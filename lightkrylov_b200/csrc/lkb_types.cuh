@@ -100,6 +100,17 @@ LKB_HDI bool is_zero_v(double a)  { return a == 0.0; }
 LKB_HDI bool is_zero_v(float2 a)  { return a.x == 0.f && a.y == 0.f; }
 LKB_HDI bool is_zero_v(double2 a) { return a.x == 0.0 && a.y == 0.0; }
 
+// One step of the GMRES-polynomial preconditioner (lkb_poly.cu) on the matvec input x, its image t = (A x)_i and a held
+// vector v:  out = a0 x + a1 t + a2 v ;  acc = [acc] + b0 x + b1 t + b2 v.  Shared by the fused stencil epilogue
+// (kernels_ops.cu) and k_poly_update (kernels_vec.cu), so both paths round alike.
+template <typename E> struct PolyCoef { E a[3], b[3]; };
+template <typename E> LKB_DI E poly_comb(E x, E t, E v, E c0, E c1, E c2) {
+    E s = mul_v(c0, x);
+    fmacc(s, t, c1);
+    fmacc(s, v, c2);
+    return s;
+}
+
 // widen element -> reduction type W, and narrow back
 LKB_HDI double  widen(float a)   { return (double)a; }
 LKB_HDI double  widen(double a)  { return a; }
