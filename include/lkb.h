@@ -206,7 +206,34 @@ int lkb_op_gmres_poly_create(lkb_op_t A, int32_t degree, uint64_t seed, lkb_op_t
 /* The roots of a polynomial operator in application order: *nroots of them as (re, im) pairs.  LKB_ERR_ARG when M is
  * not a polynomial operator or cap < *nroots (*nroots is still set).  Feed them to lkb_op_poly_create to rebuild M. */
 int lkb_op_poly_roots(lkb_op_t M, int32_t cap, int32_t* nroots, double* roots);
-/* LKB_ERR_ARG, and A stays, while a Chebyshev or GMRES-polynomial preconditioner built on A is alive */
+/* Geometric multigrid preconditioner M of a 5- or 7-point stencil A: M r is one V-cycle from a zero initial guess on a
+ * hierarchy built from A (Trottenberg, Oosterlee & Schueller, Multigrid, 2001).
+ *   Level 0 is A: grid (nx, ny[, nz]), coefficients (c0, c-x, c+x, c-y, c+y[, c-z, c+z]).  Write A = rho I + sum_d T_d with
+ *   T_d = tri(c-d, -(c-d + c+d), c+d) acting along axis d and rho = c0 + sum_d (c-d + c+d).
+ *   Coarsening: every axis at once, n -> n_c = floor(n/2), coarse point i at fine point 2i+1.  P_d is 1-D linear
+ *   interpolation (fine 2i+1 takes coarse i, fine 2i and 2i+2 half of it, coarse points outside the grid are zero), P the
+ *   tensor product of the P_d, and R = 2^-dim P^T, boundaries included.
+ *   Coarse operators: T_d' = 1/2 P_d^T T_d P_d along each axis, rho unchanged.  T_d' has constant off-diagonals and a
+ *   constant diagonal except its last entry, so every level is a 5- / 7-point stencil whose centre at (i, j, k) is
+ *   c0 + sum_d [i_d = n_d - 1] e_d.  The hierarchy is built on the host in double (complex for the complex kinds).
+ *   Coarsening stops at the first level with <= 512 unknowns or an axis below 2 points; that level's operator is
+ *   inverted densely on the host in double with partial pivoting, stored in the kind, and applied as a dense matvec.
+ *   Smoother on level l: Chebyshev of degree m (`degree`) in D_l^-1 A_l with lkb_op_chebyshev_create's recurrence on
+ *   [b_l / (2 dim), b_l], b_l the Gershgorin bound of D_l^-1 A_l.  Pre-smoothing starts from 0; post-smoothing starts from
+ *   the corrected x with d_0 = D^-1 (b - A x) / theta, z_1 = x + d_0, and continues as before.
+ *   V-cycle:  V(l, b) = A_L^-1 b if l = L, else  x = S(b, 0) ;  x += P V(l+1, R (b - A_l x)) ;  x = S(b, x).
+ * lkb_op_rmatvec applies M^H: the same cycle on A_l^H with conj(D) and (A_L^-1)^H.  M is Hermitian for Hermitian A, and
+ * positive definite as well when b_l >= lambda_max on every level (always, with the Gershgorin bound), so CG may use it.
+ * On each level but the coarsest one application costs: pre-smoothing m launches (m - 1 when m >= 2 and the level has no
+ * edge correction), one restriction (k_mg_restrict), one prolongation (k_mg_prolong) and m post-smoothing launches; plus
+ * one launch for the coarsest solve.  Every smoothing step is one fused stencil kernel.  All buffers are allocated here;
+ * M may be captured into a CUDA graph.  M keeps a pointer to A: lkb_op_destroy(A) returns LKB_ERR_ARG while M is alive.
+ * M's matvec counter counts applications of M, A's counters are not touched.
+ * LKB_ERR_ARG for an A that is not a stencil (use the Chebyshev or GMRES-polynomial preconditioner), a row-sharded stencil
+ * whose slab is not the whole grid, degree < 1, a zero or non-finite centre on any level (the message names the level), a
+ * coarsest level above 512 unknowns (the message names the grid) and a singular coarsest matrix. */
+int lkb_op_multigrid_create(lkb_op_t A, int32_t degree, lkb_op_t* M);
+/* LKB_ERR_ARG, and A stays, while a Chebyshev, GMRES-polynomial or multigrid preconditioner built on A is alive */
 int lkb_op_destroy(lkb_op_t A);
 int lkb_op_matvec(lkb_op_t A, lkb_vec_t x, lkb_vec_t y);    /* apply_matvec  :391-407 (bumps counter) */
 int lkb_op_rmatvec(lkb_op_t A, lkb_vec_t x, lkb_vec_t y);   /* apply_rmatvec :409-424 */

@@ -100,6 +100,7 @@ SIGNATURES = {
     "lkb_op_chebyshev_create": (_i, [_vp, _i32, _d, _d, _P(_vp)]),
     "lkb_op_poly_create": (_i, [_vp, _i32, _P(_d), _P(_vp)]),
     "lkb_op_gmres_poly_create": (_i, [_vp, _i32, _u64, _P(_vp)]),
+    "lkb_op_multigrid_create": (_i, [_vp, _i32, _P(_vp)]),
     "lkb_op_poly_roots": (_i, [_vp, _i32, _P(_i32), _P(_d)]),
     "lkb_op_destroy": (_i, [_vp]),
     "lkb_op_matvec": (_i, [_vp, _vp, _vp]),

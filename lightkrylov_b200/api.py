@@ -478,6 +478,14 @@ class LinOp:
         return cls._on(A, h)
 
     @classmethod
+    def multigrid(cls, A: "LinOp", degree: int = 2) -> "LinOp":
+        """Geometric multigrid preconditioner of a 5- / 7-point stencil (include/lkb.h: lkb_op_multigrid_create): one
+        V-cycle with Chebyshev smoothing of `degree` on every level.  Keeps A alive."""
+        h = C.c_void_p()
+        check(A.ctx.lib.lkb_op_multigrid_create(A.h, int(degree), C.byref(h)), "multigrid")
+        return cls._on(A, h)
+
+    @classmethod
     def _on(cls, A: "LinOp", h) -> "LinOp":
         op = cls(A.ctx, A.kind, h, A.m, A.m, keep=A)
         op.row0 = getattr(A, "out_row0", A.row0)

@@ -14,7 +14,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(CSRC, "liblkb.so")
-SOURCES = ["kernels_gs.cu", "kernels_vec.cu", "kernels_ops.cu", "kernels_gemm.cu", "kernels_fused.cu", "lkb_core.cu", "lkb_cheb.cu", "lkb_poly.cu", "lkb_csr.cu", "lkb_krylov.cu",
+SOURCES = ["kernels_gs.cu", "kernels_vec.cu", "kernels_ops.cu", "kernels_gemm.cu", "kernels_fused.cu", "lkb_core.cu", "lkb_cheb.cu", "lkb_poly.cu", "lkb_mg.cu", "lkb_csr.cu", "lkb_krylov.cu",
            "lkb_solvers.cu", "lkb_eig.cu", "lkb_expm.cu"]
 # every header in csrc/ (globbed: a forgotten header once left objects stale) + the public C ABI
 HEADERS = sorted(f for f in os.listdir(CSRC) if f.endswith((".h", ".cuh", ".inc"))) + [os.path.join("..", "..", "include", "lkb.h")]

@@ -115,6 +115,57 @@ LKB_DI void poly_store(const PolyStep<E>& c, E* y, int64_t q, const Pack<E, PW>&
     if (y) PO::st(y + q, o);
     if (c.acc) PO::st(c.acc + q, a);
 }
+// MgStep: one Chebyshev smoothing step on a level of the multigrid preconditioner (lkb_mg.cu), on t = (A x)_i and x_i.  A
+// coarse level's centre is c0 + ecor[mask] on the points that sit on the last index of the axes in mask (bit 0 x, 1 y, 2 z):
+// t gains ecor[mask] x_i there, and D^-1 there is invd[mask] (ecor[0] = 0, invd[0] = 1 / c0).  Modes:
+//   MG_SCALE    y = b0 D^-1 x: z_1 of a smoothing from zero (t is not used)
+//   MG_FIRST_R  ChebStep's first step on x = r, valid only where D is constant (a level without edge corrections)
+//   MG_STEP     s = D^-1 (r - t) ; d = alpha d_in + beta s ; y = x + d.  With d_in nullptr, d = beta s and d_in is not
+//               read (the first post-smoothing step, from a nonzero guess: stale memory must not enter as 0 * NaN).
+// d goes to d_out unless that is nullptr.  HBM traffic per step as ChebStep's.  (The modes: lkb_kernels.h.)
+template <typename E> struct MgStep {
+    const E* r; const E* d_in; E* d_out;
+    E invd[8], ecor[8];
+    double alpha, beta, b0;
+    int mode;
+};
+// a[mk] by selects: a dynamic index into a kernel parameter would copy the whole array to local memory
+template <typename E> LKB_DI E pick8(const E (&a)[8], int mk) {
+    E v = a[0];
+#pragma unroll
+    for (int q = 1; q < 8; ++q) if (mk == q) v = a[q];
+    return v;
+}
+// myz: the y / z mask bits of this row; xlast: the pack element on the last x index (outside 0 .. PW-1: none)
+template <typename E, int PW, typename Rl>
+LKB_DI void mg_store(const MgStep<E>& c, E* y, int64_t q, const Pack<E, PW>& t, const Pack<E, PW>& x, int myz, int64_t xlast) {
+    using PO = PackOps<E, PW>;
+    using P = Pack<E, PW>;
+    const Rl alpha = (Rl)c.alpha, beta = (Rl)c.beta, b0 = (Rl)c.b0;
+    P zn;
+    if (c.mode == MG_SCALE) {
+#pragma unroll
+        for (int e = 0; e < PW; ++e) zn.v[e] = rscale(mul_v(pick8(c.invd, myz | (e == xlast ? 1 : 0)), x.v[e]), b0);
+        PO::st(y + q, zn);
+        return;
+    }
+    const P rv = c.mode == MG_FIRST_R ? x : PO::ld_nc(c.r + q);
+    P dv = PO::zero();
+    if (c.mode == MG_STEP && c.d_in) dv = PO::ld_nc(c.d_in + q);
+#pragma unroll
+    for (int e = 0; e < PW; ++e) {
+        const int mk = myz | (e == xlast ? 1 : 0);
+        const E iv = mk ? pick8(c.invd, mk) : c.invd[0];
+        E tk = t.v[e], zk = x.v[e];
+        if (mk) fmacc(tk, x.v[e], pick8(c.ecor, mk));
+        if (c.mode == MG_FIRST_R) { zk = rscale(mul_v(iv, x.v[e]), b0); tk = rscale(mul_v(iv, tk), b0); dv.v[e] = zk; }
+        const E s = mul_v(iv, add_v(rv.v[e], rscale(tk, (Rl)-1)));
+        dv.v[e] = add_v(rscale(dv.v[e], alpha), rscale(s, beta));
+        zn.v[e] = add_v(zk, dv.v[e]);
+    }
+    if (c.d_out) PO::st(c.d_out + q, dv);
+    PO::st(y + q, zn);
+}
 
 // Both stencil kernels take one CTA per (column block, row block[, plane]) of a 1-D grid, column block fastest
 // (consecutive CTAs stream consecutive segments of the same grid rows).  The row blocks (2-D) / planes (3-D) are rotated
@@ -213,6 +264,9 @@ k_stencil(const typename Tr<K>::E* __restrict__ x, typename Tr<K>::E* __restrict
             if (active) PO::st_w(y + k * plane + p, out, keep, pol);
         } else if constexpr (std::is_same_v<EPI, PolyStep<E>>) {
             if (active) poly_store<E, PW>(epi, y, k * plane + p, out, center);
+        } else if constexpr (std::is_same_v<EPI, MgStep<E>>) {
+            if (active) mg_store<E, PW, typename Tr<K>::Rl>(epi, y, k * plane + p, out, center,
+                                                             (j == ny - 1 ? 2 : 0) | (k == nz - 1 ? 4 : 0), nx - 1 - i0);
         } else {
             if (active) cheb_store<E, PW, typename Tr<K>::Rl>(epi, y, k * plane + p, out, center);
         }
@@ -317,13 +371,13 @@ k_stencil_smem(const typename Tr<K>::E* __restrict__ x, typename Tr<K>::E* __res
         }
         if constexpr (std::is_same_v<EPI, StorePlain>) PackOps<E, PW>::st_w(y + p, out, keep, pol);
         else if constexpr (std::is_same_v<EPI, PolyStep<E>>) poly_store<E, PW>(epi, y, p, out, center);
+        else if constexpr (std::is_same_v<EPI, MgStep<E>>)
+            mg_store<E, PW, typename Tr<K>::Rl>(epi, y, p, out, center, j == ny - 1 ? 2 : 0, nx - 1 - i0);
         else cheb_store<E, PW, typename Tr<K>::Rl>(epi, y, p, out, center);
     }
 }
 
-template <int K, int PW, int DIM, class EPI>
-static void stencil_launch(cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans, const int* flags, const EPI& epi) {
-    using E = typename Tr<K>::E;
+template <typename E> static Coef7<E> stencil_coef(const StencilArgs& a, bool trans) {
     Coef7<E> cf;
     Scalar c[7];
     for (int q = 0; q < 7; ++q) c[q] = a.coef[q];
@@ -333,6 +387,13 @@ static void stencil_launch(cudaStream_t s, const StencilArgs& a, const void* x, 
         for (int q = 0; q < 7; ++q) c[q].im = -c[q].im;
     }
     for (int q = 0; q < 7; ++q) from_scalar(c[q], cf.c[q]);
+    return cf;
+}
+
+template <int K, int PW, int DIM, class EPI>
+static void stencil_launch(cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans, const int* flags, const EPI& epi) {
+    using E = typename Tr<K>::E;
+    const Coef7<E> cf = stencil_coef<E>(a, trans);
     const int64_t npk_row = a.nx / PW;
     const int64_t nyb = (a.ny + ST_RY - 1) / ST_RY;
     const int keep_w = ((size_t)a.nx * (size_t)a.ny * (size_t)a.nz * sizeof(E) <= W_KEEP_BYTES) ? 1 : 0;
@@ -414,6 +475,156 @@ void launch_stencil_poly(int kind, cudaStream_t s, const StencilArgs& a, const v
         case KD: stencil_poly_t<KD>(s, a, x, y, trans, flags, pa); break;
         case KC: stencil_poly_t<KC>(s, a, x, y, trans, flags, pa); break;
         default: stencil_poly_t<KZ>(s, a, x, y, trans, flags, pa); break;
+    }
+}
+// One fused multigrid smoothing step (MgStep above)
+template <int K>
+static void stencil_mg_t(cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans, const int* flags,
+                         const MgArgs& ma) {
+    using E = typename Tr<K>::E;
+    MgStep<E> epi;
+    epi.r = (const E*)ma.r; epi.d_in = (const E*)ma.d_in; epi.d_out = (E*)ma.d_out;
+    for (int q = 0; q < 8; ++q) { from_scalar(ma.invd[q], epi.invd[q]); from_scalar(ma.ecor[q], epi.ecor[q]); }
+    epi.alpha = ma.alpha; epi.beta = ma.beta; epi.b0 = ma.b0; epi.mode = ma.mode;
+    stencil_t<K>(s, a, x, y, trans, flags, epi);
+}
+void launch_stencil_mg(int kind, cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans, const int* flags,
+                       const MgArgs& ma) {
+    switch (kind) {
+        case KS: stencil_mg_t<KS>(s, a, x, y, trans, flags, ma); break;
+        case KD: stencil_mg_t<KD>(s, a, x, y, trans, flags, ma); break;
+        case KC: stencil_mg_t<KC>(s, a, x, y, trans, flags, ma); break;
+        default: stencil_mg_t<KZ>(s, a, x, y, trans, flags, ma); break;
+    }
+}
+
+// ------------------------------------------------------------------------------------------
+// Grid transfers of the multigrid preconditioner (lkb_mg.cu).  Every axis n -> n / 2, coarse point c at fine point 2c+1;
+// 1-D interpolation P: fine 2c+1 takes coarse c, fine 2c and 2c+2 take half of it, coarse points outside the grid are zero.
+// k_mg_restrict: bc = 2^-dim P^T (b - A x), one thread per coarse point, which gathers the residuals of the fine points
+// 2c .. 2c+2 along each axis (weights 1/2, 1, 1/2; 2c+2 may lie past the grid).  A residual is formed where it is used, from
+// x through L1 (a fine point on an even index serves two coarse points): b and x are read from HBM once and the fine
+// residual is never stored.  The centre of the fine level is c0 + ecor[mask] as in MgStep, ecor[mask] the sum of the
+// per-axis corrections ed.c[d] = ecor[1 << d].
+template <typename E> struct Edge3 { E c[3]; };
+template <int K>
+__global__ void __launch_bounds__(256, 1)
+k_mg_restrict(const typename Tr<K>::E* __restrict__ x, const typename Tr<K>::E* __restrict__ b, typename Tr<K>::E* __restrict__ bc,
+              int64_t nx, int64_t ny, int64_t nz, bool three, Coef7<typename Tr<K>::E> cf, Edge3<typename Tr<K>::E> ed,
+              const int* __restrict__ flags)
+{
+    using E = typename Tr<K>::E;
+    using Rl = typename Tr<K>::Rl;
+    if (flags && flags[F_STOP]) return;
+    const int64_t cx = nx / 2, cy = ny / 2, cz = three ? nz / 2 : 1;
+    const int64_t ncoarse = cx * cy * cz;
+    auto res = [&](int64_t i, int64_t j, int64_t k) -> E {
+        const int64_t p = i + nx * (j + ny * k);
+        const E xc = __ldg(x + p);
+        E s = mul_v(cf.c[0], xc);
+        if (i > 0) fmacc(s, __ldg(x + p - 1), cf.c[1]);
+        if (i < nx - 1) fmacc(s, __ldg(x + p + 1), cf.c[2]); else fmacc(s, xc, ed.c[0]);
+        if (j > 0) fmacc(s, __ldg(x + p - nx), cf.c[3]);
+        if (j < ny - 1) fmacc(s, __ldg(x + p + nx), cf.c[4]); else fmacc(s, xc, ed.c[1]);
+        if (three) {
+            if (k > 0) fmacc(s, __ldg(x + p - nx * ny), cf.c[5]);
+            if (k < nz - 1) fmacc(s, __ldg(x + p + nx * ny), cf.c[6]); else fmacc(s, xc, ed.c[2]);
+        }
+        return add_v(__ldg(b + p), rscale(s, (Rl)-1));
+    };
+    for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < ncoarse; q += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t ic = q % cx, jc = (q / cx) % cy, kc = q / (cx * cy);
+        E acc = zero_v(E());
+#pragma unroll 1
+        for (int dz = 0; dz < (three ? 3 : 1); ++dz) {
+            const int64_t k = three ? 2 * kc + dz : 0;
+            if (k >= nz) break;
+            const Rl wz = (three && dz != 1) ? (Rl)0.5 : (Rl)1;
+            for (int dy = 0; dy < 3; ++dy) {
+                const int64_t j = 2 * jc + dy;
+                if (j >= ny) break;
+                const Rl wyz = dy == 1 ? wz : wz * (Rl)0.5;
+                for (int dx = 0; dx < 3; ++dx) {
+                    const int64_t i = 2 * ic + dx;
+                    if (i >= nx) break;
+                    acc = add_v(acc, rscale(res(i, j, k), dx == 1 ? wyz : wyz * (Rl)0.5));
+                }
+            }
+        }
+        bc[q] = rscale(acc, three ? (Rl)0.125 : (Rl)0.25);
+    }
+}
+// k_mg_prolong: x += P e on the fine grid, one thread per fine point; e is the coarse vector (cached in L1 / L2)
+template <int K>
+__global__ void __launch_bounds__(256)
+k_mg_prolong(typename Tr<K>::E* __restrict__ x, const typename Tr<K>::E* __restrict__ e, int64_t nx, int64_t ny, int64_t nz,
+             bool three, const int* __restrict__ flags)
+{
+    using E = typename Tr<K>::E;
+    using Rl = typename Tr<K>::Rl;
+    if (flags && flags[F_STOP]) return;
+    const int64_t cx = nx / 2, cy = ny / 2, cz = three ? nz / 2 : 1;
+    const int64_t n = nx * ny * nz;
+    // the coarse points of fine index i along an axis of nc coarse points: c0 (weight w0) and c0 + 1 (weight w1); a weight is
+    // zero where the point is outside the coarse grid or not a neighbour
+    auto axis = [](int64_t i, int64_t nc, int64_t& c0, Rl& w0, Rl& w1) {
+        if (i & 1) { c0 = i >> 1; w0 = (Rl)1; w1 = (Rl)0; return; }
+        c0 = (i >> 1) - 1;
+        w0 = i > 0 ? (Rl)0.5 : (Rl)0;
+        w1 = (i >> 1) < nc ? (Rl)0.5 : (Rl)0;
+    };
+    for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < n; p += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t i = p % nx, j = (p / nx) % ny, k = p / (nx * ny);
+        int64_t ci, cj, ck = 0;
+        Rl wi[2], wj[2], wk[2] = {(Rl)1, (Rl)0};
+        axis(i, cx, ci, wi[0], wi[1]); axis(j, cy, cj, wj[0], wj[1]);
+        if (three) axis(k, cz, ck, wk[0], wk[1]);
+        E acc = zero_v(E());
+#pragma unroll
+        for (int a = 0; a < 2; ++a)
+#pragma unroll
+            for (int bb = 0; bb < 2; ++bb)
+#pragma unroll
+                for (int c = 0; c < 2; ++c) {
+                    const Rl w = wi[c] * wj[bb] * wk[a];
+                    if (w != (Rl)0) acc = add_v(acc, rscale(__ldg(e + (ci + c) + cx * ((cj + bb) + cy * (ck + a))), w));
+                }
+        x[p] = add_v(x[p], acc);
+    }
+}
+template <int K>
+static void mg_transfer_t(cudaStream_t s, const StencilArgs& a, const Scalar* ecor, const void* x, const void* b, void* out,
+                          bool trans, bool restrict_, const int* flags, int sms) {
+    using E = typename Tr<K>::E;
+    const bool three = a.dim == 3;
+    const int64_t work = restrict_ ? (a.nx / 2) * (a.ny / 2) * (three ? a.nz / 2 : 1) : a.nx * a.ny * a.nz;
+    int64_t nb = (work + 255) / 256;
+    if (nb < 1) nb = 1;
+    if (nb > (int64_t)sms * 32) nb = (int64_t)sms * 32;
+    if (restrict_) {
+        Edge3<E> ed;
+        for (int d = 0; d < 3; ++d) from_scalar(ecor[1 << d], ed.c[d]);
+        k_mg_restrict<K><<<(int)nb, 256, 0, s>>>((const E*)x, (const E*)b, (E*)out, a.nx, a.ny, a.nz, three, stencil_coef<E>(a, trans),
+                                                  ed, flags);
+    } else {
+        k_mg_prolong<K><<<(int)nb, 256, 0, s>>>((E*)out, (const E*)x, a.nx, a.ny, a.nz, three, flags);
+    }
+}
+void launch_mg_restrict(int kind, cudaStream_t s, const StencilArgs& a, const Scalar* ecor, const void* x, const void* b, void* bc,
+                        bool trans, const int* flags, int sms) {
+    switch (kind) {
+        case KS: mg_transfer_t<KS>(s, a, ecor, x, b, bc, trans, true, flags, sms); break;
+        case KD: mg_transfer_t<KD>(s, a, ecor, x, b, bc, trans, true, flags, sms); break;
+        case KC: mg_transfer_t<KC>(s, a, ecor, x, b, bc, trans, true, flags, sms); break;
+        default: mg_transfer_t<KZ>(s, a, ecor, x, b, bc, trans, true, flags, sms); break;
+    }
+}
+void launch_mg_prolong(int kind, cudaStream_t s, const StencilArgs& a, const void* e, void* x, const int* flags, int sms) {
+    switch (kind) {
+        case KS: mg_transfer_t<KS>(s, a, nullptr, e, nullptr, x, false, false, flags, sms); break;
+        case KD: mg_transfer_t<KD>(s, a, nullptr, e, nullptr, x, false, false, flags, sms); break;
+        case KC: mg_transfer_t<KC>(s, a, nullptr, e, nullptr, x, false, false, flags, sms); break;
+        default: mg_transfer_t<KZ>(s, a, nullptr, e, nullptr, x, false, false, flags, sms); break;
     }
 }
 

@@ -20,6 +20,19 @@ namespace lkb {
 // step reads and writes the same buffer (the stencil's neighbours read z_k while z_{k+1} is written)
 static void* stencil_z(lkb_op_s* M, void* y, int j) { return ((M->cheb_m - j) % 2 == 0) ? y : M->cheb_z.get(); }
 
+void cheb_coefficients(int m, double a, double b, std::vector<double>& ca, std::vector<double>& cb) {
+    const double theta = (b + a) / 2, delta = (b - a) / 2, sigma = theta / delta;
+    ca.assign(m, 0.0); cb.assign(m, 0.0);
+    cb[0] = 1.0 / theta;
+    double rho = 1.0 / sigma;
+    for (int k = 1; k < m; ++k) {
+        const double rho_k = 1.0 / (2.0 * sigma - rho);
+        ca[k] = rho_k * rho;
+        cb[k] = 2.0 * rho_k / delta;
+        rho = rho_k;
+    }
+}
+
 int cheb_apply_enqueue(lkb_op_s* M, const void* r, void* y, bool trans, const int* flags) {
     lkb_op_s* A = M->base;
     lkb_ctx_s* c = M->ctx;
@@ -113,16 +126,7 @@ int lkb_op_chebyshev_create(lkb_op_t A, int32_t degree, double lmin, double lmax
     const double b = want_bound ? bound : lmax;
     const double a = lmin > 0.0 ? lmin : b / 100.0;
     if (!(a < b) || !isfinite(b)) { set_error("chebyshev_create: lmin = %g is not below lmax = %g", a, b); return LKB_ERR_ARG; }
-    const double theta = (b + a) / 2, delta = (b - a) / 2, sigma = theta / delta;
-    op->cheb_a.assign(degree, 0.0); op->cheb_b.assign(degree, 0.0);
-    op->cheb_b[0] = 1.0 / theta;
-    double rho = 1.0 / sigma;
-    for (int k = 1; k < degree; ++k) {
-        const double rho_k = 1.0 / (2.0 * sigma - rho);
-        op->cheb_a[k] = rho_k * rho;
-        op->cheb_b[k] = 2.0 * rho_k / delta;
-        rho = rho_k;
-    }
+    cheb_coefficients(degree, a, b, op->cheb_a, op->cheb_b);
     const size_t bytes = std::max<size_t>((size_t)A->m * kind_size(A->kind), 16);
     if (degree >= 3) LKB_TRY(cuda_alloc(op->cheb_d, bytes));
     if (degree >= 3 && A->type == OP_STENCIL) LKB_TRY(cuda_alloc(op->cheb_z, bytes));

@@ -760,7 +760,7 @@ int lkb_op_jacobi_create(lkb_op_t A, lkb_op_t* M) {
 int lkb_op_destroy(lkb_op_t A) {
     if (!A) return LKB_ERR_ARG;
     if (A->users > 0) {
-        set_error("op_destroy: %d Chebyshev or GMRES-polynomial preconditioner(s) built on this operator are still alive "
+        set_error("op_destroy: %d Chebyshev, GMRES-polynomial or multigrid preconditioner(s) built on this operator are still alive "
                   "(destroy them first)", A->users);
         return LKB_ERR_ARG;
     }
@@ -866,6 +866,7 @@ const HaloP2P* op_halo_desc(const lkb_op_s* A, int j) {
 int op_apply_enqueue(lkb_op_s* A, const void* x, void* y, bool trans, const int* flags, bool halo_prepushed) {
     if (A->type == OP_CHEB) return cheb_apply_enqueue(A, x, y, trans, flags);     // brackets each of its launches itself
     if (A->type == OP_POLY) return poly_apply_enqueue(A, x, y, trans, flags);     // the same
+    if (A->type == OP_MG) return mg_apply_enqueue(A, x, y, trans, flags);         // the same
     lkb_ctx_s* c = A->ctx;
     const size_t es = kind_size(A->kind);
     int nl = 1;

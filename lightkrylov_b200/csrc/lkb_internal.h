@@ -37,7 +37,7 @@ NcclApi* nccl_api();   // nullptr (+ error set) when libnccl cannot be loaded
 
 enum ProfClass { PC_MATVEC = 0, PC_DOT = 1, PC_AXPY = 2, PC_OTHER = 3, PC_FUSED = 4, PC_COUNT = 8 };
 // lkb_op_s::type.  The values are printed by lkb_op_jacobi_create's error message.
-enum OpType { OP_DENSE = 0, OP_STENCIL = 1, OP_CSR = 3, OP_DIAG = 4, OP_CHEB = 5, OP_POLY = 6, OP_CALLBACK = 9 };
+enum OpType { OP_DENSE = 0, OP_STENCIL = 1, OP_CSR = 3, OP_DIAG = 4, OP_CHEB = 5, OP_POLY = 6, OP_MG = 7, OP_CALLBACK = 9 };
 
 // ---- owners: every raw CUDA resource and every solver work object has exactly one, and goes with it ------------------
 // Members and locals are released in reverse order of declaration.  (The host-shell test mocks replace lkb_basis_destroy,
@@ -80,6 +80,18 @@ struct CsrBlockedMem { CudaPtr<uint32_t> tab; CudaPtr<int32_t> col; CudaPtr<void
 // coefficients of (x, t, v) of out and acc (lkb_kernels.h: PolyArgs), conjugated for the rmatvec.
 enum { POLY_NONE = -1, POLY_R = -2 };
 struct PolyStepPlan { int x, dst, v, acc; bool matvec, out; Scalar a[3], b[3]; };
+// One level ell < L of the multigrid preconditioner (lkb_mg.cu): its stencil, the centre corrections ecor[mask] and D^-1 =
+// invd[mask] by last-index mask (kernels_ops.cu: MgStep), whether any correction is nonzero, the Chebyshev coefficients of
+// its smoother (b0 = 1 / theta, step k = 1 .. m-1: ca[k], cb[k]) and its vectors: b, e the level's input and output (ell >
+// 0), xa, xb, d the smoother's iterates and direction (xb, d for m >= 2).  The coarsest level keeps only st, b and e.
+struct MgLevel {
+    StencilArgs st = {};
+    Scalar ecor[8] = {}, invd[8] = {};
+    bool edges = false;
+    double b0 = 0.0;
+    std::vector<double> ca, cb;
+    CudaPtr<void> b, e, xa, xb, d;
+};
 }  // namespace lkb
 
 struct lkb_ctx_s {
@@ -175,6 +187,11 @@ struct lkb_op_s {
     std::vector<lkb::Scalar> poly_roots;
     std::vector<lkb::PolyStepPlan> poly_plan;
     lkb::CudaPtr<void> poly_w[3];
+    // geometric multigrid preconditioner (lkb_mg.cu) on the stencil `base`: smoother degree, the levels (mg[0] is base's
+    // grid) and the inverse of the coarsest operator (column-major, in the kind)
+    int mg_m = 0;
+    std::vector<lkb::MgLevel> mg;
+    lkb::CudaPtr<void> mg_inv;
     uint64_t uid = 0;
 };
 
@@ -230,6 +247,11 @@ int stencil_halo_exchange(lkb_op_s* A, const void* x, const int* flags, bool hal
 int cheb_apply_enqueue(lkb_op_s* M, const void* r, void* y, bool trans, const int* flags);
 // y = M r (trans: M^H r) for a GMRES-polynomial operator M (lkb_poly.cu); op_apply_enqueue dispatches here
 int poly_apply_enqueue(lkb_op_s* M, const void* r, void* y, bool trans, const int* flags);
+// y = M r (trans: M^H r) for a multigrid operator M, one V-cycle (lkb_mg.cu); op_apply_enqueue dispatches here
+int mg_apply_enqueue(lkb_op_s* M, const void* r, void* y, bool trans, const int* flags);
+// theta and the step coefficients of a Chebyshev iteration of degree m on [a, b] (lkb_cheb.cu): cb[0] = 1 / theta, step
+// k = 1 .. m-1 uses ca[k], cb[k]
+void cheb_coefficients(int m, double a, double b, std::vector<double>& ca, std::vector<double>& cb);
 // Jacobi set-up, shared by lkb_op_jacobi_create and lkb_op_chebyshev_create (`what` prefixes the messages): where A keeps
 // its diagonal, for k_jacobi / k_gershgorin; LKB_ERR_ARG for an operator without one (callback, non-square, ...)
 int jacobi_source(const lkb_op_s* A, const char* what, JacobiSrc* src, int64_t* n_global);
@@ -307,6 +329,12 @@ inline Scalar to_scalar(cd v) { return Scalar{v.real(), v.imag()}; }
 // product of the other factors exceeds 1e4 at them, modified Leja order (real kinds: conjugate pairs adjacent, im > 0
 // first).  LKB_ERR_ARG for a singular H_k or a zero / non-finite root, LKB_ERR_LAPACK without a LAPACK provider.
 int gmres_poly_roots(int kind, const cd* H, int ldh, int k, std::vector<cd>& roots);
+// The multigrid hierarchy of a dim-D stencil on grid n with coefficients coef (lkb_mg.cu; host only, in complex double).
+// Level ell: grid n, stencil (c0, cm[d], cp[d]) with centre c0 + sum_d [i_d = n_d - 1] e[d], and the Gershgorin bound lmax
+// of its D^-1 A; inv: the inverse of the last level's operator, column-major.  LKB_ERR_ARG (with the message) for a zero or
+// non-finite centre, a coarsest level above 512 unknowns or a singular coarsest matrix.
+struct MgHostLevel { int64_t n[3]; cd c0, cm[3], cp[3], e[3]; double lmax; };
+int mg_hierarchy(int dim, const int64_t* n, const cd* coef, std::vector<MgHostLevel>& levels, std::vector<cd>& inv);
 // eigenvalues of the k x k complex-double matrix A (real when !cplx) by the double-precision geev (lkb_eig.cu)
 int host_eig_double(bool cplx, int k, const std::vector<cd>& A, int lda, std::vector<cd>& vals);
 

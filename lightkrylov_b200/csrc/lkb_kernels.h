@@ -262,6 +262,18 @@ void launch_poly_update(int kind, cudaStream_t s, const void* x, const void* t, 
 // Neither y, v nor acc may be x.
 void launch_stencil_poly(int kind, cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans, const int* flags,
                          const PolyArgs& pa);
+// One Chebyshev smoothing step on a level of the multigrid preconditioner (lkb_mg.cu), fused into the stencil kernels
+// (kernels_ops.cu: MgStep): a.coef is the level's stencil, and the centre on the last index of the axes in mask (bit 0 x,
+// 1 y, 2 z) is c0 + ecor[mask], with D^-1 = invd[mask] there (both already conjugated for trans).  mode: MG_SCALE,
+// MG_FIRST_R or MG_STEP (kernels_ops.cu).  Neither y, r, d_in nor d_out may be x, except d_in.
+enum { MG_SCALE = 0, MG_FIRST_R = 1, MG_STEP = 2 };
+struct MgArgs { const void* r; const void* d_in; void* d_out; Scalar invd[8], ecor[8]; double alpha, beta, b0; int mode; };
+void launch_stencil_mg(int kind, cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans, const int* flags,
+                       const MgArgs& ma);
+// bc = 2^-dim P^T (b - A x) from a level (a, ecor as above) to its coarse grid (k_mg_restrict); x += P e (k_mg_prolong)
+void launch_mg_restrict(int kind, cudaStream_t s, const StencilArgs& a, const Scalar* ecor, const void* x, const void* b, void* bc,
+                        bool trans, const int* flags, int sms);
+void launch_mg_prolong(int kind, cudaStream_t s, const StencilArgs& a, const void* e, void* x, const int* flags, int sms);
 void launch_stencil(int kind, cudaStream_t s, const StencilArgs& a, const void* x, void* y, bool trans,
                     const int* flags, int sms);
 // CSR SpMV y = A x (vector-per-row); conj_vals: use conj(A) values (for the explicit-transpose rmatvec)
